@@ -72,7 +72,27 @@ def parse():
     ap.add_argument("--mixed", action="store_true",
                     help="config 5: half of the batch are 'combined' queries normalise(2.0*t + 1.0*i - 0.2*n) "
                          "(/root/reference/api/routes.py:759-850)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the (D, I) the last one returned as DIR/D.npy and DIR/I.npy")
     return ap.parse_args()
+
+
+DUMP_MAX_BYTES = 60 << 20  # keeps the two files, headers included, under 64 MB
+
+
+def dump_outputs(out_dir, D, I):
+    """--dump-outputs: the scores D (float32) and ids I (int64 stored as float64, exact below 2**53) of the last timed
+    step, so that two builds can be compared output for output on the same seeded inputs.  When the pair exceeds
+    DUMP_MAX_BYTES, a fixed seeded sample of the query rows is written instead (the same rows for the same arguments)."""
+    D = np.asarray(D, dtype=np.float32)
+    I = np.asarray(I).astype(np.float64)
+    row_bytes = D.shape[1] * (D.itemsize + I.itemsize)
+    if D.shape[0] * row_bytes > DUMP_MAX_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(D.shape[0], DUMP_MAX_BYTES // row_bytes, replace=False))
+        D, I = D[rows], I[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "D.npy"), D)
+    np.save(os.path.join(out_dir, "I.npy"), I)
 
 
 def workload_name(a, batch=None):
@@ -375,8 +395,10 @@ def run_reference(a):
         step()
     t0 = time.perf_counter()
     for _ in range(a.steps):
-        step()
+        D, I = step()
     dt = time.perf_counter() - t0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, D, I)
     scale = a.rows / n_s
     ms_step = dt / a.steps * 1e3 * scale
     qps = a.batch / (ms_step / 1e3)
@@ -724,6 +746,8 @@ def run_ours(a):
     preroll(a.batch)
     ms_step, scan_ms, launches, q_last, D_last, I_last = timed_steps(a.batch, a.steps, a.warmup)
     clocks = sampler.finish() if sampler else None
+    if a.dump_outputs and rank == 0:  # every rank holds the same merged (D, I)
+        dump_outputs(a.dump_outputs, D_last.cpu().numpy(), I_last.cpu().numpy())
     e2e_ms, q_e2e, D_e2e, I_e2e = timed_e2e(a.batch, a.steps, a.warmup)
 
     parity = None

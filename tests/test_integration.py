@@ -57,15 +57,20 @@ def test_batched_join_reports_unknown_ids():
         join_hits_batched(conn, np.array([5, 999999, -1]), np.array([0.9, 0.8, 0.0], np.float32))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src/index") or shutil.which("patch") is None,
-                    reason="needs the reference tree and patch(1) (dev container only)")
+# A checkout of the WISE 2 sources (https://github.com/ox-vgg/wise) that integration/wise_b200.patch targets.
+WISE_SRC = os.environ.get("WISE_SRC", "")
+
+
+@pytest.mark.skipif(not WISE_SRC or not os.path.isdir(os.path.join(WISE_SRC, "src", "index"))
+                    or shutil.which("patch") is None,
+                    reason="needs WISE_SRC set to a WISE 2 checkout, and patch(1)")
 def test_integration_patch_applies_to_the_reference(tmp_path):
     """integration/wise_b200.patch: backend switch (src/index/feature_search_index.py:1), request batcher
     (api/routes.py:1407) and batched metadata join (search.py:137-153) - applies cleanly and leaves valid python."""
     import ast
     for f in ("src/index/feature_search_index.py", "search.py", "api/routes.py"):
         os.makedirs(tmp_path / os.path.dirname(f), exist_ok=True)
-        shutil.copy(os.path.join("/root/reference", f), tmp_path / f)
+        shutil.copy(os.path.join(WISE_SRC, f), tmp_path / f)
     r = subprocess.run(["patch", "-p1", "--dry-run", "-i", os.path.join(ROOT, "integration", "wise_b200.patch")], cwd=tmp_path,
                        capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
