@@ -1,5 +1,5 @@
 """Where the time of a one-query scan goes: per-CTA %globaltimer stamps (WB_PHASE_TS=1, wb_phase_stamps) of the fused
-scan kernel for a flat store and an IVF index, with the heads merge + rank-counting sort on and off.  Prints, per case, the
+scan kernel for a flat store and an IVF index.  Prints, per case, the
 median / max over CTAs of every phase boundary relative to the earliest CTA start, and the last CTA's merge time.
     python scripts/phase_times.py"""
 import ctypes as C
@@ -54,9 +54,7 @@ def main():
         flat = faiss.IndexIDMap(faiss.IndexFlatIP(d))
         centres, _ = fill_index_clustered(flat, 0, n, d, 50, dev)
         q = make_queries(centres, 1, d, 7, dev)
-        for new in ("0", "1"):
-            os.environ["WB_MERGE_HEADS"] = os.environ["WB_RANK_SORT"] = new
-            report("flat", stamps(flat, q, 100, 1), {"rows": n, "d": d, "heads_merge_and_rank_sort": int(new)})
+        report("flat", stamps(flat, q, 100, 1), {"rows": n, "d": d})
         del flat
         torch.cuda.empty_cache()
     n, d, nlist = 2_000_000, 512, 1024
@@ -68,10 +66,7 @@ def main():
     fill_index_clustered(ivf, 0, n, d, 50, dev)
     q = make_queries(centres, 1, d, 8, dev)
     for nprobe in (8, 32):
-        for new in ("0", "1"):
-            os.environ["WB_MERGE_HEADS"] = os.environ["WB_RANK_SORT"] = new
-            report("ivf", stamps(ivf, q, 100, nprobe), {"rows": n, "nlist": nlist, "nprobe": nprobe,
-                                                        "heads_merge_and_rank_sort": int(new)})
+        report("ivf", stamps(ivf, q, 100, nprobe), {"rows": n, "nlist": nlist, "nprobe": nprobe})
 
 
 if __name__ == "__main__":

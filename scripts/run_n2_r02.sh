@@ -1,18 +1,15 @@
 # Round-2 2-GPU check (gpurun --gpus 2): the multi-GPU tests (fused NVLink exchange in the scan tail, merge through the
-# heads of the per-rank rows) and the batch-1 bench with its in-run parity check, heads merge on / off.
+# heads of the per-rank rows) and the batch-1 bench with its in-run parity check.
 mkdir -p gpurun_out/n2
 O=gpurun_out/n2
 timeout 600 python -m pytest tests/test_multigpu_gpu.py -m gpu -q > $O/test_multigpu.log 2>&1
 echo "multigpu tests rc=$?" | tee $O/status.txt
 tail -4 $O/test_multigpu.log
 T="python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29533"
-for H in 1 0; do
-  WB_MERGE_HEADS=$H WB_RANK_SORT=$H timeout 300 $T bench.py --gpus 2 --steps 50 --warmup 5 --no-cpu-baseline --secondary none > $O/bench_n2_heads$H.json 2> $O/bench_n2_heads$H.err
-  echo "bench heads=$H rc=$?" | tee -a $O/status.txt
-  python - <<P
+timeout 300 $T bench.py --gpus 2 --steps 50 --warmup 5 --no-cpu-baseline --secondary none > $O/bench_n2.json 2> $O/bench_n2.err
+echo "bench rc=$?" | tee -a $O/status.txt
+python - <<P
 import json
-d=json.loads(open("$O/bench_n2_heads$H.json").read().strip().splitlines()[-1])
-print("heads=$H", d["value"], d["ms_per_step"], d["e2e"]["ms_per_step"], d["parity_check"]["ok"], d["roofline"]["launch_ms"])
+d=json.loads(open("$O/bench_n2.json").read().strip().splitlines()[-1])
+print(d["value"], d["ms_per_step"], d["e2e"]["ms_per_step"], d["parity_check"]["ok"], d["roofline"]["launch_ms"])
 P
-done
-cp $O/bench_n2_heads1.json $O/bench_n2.json

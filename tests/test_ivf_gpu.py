@@ -259,6 +259,103 @@ def test_ivf_batched_listmajor_matches_oracle(faiss, monkeypatch, n, d, nlist, k
     O.compare_topk(D, I, Dr, Ir)
 
 
+def test_ivf_ungrouped_store_matches_grouped(faiss, monkeypatch, tmp_path):
+    """When the second copy of the rows does not fit, the IVF store stays un-grouped: the list scan gathers rows through
+    the CSR of row indices (`perm`).  WB_IVF_CONTIGUOUS=0 forces that.  An un-grouped index B returns the same bytes as
+    a grouped twin A (selection keys carry the insertion position, not the storage row): in the fused coarse launch
+    (1 and 4 queries) and in the query-major scan of a batch, where the list-major kernel refuses an un-grouped store.
+    Then B is grouped once, takes more rows and is left un-grouped again (`perm` over a store described by `row_pos`).
+    reconstruct_batch and a write_index / read_index round trip agree with A."""
+    from wise_b200 import _capi
+    L = _capi.lib()
+    n, d, nlist, k = 20000, 128, 32, 50
+    cent = O.unit_gaussian(nlist, d, 80)
+    xs, ids, assigns = [], [], []
+
+    def add(m, seed):  # the same rows into A and B, with an exact duplicate of row 11 in another list
+        x = O.clustered_unit(m, d, 3 * nlist, seed)
+        x[m - 7] = xs[0][11] if xs else x[11]
+        a = O.ivf_assign(x, cent).astype(np.int32)
+        a[m - 7] = (assigns[0][11] if assigns else a[11]) + 1
+        a[m - 7] %= nlist
+        i = np.arange(sum(len(v) for v in ids), sum(len(v) for v in ids) + m, dtype=np.int64)
+        for index in (A, B):
+            _capi.check(L.wb_ivf_add_preassigned(index._h, m, _capi.ptr(x), _capi.ptr(i), _capi.ptr(a)))
+        xs.append(x)
+        ids.append(i)
+        assigns.append(a)
+
+    def grouped(index):
+        off = np.empty(nlist + 1, np.int64)
+        g = C.c_int(-1)
+        _capi.check(L.wb_ivf_list_offsets(index._h, _capi.ptr(off), C.byref(g)))
+        return g.value
+
+    def regroup(ungrouped_b):
+        assert grouped(A) == 1
+        if ungrouped_b:
+            monkeypatch.setenv("WB_IVF_CONTIGUOUS", "0")
+        assert grouped(B) == (0 if ungrouped_b else 1)
+        monkeypatch.delenv("WB_IVF_CONTIGUOUS", raising=False)
+
+    def same(D, I, D2, I2):
+        return np.array_equal(I, I2) and np.array_equal(D.view(np.uint32), D2.view(np.uint32))
+
+    def check_searches():
+        xa, ia, aa = np.concatenate(xs), np.concatenate(ids), np.concatenate(assigns).astype(np.int64)
+        xq = np.concatenate([xa[11:12], O.clustered_unit(63, d, 3 * nlist, 81)])
+        for nq in (1, 4, 64):
+            for nprobe in (1, 8, nlist):
+                A.nprobe = B.nprobe = nprobe
+                DA, IA = A.search(xq[:nq], k)
+                f0 = L.wb_ivf_fused_searches(B._h)
+                DB, IB = B.search(xq[:nq], k)
+                Dr, Ir = O.ivf_search(xa, ia, aa, cent, xq[:nq], k, nprobe)
+                O.compare_topk(DA, IA, Dr, Ir)
+                O.compare_topk(DB, IB, Dr, Ir)
+                if nq <= 4:  # both take the fused coarse launch
+                    assert L.wb_ivf_fused_searches(B._h) - f0 == 1, "the fused path was not taken"
+                else:  # A takes the list-major kernel by default; compare the same query-major kernel
+                    monkeypatch.setenv("WB_IVF_LISTMAJOR", "0")
+                    DA, IA = A.search(xq[:nq], k)
+                    monkeypatch.delenv("WB_IVF_LISTMAJOR")
+                assert same(DA, IA, DB, IB), (nq, nprobe)
+                if nprobe == nlist:  # equal scores in different lists: insertion order
+                    assert IB[0, 0] == 11 and IB[0, 1] == len(xs[0]) - 7 and DB[0, 0] == DB[0, 1]
+
+    A = faiss.IndexIVFFlat(faiss.IndexFlatIP(d), d, nlist, faiss.METRIC_INNER_PRODUCT)
+    B = faiss.IndexIVFFlat(faiss.IndexFlatIP(d), d, nlist, faiss.METRIC_INNER_PRODUCT)
+    A.set_centroids(cent)
+    B.set_centroids(cent)
+    monkeypatch.delenv("WB_IVF_CONTIGUOUS", raising=False)
+    add(n, 82)
+    regroup(ungrouped_b=True)
+    check_searches()
+    # B grouped (row_pos set), then more rows and un-grouped again: perm over a store that row_pos describes
+    add(3000, 83)
+    regroup(ungrouped_b=False)
+    add(2000, 84)
+    regroup(ungrouped_b=True)
+    check_searches()
+    xa = np.concatenate(xs)
+    A.make_direct_map(True)
+    B.make_direct_map(True)
+    keys = [11, n - 7, n + 2999, n + 3000, xa.shape[0] - 1, 0, 12345]
+    assert np.array_equal(B.reconstruct_batch(keys), xa[keys])
+    assert np.array_equal(B.reconstruct_batch(keys), A.reconstruct_batch(keys))
+    fa, fb = str(tmp_path / "a.faiss"), str(tmp_path / "b.faiss")
+    faiss.write_index(A, fa)
+    faiss.write_index(B, fb)
+    assert grouped(B) == 0  # writing did not regroup B
+    with open(fa, "rb") as f1, open(fb, "rb") as f2:
+        assert f1.read() == f2.read()
+    B2 = faiss.read_index(fb, faiss.IO_FLAG_READ_ONLY)
+    xq = O.clustered_unit(8, d, 3 * nlist, 85)
+    A.nprobe = B2.nprobe = 8
+    assert same(*A.search(xq, k), *B2.search(xq, k))
+    assert np.array_equal(B2.reconstruct_batch(keys), xa[keys])
+
+
 def test_kmeans_split_clusters_matches_oracle(faiss):
     """Empty lists: the host draws the (empty, donor) pairs from the list sizes with the faiss procedure (mt19937, same
     stream as the oracle), split_apply_kernel applies them on the device.  Several empties, one donor hit twice."""

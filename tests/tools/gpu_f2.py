@@ -1,5 +1,6 @@
-"""Dev script (round 2): the 256-query SS filter kernel (gemm_ss.cuh) - TF32 peak microbenchmark, parity of large
-batches against the oracle, then A/B timing against the 128-query TS kernel on 10M x 768 (WB_GEMM_F2=0/1)."""
+"""Dev script (round 2): the 256-query SS filter kernel (gemm_ss.cuh) - TF32 peak microbenchmark and parity of large
+batches against the oracle.
+    python tests/tools/gpu_f2.py [all|peak|check]"""
 import ctypes as C, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import numpy as np
@@ -42,30 +43,3 @@ if __name__ == "__main__":
         for cfg in [(100000, 512, 200, 100), (131072, 768, 300, 100, True), (300000, 64, 1000, 10), (60000, 70, 129, 100, True),
                     (200000, 768, 1024, 100, True), (150001, 772, 257, 10)]:
             check(*cfg)
-    if what in ("all", "time"):
-        import torch
-        n, d = int(os.environ.get("F2_ROWS", 10_000_000)), 768
-        gen = torch.Generator(device="cuda"); gen.manual_seed(1)
-        idx = faiss.IndexFlatIP(d); idx.reserve(n)
-        for s in range(0, n, 1_000_000):
-            x = torch.randn(min(1_000_000, n - s), d, device="cuda", generator=gen); x /= x.norm(dim=1, keepdim=True)
-            _capi.check(L.wb_add_with_ids_dev(idx._h, x.shape[0], x.data_ptr(), None, None)); torch.cuda.synchronize()
-        del x
-        L.wb_set_timing(idx._h, 1)
-        st = torch.cuda.current_stream().cuda_stream
-        for nq in [int(t) for t in os.environ.get("F2_NQ", "256,512,1024,2048").split(",")]:
-            q = torch.randn(nq, d, device="cuda"); q /= q.norm(dim=1, keepdim=True)
-            D = torch.empty(nq, 100, device="cuda"); I = torch.empty(nq, 100, dtype=torch.int64, device="cuda")
-            ref = None
-            for f2 in os.environ.get("F2_MODES", "0,1").split(","):
-                os.environ["WB_GEMM_F2"] = f2
-                ts = []
-                for _ in range(int(os.environ.get("F2_REPS", 12))):
-                    _capi.check(L.wb_search_dev(idx._h, nq, q.data_ptr(), 100, 1, D.data_ptr(), I.data_ptr(), st)); torch.cuda.synchronize()
-                    ts.append(L.wb_last_scan_ms(idx._h))
-                ms, med = min(ts[1:]), float(np.median(ts[6:]))
-                if ref is None:
-                    ref = (D.clone(), I.clone())
-                same = bool((ref[1] == I).all().item()) and bool((ref[0] == D).all().item())
-                print(f"nq={nq} F2={f2}: min {ms:.3f} ms, sustained median {med:.3f} ms  {nq/med*1e3:.0f} QPS  "
-                      f"{2*nq*n*d/med/1e9:.1f} TFLOP/s algorithmic  same_as_F2=0: {same}  stats={stats(idx)}", flush=True)

@@ -37,17 +37,29 @@ static int fail(const char* fmt, ...) {
     g_err = buf;
     return 1;
 }
-#define CK(call)                                                                                     \
-    do {                                                                                             \
-        cudaError_t e_ = (call);                                                                     \
-        if (e_ != cudaSuccess)                                                                       \
-            return fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
+#define CK(...) /* variadic: the call may hold template-argument commas */                                  \
+    do {                                                                                                    \
+        cudaError_t e_ = (__VA_ARGS__);                                                                     \
+        if (e_ != cudaSuccess)                                                                              \
+            return fail("%s failed: %s (%s:%d)", #__VA_ARGS__, cudaGetErrorString(e_), __FILE__, __LINE__); \
     } while (0)
 #define TRY(call)              \
     do {                       \
         int r_ = (call);       \
         if (r_ != 0) return r_; \
     } while (0)
+
+// Opt `Kernel` in to `bytes` of dynamic shared memory, once per device and host thread.
+template <auto Kernel>
+static cudaError_t smem_optin(int bytes) {
+    static thread_local bool done[64] = {};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess || (dev < 64 && done[dev])) return e;
+    e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess && dev < 64) done[dev] = true;
+    return e;
+}
 
 extern "C" const char* wb_last_error(void) { return g_err.c_str(); }
 extern "C" const char* wb_version(void) { return "wise_b200 0.1 (sm_100a)"; }
@@ -344,35 +356,30 @@ static int env_int(const char* name, int dflt) {
 // chunked stages (one 1 KB copy per row and chunk) top out at 4.0 TB/s and are only the fallback
 // for rows too wide for two whole-row stages.
 static int plan_scan(const wb_index* h, int64_t nq, int k, bool gather, int nprobe, ScanCfg* c) {
+    constexpr int kMaxStages = 8;
     const int ld = h->ld;
     int NQ = gather ? 1 : (nq >= 8 ? 8 : nq > 2 ? 4 : nq > 1 ? 2 : 1);
-    NQ = std::min(NQ, std::max(1, env_int("WB_SCAN_NQ", 8)));
     const int P = pow2_ceil(k + kMinQueue);
-    const int max_stages = std::max(2, env_int("WB_SCAN_STAGES", 8));
-    const int rw_max = std::min(4, std::max(1, env_int("WB_SCAN_RW", 4)));
-    const int ck_env = env_int("WB_SCAN_CK", 0) & ~3;
     const int np = gather ? nprobe : 0;
     for (; NQ >= 1; NQ >>= 1) {
-        if (ck_env == 0 || ck_env >= ld) {
-            for (int RW = rw_max; RW >= 1; RW >>= 1) {  // whole-row stages
-                const int gr = kConsumerWarps * RW;
-                const size_t fixed = scan_smem_layout(NQ, ld, P, ld, 0, np, gr).total;
-                const size_t stage_bytes = (size_t)gr * ld * 4;
-                if (fixed + 2 * stage_bytes + 64 > (size_t)h->smem_max) continue;
-                if (stage_bytes >= (1u << 20)) continue;  // mbarrier tx-count limit
-                const int stages = (int)std::min<size_t>(max_stages, ((size_t)h->smem_max - fixed - 64) / (stage_bytes + 24));
-                *c = ScanCfg{NQ, RW, P, ld, 1, stages, gather ? 0 : 1, 0};
-                c->smem = scan_smem_layout(NQ, ld, P, ld, stages, np, gr).total;
-                return 0;
-            }
+        for (int RW = kMaxRowsPerWarp; RW >= 1; RW >>= 1) {  // whole-row stages
+            const int gr = kConsumerWarps * RW;
+            const size_t fixed = scan_smem_layout(NQ, ld, P, ld, 0, np, gr).total;
+            const size_t stage_bytes = (size_t)gr * ld * 4;
+            if (fixed + 2 * stage_bytes + 64 > (size_t)h->smem_max) continue;
+            if (stage_bytes >= (1u << 20)) continue;  // mbarrier tx-count limit
+            const int stages = (int)std::min<size_t>(kMaxStages, ((size_t)h->smem_max - fixed - 64) / (stage_bytes + 24));
+            *c = ScanCfg{NQ, RW, P, ld, 1, stages, gather ? 0 : 1, 0};
+            c->smem = scan_smem_layout(NQ, ld, P, ld, stages, np, gr).total;
+            return 0;
         }
-        const int RW = rw_max;  // chunked fallback: very wide rows
+        const int RW = kMaxRowsPerWarp;  // chunked fallback: very wide rows
         const int gr = kConsumerWarps * RW;
-        for (int ck = std::min(ck_env ? ck_env : 1024, ld) & ~3; ck >= 32; ck = (ck / 2) & ~3) {
+        for (int ck = std::min(1024, ld) & ~3; ck >= 32; ck = (ck / 2) & ~3) {
             const size_t fixed = scan_smem_layout(NQ, ld, P, ck, 0, np, gr).total;
             const size_t stage_bytes = (size_t)gr * ck * 4;
             if (fixed + 2 * stage_bytes + 64 > (size_t)h->smem_max) continue;
-            const int stages = (int)std::min<size_t>(max_stages, ((size_t)h->smem_max - fixed - 64) / (stage_bytes + 24));
+            const int stages = (int)std::min<size_t>(kMaxStages, ((size_t)h->smem_max - fixed - 64) / (stage_bytes + 24));
             *c = ScanCfg{NQ, RW, P, ck, (ld + ck - 1) / ck, stages, 0, 0};
             c->smem = scan_smem_layout(NQ, ld, P, ck, stages, np, gr).total;
             return 0;
@@ -383,13 +390,7 @@ static int plan_scan(const wb_index* h, int64_t nq, int k, bool gather, int npro
 
 template <int NQ, int RW, bool GATHER>
 static int launch_scan_t(const ScanParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-    static thread_local bool attr_done[64] = {};
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (dev >= 64 || !attr_done[dev]) {
-        CK(cudaFuncSetAttribute(scan_topk_kernel<NQ, RW, GATHER>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-        if (dev < 64) attr_done[dev] = true;
-    }
+    CK(smem_optin<scan_topk_kernel<NQ, RW, GATHER>>(232448));
     scan_topk_kernel<NQ, RW, GATHER><<<grid, kScanThreads, smem, st>>>(p);
     CK(cudaGetLastError());
     return 0;
@@ -409,15 +410,8 @@ static int launch_scan_rw(int RW, const ScanParams& p, dim3 grid, size_t smem, c
 // of them must be resident - the cooperative launch guarantees it or fails).
 template <int RW>
 static cudaError_t launch_scan_coop_t(const ScanParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-    static thread_local bool attr_done[64] = {};
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
+    const cudaError_t e = smem_optin<scan_topk_kernel<1, RW, true>>(232448);
     if (e != cudaSuccess) return e;
-    if (dev >= 64 || !attr_done[dev]) {
-        e = cudaFuncSetAttribute(scan_topk_kernel<1, RW, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-        if (e != cudaSuccess) return e;
-        if (dev < 64) attr_done[dev] = true;
-    }
     void* args[] = {const_cast<ScanParams*>(&p)};
     return cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(scan_topk_kernel<1, RW, true>), grid,
                                        dim3(kScanThreads), args, smem, st);
@@ -430,8 +424,7 @@ static void apply_scan_cfg(const ScanCfg& c, ScanParams& p) {
     p.stages = c.stages;
     p.single_copy = c.single_copy;
     p.rw = c.RW;
-    p.prefetch_idx = env_int("WB_GATHER_PREFETCH", 1);
-    p.rank_sort = c.P <= kConsumerThreads && env_int("WB_RANK_SORT", 1);  // measured: slower than bitonic at P = 512
+    p.rank_sort = c.P <= kConsumerThreads;  // measured: slower than bitonic at P = 512
 }
 
 static cudaError_t launch_scan_coop(const ScanCfg& c, ScanParams& p, dim3 grid, cudaStream_t st) {
@@ -463,18 +456,6 @@ static int merge_buffer_entries(int k, int64_t nparts, int nthreads = kMergeThre
     return full;
 }
 
-template <bool FROM_KEYS>
-static int merge_smem_optin() {
-    static thread_local bool done[64] = {};
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (dev >= 64 || !done[dev]) {
-        CK(cudaFuncSetAttribute(merge_topk_kernel<FROM_KEYS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8192 * 8));
-        if (dev < 64) done[dev] = true;
-    }
-    return 0;
-}
-
 static int launch_merge_keys(wb_index* h, int64_t nq, int k, int64_t nparts, const uint64_t* keys, const int64_t* ids,
                              float* D, int64_t* I, cudaStream_t st) {
     MergeParams m{};
@@ -486,7 +467,7 @@ static int launch_merge_keys(wb_index* h, int64_t nq, int k, int64_t nparts, con
     m.ids = ids;
     m.D = D;
     m.I = I;
-    TRY(merge_smem_optin<true>());
+    CK(smem_optin<merge_topk_kernel<true>>(8192 * 8));
     merge_topk_kernel<true><<<(unsigned)nq, kMergeThreads, (size_t)m.S * 8, st>>>(m);
     CK(cudaGetLastError());
     h->launches++;
@@ -508,7 +489,6 @@ static int ensure_tail_counters(wb_index* h, cudaStream_t st) {
 static bool tail_fusable(const ScanCfg& c, int k, int64_t nparts, int world, int* S_merge, int* heads_bytes) {
     *S_merge = 0;
     *heads_bytes = 0;
-    if (env_int("WB_FUSE_TAIL", 1) == 0) return false;
     const size_t ring_bytes = (size_t)c.stages * kConsumerWarps * c.RW * c.ck * 4;
     const int S = std::max(merge_buffer_entries(k, nparts, kConsumerThreads),
                            world > 1 ? merge_buffer_entries(k, world, kConsumerThreads) : 2);
@@ -516,7 +496,7 @@ static bool tail_fusable(const ScanCfg& c, int k, int64_t nparts, int world, int
     *S_merge = S;
     // merge through the heads of the sorted lists first (block_merge_heads, merge.cuh); the sort-based merge stays
     // behind it as the fallback, so both regions must fit
-    if (env_int("WB_MERGE_HEADS", 1) && nparts <= 256) {
+    if (nparts <= 256) {
         const HeadsPlan a = heads_plan(k, (int)nparts);
         if (a.ok && std::max(a.bytes, (size_t)S * 8) + (size_t)k * 12 + 64 <= ring_bytes) *heads_bytes = (int)a.bytes;
     }
@@ -532,7 +512,7 @@ static void set_tail(ScanParams& p, wb_index* h, const ScanCfg& c, int S_merge, 
     if (env_int("WB_PHASE_TS", 0) && h->phase.ensure(kPhaseCtas * 16 * sizeof(unsigned long long)) == 0)
         p.phase_ts = h->phase.as<unsigned long long>();
     p.tail_count = h->tailcnt.as<unsigned int>();
-    p.group_count = (c.nchunks == 1 && env_int("WB_SCAN_DYNAMIC", 1)) ? h->tailcnt.as<unsigned int>() + kMaxGridY : nullptr;
+    p.group_count = c.nchunks == 1 ? h->tailcnt.as<unsigned int>() + kMaxGridY : nullptr;
     p.ids = ids;
     p.D = D;
     p.I = I;
@@ -556,11 +536,10 @@ static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const fl
     const int gr = kConsumerWarps * c.RW;
     const int64_t ngroups = (nrows + gr - 1) / gr;
     const int64_t qgroups_total = (nq + c.NQ - 1) / c.NQ;
-    const int waves = std::max(1, env_int("WB_SCAN_WAVES", 1));
     int64_t S = std::min<int64_t>(std::max<int64_t>(ngroups, 1),
-                                  std::max<int64_t>(1, ((int64_t)h->sm_count * waves * (qgroups_total > 1 ? 2 : 1) +
+                                  std::max<int64_t>(1, ((int64_t)h->sm_count * (qgroups_total > 1 ? 2 : 1) +
                                                         qgroups_total - 1) / qgroups_total));
-    S = std::min<int64_t>(S, (int64_t)h->sm_count * waves);
+    S = std::min<int64_t>(S, (int64_t)h->sm_count);
     TRY(h->parts.ensure((size_t)nq * S * k * sizeof(uint64_t)));
     ScanParams p{};
     p.rows = rows;
@@ -606,16 +585,24 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-static int get_tensormap_encoder(PFN_encodeTiled* out) {
-    static PFN_encodeTiled fn = nullptr;
-    if (!fn) {
+// 2-D TMA map of a row matrix [nrows, ld] (fp32) in kGemmBM x kGemmBK boxes: the A operand of every K2 kernel.
+static int encode_rows_tmap(const float* rows, int ld, int64_t nrows, CUtensorMap* out) {
+    static PFN_encodeTiled encode = nullptr;
+    if (!encode) {
         void* p = nullptr;
         cudaDriverEntryPointQueryResult qres;
         CK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres));
         if (qres != cudaDriverEntryPointSuccess || !p) return fail("cuTensorMapEncodeTiled is not available in this driver");
-        fn = (PFN_encodeTiled)p;
+        encode = (PFN_encodeTiled)p;
     }
-    *out = fn;
+    cuuint64_t gdim[2] = {(cuuint64_t)ld, (cuuint64_t)nrows};
+    cuuint64_t gstr[1] = {(cuuint64_t)ld * 4};
+    cuuint32_t box[2] = {(cuuint32_t)kGemmBK, (cuuint32_t)kGemmBM};
+    cuuint32_t estr[2] = {1, 1};
+    CUresult r = encode(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)rows, gdim, gstr, box, estr,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
     return 0;
 }
 
@@ -626,11 +613,11 @@ static int get_tensormap_encoder(PFN_encodeTiled* out) {
 constexpr double kK1BatchBytesPerS = 4.2e12;
 constexpr double kK2StreamBytesPerS = 6.0e12;
 constexpr double kK2FixedSeconds = 0.3e-3;
+constexpr int64_t kK2MinBatch = 5;  // measured: K2 5.8 ms vs K1 8.1 ms at 5..8 queries (10M x 768)
 
 // Can the tensor-core path take this problem?  (candidate capacity `cap` rows form epoch 0)
 static bool gemm_eligible(const wb_index* h, int64_t nrows, int64_t nq, int k, int* cap_out) {
-    if (env_int("WB_GEMM", 1) == 0) return false;
-    if (nq < env_int("WB_GEMM_MIN_NQ", 5)) return false;  // measured: K2 5.8 ms vs K1 8.1 ms at 5..8 queries (10M x 768)
+    if (nq < kK2MinBatch) return false;
     if (nrows >= ((int64_t)1 << 31) - 256) return false;  // TMA coordinates are int32
     int64_t cap = std::min<int64_t>(4096, std::max<int64_t>(256, ((nrows / 64) + 127) / 128 * 128));
     if (cap < 2 * (int64_t)k || nrows < 4 * cap) return false;
@@ -662,13 +649,12 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
     const int nqb = (int)((nq + kGemmBN - 1) / kGemmBN);
     const int kstride = k + cap;
     // measured (10M x 768): 40 / 64 queries 5.9 / 6.3 ms on one CTA vs 6.2 / 6.4 ms on the pair; 128 queries 8.8 vs 8.1 ms
-    const bool use2 = BN >= 128 && env_int("WB_GEMM_2CTA", 1) != 0 && (h->sm_count % 2) == 0;
+    const bool use2 = BN >= 128 && (h->sm_count % 2) == 0;
     // Batches above 128 queries run their filter epochs in 256-query blocks on the SS kernel (gemm_ss.cuh): half as many
     // passes over the rows and 1.5x fewer L2 bytes per MAC than 128-query blocks.
-    const bool use_f2 = BN >= 128 && filter && use2 && nq > 128 && env_int("WB_GEMM_F2", 1) != 0;
+    const bool use_f2 = use2 && filter && nq > 128;
     // a single block of 65..128 queries: the same SS kernel with 64 queries per CTA (one pass over the rows, HBM-bound)
-    const bool use_f2h = BN >= 128 && filter && use2 && nq <= 128 && env_int("WB_GEMM_F2", 1) != 0 &&
-                         env_int("WB_GEMM_F2H", 1) != 0;
+    const bool use_f2h = use2 && filter && nq <= 128;
     const int nqb2 = (int)((nq + kF2BN - 1) / kF2BN);
     const int nq_pad = use_f2 ? nqb2 * kF2BN : nqb * kGemmBN;  // thresholds / margins of padding queries: +inf / 0
     TRY(h->gimg.ensure((size_t)nqb * nchunks * kGemmBBytes));
@@ -705,8 +691,7 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
     int* cnt = reinterpret_cast<int*>(thr + (size_t)nq_pad);
     int* overflow = cnt + nq;
     unsigned int* dispensers = reinterpret_cast<unsigned int*>(overflow + 16);  // [64], zeroed once per search
-    const bool dyn_work = env_int("WB_GEMM_DYNAMIC", 1) != 0;
-    if (dyn_work) CK(cudaMemsetAsync(dispensers, 0, 64 * sizeof(unsigned int), st));
+    CK(cudaMemsetAsync(dispensers, 0, 64 * sizeof(unsigned int), st));
     int epoch_no = 0;
     uint64_t* keys = h->gkeys.as<uint64_t>();
     {
@@ -735,34 +720,21 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
         CK(cudaGetLastError());
         h->launches += 2;
     }
-    PFN_encodeTiled encode = nullptr;
-    TRY(get_tensormap_encoder(&encode));
     CUtensorMap tmap;
-    {
-        cuuint64_t gdim[2] = {(cuuint64_t)ld, (cuuint64_t)nrows};
-        cuuint64_t gstr[1] = {(cuuint64_t)ld * 4};
-        cuuint32_t box[2] = {(cuuint32_t)kGemmBK, (cuuint32_t)kGemmBM};
-        cuuint32_t estr[2] = {1, 1};
-        CUresult r = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)rows, gdim, gstr, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
+    TRY(encode_rows_tmap(rows, ld, nrows, &tmap));
+    if constexpr (BN >= 128) {  // the CTA pair exists for 128-query blocks only
+        if (use2) {
+            CK(smem_optin<gemm2_topk_kernel<BN, false>>((int)Gemm2Cfg<BN>::kSmemBytes));
+            if (use_f2) CK(smem_optin<filter2_topk_kernel<128, false, false>>((int)kF2SmemBytes));
+            if (use_f2h) CK(smem_optin<filter2_topk_kernel<64, false, false>>((int)F2Cfg<64>::kSmemBytes));
+        }
     }
-    static thread_local bool attr_done[64] = {};
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (dev >= 64 || !attr_done[dev]) {
-        CK(cudaFuncSetAttribute(gemm_topk_kernel<BN, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes));
-        CK(cudaFuncSetAttribute(gemm_topk_kernel<BN, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)GemmCfg<BN, false>::kSmemBytes));
-        if (dev < 64) attr_done[dev] = true;
+    if (!use2) {
+        CK(smem_optin<gemm_topk_kernel<BN, false>>((int)kGemmSmemBytes));
+        CK(smem_optin<gemm_topk_kernel<BN, false, 1>>((int)GemmCfg<BN, false>::kSmemBytes));
     }
-    TRY(merge_smem_optin<true>());
-    static thread_local bool cattr_done[64] = {};
-    if (dev >= 64 || !cattr_done[dev]) {
-        CK(cudaFuncSetAttribute(compact_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 8192 * 8));
-        if (dev < 64) cattr_done[dev] = true;
-    }
+    CK(smem_optin<merge_topk_kernel<true>>(8192 * 8));
+    CK(smem_optin<compact_topk_kernel>(8192 * 8));
     GemmParams g{};
     g.nchunks = nchunks;
     g.nq = (int)nq;
@@ -809,56 +781,28 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
         // first epoch: 3xTF32 scores select, the winners are re-scored; later epochs: one-term filter, candidates re-scored
         const bool one_term = filter && r0 > 0;
         c.rescore = filter ? (r0 == 0 ? 2 : 1) : 0;
-        bool launched = false;
         if constexpr (BN >= 128) {
+            // with the pair, every filter epoch (one_term) goes to the SS kernel: use_f2 or use_f2h is set
+            const int64_t ntp = ((r1 - r0 + kGemmBM - 1) / kGemmBM + 1) / 2;
             if (use_f2 && one_term) {  // 256-query blocks, both operands from shared memory
-                static thread_local bool a3[64] = {};
-                if (dev >= 64 || !a3[dev]) {
-                    CK(cudaFuncSetAttribute(filter2_topk_kernel<128, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            (int)kF2SmemBytes));
-                    if (dev < 64) a3[dev] = true;
-                }
                 GemmParams g2 = g;
                 g2.nqb = nqb2;
                 g2.bimg = h->gimg2.as<float>();
-                const int64_t ntp = ((r1 - r0 + kGemmBM - 1) / kGemmBM + 1) / 2;
                 const unsigned grid3 = 2u * (unsigned)std::min<int64_t>(ntp * nqb2, h->sm_count / 2);
                 filter2_topk_kernel<128, false, false><<<grid3, kF2Threads, kF2SmemBytes, st>>>(tmap, g2);
-                launched = true;
             } else if (use_f2h && one_term) {
-                static thread_local bool a5[64] = {};
-                if (dev >= 64 || !a5[dev]) {
-                    CK(cudaFuncSetAttribute(filter2_topk_kernel<64, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            (int)F2Cfg<64>::kSmemBytes));
-                    if (dev < 64) a5[dev] = true;
-                }
                 GemmParams g2 = g;
                 g2.bimg = h->gimg2.as<float>();
-                const int64_t ntp = ((r1 - r0 + kGemmBM - 1) / kGemmBM + 1) / 2;
                 const unsigned grid3 = 2u * (unsigned)std::min<int64_t>(ntp * nqb, h->sm_count / 2);
                 filter2_topk_kernel<64, false, false><<<grid3, kF2Threads, F2Cfg<64>::kSmemBytes, st>>>(tmap, g2);
-                launched = true;
-            }
-        }
-        if constexpr (BN >= 128) {  // the CTA pair exists for 128-query blocks only
-            if (use2 && !launched) {
-                static thread_local bool a2[64] = {};
-                if (dev >= 64 || !a2[dev]) {
-                    CK(cudaFuncSetAttribute(gemm2_topk_kernel<BN, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            (int)Gemm2Cfg<BN>::kSmemBytes));
-                    CK(cudaFuncSetAttribute(gemm2_topk_kernel<BN, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            (int)Gemm2Cfg<BN>::kSmemBytes));
-                    if (dev < 64) a2[dev] = true;
-                }
-                const int64_t ntp = ((r1 - r0 + kGemmBM - 1) / kGemmBM + 1) / 2;
+            } else if (use2) {
                 const unsigned grid2 = 2u * (unsigned)std::min<int64_t>(ntp * nqb, h->sm_count / 2);
-                if (one_term) gemm2_topk_kernel<BN, false, 1><<<grid2, kGemmThreads, Gemm2Cfg<BN>::kSmemBytes, st>>>(tmap, g);
-                else gemm2_topk_kernel<BN, false><<<grid2, kGemmThreads, Gemm2Cfg<BN>::kSmemBytes, st>>>(tmap, g);
+                gemm2_topk_kernel<BN, false><<<grid2, kGemmThreads, Gemm2Cfg<BN>::kSmemBytes, st>>>(tmap, g);
             }
         }
-        if (!use2 && !launched) {
+        if (!use2) {
             // SMs stream at different rates: (tile, block) items are drawn from a dispenser, not dealt out statically
-            g.work_counter = dyn_work && epoch_no < 64 ? dispensers + epoch_no : nullptr;
+            g.work_counter = epoch_no < 64 ? dispensers + epoch_no : nullptr;
             if (one_term) {
                 GemmParams g1 = g;
                 if (kFold) g1.bimg = h->gimg2.as<float>();
@@ -897,14 +841,11 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
 
 static int run_flat_gemm(wb_index* h, const float* rows, int64_t nrows, const float* q_ld, int64_t nq, int k, int cap,
                          const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, bool* overflowed) {
-    const int bn_max = env_int("WB_GEMM_BN", 128);
     // 16-query blocks halve the image traffic and the MMA work of a half-empty 32-query block (K2 is power-capped at
     // small batches: 992 W and 1.37 GHz at batch 16)
-    if (nq <= 16 && bn_max >= 16 && env_int("WB_GEMM_BN16", 1))
-        return run_flat_gemm_t<16>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
-    if (nq <= 32 && bn_max >= 32) return run_flat_gemm_t<32>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
-    if ((nq <= 64 && bn_max >= 64) || bn_max < 128)
-        return run_flat_gemm_t<64>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
+    if (nq <= 16) return run_flat_gemm_t<16>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
+    if (nq <= 32) return run_flat_gemm_t<32>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
+    if (nq <= 64) return run_flat_gemm_t<64>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
     return run_flat_gemm_t<128>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
 }
 
@@ -912,8 +853,7 @@ static int run_flat_gemm(wb_index* h, const float* rows, int64_t nrows, const fl
 // One launch, no epochs, no host synchronisation: the points are the A operand (streamed once from HBM), the
 // centroids are the query images (L2 resident), each row keeps its running maximum in the epilogue.
 static bool assign_gemm_eligible(const wb_index* h, int64_t n) {
-    return env_int("WB_GEMM", 1) != 0 && env_int("WB_GEMM_ASSIGN", 1) != 0 && n >= 1024 && h->nlist >= 64 &&
-           n < ((int64_t)1 << 31) - 256;
+    return n >= 1024 && h->nlist >= 64 && n < ((int64_t)1 << 31) - 256;
 }
 
 static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* assign_out, float* best_out,
@@ -922,7 +862,9 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
     using Cfg = GemmCfg<BN>;
     const int ld = h->ld;
     const int nchunks = (ld + kGemmBK - 1) / kGemmBK;
-    if (tf32 && (h->sm_count % 2) == 0 && env_int("WB_GEMM_2CTA", 1) != 0) {
+    const bool use2 = (h->sm_count % 2) == 0;
+    CUtensorMap tmap;
+    if (tf32 && use2) {
         // k-means TRAINING assignment: plain TF32 on the SS pair kernel, 256 centroids per block (gemm_ss.cuh)
         const int nqb2 = (int)((h->nlist + kF2BN - 1) / kF2BN);
         TRY(h->gimg2.ensure((size_t)nqb2 * 2 * nchunks * kF2BBytes));
@@ -930,25 +872,8 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
         image_queries_f2_kernel<<<(unsigned)((n4 + 255) / 256), 256, 0, st>>>(h->centroids, (int)h->nlist, ld, nchunks, nqb2,
                                                                              h->gimg2.as<float>());
         CK(cudaGetLastError());
-        PFN_encodeTiled enc = nullptr;
-        TRY(get_tensormap_encoder(&enc));
-        CUtensorMap tm;
-        cuuint64_t gdim[2] = {(cuuint64_t)ld, (cuuint64_t)n};
-        cuuint64_t gstr[1] = {(cuuint64_t)ld * 4};
-        cuuint32_t box[2] = {(cuuint32_t)kGemmBK, (cuuint32_t)kGemmBM};
-        cuuint32_t estr[2] = {1, 1};
-        CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)x_ld, gdim, gstr, box, estr,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-        static thread_local bool a4[64] = {};
-        int dev = 0;
-        CK(cudaGetDevice(&dev));
-        if (dev >= 64 || !a4[dev]) {
-            CK(cudaFuncSetAttribute(filter2_topk_kernel<128, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)kF2SmemBytes));
-            if (dev < 64) a4[dev] = true;
-        }
+        TRY(encode_rows_tmap(x_ld, ld, n, &tmap));
+        CK(smem_optin<filter2_topk_kernel<128, true, false>>((int)kF2SmemBytes));
         GemmParams g{};
         g.row_begin = 0;
         g.row_end = n;
@@ -959,7 +884,7 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
         g.assign_out = assign_out;
         g.best_out = best_out;
         const int64_t ntp = ((n + kGemmBM - 1) / kGemmBM + 1) / 2;
-        filter2_topk_kernel<128, true, false><<<2u * (unsigned)std::min<int64_t>(ntp, h->sm_count / 2), kF2Threads, kF2SmemBytes, st>>>(tm, g);
+        filter2_topk_kernel<128, true, false><<<2u * (unsigned)std::min<int64_t>(ntp, h->sm_count / 2), kF2Threads, kF2SmemBytes, st>>>(tmap, g);
         CK(cudaGetLastError());
         h->launches += 2;
         h->gemm_launches++;
@@ -968,7 +893,6 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
     const int nqb = (int)((h->nlist + BN - 1) / BN);
     TRY(h->gimg.ensure((size_t)nqb * nchunks * Cfg::kBBytes));
     const int64_t n2 = (int64_t)nqb * nchunks * 8 * BN;
-    const bool use2 = env_int("WB_GEMM_2CTA", 1) != 0 && (h->sm_count % 2) == 0;
     if (use2) {
         const int64_t n3 = (int64_t)(2 * nqb) * nchunks * 8 * (BN / 2);
         split_queries_kernel<BN / 2><<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(h->centroids, (int)h->nlist, ld, nchunks,
@@ -978,24 +902,7 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
                                                                               h->gimg.as<float>());
     }
     CK(cudaGetLastError());
-    PFN_encodeTiled encode = nullptr;
-    TRY(get_tensormap_encoder(&encode));
-    CUtensorMap tmap;
-    cuuint64_t gdim[2] = {(cuuint64_t)ld, (cuuint64_t)n};
-    cuuint64_t gstr[1] = {(cuuint64_t)ld * 4};
-    cuuint32_t box[2] = {(cuuint32_t)kGemmBK, (cuuint32_t)kGemmBM};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)x_ld, gdim, gstr, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-    static thread_local bool attr_done[64] = {};
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (dev >= 64 || !attr_done[dev]) {
-        CK(cudaFuncSetAttribute(gemm_topk_kernel<BN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
-        if (dev < 64) attr_done[dev] = true;
-    }
+    TRY(encode_rows_tmap(x_ld, ld, n, &tmap));
     GemmParams g{};
     g.row_begin = 0;
     g.row_end = n;
@@ -1007,16 +914,12 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
     g.best_out = best_out;
     const int64_t ntiles = (n + kGemmBM - 1) / kGemmBM;
     if (use2) {
-        static thread_local bool a2[64] = {};
-        if (dev >= 64 || !a2[dev]) {
-            CK(cudaFuncSetAttribute(gemm2_topk_kernel<BN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)Gemm2Cfg<BN>::kSmemBytes));
-            if (dev < 64) a2[dev] = true;
-        }
+        CK(smem_optin<gemm2_topk_kernel<BN, true>>((int)Gemm2Cfg<BN>::kSmemBytes));
         const int64_t ntp = (ntiles + 1) / 2;
         gemm2_topk_kernel<BN, true><<<2u * (unsigned)std::min<int64_t>(ntp, h->sm_count / 2), kGemmThreads,
                                      Gemm2Cfg<BN>::kSmemBytes, st>>>(tmap, g);
     } else {
+        CK(smem_optin<gemm_topk_kernel<BN, true>>((int)Cfg::kSmemBytes));
         gemm_topk_kernel<BN, true><<<(unsigned)std::min<int64_t>(ntiles, h->sm_count), kGemmThreads, Cfg::kSmemBytes, st>>>(tmap, g);
     }
     CK(cudaGetLastError());
@@ -1047,7 +950,7 @@ static int run_flat_any(wb_index* h, const float* rows, int64_t nrows, const flo
         h->gemm_fallbacks++;
     }
     return run_flat_scan(h, rows, nrows, q_dev, nq, k, ids, D, I, st, timed,
-                         ex && nq <= kMaxGridY && env_int("WB_FUSE_EXCH", 1) ? ex : nullptr, exchanged);
+                         ex && nq <= kMaxGridY ? ex : nullptr, exchanged);
 }
 
 // ---- K8: CSR inverted lists, built on the device (csr.cuh) -------------------------------------------------------
@@ -1311,13 +1214,7 @@ extern "C" int wb_ivf_add_preassigned(wb_index* h, int64_t n, const float* x_hos
 // ---- K5 for batches: list-major scan (ivf_lm.cuh) ------------------------------------------------------------------
 template <int RW>
 static int launch_lm_t(const LmParams& p, int grid, size_t smem, cudaStream_t st) {
-    static thread_local bool attr_done[64] = {};
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (dev >= 64 || !attr_done[dev]) {
-        CK(cudaFuncSetAttribute(ivf_listmajor_kernel<8, RW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-        if (dev < 64) attr_done[dev] = true;
-    }
+    CK(smem_optin<ivf_listmajor_kernel<8, RW>>(232448));
     ivf_listmajor_kernel<8, RW><<<grid, kScanThreads, smem, st>>>(p);
     CK(cudaGetLastError());
     return 0;
@@ -1423,6 +1320,8 @@ static int run_gather_scan(wb_index* h, const ScanCfg& c, ScanParams& p, int64_t
 }
 
 // ---- search --------------------------------------------------------------------------------
+constexpr int64_t kIvfFuseCoarseMaxQ = 4;  // largest IVF batch that runs the coarse quantizer inside the list-scan launch
+
 static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld] */, int64_t k, int64_t nprobe, float* D,
                            int64_t* I, cudaStream_t st, const ExchParams* ex = nullptr, bool* exchanged = nullptr) {
     if (exchanged) *exchanged = false;
@@ -1437,12 +1336,12 @@ static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld
     ScanCfg c;
     TRY(plan_scan(h, 1, (int)k, true, np, &c));
     int64_t S = nq >= h->sm_count ? 1 : std::max<int64_t>(1, (int64_t)h->sm_count / nq);
-    if (ex && (nq > kMaxGridY || !env_int("WB_FUSE_EXCH", 1))) ex = nullptr;
+    if (ex && nq > kMaxGridY) ex = nullptr;
     int S_merge = 0, heads_bytes = 0;
     const bool fuse = tail_fusable(c, (int)k, S, ex ? ex->world : 1, &S_merge, &heads_bytes);
     // K4 + K5 in one launch (coarse.cuh): a few queries, every CTA resident, the selection scratch fits the idle ring
     const size_t ring_bytes = (size_t)c.stages * kConsumerWarps * c.RW * c.ck * 4;
-    bool fuse_coarse = fuse && h->coop_ok && nq <= env_int("WB_IVF_FUSE_COARSE_MAXQ", 4) && S * nq <= h->sm_count &&
+    bool fuse_coarse = fuse && h->coop_ok && nq <= kIvfFuseCoarseMaxQ && S * nq <= h->sm_count &&
                        h->nlist < ((int64_t)1 << 30) && coarse_smem_layout(h->nlist, np).total <= ring_bytes &&
                        env_int("WB_IVF_FUSE_COARSE", 1) && env_int("WB_IVF_LISTMAJOR", -1) != 1;
     for (int attempt = 0; attempt < 2; ++attempt) {
@@ -1639,7 +1538,7 @@ extern "C" int wb_merge_topk_dev(int device, int64_t nq, int64_t k, int64_t npar
     m.Ip = I_parts_dev;
     m.D = D_dev;
     m.I = I_dev;
-    TRY(merge_smem_optin<false>());
+    CK(smem_optin<merge_topk_kernel<false>>(8192 * 8));
     merge_topk_kernel<false><<<(unsigned)nq, kMergeThreads, (size_t)m.S * 8, (cudaStream_t)stream>>>(m);
     CK(cudaGetLastError());
     return 0;
@@ -2151,11 +2050,7 @@ static int launch_exchange_kernel(wb_exchange* ex, ExchParams& p, const float* D
     p.D_local = D_local;
     p.I_local = I_local;
     p.S = merge_buffer_entries(p.k, p.world);
-    static thread_local bool attr_done[64] = {};
-    if (ex->device >= 64 || !attr_done[ex->device]) {
-        CK(cudaFuncSetAttribute(exchange_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 8192 * 8));
-        if (ex->device < 64) attr_done[ex->device] = true;
-    }
+    CK(smem_optin<exchange_merge_kernel>(8192 * 8));
     int sms = 148;
     CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ex->device));
     const unsigned grid = (unsigned)std::min<int64_t>(p.nq, sms);  // one resident CTA per SM at most (1024 threads)

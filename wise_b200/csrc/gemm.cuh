@@ -683,10 +683,9 @@ __device__ __forceinline__ void umma_tf32_ts_2cta(uint32_t d_tmem, uint32_t a_tm
         : "memory");
 }
 
-template <int BN, bool ARGMAX, int TERMS = 3>
+template <int BN, bool ARGMAX>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kGemmThreads, 1)
 gemm2_topk_kernel(const __grid_constant__ CUtensorMap tmap, const GemmParams p) {
-    static_assert(TERMS == 3 || (TERMS == 1 && !ARGMAX), "one-term scores are only a filter");
     using Cfg2 = Gemm2Cfg<BN>;
     constexpr int kG2Half = Cfg2::kHalf;
     constexpr int kRaw = Cfg2::kRaw;
@@ -795,11 +794,8 @@ gemm2_topk_kernel(const __grid_constant__ CUtensorMap tmap, const GemmParams p) 
             for (int c = 0; c < p.nchunks; ++c) {
                 mbar_wait_cluster(&b_empty[s], ph ^ 1u);
                 if (elect_one_sync()) {
-                    // one-term epochs read only the hi half of the image (the first half of a chunk's image): half
-                    // the L2 -> SM bytes of the query operand, which is what bounds a single 128-query block
-                    constexpr uint32_t kCopy = TERMS == 1 ? kBBytes / 2 : kBBytes;
-                    mbar_arrive_expect_tx(&b_full[s], kCopy);
-                    bulk_g2s(bimg_s + (size_t)s * kBBytes, bsrc + (size_t)c * (kBBytes / 4), kCopy, &b_full[s]);
+                    mbar_arrive_expect_tx(&b_full[s], kBBytes);
+                    bulk_g2s(bimg_s + (size_t)s * kBBytes, bsrc + (size_t)c * (kBBytes / 4), kBBytes, &b_full[s]);
                 }
                 __syncwarp();
                 if (++s == kBSlots) { s = 0; ph ^= 1u; }
@@ -844,10 +840,8 @@ gemm2_topk_kernel(const __grid_constant__ CUtensorMap tmap, const GemmParams p) 
                         const uint64_t dh = dh0 + (uint64_t)((j * 2 * kG2Half * 16) >> 4);
                         const uint64_t dl = dl0 + (uint64_t)((j * 2 * kG2Half * 16) >> 4);
                         umma_tf32_ts_2cta(d_tmem, a_hi + j * 8, dh, idesc, (c | j) != 0);
-                        if constexpr (TERMS == 3) {
-                            umma_tf32_ts_2cta(d_tmem, a_hi + j * 8, dl, idesc, 1);
-                            umma_tf32_ts_2cta(d_tmem, a_lo + j * 8, dh, idesc, 1);
-                        }
+                        umma_tf32_ts_2cta(d_tmem, a_hi + j * 8, dl, idesc, 1);
+                        umma_tf32_ts_2cta(d_tmem, a_lo + j * 8, dh, idesc, 1);
                     }
                     umma_commit_2cta(&b_empty[s]);
                     umma_commit_2cta(&a_empty[sa]);
@@ -883,14 +877,14 @@ gemm2_topk_kernel(const __grid_constant__ CUtensorMap tmap, const GemmParams p) 
                     for (int e = 0; e < 4; ++e) {
                         const uint32_t h = __float_as_uint(x[e]) & 0xFFFFE000u;
                         hi[ch * 4 + e] = h;
-                        if constexpr (TERMS != 1) lo[ch * 4 + e] = __float_as_uint(x[e] - __uint_as_float(h));
+                        lo[ch * 4 + e] = __float_as_uint(x[e] - __uint_as_float(h));
                     }
                 }
                 mbar_wait_cluster(&a_empty[ss], phs ^ 1u);
                 tc_fence_after();
                 const uint32_t ta = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(kTmemAOff + ss * 64);
                 tmem_st32(ta, hi);
-                if constexpr (TERMS != 1) tmem_st32(ta + 32, lo);
+                tmem_st32(ta + 32, lo);
                 asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
                 tc_fence_before();
                 __syncwarp();
@@ -915,11 +909,7 @@ gemm2_topk_kernel(const __grid_constant__ CUtensorMap tmap, const GemmParams p) 
             const int64_t row = p.row_begin + tile * kGemmBM + quarter * 32 + lane;
             const bool row_ok = row < p.row_end;
             if constexpr (!ARGMAX) {
-                if (etid < BN) {
-                    float t = p.thr[qb * BN + etid];
-                    if constexpr (TERMS == 1) t -= p.margin[qb * BN + etid];
-                    thr_s[buf * BN + etid] = t;
-                }
+                if (etid < BN) thr_s[buf * BN + etid] = p.thr[qb * BN + etid];
                 named_bar_sync(kBarEpilogue, 128);
             } else if (qb == 0) {
                 best = -INFINITY;

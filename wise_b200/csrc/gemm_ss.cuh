@@ -1,7 +1,7 @@
 // gemm_ss.cuh - K2 "filter" epochs for large batches: 256-query blocks on a CTA pair, BOTH operands read by the
 // tensor core straight from shared memory (tcgen05.mma.cta_group::2.kind::tf32, SS form, M = 256, N = 256).
 //
-// Same contract as gemm2_topk_kernel<128, false, TERMS = 1> (gemm.cuh): one-term TF32 scores are only a filter, a row
+// Same contract as the one-term gemm_topk_kernel<BN, false, TERMS = 1> (gemm.cuh): one-term TF32 scores are only a filter, a row
 // becomes a candidate when its score exceeds thr - margin and rescore_candidates_kernel / compact_topk_kernel
 // (merge.cuh) re-score the candidates exactly in fp32, so the result is the exact top-k.  Replaces faiss
 // exhaustive_inner_product_blas [faiss-upstream] reached from /root/reference/src/index/feature_search_index.py:113.

@@ -46,7 +46,6 @@ struct ScanParams {
     int stages;
     int single_copy;        // flat && nchunks == 1: one bulk copy per group
     int rw;                 // rows per consumer warp (4, 2 or 1); a row group is 8 * rw rows
-    int prefetch_idx;       // gather: look up the next group's row indices one iteration ahead
     uint64_t* parts;        // [nq][nparts][k] keys
     int nparts;             // == gridDim.x
     // gather mode (IVF): candidates = concatenation of the probed lists of query blockIdx.y
@@ -318,15 +317,11 @@ __global__ void __launch_bounds__(kScanThreads, 1) scan_topk_kernel(const ScanPa
         for (; g < ngroups;) {
             const int64_t p0 = g * kGroupRows;
             const int nvalid = (int)min((int64_t)kGroupRows, total - p0);
-            int64_t row = row_next;
+            const int64_t row = row_next;
             // the next group is drawn (and its row indices looked up) now, one iteration ahead: the atomic and the
             // CSR loads are in flight while this group's copies are issued
             const int64_t g_next = draw(g);
-            if (p.prefetch_idx || dyn) {
-                if (g_next < ngroups) row_next = lookup(g_next);
-            } else if (g != (int64_t)blockIdx.x) {
-                row = lookup(g);
-            }
+            if (g_next < ngroups) row_next = lookup(g_next);
             const float* src = p.rows + (size_t)row * ld;
             for (int ch = 0; ch < p.nchunks; ++ch) {
                 if (lane == 0) {
