@@ -9,8 +9,10 @@
 #include <string.h>
 
 #include <algorithm>
+#include <memory>
 #include <random>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/wise_b200.h"
@@ -68,50 +70,59 @@ extern "C" int wb_device_count(int* count) {
     return 0;
 }
 
-// ---- grow-only device scratch --------------------------------------------------------------
-struct DevBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-    int ensure(size_t bytes) {
-        if (bytes <= cap) return 0;
-        if (p) CK(cudaFree(p));
-        p = nullptr;
-        cap = 0;
-        size_t want = std::max(bytes, (size_t)1 << 16);
-        CK(cudaMalloc(&p, want));
-        cap = want;
-        return 0;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-    template <class T>
-    T* as() { return reinterpret_cast<T*>(p); }
+// ---- owned device / pinned memory ----------------------------------------------------------
+struct DevFree {
+    void operator()(void* p) const { cudaFree(p); }
 };
+struct HostFree {
+    void operator()(void* p) const { cudaFreeHost(p); }
+};
+template <class T>
+using DevPtr = std::unique_ptr<T, DevFree>;
+template <class T>
+using PinPtr = std::unique_ptr<T, HostFree>;
+struct EventDestroy {
+    void operator()(cudaEvent_t e) const { cudaEventDestroy(e); }
+};
+using EventPtr = std::unique_ptr<CUevent_st, EventDestroy>;
 
-// Grow-only pinned host buffer (cudaHostAlloc): a copy between pageable memory and the device is staged by the
-// driver and blocks the call; small transfers go through this buffer instead and stay asynchronous.
-struct PinBuf {
-    void* p = nullptr;
+// cudaMalloc into an owner; `out` keeps what it held when the allocation fails
+template <class T>
+static cudaError_t dev_alloc(DevPtr<T>* out, size_t bytes) {
+    T* p = nullptr;
+    const cudaError_t e = cudaMalloc(&p, bytes);
+    if (e == cudaSuccess) out->reset(p);
+    return e;
+}
+
+// Grow-only scratch (at least 64 KB, contents not kept when it grows) in device memory, or, when `Pinned`, in pinned
+// host memory: a copy between pageable memory and the device is staged by the driver and blocks the call; small
+// transfers go through a pinned buffer instead and stay asynchronous.
+template <bool Pinned>
+struct GrowBuf {
+    std::unique_ptr<void, std::conditional_t<Pinned, HostFree, DevFree>> mem;
     size_t cap = 0;
     int ensure(size_t bytes) {
         if (bytes <= cap) return 0;
-        if (p) CK(cudaFreeHost(p));
-        p = nullptr;
+        mem.reset();
         cap = 0;
         const size_t want = std::max(bytes, (size_t)1 << 16);
-        CK(cudaHostAlloc(&p, want, cudaHostAllocMapped | cudaHostAllocPortable));  // kernels may write into it (UVA)
+        void* p = nullptr;
+        if constexpr (Pinned)
+            CK(cudaHostAlloc(&p, want, cudaHostAllocMapped | cudaHostAllocPortable));  // kernels may write into it (UVA)
+        else
+            CK(cudaMalloc(&p, want));
+        mem.reset(p);
         cap = want;
         return 0;
     }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-    }
+    void* get() const { return mem.get(); }
+    template <class T>
+    T* as() const { return reinterpret_cast<T*>(mem.get()); }
 };
+using DevBuf = GrowBuf<false>;
+using PinBuf = GrowBuf<true>;
+
 struct wb_index {
     int device = 0;
     int d = 0, ld = 0;
@@ -121,20 +132,20 @@ struct wb_index {
     bool spherical = false;  // k-means: L2-renormalise the centroids after every update (faiss cp.spherical)
     cudaStream_t stream = nullptr;
     // row store (insertion order)
-    float* rows = nullptr;
-    int64_t* ids = nullptr;
-    int32_t* assign = nullptr;  // IVF: list of each row
+    DevPtr<float> rows;
+    DevPtr<int64_t> ids;
+    DevPtr<int32_t> assign;  // IVF: list of each row
     int64_t n = 0, cap = 0;
-    float* norm2_max = nullptr;  // device scalar: max |row|^2 over everything ever added (K2 filter margin)
+    DevPtr<float> norm2_max;  // device scalar: max |row|^2 over everything ever added (K2 filter margin)
     // IVF quantizer + inverted lists.  `ids` always stay in INSERTION order.  After a (re)grouping the rows are
     // stored list by list (insertion order kept inside a list): row_pos[row] is then the insertion position of a
     // storage row - the tie rule and the id lookup - and slot_row is null.  When the transient second copy of the rows
     // does not fit, the rows stay where they are and slot_row[CSR slot] is the storage row of each list slot.
-    float* centroids = nullptr;   // [nlist, ld]
-    uint32_t* slot_row = nullptr; // [n] or null (slot == storage row)
-    uint32_t* row_pos = nullptr;  // [map_cap] or null (storage row == insertion position)
+    DevPtr<float> centroids;   // [nlist, ld]
+    DevPtr<uint32_t> slot_row; // [n] or null (slot == storage row)
+    DevPtr<uint32_t> row_pos;  // [map_cap] or null (storage row == insertion position)
     int64_t map_cap = 0;
-    int64_t* list_off = nullptr;  // [nlist + 1]
+    DevPtr<int64_t> list_off;  // [nlist + 1]
     bool csr_dirty = true;
     // scratch
     DevBuf parts, qbuf, dbuf, ibuf, pD, pI, xbuf, idbuf, misc, kperm, koff, gimg, gimg2, gkeys, gstate, gmargin, eD, eI, tailcnt, ccnt, ctot, lmA, lmB, lmC, lmD, lmE, lmF, lmG;
@@ -156,6 +167,19 @@ struct wb_index {
     static constexpr int kEvRing = 128;  // event pairs of the most recent timed scan launches
     cudaEvent_t ev0[kEvRing] = {}, ev1[kEvRing] = {};
     int64_t ev_count = 0;
+
+    // The caller has made `device` current.  The members free the memory once the stream is gone.
+    ~wb_index() {
+        if (!stream) return;
+        cudaStreamSynchronize(stream);
+        for (cudaEvent_t e : add_ev)
+            if (e) cudaEventDestroy(e);
+        for (int i = 0; i < kEvRing; ++i) {
+            if (ev0[i]) cudaEventDestroy(ev0[i]);
+            if (ev1[i]) cudaEventDestroy(ev1[i]);
+        }
+        cudaStreamDestroy(stream);
+    }
 };
 
 static int set_dev(const wb_index* h) {
@@ -177,7 +201,7 @@ static int create_common(int d, int device, bool ivf, int64_t nlist, wb_index** 
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, device));
     if (prop.major != 10) return fail("device %d is sm_%d%d; this library is built for sm_100a only", device, prop.major, prop.minor);
-    wb_index* h = new wb_index();
+    std::unique_ptr<wb_index> h(new wb_index());
     h->device = device;
     h->d = d;
     h->ld = (d + 3) & ~3;
@@ -192,16 +216,16 @@ static int create_common(int d, int device, bool ivf, int64_t nlist, wb_index** 
         CK(cudaEventCreate(&h->ev0[i]));
         CK(cudaEventCreate(&h->ev1[i]));
     }
-    CK(cudaMalloc(&h->norm2_max, sizeof(float)));
-    CK(cudaMemsetAsync(h->norm2_max, 0, sizeof(float), h->stream));
+    CK(dev_alloc(&h->norm2_max, sizeof(float)));
+    CK(cudaMemsetAsync(h->norm2_max.get(), 0, sizeof(float), h->stream));
     if (ivf) {
-        CK(cudaMalloc(&h->centroids, (size_t)nlist * h->ld * sizeof(float)));
-        CK(cudaMemsetAsync(h->centroids, 0, (size_t)nlist * h->ld * sizeof(float), h->stream));
-        CK(cudaMalloc(&h->list_off, (size_t)(nlist + 1) * sizeof(int64_t)));
-        CK(cudaMemsetAsync(h->list_off, 0, (size_t)(nlist + 1) * sizeof(int64_t), h->stream));
+        CK(dev_alloc(&h->centroids, (size_t)nlist * h->ld * sizeof(float)));
+        CK(cudaMemsetAsync(h->centroids.get(), 0, (size_t)nlist * h->ld * sizeof(float), h->stream));
+        CK(dev_alloc(&h->list_off, (size_t)(nlist + 1) * sizeof(int64_t)));
+        CK(cudaMemsetAsync(h->list_off.get(), 0, (size_t)(nlist + 1) * sizeof(int64_t), h->stream));
     }
     CK(cudaStreamSynchronize(h->stream));  // the zero-fills above must not race a first add on another stream
-    *out = h;
+    *out = h.release();
     return 0;
 }
 
@@ -214,28 +238,6 @@ extern "C" int wb_ivf_create(int d, int64_t nlist, int device, wb_index** out) {
 extern "C" int wb_free(wb_index* h) {
     if (!h) return 0;
     cudaSetDevice(h->device);
-    cudaStreamSynchronize(h->stream);
-    cudaFree(h->rows);
-    cudaFree(h->ids);
-    cudaFree(h->assign);
-    cudaFree(h->centroids);
-    cudaFree(h->norm2_max);
-    cudaFree(h->slot_row);
-    cudaFree(h->row_pos);
-    cudaFree(h->list_off);
-    for (DevBuf* b : {&h->parts, &h->qbuf, &h->dbuf, &h->ibuf, &h->pD, &h->pI, &h->xbuf, &h->idbuf, &h->misc,
-                      &h->kperm, &h->koff, &h->gimg, &h->gimg2, &h->gkeys, &h->gstate, &h->gmargin, &h->eD, &h->eI, &h->tailcnt, &h->ccnt, &h->ctot, &h->lmA, &h->lmB, &h->lmC,
-                      &h->lmD, &h->lmE, &h->lmF, &h->lmG, &h->ckeys, &h->phase})
-        b->release();
-    h->pin_q.release();
-    h->pin_o.release();
-    for (int i = 0; i < wb_index::kAddSlots; ++i)
-        if (h->add_ev[i]) cudaEventDestroy(h->add_ev[i]);
-    for (int i = 0; i < wb_index::kEvRing; ++i) {
-        cudaEventDestroy(h->ev0[i]);
-        cudaEventDestroy(h->ev1[i]);
-    }
-    cudaStreamDestroy(h->stream);
     delete h;
     return 0;
 }
@@ -250,11 +252,11 @@ extern "C" int64_t wb_ivf_fused_searches(const wb_index* h) { return h ? h->coar
 constexpr size_t kPhaseCtas = 1024;  // phase stamps: CTAs of query group 0 (the kernel ignores blockIdx.x >= 1024)
 extern "C" int wb_phase_stamps(wb_index* h, uint64_t* out_host, int ctas) {
     if (!h || !out_host) return fail("NULL argument");
-    if (!h->phase.p) return fail("no phase stamps: set WB_PHASE_TS=1 before the search");
+    if (!h->phase.get()) return fail("no phase stamps: set WB_PHASE_TS=1 before the search");
     if (ctas < 1 || (size_t)ctas > kPhaseCtas) return fail("ctas out of range");
     TRY(set_dev(h));
     CK(cudaStreamSynchronize(h->stream));
-    CK(cudaMemcpy(out_host, h->phase.p, (size_t)ctas * 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(out_host, h->phase.get(), (size_t)ctas * 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost));
     return 0;
 }
 extern "C" int wb_gemm_stats(const wb_index* h, int64_t* epochs, int64_t* fallbacks) {
@@ -267,6 +269,17 @@ extern "C" int wb_set_timing(wb_index* h, int on) {
     if (!h) return fail("NULL index");
     h->timing = on != 0;
     h->ev_count = 0;
+    return 0;
+}
+// The event pair around one timed scan, in the ring slot that wb_last_scan_ms / wb_scan_ms_history read.
+static int timing_begin(wb_index* h, bool on, cudaStream_t st) {
+    if (on) CK(cudaEventRecord(h->ev0[h->ev_count % wb_index::kEvRing], st));
+    return 0;
+}
+static int timing_end(wb_index* h, bool on, cudaStream_t st) {
+    if (!on) return 0;
+    CK(cudaEventRecord(h->ev1[h->ev_count % wb_index::kEvRing], st));
+    h->ev_count++;
     return 0;
 }
 static float scan_ms_at(wb_index* h, int64_t i) {
@@ -290,7 +303,7 @@ extern "C" int wb_scan_ms_history(wb_index* h, float* out_ms, int cap) {
 }
 extern "C" int wb_storage(wb_index* h, void** rows_dev, int64_t* ld) {
     if (!h) return fail("NULL index");
-    if (rows_dev) *rows_dev = h->rows;
+    if (rows_dev) *rows_dev = h->rows.get();
     if (ld) *ld = h->ld;
     return 0;
 }
@@ -300,34 +313,32 @@ static int ensure_capacity(wb_index* h, int64_t need) {
     if (need <= h->cap) return 0;
     if (need >= (int64_t)0xFFFFFFFEll) return fail("an index shard is limited to 2^32-2 rows per GPU");
     int64_t newcap = std::max<int64_t>(need, std::max<int64_t>(1024, h->cap + h->cap / 2));
-    float* nrows = nullptr;
-    int64_t* nids = nullptr;
-    int32_t* nas = nullptr;
-    CK(cudaMalloc(&nrows, (size_t)newcap * h->ld * sizeof(float)));
-    CK(cudaMalloc(&nids, (size_t)newcap * sizeof(int64_t)));
-    if (h->ivf) CK(cudaMalloc(&nas, (size_t)newcap * sizeof(int32_t)));
-    if (h->row_pos && newcap > h->map_cap) {
-        uint32_t* np_ = nullptr;
-        CK(cudaMalloc(&np_, (size_t)newcap * sizeof(uint32_t)));
-        if (h->n > 0) CK(cudaMemcpyAsync(np_, h->row_pos, (size_t)h->n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        cudaFree(h->row_pos);
-        h->row_pos = np_;
-        h->map_cap = newcap;
-    }
+    // everything is allocated and copied before the handle changes: a failure leaves it as it was
+    DevPtr<float> nrows;
+    DevPtr<int64_t> nids;
+    DevPtr<int32_t> nas;
+    DevPtr<uint32_t> npos;
+    const bool grow_pos = h->row_pos && newcap > h->map_cap;
+    CK(dev_alloc(&nrows, (size_t)newcap * h->ld * sizeof(float)));
+    CK(dev_alloc(&nids, (size_t)newcap * sizeof(int64_t)));
+    if (h->ivf) CK(dev_alloc(&nas, (size_t)newcap * sizeof(int32_t)));
+    if (grow_pos) CK(dev_alloc(&npos, (size_t)newcap * sizeof(uint32_t)));
     if (h->n > 0) {
-        CK(cudaMemcpyAsync(nrows, h->rows, (size_t)h->n * h->ld * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
-        CK(cudaMemcpyAsync(nids, h->ids, (size_t)h->n * sizeof(int64_t), cudaMemcpyDeviceToDevice, h->stream));
+        if (grow_pos)
+            CK(cudaMemcpyAsync(npos.get(), h->row_pos.get(), (size_t)h->n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpyAsync(nrows.get(), h->rows.get(), (size_t)h->n * h->ld * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpyAsync(nids.get(), h->ids.get(), (size_t)h->n * sizeof(int64_t), cudaMemcpyDeviceToDevice, h->stream));
         if (h->ivf)
-            CK(cudaMemcpyAsync(nas, h->assign, (size_t)h->n * sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));
+            CK(cudaMemcpyAsync(nas.get(), h->assign.get(), (size_t)h->n * sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));
     }
     CK(cudaStreamSynchronize(h->stream));
-    cudaFree(h->rows);
-    cudaFree(h->ids);
-    cudaFree(h->assign);
-    h->rows = nrows;
-    h->ids = nids;
-    h->assign = nas;
+    if (grow_pos) {
+        h->row_pos = std::move(npos);
+        h->map_cap = newcap;
+    }
+    h->rows = std::move(nrows);
+    h->ids = std::move(nids);
+    h->assign = std::move(nas);
     h->cap = newcap;
     return 0;
 }
@@ -477,10 +488,10 @@ static int launch_merge_keys(wb_index* h, int64_t nq, int k, int64_t nparts, con
 // Arrival counters of the fused tail merge: zero between launches (the last CTA of a group resets its own).
 constexpr int64_t kMaxGridY = 32768;
 static int ensure_tail_counters(wb_index* h, cudaStream_t st) {
-    if (h->tailcnt.p) return 0;
+    if (h->tailcnt.get()) return 0;
     // [arrivals | row-group dispensers | coarse-barrier arrivals]
     TRY(h->tailcnt.ensure((size_t)3 * kMaxGridY * sizeof(unsigned int)));
-    CK(cudaMemsetAsync(h->tailcnt.p, 0, (size_t)3 * kMaxGridY * sizeof(unsigned int), st));
+    CK(cudaMemsetAsync(h->tailcnt.get(), 0, (size_t)3 * kMaxGridY * sizeof(unsigned int), st));
     return 0;
 }
 
@@ -553,8 +564,7 @@ static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const fl
         TRY(ensure_tail_counters(h, st));
         set_tail(p, h, c, S_merge, heads_bytes, ids, ex ? ex->D : D, ex ? ex->I : I, k, ex);
     }
-    const int evs = (int)(h->ev_count % wb_index::kEvRing);
-    if (timed && h->timing) CK(cudaEventRecord(h->ev0[evs], st));
+    TRY(timing_begin(h, timed && h->timing, st));
     for (int64_t g0 = 0; g0 < qgroups_total; g0 += kMaxGridY) {
         const int64_t gy = std::min(kMaxGridY, qgroups_total - g0);
         const int64_t qoff = g0 * c.NQ;
@@ -569,10 +579,7 @@ static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const fl
         TRY(launch_scan(c, false, p, dim3((unsigned)S, (unsigned)gy), st));
         h->launches++;
     }
-    if (timed && h->timing) {
-        CK(cudaEventRecord(h->ev1[evs], st));
-        h->ev_count++;
-    }
+    TRY(timing_end(h, timed && h->timing, st));
     if (fuse) {
         if (ex && exchanged) *exchanged = true;
         return 0;
@@ -638,7 +645,7 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
                          const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, bool* overflowed) {
     // Filter-and-refine (main row store only, whose norms are tracked): after the first epoch the GEMM issues only
     // the hi x hi term and the compaction re-scores the few hundred candidates per query exactly in fp32.
-    const bool filter = rows == h->rows && env_int("WB_GEMM_FILTER", 1) != 0;
+    const bool filter = rows == h->rows.get() && env_int("WB_GEMM_FILTER", 1) != 0;
     constexpr bool kFold = kGemmFold<BN, false>;
     using Cfg = GemmCfg<BN, kFold>;
     constexpr int kGemmBN = BN;
@@ -668,7 +675,7 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
         // |exact - hi.hi| <= 2^-9 |x||q| (two truncations to tf32, Cauchy-Schwarz) + fp32 accumulation slack
         // (n-term fp32 accumulation: <= n * 2^-23 * sum |x_i q_i| even if the tensor core truncates)
         const float c_margin = 1.953125e-3f + (float)ld * 1.1920929e-7f * 1.1f + 1e-5f;
-        query_margin_kernel<<<(unsigned)((nq_pad * 32 + 255) / 256), 256, 0, st>>>(q_ld, (int)nq, nq_pad, ld, h->norm2_max,
+        query_margin_kernel<<<(unsigned)((nq_pad * 32 + 255) / 256), 256, 0, st>>>(q_ld, (int)nq, nq_pad, ld, h->norm2_max.get(),
                                                                                  c_margin, margin);
         CK(cudaGetLastError());
         h->launches++;
@@ -767,8 +774,7 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
     // next epoch = growth x (rows seen so far): a query then collects ~k*ln(1+growth) survivors per epoch, far
     // below `cap`; fewer, larger epochs mean fewer launch gaps and compactions (each costs ~50 us)
     const double growth = std::min(12.0, std::max(0.25, (double)cap / (4.0 * k)));
-    const int evs = (int)(h->ev_count % wb_index::kEvRing);
-    if (timed && h->timing) CK(cudaEventRecord(h->ev0[evs], st));
+    TRY(timing_begin(h, timed && h->timing, st));
     int64_t r0 = 0;
     while (r0 < nrows) {
         int64_t len = r0 == 0 ? cap : (int64_t)((double)r0 * growth);
@@ -828,10 +834,7 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
         epoch_no++;
         r0 = r1;
     }
-    if (timed && h->timing) {
-        CK(cudaEventRecord(h->ev1[evs], st));
-        h->ev_count++;
-    }
+    TRY(timing_end(h, timed && h->timing, st));
     int ovf = 0;
     CK(cudaMemcpyAsync(&ovf, overflow, sizeof(int), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
@@ -869,7 +872,7 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
         const int nqb2 = (int)((h->nlist + kF2BN - 1) / kF2BN);
         TRY(h->gimg2.ensure((size_t)nqb2 * 2 * nchunks * kF2BBytes));
         const int64_t n4 = (int64_t)nqb2 * 2 * nchunks * 8 * kF2Half;
-        image_queries_f2_kernel<<<(unsigned)((n4 + 255) / 256), 256, 0, st>>>(h->centroids, (int)h->nlist, ld, nchunks, nqb2,
+        image_queries_f2_kernel<<<(unsigned)((n4 + 255) / 256), 256, 0, st>>>(h->centroids.get(), (int)h->nlist, ld, nchunks, nqb2,
                                                                              h->gimg2.as<float>());
         CK(cudaGetLastError());
         TRY(encode_rows_tmap(x_ld, ld, n, &tmap));
@@ -895,10 +898,10 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
     const int64_t n2 = (int64_t)nqb * nchunks * 8 * BN;
     if (use2) {
         const int64_t n3 = (int64_t)(2 * nqb) * nchunks * 8 * (BN / 2);
-        split_queries_kernel<BN / 2><<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(h->centroids, (int)h->nlist, ld, nchunks,
+        split_queries_kernel<BN / 2><<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(h->centroids.get(), (int)h->nlist, ld, nchunks,
                                                                               2 * nqb, h->gimg.as<float>());
     } else {
-        split_queries_kernel<BN><<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>(h->centroids, (int)h->nlist, ld, nchunks, nqb,
+        split_queries_kernel<BN><<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>(h->centroids.get(), (int)h->nlist, ld, nchunks, nqb,
                                                                               h->gimg.as<float>());
     }
     CK(cudaGetLastError());
@@ -998,75 +1001,58 @@ static int device_csr(wb_index* h, const int32_t* assign, int64_t n, const uint3
 // contiguous span, insertion order kept inside a list), so the list scan is a sequential HBM stream instead of
 // a gather of 2-3 KB rows (measured 3.3-4.3 TB/s gathered).  Needs a second copy of the rows while it runs; if
 // that does not fit, the lists stay a CSR of row indices (slot_row) over the store as it is.
+// A failure leaves the store as it was and the lists dirty (list_off and slot_row describe nothing until then).
 static int ensure_csr(wb_index* h) {
     if (!h->csr_dirty) return 0;
     cudaStream_t st = h->stream;
     const int64_t n = h->n;
-    cudaFree(h->slot_row);
-    h->slot_row = nullptr;
+    h->slot_row.reset();
     if (n == 0) {
-        CK(cudaMemsetAsync(h->list_off, 0, (size_t)(h->nlist + 1) * sizeof(int64_t), st));
+        CK(cudaMemsetAsync(h->list_off.get(), 0, (size_t)(h->nlist + 1) * sizeof(int64_t), st));
         CK(cudaStreamSynchronize(st));
         h->csr_dirty = false;
         return 0;
     }
-    uint32_t* src = nullptr;
-    uint32_t* pos_out = nullptr;
+    DevPtr<uint32_t> src, pos_out;
     const int64_t mcap = std::max<int64_t>(h->cap, n);
-    CK(cudaMalloc(&src, (size_t)n * sizeof(uint32_t)));
-    CK(cudaMalloc(&pos_out, (size_t)mcap * sizeof(uint32_t)));
-    int rc = device_csr(h, h->assign, n, h->row_pos, h->list_off, src, pos_out, st, true);
-    if (rc) {
-        cudaFree(src);
-        cudaFree(pos_out);
-        return rc;
-    }
-    bool grouped = false;
+    CK(dev_alloc(&src, (size_t)n * sizeof(uint32_t)));
+    CK(dev_alloc(&pos_out, (size_t)mcap * sizeof(uint32_t)));
+    TRY(device_csr(h, h->assign.get(), n, h->row_pos.get(), h->list_off.get(), src.get(), pos_out.get(), st, true));
     if (env_int("WB_IVF_CONTIGUOUS", 1)) {
         const int64_t ncap = std::max<int64_t>(h->cap, std::max<int64_t>(n, 1024));
         const size_t need = (size_t)ncap * h->ld * 4 + (size_t)ncap * 4;
         size_t free_b = 0, total_b = 0;
         CK(cudaMemGetInfo(&free_b, &total_b));
         if (free_b > need + ((size_t)1 << 30)) {
-            float* nrows = nullptr;
-            int32_t* nas = nullptr;
-            CK(cudaMalloc(&nrows, (size_t)ncap * h->ld * 4));
-            CK(cudaMalloc(&nas, (size_t)ncap * 4));
+            DevPtr<float> nrows;
+            DevPtr<int32_t> nas;
+            DevPtr<int64_t> nids;  // ids keep their insertion order; they only follow the capacity
+            CK(dev_alloc(&nrows, (size_t)ncap * h->ld * 4));
+            CK(dev_alloc(&nas, (size_t)ncap * 4));
+            if (ncap > h->cap) CK(dev_alloc(&nids, (size_t)ncap * 8));
             const int ld4 = h->ld / 4;
             const int64_t tot = n * ld4;
             permute_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(
-                reinterpret_cast<const float4*>(h->rows), reinterpret_cast<float4*>(nrows), src, n, ld4);
+                reinterpret_cast<const float4*>(h->rows.get()), reinterpret_cast<float4*>(nrows.get()), src.get(), n, ld4);
             CK(cudaGetLastError());
-            permute_i32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->assign, nas, src, n);
+            permute_i32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->assign.get(), nas.get(), src.get(), n);
             CK(cudaGetLastError());
             h->launches += 2;
+            if (nids) CK(cudaMemcpyAsync(nids.get(), h->ids.get(), (size_t)n * 8, cudaMemcpyDeviceToDevice, st));
             CK(cudaStreamSynchronize(st));
-            cudaFree(h->rows);
-            cudaFree(h->assign);
-            h->rows = nrows;
-            h->assign = nas;
-            if (ncap > h->cap) {  // ids keep their insertion order; they only follow the capacity
-                int64_t* nids = nullptr;
-                CK(cudaMalloc(&nids, (size_t)ncap * 8));
-                CK(cudaMemcpy(nids, h->ids, (size_t)n * 8, cudaMemcpyDeviceToDevice));
-                cudaFree(h->ids);
-                h->ids = nids;
-            }
+            h->rows = std::move(nrows);
+            h->assign = std::move(nas);
+            if (nids) h->ids = std::move(nids);
             h->cap = ncap;
-            cudaFree(h->row_pos);
-            h->row_pos = pos_out;  // storage row -> insertion position
+            h->row_pos = std::move(pos_out);  // storage row -> insertion position
             h->map_cap = mcap;
-            pos_out = nullptr;
-            cudaFree(src);
-            src = nullptr;
-            grouped = true;
+            h->csr_dirty = false;
+            return 0;
         }
     }
-    if (!grouped) {  // rows stay put: lists are row indices, row_pos (if any) still describes the storage
-        CK(cudaStreamSynchronize(st));
-        h->slot_row = src;
-        cudaFree(pos_out);
-    }
+    // rows stay put: lists are row indices, row_pos (if any) still describes the storage
+    CK(cudaStreamSynchronize(st));
+    h->slot_row = std::move(src);
     h->csr_dirty = false;
     return 0;
 }
@@ -1079,7 +1065,7 @@ static int assign_rows(wb_index* h, const float* x_dev, int64_t n, int32_t* assi
     TRY(h->pD.ensure((size_t)n * sizeof(float)));
     TRY(h->pI.ensure((size_t)n * sizeof(int64_t)));
     float* D = best_out ? best_out : h->pD.as<float>();
-    TRY(run_flat_any(h, h->centroids, h->nlist, x_dev, n, 1, nullptr, D, h->pI.as<int64_t>(), st, false));
+    TRY(run_flat_any(h, h->centroids.get(), h->nlist, x_dev, n, 1, nullptr, D, h->pI.as<int64_t>(), st, false));
     labels_to_lists_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->pI.as<int64_t>(), assign_out, n);
     CK(cudaGetLastError());
     h->launches++;
@@ -1097,7 +1083,7 @@ static int add_common(wb_index* h, int64_t n, const float* x, const int64_t* ids
     if (h->n + n > h->cap && st != h->stream) CK(cudaStreamSynchronize(st));  // growth copies run on the handle's stream
     TRY(ensure_capacity(h, h->n + n));
     const int64_t n0 = h->n;
-    float* dst = h->rows + (size_t)n0 * h->ld;
+    float* dst = h->rows.get() + (size_t)n0 * h->ld;
     const cudaMemcpyKind kind = host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
     if (h->ld == h->d) {
         CK(cudaMemcpyAsync(dst, x, (size_t)n * h->d * sizeof(float), kind, st));
@@ -1105,7 +1091,7 @@ static int add_common(wb_index* h, int64_t n, const float* x, const int64_t* ids
         const float* src = x;
         if (host) {
             TRY(h->xbuf.ensure((size_t)n * h->d * sizeof(float)));
-            CK(cudaMemcpyAsync(h->xbuf.p, x, (size_t)n * h->d * sizeof(float), kind, st));
+            CK(cudaMemcpyAsync(h->xbuf.get(), x, (size_t)n * h->d * sizeof(float), kind, st));
             src = h->xbuf.as<float>();
         }
         const int64_t tot = n * h->ld;
@@ -1115,27 +1101,27 @@ static int add_common(wb_index* h, int64_t n, const float* x, const int64_t* ids
     }
     {   // running max of |row|^2: the K2 filter epochs derive their safety margin from it
         const unsigned blocks = (unsigned)std::min<int64_t>((n + 7) / 8, (int64_t)h->sm_count * 8);
-        row_norm2_max_kernel<<<blocks, 256, 0, st>>>(dst, n, h->ld, h->norm2_max);
+        row_norm2_max_kernel<<<blocks, 256, 0, st>>>(dst, n, h->ld, h->norm2_max.get());
         CK(cudaGetLastError());
         h->launches++;
     }
     if (ids) {
-        CK(cudaMemcpyAsync(h->ids + n0, ids, (size_t)n * sizeof(int64_t), kind, st));
+        CK(cudaMemcpyAsync(h->ids.get() + n0, ids, (size_t)n * sizeof(int64_t), kind, st));
     } else {
-        iota_ids_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->ids + n0, n0, n);
+        iota_ids_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->ids.get() + n0, n0, n);
         CK(cudaGetLastError());
         h->launches++;
     }
     if (h->row_pos) {  // the store has been grouped before: new rows sit at their insertion position
-        iota_u32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->row_pos, n0, n);
+        iota_u32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->row_pos.get(), n0, n);
         CK(cudaGetLastError());
         h->launches++;
     }
     if (h->ivf) {
         if (preassign) {
-            CK(cudaMemcpyAsync(h->assign + n0, preassign, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(h->assign.get() + n0, preassign, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         } else {
-            TRY(assign_rows(h, dst, n, h->assign + n0, nullptr, st));
+            TRY(assign_rows(h, dst, n, h->assign.get() + n0, nullptr, st));
         }
         h->csr_dirty = true;
     }
@@ -1162,28 +1148,26 @@ extern "C" int wb_pinned_free(void* p) {
     if (p) CK(cudaFreeHost(p));
     return 0;
 }
-extern "C" int wb_add_with_ids_pinned(wb_index* h, int64_t n, const float* x_pinned, const int64_t* ids_pinned, int slot) {
-    if (!h) return fail("NULL index");
+static int add_pinned(wb_index* h, int64_t n, const float* x_pinned, const int64_t* ids_pinned, const int32_t* preassign,
+                      int slot) {
     if (slot < 0 || slot >= wb_index::kAddSlots) return fail("slot %d out of range [0, %d)", slot, wb_index::kAddSlots);
     TRY(set_dev(h));
     if (!h->add_ev[slot]) CK(cudaEventCreateWithFlags(&h->add_ev[slot], cudaEventDisableTiming));
-    TRY(add_common(h, n, x_pinned, ids_pinned, true, nullptr, h->stream, false));
+    TRY(add_common(h, n, x_pinned, ids_pinned, true, preassign, h->stream, false));
     CK(cudaEventRecord(h->add_ev[slot], h->stream));
     h->add_pending[slot] = true;
     return 0;
+}
+extern "C" int wb_add_with_ids_pinned(wb_index* h, int64_t n, const float* x_pinned, const int64_t* ids_pinned, int slot) {
+    if (!h) return fail("NULL index");
+    return add_pinned(h, n, x_pinned, ids_pinned, nullptr, slot);
 }
 // Same for rows whose list is already known (faiss.read_index of an IndexIVFFlat file): no coarse quantisation.
 extern "C" int wb_ivf_add_preassigned_pinned(wb_index* h, int64_t n, const float* x_pinned, const int64_t* ids_pinned,
                                              const int32_t* assign_pinned, int slot) {
     if (!h || !h->ivf) return fail("not an IVF index");
     if (!assign_pinned) return fail("assign is NULL");
-    if (slot < 0 || slot >= wb_index::kAddSlots) return fail("slot %d out of range [0, %d)", slot, wb_index::kAddSlots);
-    TRY(set_dev(h));
-    if (!h->add_ev[slot]) CK(cudaEventCreateWithFlags(&h->add_ev[slot], cudaEventDisableTiming));
-    TRY(add_common(h, n, x_pinned, ids_pinned, true, assign_pinned, h->stream, false));
-    CK(cudaEventRecord(h->add_ev[slot], h->stream));
-    h->add_pending[slot] = true;
-    return 0;
+    return add_pinned(h, n, x_pinned, ids_pinned, assign_pinned, slot);
 }
 extern "C" int wb_add_slot_wait(wb_index* h, int slot) {
     if (!h) return fail("NULL index");
@@ -1252,9 +1236,9 @@ static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, 
     CK(cudaGetLastError());
     lm_item_fill_kernel<<<(unsigned)((nlist + 255) / 256), 256, 0, st>>>(h->lmE.as<int64_t>(), nlist, h->lmF.as<int32_t>());
     CK(cudaGetLastError());
-    CK(cudaMemsetAsync(h->lmG.p, 0, (size_t)nq * 4 + 64, st));
+    CK(cudaMemsetAsync(h->lmG.get(), 0, (size_t)nq * 4 + 64, st));
     LmParams p{};
-    p.rows = h->rows;
+    p.rows = h->rows.get();
     p.ld = h->ld;
     p.queries = q_ld;
     p.nq = (int)nq;
@@ -1263,8 +1247,8 @@ static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, 
     p.stages = c.stages;
     p.nprobe = np;
     p.nlist = nlist;
-    p.list_off = h->list_off;
-    p.row_pos = h->row_pos;
+    p.list_off = h->list_off.get();
+    p.row_pos = h->row_pos.get();
     p.pl_off = h->lmC.as<int64_t>();
     p.pair_src = h->lmB.as<uint32_t>();
     p.item_off = h->lmE.as<int64_t>();
@@ -1272,20 +1256,16 @@ static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, 
     p.gthr = h->lmG.as<uint32_t>();
     p.counter = reinterpret_cast<unsigned int*>(h->lmG.as<unsigned char>() + (size_t)nq * 4 + 16);
     p.parts = h->parts.as<uint64_t>();
-    const int evs = (int)(h->ev_count % wb_index::kEvRing);
-    if (h->timing) CK(cudaEventRecord(h->ev0[evs], st));
+    TRY(timing_begin(h, h->timing, st));
     const int grid = (int)std::min<int64_t>(h->sm_count, max_items);
     switch (c.RW) {
         case 4: TRY(launch_lm_t<4>(p, grid, c.smem, st)); break;
         case 2: TRY(launch_lm_t<2>(p, grid, c.smem, st)); break;
         default: TRY(launch_lm_t<1>(p, grid, c.smem, st)); break;
     }
-    if (h->timing) {
-        CK(cudaEventRecord(h->ev1[evs], st));
-        h->ev_count++;
-    }
+    TRY(timing_end(h, h->timing, st));
     h->launches += 4;
-    TRY(launch_merge_keys(h, nq, k, np, h->parts.as<uint64_t>(), h->ids, D, I, st));
+    TRY(launch_merge_keys(h, nq, k, np, h->parts.as<uint64_t>(), h->ids.get(), D, I, st));
     *done = true;
     return 0;
 }
@@ -1293,8 +1273,7 @@ static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, 
 // The query-major list scan: one launch per <= 32768 queries (the probe table is in h->pI), tail merge fused or not.
 static int run_gather_scan(wb_index* h, const ScanCfg& c, ScanParams& p, int64_t S, bool fuse, int64_t nq, const float* q_ld,
                            int k, int np, float* D, int64_t* I, cudaStream_t st, const ExchParams* ex, bool* exchanged) {
-    const int evs = (int)(h->ev_count % wb_index::kEvRing);
-    if (h->timing) CK(cudaEventRecord(h->ev0[evs], st));
+    TRY(timing_begin(h, h->timing, st));
     for (int64_t q0 = 0; q0 < nq; q0 += kMaxGridY) {
         const int64_t gy = std::min(kMaxGridY, nq - q0);
         p.queries = q_ld + (size_t)q0 * h->ld;
@@ -1308,15 +1287,12 @@ static int run_gather_scan(wb_index* h, const ScanCfg& c, ScanParams& p, int64_t
         TRY(launch_scan(c, true, p, dim3((unsigned)S, (unsigned)gy), st));
         h->launches++;
     }
-    if (h->timing) {
-        CK(cudaEventRecord(h->ev1[evs], st));
-        h->ev_count++;
-    }
+    TRY(timing_end(h, h->timing, st));
     if (fuse) {
         if (ex && exchanged) *exchanged = true;
         return 0;
     }
-    return launch_merge_keys(h, nq, (int)k, S, h->parts.as<uint64_t>(), h->ids, D, I, st);
+    return launch_merge_keys(h, nq, (int)k, S, h->parts.as<uint64_t>(), h->ids.get(), D, I, st);
 }
 
 // ---- search --------------------------------------------------------------------------------
@@ -1325,7 +1301,7 @@ constexpr int64_t kIvfFuseCoarseMaxQ = 4;  // largest IVF batch that runs the co
 static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld] */, int64_t k, int64_t nprobe, float* D,
                            int64_t* I, cudaStream_t st, const ExchParams* ex = nullptr, bool* exchanged = nullptr) {
     if (exchanged) *exchanged = false;
-    if (!h->ivf) return run_flat_any(h, h->rows, h->n, q_ld, nq, (int)k, h->ids, D, I, st, true, ex, exchanged);
+    if (!h->ivf) return run_flat_any(h, h->rows.get(), h->n, q_ld, nq, (int)k, h->ids.get(), D, I, st, true, ex, exchanged);
     if (!h->trained) return fail("IndexIVFFlat is not trained");
     int np = (int)std::min<int64_t>(std::max<int64_t>(nprobe, 1), std::min<int64_t>(h->nlist, WB_MAX_K));
     if (h->csr_dirty) {
@@ -1349,7 +1325,7 @@ static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld
             // K4: coarse quantizer = exhaustive scan of the centroids, top-nprobe
             TRY(h->pD.ensure((size_t)nq * np * sizeof(float)));
             TRY(h->pI.ensure((size_t)nq * np * sizeof(int64_t)));
-            TRY(run_flat_any(h, h->centroids, h->nlist, q_ld, nq, np, nullptr, h->pD.as<float>(), h->pI.as<int64_t>(), st, false));
+            TRY(run_flat_any(h, h->centroids.get(), h->nlist, q_ld, nq, np, nullptr, h->pD.as<float>(), h->pI.as<int64_t>(), st, false));
             // K5, batches: list-major - the probe table is inverted on the device and every probed list is streamed once
             // per group of 8 of the queries that probe it (ivf_lm.cuh)
             bool done = false;
@@ -1358,30 +1334,29 @@ static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld
         }
         TRY(h->parts.ensure((size_t)nq * S * k * sizeof(uint64_t)));
         ScanParams p{};
-        p.rows = h->rows;
+        p.rows = h->rows.get();
         p.nrows = 0;
         p.ld = h->ld;
         p.k = (int)k;
         p.nparts = (int)S;
-        p.perm = h->slot_row;
-        p.row_pos = h->row_pos;
-        p.list_off = h->list_off;
+        p.perm = h->slot_row.get();
+        p.row_pos = h->row_pos.get();
+        p.list_off = h->list_off.get();
         p.nprobe = np;
         if (fuse) {
             TRY(ensure_tail_counters(h, st));
-            set_tail(p, h, c, S_merge, heads_bytes, h->ids, ex ? ex->D : D, ex ? ex->I : I, (int)k, ex);
+            set_tail(p, h, c, S_merge, heads_bytes, h->ids.get(), ex ? ex->D : D, ex ? ex->I : I, (int)k, ex);
         }
         if (fuse_coarse) {
             TRY(h->ckeys.ensure((size_t)nq * h->nlist * sizeof(uint32_t)));
-            p.centroids = h->centroids;
+            p.centroids = h->centroids.get();
             p.nlist = h->nlist;
             p.coarse_keys = h->ckeys.as<uint32_t>();
             p.coarse_count = h->tailcnt.as<unsigned int>() + 2 * kMaxGridY;
             p.queries = q_ld;
             p.nq = (int)nq;
             p.parts = h->parts.as<uint64_t>();
-            const int evs = (int)(h->ev_count % wb_index::kEvRing);
-            if (h->timing) CK(cudaEventRecord(h->ev0[evs], st));
+            TRY(timing_begin(h, h->timing, st));
             const cudaError_t e = launch_scan_coop(c, p, dim3((unsigned)S, (unsigned)nq), st);
             if (e != cudaSuccess) {
                 // (a partitioned device can refuse a full-width cooperative grid: two launches from now on)
@@ -1390,10 +1365,7 @@ static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld
                 fuse_coarse = false;
                 continue;
             }
-            if (h->timing) {
-                CK(cudaEventRecord(h->ev1[evs], st));
-                h->ev_count++;
-            }
+            TRY(timing_end(h, h->timing, st));
             h->launches++;
             h->coarse_fused++;
             if (ex && exchanged) *exchanged = true;
@@ -1424,17 +1396,17 @@ static int stage_queries(wb_index* h, int64_t nq, const float* q, bool host, cud
     if (host && qbytes <= kPinStageMax) {  // pageable -> pinned (host memcpy) -> device (async)
         PinBuf& pb = h->pin_q;
         TRY(pb.ensure(qbytes));
-        memcpy(pb.p, q, qbytes);
-        q = reinterpret_cast<const float*>(pb.p);
+        memcpy(pb.get(), q, qbytes);
+        q = reinterpret_cast<const float*>(pb.get());
     }
     TRY(h->qbuf.ensure((size_t)nq * h->ld * sizeof(float)));
     if (h->ld == h->d) {
-        CK(cudaMemcpyAsync(h->qbuf.p, q, qbytes, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(h->qbuf.get(), q, qbytes, cudaMemcpyHostToDevice, st));
     } else {
         const float* src = q;
         if (host) {
             TRY(h->xbuf.ensure(qbytes));
-            CK(cudaMemcpyAsync(h->xbuf.p, q, qbytes, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(h->xbuf.get(), q, qbytes, cudaMemcpyHostToDevice, st));
             src = h->xbuf.as<float>();
         }
         const int64_t tot = nq * h->ld;
@@ -1455,7 +1427,7 @@ static int fetch_results(wb_index* h, int64_t nq, int64_t k, const float* D_dev,
     PinBuf& pb = h->pin_o;
     if (dbytes + ibytes <= kPinStageMax) {
         TRY(pb.ensure(dbytes + ibytes));
-        unsigned char* stage = reinterpret_cast<unsigned char*>(pb.p);
+        unsigned char* stage = reinterpret_cast<unsigned char*>(pb.get());
         CK(cudaMemcpyAsync(stage, I_dev, ibytes, cudaMemcpyDeviceToHost, st));
         CK(cudaMemcpyAsync(stage + ibytes, D_dev, dbytes, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
@@ -1469,26 +1441,30 @@ static int fetch_results(wb_index* h, int64_t nq, int64_t k, const float* D_dev,
     return 0;
 }
 
+// Runs `search(D, I)`, which enqueues a search on `st`, and delivers its results to the caller's host buffers.
 // Small result sets skip the device buffer and its two D2H copies: the kernel that emits the final (D, I) rows writes
 // them straight into the pinned staging buffer (a few KB of posted PCIe writes), which the host reads after the
-// stream synchronisation.  At one query this takes ~10 us off a 60 us IVF call.
+// stream synchronisation.  At one query this takes ~10 us off a 60 us IVF call.  Larger ones go through
+// (D_dev, I_dev) and fetch_results.
 constexpr size_t kDirectResultMax = (size_t)64 << 10;
-static bool direct_results(wb_index* h, int64_t nq, int64_t k) {
-    return (size_t)nq * k * 12 <= kDirectResultMax && env_int("WB_DIRECT_RESULTS", 1);
-}
-static int direct_result_buffers(wb_index* h, int64_t nq, int64_t k, float** D_pin, int64_t** I_pin) {
+template <class Search>
+static int search_to_host(wb_index* h, int64_t nq, int64_t k, DevBuf& D_dev, DevBuf& I_dev, float* D_host, int64_t* I_host,
+                          cudaStream_t st, const Search& search) {
     const size_t dbytes = (size_t)nq * k * sizeof(float), ibytes = (size_t)nq * k * sizeof(int64_t);
-    TRY(h->pin_o.ensure(dbytes + ibytes));
-    *I_pin = reinterpret_cast<int64_t*>(h->pin_o.p);
-    *D_pin = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(h->pin_o.p) + ibytes);
-    return 0;
-}
-static int finish_direct_results(int64_t nq, int64_t k, const float* D_pin, const int64_t* I_pin, float* D_host,
-                                 int64_t* I_host, cudaStream_t st) {
-    CK(cudaStreamSynchronize(st));
-    memcpy(I_host, I_pin, (size_t)nq * k * sizeof(int64_t));
-    memcpy(D_host, D_pin, (size_t)nq * k * sizeof(float));
-    return 0;
+    if (dbytes + ibytes <= kDirectResultMax && env_int("WB_DIRECT_RESULTS", 1)) {
+        TRY(h->pin_o.ensure(dbytes + ibytes));
+        int64_t* I_pin = h->pin_o.as<int64_t>();
+        float* D_pin = reinterpret_cast<float*>(h->pin_o.as<unsigned char>() + ibytes);
+        TRY(search(D_pin, I_pin));
+        CK(cudaStreamSynchronize(st));
+        memcpy(I_host, I_pin, ibytes);
+        memcpy(D_host, D_pin, dbytes);
+        return 0;
+    }
+    TRY(D_dev.ensure(dbytes));
+    TRY(I_dev.ensure(ibytes));
+    TRY(search(D_dev.as<float>(), I_dev.as<int64_t>()));
+    return fetch_results(h, nq, k, D_dev.as<float>(), I_dev.as<int64_t>(), D_host, I_host, st);
 }
 
 extern "C" int wb_search_dev(wb_index* h, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe, float* D_dev,
@@ -1510,17 +1486,9 @@ extern "C" int wb_search(wb_index* h, int64_t nq, const float* q_host, int64_t k
     cudaStream_t st = h->stream;
     const float* q = nullptr;
     TRY(stage_queries(h, nq, q_host, true, st, &q));
-    if (direct_results(h, nq, k)) {
-        float* Dp = nullptr;
-        int64_t* Ip = nullptr;
-        TRY(direct_result_buffers(h, nq, k, &Dp, &Ip));
-        TRY(search_dev_impl(h, nq, q, k, nprobe, Dp, Ip, st));
-        return finish_direct_results(nq, k, Dp, Ip, D_host, I_host, st);
-    }
-    TRY(h->dbuf.ensure((size_t)nq * k * sizeof(float)));
-    TRY(h->ibuf.ensure((size_t)nq * k * sizeof(int64_t)));
-    TRY(search_dev_impl(h, nq, q, k, nprobe, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st));
-    return fetch_results(h, nq, k, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), D_host, I_host, st);
+    return search_to_host(h, nq, k, h->dbuf, h->ibuf, D_host, I_host, st, [&](float* D, int64_t* I) {
+        return search_dev_impl(h, nq, q, k, nprobe, D, I, st);
+    });
 }
 
 extern "C" int wb_merge_topk_dev(int device, int64_t nq, int64_t k, int64_t nparts, const float* D_parts_dev,
@@ -1559,13 +1527,28 @@ extern "C" int wb_ivf_list_offsets(wb_index* h, int64_t* list_off_host, int* gro
     if (!list_off_host) return fail("NULL buffer");
     TRY(set_dev(h));
     TRY(ensure_csr(h));
-    CK(cudaMemcpyAsync(list_off_host, h->list_off, (size_t)(h->nlist + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(list_off_host, h->list_off.get(), (size_t)(h->nlist + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (grouped_out) *grouped_out = h->slot_row == nullptr;
     return 0;
 }
 
 // ---- row access ----------------------------------------------------------------------------
+// pos[j] = the index of tgt[j] in keys[0, h->n), all ones when it is absent; `kernel` (find_ids_kernel<T>) takes 64
+// targets per launch
+template <class T>
+static int find_positions(wb_index* h, void (*kernel)(const T*, int64_t, const int64_t*, int, unsigned long long*),
+                          const T* keys, const int64_t* tgt, int64_t m, unsigned long long* pos, cudaStream_t st) {
+    CK(cudaMemsetAsync(pos, 0xFF, (size_t)m * sizeof(int64_t), st));
+    for (int64_t j0 = 0; j0 < m; j0 += 64) {
+        const int mm = (int)std::min<int64_t>(64, m - j0);
+        const unsigned grid = (unsigned)std::min<int64_t>(std::max<int64_t>((h->n + 255) / 256, 1), h->sm_count * 8);
+        kernel<<<grid, 256, 0, st>>>(keys, h->n, tgt + j0, mm, pos + j0);
+        CK(cudaGetLastError());
+        h->launches++;
+    }
+    return 0;
+}
 extern "C" int wb_reconstruct_batch(wb_index* h, int64_t m, const int64_t* ids_host, float* out_host) {
     if (!h) return fail("NULL index");
     if (m < 0) return fail("negative m");
@@ -1578,14 +1561,7 @@ extern "C" int wb_reconstruct_batch(wb_index* h, int64_t m, const int64_t* ids_h
     int64_t* tgt = h->idbuf.as<int64_t>();
     unsigned long long* pos = reinterpret_cast<unsigned long long*>(tgt + m);
     CK(cudaMemcpyAsync(tgt, ids_host, (size_t)m * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    CK(cudaMemsetAsync(pos, 0xFF, (size_t)m * sizeof(int64_t), st));
-    for (int64_t j0 = 0; j0 < m; j0 += 64) {
-        const int mm = (int)std::min<int64_t>(64, m - j0);
-        const unsigned grid = (unsigned)std::min<int64_t>(std::max<int64_t>((h->n + 255) / 256, 1), h->sm_count * 8);
-        find_ids_kernel<int64_t><<<grid, 256, 0, st>>>(h->ids, h->n, tgt + j0, mm, pos + j0);
-        CK(cudaGetLastError());
-        h->launches++;
-    }
+    TRY(find_positions(h, find_ids_kernel<int64_t>, h->ids.get(), tgt, m, pos, st));
     std::vector<int64_t> hpos((size_t)m);
     CK(cudaMemcpyAsync(hpos.data(), pos, (size_t)m * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
@@ -1593,21 +1569,14 @@ extern "C" int wb_reconstruct_batch(wb_index* h, int64_t m, const int64_t* ids_h
         if (hpos[j] < 0) return fail("reconstruct: id %lld not found in the index", (long long)ids_host[j]);
     if (h->row_pos) {  // grouped IVF store: insertion position -> storage row
         CK(cudaMemcpyAsync(tgt, pos, (size_t)m * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
-        CK(cudaMemsetAsync(pos, 0xFF, (size_t)m * sizeof(int64_t), st));
-        for (int64_t j0 = 0; j0 < m; j0 += 64) {
-            const int mm = (int)std::min<int64_t>(64, m - j0);
-            const unsigned grid = (unsigned)std::min<int64_t>(std::max<int64_t>((h->n + 255) / 256, 1), h->sm_count * 8);
-            find_ids_kernel<uint32_t><<<grid, 256, 0, st>>>(h->row_pos, h->n, tgt + j0, mm, pos + j0);
-            CK(cudaGetLastError());
-            h->launches++;
-        }
+        TRY(find_positions(h, find_ids_kernel<uint32_t>, h->row_pos.get(), tgt, m, pos, st));
     }
     const int64_t tot = m * h->d;
-    gather_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(h->rows, h->ld, h->d, (const int64_t*)pos, m,
+    gather_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(h->rows.get(), h->ld, h->d, (const int64_t*)pos, m,
                                                                        h->xbuf.as<float>());
     CK(cudaGetLastError());
     h->launches++;
-    CK(cudaMemcpyAsync(out_host, h->xbuf.p, (size_t)tot * sizeof(float), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(out_host, h->xbuf.get(), (size_t)tot * sizeof(float), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return 0;
 }
@@ -1621,22 +1590,22 @@ extern "C" int wb_export_rows(wb_index* h, int64_t start, int64_t n, float* x_ho
     TRY(set_dev(h));
     cudaStream_t st = h->stream;
     if (x_host)
-        CK(cudaMemcpy2DAsync(x_host, (size_t)h->d * 4, h->rows + (size_t)start * h->ld, (size_t)h->ld * 4,
+        CK(cudaMemcpy2DAsync(x_host, (size_t)h->d * 4, h->rows.get() + (size_t)start * h->ld, (size_t)h->ld * 4,
                              (size_t)h->d * 4, (size_t)n, cudaMemcpyDeviceToHost, st));
     if (ids_host) {
         if (h->row_pos) {  // grouped IVF store: the id of storage row r is ids[row_pos[r]]
             TRY(h->idbuf.ensure((size_t)n * 8));
-            gather_ids_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->ids, h->row_pos, start, n, h->idbuf.as<int64_t>());
+            gather_ids_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->ids.get(), h->row_pos.get(), start, n, h->idbuf.as<int64_t>());
             CK(cudaGetLastError());
             h->launches++;
-            CK(cudaMemcpyAsync(ids_host, h->idbuf.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(ids_host, h->idbuf.get(), (size_t)n * 8, cudaMemcpyDeviceToHost, st));
         } else {
-            CK(cudaMemcpyAsync(ids_host, h->ids + start, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(ids_host, h->ids.get() + start, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
         }
     }
     if (assign_host) {
         if (!h->ivf) return fail("assignments exist only for IVF indices");
-        CK(cudaMemcpyAsync(assign_host, h->assign + start, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(assign_host, h->assign.get() + start, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
     }
     CK(cudaStreamSynchronize(st));
     return 0;
@@ -1648,8 +1617,8 @@ extern "C" int wb_ivf_set_centroids(wb_index* h, const float* c) {
     if (!c) return fail("NULL centroids");
     if (h->n > 0) return fail("cannot replace the centroids of a non-empty index");
     TRY(set_dev(h));
-    CK(cudaMemsetAsync(h->centroids, 0, (size_t)h->nlist * h->ld * 4, h->stream));
-    CK(cudaMemcpy2DAsync(h->centroids, (size_t)h->ld * 4, c, (size_t)h->d * 4, (size_t)h->d * 4, (size_t)h->nlist,
+    CK(cudaMemsetAsync(h->centroids.get(), 0, (size_t)h->nlist * h->ld * 4, h->stream));
+    CK(cudaMemcpy2DAsync(h->centroids.get(), (size_t)h->ld * 4, c, (size_t)h->d * 4, (size_t)h->d * 4, (size_t)h->nlist,
                          cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->trained = true;
@@ -1675,7 +1644,7 @@ extern "C" int wb_ivf_get_centroids(const wb_index* h, float* c) {
     if (!h || !h->ivf) return fail("not an IVF index");
     if (!c) return fail("NULL centroids");
     TRY(set_dev(h));
-    CK(cudaMemcpy2DAsync(c, (size_t)h->d * 4, h->centroids, (size_t)h->ld * 4, (size_t)h->d * 4, (size_t)h->nlist,
+    CK(cudaMemcpy2DAsync(c, (size_t)h->d * 4, h->centroids.get(), (size_t)h->ld * 4, (size_t)h->d * 4, (size_t)h->nlist,
                          cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return 0;
@@ -1719,12 +1688,12 @@ static int kmeans_assign_impl(wb_index* h, int64_t n, const float* x_dev, int32_
     TRY(assign_rows(h, x, n, assign_dev, h->dbuf.as<float>(), st, tf32));
     if (objective_host) {
         TRY(h->misc.ensure(sizeof(double)));
-        CK(cudaMemsetAsync(h->misc.p, 0, sizeof(double), st));
+        CK(cudaMemsetAsync(h->misc.get(), 0, sizeof(double), st));
         sum_f32_kernel<<<(unsigned)std::min<int64_t>((n + 255) / 256, 1024), 256, 0, st>>>(h->dbuf.as<float>(), n,
                                                                                           h->misc.as<double>());
         CK(cudaGetLastError());
         h->launches++;
-        CK(cudaMemcpyAsync(objective_host, h->misc.p, sizeof(double), cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(objective_host, h->misc.get(), sizeof(double), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
     }
     return 0;
@@ -1756,7 +1725,7 @@ extern "C" int wb_kmeans_update_dev(wb_index* h, const float* sums_dev, const in
     const int64_t k = h->nlist;
     const int d = h->d, ld = h->ld;
     const int64_t tot = k * d;
-    centroid_mean_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(sums_dev, counts_dev, h->centroids, ld, d, k);
+    centroid_mean_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(sums_dev, counts_dev, h->centroids.get(), ld, d, k);
     CK(cudaGetLastError());
     h->launches++;
     // split_clusters [faiss-upstream]: an empty list takes a perturbed copy of a list picked with probability ~ its
@@ -1793,18 +1762,73 @@ extern "C" int wb_kmeans_update_dev(wb_index* h, const float* sums_dev, const in
             nsplit++;
         }
         TRY(h->misc.ensure(pairs.size() * sizeof(int32_t) + 16));
-        CK(cudaMemcpyAsync(h->misc.p, pairs.data(), pairs.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        split_apply_kernel<<<(unsigned)((d + 255) / 256), 256, 0, st>>>(h->centroids, ld, d, h->misc.as<int32_t>(), (int)nsplit);
+        CK(cudaMemcpyAsync(h->misc.get(), pairs.data(), pairs.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        split_apply_kernel<<<(unsigned)((d + 255) / 256), 256, 0, st>>>(h->centroids.get(), ld, d, h->misc.as<int32_t>(), (int)nsplit);
         CK(cudaGetLastError());
         h->launches++;
         CK(cudaStreamSynchronize(st));  // `pairs` (host) is read by the copy above
     }
     if (h->spherical) {
-        renorm_rows_kernel<<<(unsigned)k, 256, 0, st>>>(h->centroids, ld, d);
+        renorm_rows_kernel<<<(unsigned)k, 256, 0, st>>>(h->centroids.get(), ld, d);
         CK(cudaGetLastError());
         h->launches++;
     }
     if (nsplit_host) *nsplit_host = nsplit;
+    return 0;
+}
+
+// The k-means iterations of wb_ivf_train, on device buffers that the caller owns: x [n, d], assign [n],
+// sums [nlist, d], counts [nlist] and the non-finite flag.
+static int kmeans_train(wb_index* h, int64_t n, const float* x_host, int niter, int64_t seed, float* x, int32_t* assign,
+                        float* sums, int64_t* counts, int* nonfinite) {
+    cudaStream_t st = h->stream;
+    const int64_t k = h->nlist;
+    const int d = h->d;
+    CK(cudaMemcpyAsync(x, x_host, (size_t)n * d * 4, cudaMemcpyHostToDevice, st));
+    // faiss Clustering::train: "input contains NaN's or Inf's" - checked on the device, read at the first sync
+    CK(cudaMemsetAsync(nonfinite, 0, sizeof(int), st));
+    nonfinite_flag_kernel<<<(unsigned)(h->sm_count * 8), 256, 0, st>>>(x, n * (int64_t)d, nonfinite);
+    CK(cudaGetLastError());
+    // initial centroids: first k rows of the faiss-style random permutation, seed + 1
+    std::mt19937 mt((uint32_t)(seed + 1));
+    std::vector<int64_t> perm((size_t)n);
+    for (int64_t i = 0; i < n; ++i) perm[i] = i;
+    for (int64_t i = 0; i + 1 < n; ++i) {
+        const int64_t i2 = i + (int64_t)(mt() % (uint64_t)(n - i));
+        std::swap(perm[i], perm[i2]);
+    }
+    CK(cudaMemsetAsync(h->centroids.get(), 0, (size_t)k * h->ld * 4, st));
+    {   // the k picked rows, gathered by one kernel
+        TRY(h->idbuf.ensure((size_t)k * 8));
+        CK(cudaMemcpyAsync(h->idbuf.get(), perm.data(), (size_t)k * 8, cudaMemcpyHostToDevice, st));
+        if (h->ld == d) {
+            gather_rows_kernel<<<(unsigned)((k * d + 255) / 256), 256, 0, st>>>(x, d, d, h->idbuf.as<int64_t>(), k, h->centroids.get());
+            CK(cudaGetLastError());
+        } else {
+            TRY(h->xbuf.ensure((size_t)k * d * 4));
+            gather_rows_kernel<<<(unsigned)((k * d + 255) / 256), 256, 0, st>>>(x, d, d, h->idbuf.as<int64_t>(), k, h->xbuf.as<float>());
+            CK(cudaGetLastError());
+            pad_rows_kernel<<<(unsigned)((k * h->ld + 255) / 256), 256, 0, st>>>(h->xbuf.as<float>(), h->centroids.get(), k, d, h->ld);
+            CK(cudaGetLastError());
+        }
+        h->launches++;
+        CK(cudaStreamSynchronize(st));  // perm (host) is read by the copy above
+        int bad = 0;
+        CK(cudaMemcpy(&bad, nonfinite, sizeof(int), cudaMemcpyDeviceToHost));
+        if (bad) return fail("input contains NaN's or Inf's");
+    }
+    if (h->spherical) {
+        renorm_rows_kernel<<<(unsigned)k, 256, 0, st>>>(h->centroids.get(), h->ld, d);
+        CK(cudaGetLastError());
+        h->launches++;
+    }
+    for (int it = 0; it < niter; ++it) {
+        double obj = 0;
+        TRY(wb_kmeans_assign_fast_dev(h, n, x, assign, &obj, st));
+        TRY(wb_kmeans_accumulate_dev(h, n, x, assign, sums, counts, st));
+        int64_t nsplit = 0;
+        TRY(wb_kmeans_update_dev(h, sums, counts, n, 1234, &nsplit, st));
+    }
     return 0;
 }
 
@@ -1815,76 +1839,20 @@ extern "C" int wb_ivf_train(wb_index* h, int64_t n, const float* x_host, int nit
                                    (long long)n, (long long)h->nlist);
     if (!x_host) return fail("NULL training set");
     TRY(set_dev(h));
-    cudaStream_t st = h->stream;
     const int64_t k = h->nlist;
     const int d = h->d;
-    float* x = nullptr;
-    CK(cudaMalloc(&x, (size_t)n * d * 4));
-    int rc = 0;
-    int32_t* assign = nullptr;
-    float* sums = nullptr;
-    int64_t* counts = nullptr;
-    int* nonfinite = nullptr;
-    g_err.clear();  // the error path below reports a CUDA error only when no step has already described its failure
-    do {
-        if ((rc = (cudaMemcpyAsync(x, x_host, (size_t)n * d * 4, cudaMemcpyHostToDevice, st) != cudaSuccess))) break;
-        if ((rc = (cudaMalloc(&assign, (size_t)n * 4) != cudaSuccess))) break;
-        if ((rc = (cudaMalloc(&sums, (size_t)k * d * 4) != cudaSuccess))) break;
-        if ((rc = (cudaMalloc(&counts, (size_t)k * 8) != cudaSuccess))) break;
-        // faiss Clustering::train: "input contains NaN's or Inf's" - checked on the device, read at the first sync
-        if ((rc = (cudaMalloc(&nonfinite, sizeof(int)) != cudaSuccess))) break;
-        if ((rc = (cudaMemsetAsync(nonfinite, 0, sizeof(int), st) != cudaSuccess))) break;
-        nonfinite_flag_kernel<<<(unsigned)(h->sm_count * 8), 256, 0, st>>>(x, n * (int64_t)d, nonfinite);
-        // initial centroids: first k rows of the faiss-style random permutation, seed + 1
-        std::mt19937 mt((uint32_t)(seed + 1));
-        std::vector<int64_t> perm((size_t)n);
-        for (int64_t i = 0; i < n; ++i) perm[i] = i;
-        for (int64_t i = 0; i + 1 < n; ++i) {
-            const int64_t i2 = i + (int64_t)(mt() % (uint64_t)(n - i));
-            std::swap(perm[i], perm[i2]);
-        }
-        if ((rc = (cudaMemsetAsync(h->centroids, 0, (size_t)k * h->ld * 4, st) != cudaSuccess))) break;
-        {   // the k picked rows, gathered by one kernel
-            if ((rc = h->idbuf.ensure((size_t)k * 8))) break;
-            if ((rc = (cudaMemcpyAsync(h->idbuf.p, perm.data(), (size_t)k * 8, cudaMemcpyHostToDevice, st) != cudaSuccess))) break;
-            if (h->ld == d) {
-                gather_rows_kernel<<<(unsigned)((k * d + 255) / 256), 256, 0, st>>>(x, d, d, h->idbuf.as<int64_t>(), k, h->centroids);
-            } else {
-                if ((rc = h->xbuf.ensure((size_t)k * d * 4))) break;
-                gather_rows_kernel<<<(unsigned)((k * d + 255) / 256), 256, 0, st>>>(x, d, d, h->idbuf.as<int64_t>(), k, h->xbuf.as<float>());
-                pad_rows_kernel<<<(unsigned)((k * h->ld + 255) / 256), 256, 0, st>>>(h->xbuf.as<float>(), h->centroids, k, d, h->ld);
-            }
-            h->launches++;
-            if ((rc = (cudaStreamSynchronize(st) != cudaSuccess))) break;  // perm (host) is read by the copy above
-            int bad = 0;
-            if ((rc = (cudaMemcpy(&bad, nonfinite, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess))) break;
-            if (bad) {
-                rc = fail("input contains NaN's or Inf's");
-                break;
-            }
-        }
-        if (h->spherical) {
-            renorm_rows_kernel<<<(unsigned)k, 256, 0, st>>>(h->centroids, h->ld, d);
-            h->launches++;
-        }
-        for (int it = 0; it < niter && !rc; ++it) {
-            double obj = 0;
-            if ((rc = wb_kmeans_assign_fast_dev(h, n, x, assign, &obj, st))) break;
-            if ((rc = wb_kmeans_accumulate_dev(h, n, x, assign, sums, counts, st))) break;
-            int64_t nsplit = 0;
-            if ((rc = wb_kmeans_update_dev(h, sums, counts, n, 1234, &nsplit, st))) break;
-        }
-    } while (0);
-    cudaError_t e = cudaStreamSynchronize(st);
-    cudaFree(x);
-    cudaFree(assign);
-    cudaFree(sums);
-    cudaFree(counts);
-    cudaFree(nonfinite);
-    if (rc) {
-        if (g_err.empty()) fail("k-means training failed: %s", cudaGetErrorString(cudaGetLastError()));
-        return 1;
-    }
+    DevPtr<float> x, sums;
+    DevPtr<int32_t> assign;
+    DevPtr<int64_t> counts;
+    DevPtr<int> nonfinite;
+    CK(dev_alloc(&x, (size_t)n * d * 4));
+    CK(dev_alloc(&assign, (size_t)n * 4));
+    CK(dev_alloc(&sums, (size_t)k * d * 4));
+    CK(dev_alloc(&counts, (size_t)k * 8));
+    CK(dev_alloc(&nonfinite, sizeof(int)));
+    const int rc = kmeans_train(h, n, x_host, niter, seed, x.get(), assign.get(), sums.get(), counts.get(), nonfinite.get());
+    const cudaError_t e = cudaStreamSynchronize(h->stream);  // the buffers are freed on return
+    if (rc) return rc;
     if (e != cudaSuccess) return fail("k-means training failed: %s", cudaGetErrorString(e));
     h->trained = true;
     return 0;
@@ -1907,9 +1875,11 @@ extern "C" int wb_tf32_peak(int device, int iters, int reps, double* tflops_burs
     const int constant_ops = env_int("WB_PEAK_CONSTANT", 0);  // 1: all-ones operands (no bit toggling: less power, higher clock)
     const size_t smem = (size_t)kF2StageBytes + 1024;
     CK(cudaFuncSetAttribute(tf32_peak_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaEvent_t e0, e1;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
     CK(cudaEventCreate(&e0));
+    const EventPtr own_e0(e0);
     CK(cudaEventCreate(&e1));
+    const EventPtr own_e1(e1);
     const double flop = (double)npairs * iters * 4.0 * 2.0 * 256.0 * 256.0 * 8.0;
     float best = 1e30f;
     for (int r = 0; r < 4; ++r) {  // burst: best single launch (the first one is the warm-up)
@@ -1935,8 +1905,6 @@ extern "C" int wb_tf32_peak(int device, int iters, int reps, double* tflops_burs
         CK(cudaEventElapsedTime(&ms, e0, e1));
         *tflops_sustained_out = flop * half / (ms * 1e-3) / 1e12;
     }
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
     return 0;
 }
 
@@ -1944,11 +1912,11 @@ extern "C" int wb_tf32_peak(int device, int iters, int reps, double* tflops_burs
 struct wb_exchange {
     int device = 0, rank = 0, world = 1;
     size_t region_bytes = 0, flags_bytes = 0, cap_entries = 0, nq_cap = 0, total_bytes = 0;
-    unsigned char* local = nullptr;
+    DevPtr<unsigned char> local;
     unsigned char* peers[kExchMaxWorld] = {};
     bool opened[kExchMaxWorld] = {};
     uint32_t seq = 0;       // sequence number of the last exchange that was LAUNCHED (all ranks advance in lockstep)
-    int* status = nullptr;  // pinned (device-visible) host word raised by a kernel whose wait for the peers timed out
+    PinPtr<int> status;     // pinned (device-visible) host word raised by a kernel whose wait for the peers timed out
     int64_t launches = 0;   // exchange_merge_kernel launches (the fused path needs none)
 };
 
@@ -1959,7 +1927,7 @@ extern "C" int wb_exch_create(int device, int rank, int world, int64_t max_queri
     if (world < 1 || world > kExchMaxWorld || rank < 0 || rank >= world) return fail("bad rank/world %d/%d", rank, world);
     if (max_queries < 1 || max_entries < max_queries) return fail("bad exchange capacity");
     CK(cudaSetDevice(device));
-    wb_exchange* ex = new wb_exchange();
+    std::unique_ptr<wb_exchange> ex(new wb_exchange());
     ex->device = device;
     ex->rank = rank;
     ex->world = world;
@@ -1968,13 +1936,15 @@ extern "C" int wb_exch_create(int device, int rank, int world, int64_t max_queri
     ex->flags_bytes = ((size_t)max_queries * 4 + 255) & ~(size_t)255;
     ex->region_bytes = (ex->flags_bytes + ex->cap_entries * 12 + 255) & ~(size_t)255;
     ex->total_bytes = ex->region_bytes * 2 * world;
-    CK(cudaMalloc(&ex->local, ex->total_bytes));
-    CK(cudaMemset(ex->local, 0, ex->total_bytes));
-    CK(cudaHostAlloc(&ex->status, sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
-    *ex->status = 0;
+    CK(dev_alloc(&ex->local, ex->total_bytes));
+    CK(cudaMemset(ex->local.get(), 0, ex->total_bytes));
+    int* status = nullptr;
+    CK(cudaHostAlloc(&status, sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
+    ex->status.reset(status);
+    *status = 0;
     CK(cudaDeviceSynchronize());
-    ex->peers[rank] = ex->local;
-    *out = ex;
+    ex->peers[rank] = ex->local.get();
+    *out = ex.release();
     return 0;
 }
 
@@ -1983,7 +1953,7 @@ extern "C" int wb_exch_local_handle(wb_exchange* ex, void* handle64) {
     CK(cudaSetDevice(ex->device));
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
     cudaIpcMemHandle_t hnd;
-    CK(cudaIpcGetMemHandle(&hnd, ex->local));
+    CK(cudaIpcGetMemHandle(&hnd, ex->local.get()));
     memcpy(handle64, &hnd, 64);
     return 0;
 }
@@ -2009,8 +1979,6 @@ extern "C" int wb_exch_free(wb_exchange* ex) {
     cudaDeviceSynchronize();
     for (int r = 0; r < ex->world; ++r)
         if (ex->opened[r]) cudaIpcCloseMemHandle(ex->peers[r]);
-    cudaFree(ex->local);
-    cudaFreeHost(ex->status);
     delete ex;
     return 0;
 }
@@ -2039,7 +2007,7 @@ static int exch_prepare(wb_exchange* ex, int64_t nq, int64_t k, float* D_dev, in
     p.cap_entries = ex->cap_entries;
     p.D = D_dev;
     p.I = I_dev;
-    p.status = ex->status;
+    p.status = ex->status.get();
     *out = p;
     return 0;
 }
@@ -2078,7 +2046,7 @@ extern "C" int64_t wb_exch_launch_count(const wb_exchange* ex) { return ex ? ex-
 
 extern "C" int wb_exch_status(wb_exchange* ex, int* timed_out) {
     if (!ex || !timed_out) return fail("NULL argument");
-    *timed_out = *reinterpret_cast<volatile int*>(ex->status);
+    *timed_out = *reinterpret_cast<volatile int*>(ex->status.get());
     return 0;
 }
 
@@ -2200,18 +2168,10 @@ extern "C" int wb_exch_search(wb_index* h, wb_exchange* ex, int64_t nq, const fl
     cudaStream_t st = h->stream;
     const float* q = nullptr;
     TRY(stage_queries(h, nq, q_host, true, st, &q));
-    if (direct_results(h, nq, k)) {
-        float* Dp = nullptr;
-        int64_t* Ip = nullptr;
-        TRY(direct_result_buffers(h, nq, k, &Dp, &Ip));
-        TRY(exch_search_dev_impl(h, ex, nq, q, k, nprobe, Dp, Ip, st));
-        TRY(finish_direct_results(nq, k, Dp, Ip, D_host, I_host, st));
-    } else {
-        TRY(h->eD.ensure((size_t)nq * k * sizeof(float)));
-        TRY(h->eI.ensure((size_t)nq * k * sizeof(int64_t)));
-        TRY(exch_search_dev_impl(h, ex, nq, q, k, nprobe, h->eD.as<float>(), h->eI.as<int64_t>(), st));
-        TRY(fetch_results(h, nq, k, h->eD.as<float>(), h->eI.as<int64_t>(), D_host, I_host, st));
-    }
-    if (*reinterpret_cast<volatile int*>(ex->status)) return fail("sharded search: a peer GPU did not join the exchange within 20 s (results invalid)");
+    // (eD, eI): exch_search_dev_impl keeps this rank's local results in (dbuf, ibuf)
+    TRY(search_to_host(h, nq, k, h->eD, h->eI, D_host, I_host, st, [&](float* D, int64_t* I) {
+        return exch_search_dev_impl(h, ex, nq, q, k, nprobe, D, I, st);
+    }));
+    if (*reinterpret_cast<volatile int*>(ex->status.get())) return fail("sharded search: a peer GPU did not join the exchange within 20 s (results invalid)");
     return 0;
 }
