@@ -114,6 +114,33 @@ int wb_search(wb_index* h, int64_t nq, const float* q_host, int64_t k, int64_t n
               float* D_host, int64_t* I_host);
 int wb_search_dev(wb_index* h, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
                   float* D_dev, int64_t* I_dev, void* stream);
+/* ---- filtered search ---------------------------------------------------------------------------
+ * index.search(x, k, params=faiss.SearchParameters(sel=...)) / SearchParametersIVF(sel=..., nprobe=...) [faiss-upstream]:
+ * the exact top-k over the rows a selector keeps.  A selector tests the EXTERNAL id of a row (the id given to
+ * add_with_ids; the insertion position for rows added without ids).  Order, tie rule and padding are those of
+ * wb_search; the IVF coarse quantizer is not filtered (candidates = the selected rows of the nprobe probed lists).
+ *
+ * A wb_filter is bound to the index it was created for (using it with another index is an error) and must be freed
+ * before that index.  It keeps its definition, a device bitmap with one bit per insertion position, and the number of
+ * rows it selects.  Creation evaluates it on the device and synchronises once to read that number; a search with it
+ * needs no further synchronisation, except after the index has grown: the next search re-evaluates the bitmap, and a
+ * _dev search then synchronises the caller's stream first (as an add that grows the store does).  The first flat
+ * search with a very selective filter (below 1/kSparseCutoffDen of the rows, DESIGN.md "Filtered search") also
+ * gathers the selected rows into a compact copy that the filter keeps and later searches reuse.
+ * f == NULL in the search calls means unfiltered. */
+typedef struct wb_filter wb_filter;
+/* IDSelectorBatch(ids) (invert = 0) or IDSelectorNot(IDSelectorBatch(ids)) (invert = 1): ids in any order,
+ * duplicates allowed, n may be 0. */
+int wb_filter_create_ids(wb_index* h, int64_t n, const int64_t* ids_host, int invert, wb_filter** out);
+/* IDSelectorRange(imin, imax): imin <= id < imax (empty when imin >= imax); invert = 1 for IDSelectorNot of it. */
+int wb_filter_create_range(wb_index* h, int64_t imin, int64_t imax, int invert, wb_filter** out);
+int64_t wb_filter_count(const wb_filter* f); /* rows selected when the filter was last evaluated */
+int wb_filter_free(wb_filter* f);            /* before the index it belongs to */
+int wb_search_filtered(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
+                       float* D_host, int64_t* I_host);
+int wb_search_filtered_dev(wb_index* h, wb_filter* f, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
+                           float* D_dev, int64_t* I_dev, void* stream);
+
 /* Merge `nparts` sorted partial results (layout [part][nq][k], e.g. the all-gathered per-GPU
  * top-k) into the global top-k.  Order: score desc, then part asc, then rank-in-part asc - with
  * contiguous row sharding that is exactly "lowest insertion position". */
@@ -139,6 +166,12 @@ int wb_exch_search(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_host
                    float* D_host, int64_t* I_host);
 int wb_exch_search_dev(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
                        float* D_dev, int64_t* I_dev, void* stream);
+/* Filtered sharded search: every rank passes a filter built from the same selector over its own rows.  A rank whose
+ * filter selects nothing still takes part in the exchange. */
+int wb_exch_search_filtered(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_host, int64_t k,
+                            int64_t nprobe, float* D_host, int64_t* I_host);
+int wb_exch_search_filtered_dev(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_dev, int64_t k,
+                                int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream);
 /* *timed_out = 1 when a kernel of this exchange gave up waiting for a peer (20 s): that search's results are invalid.
  * wb_exch_search checks it itself; callers of the _dev entry points check it after synchronising their stream. */
 int wb_exch_status(wb_exchange* ex, int* timed_out);

@@ -51,7 +51,15 @@ SIGNATURES = {
     "wb_kmeans_update_dev": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int64, C.POINTER(C.c_int64), _vp]),
     "wb_search": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp]),
     "wb_search_dev": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp]),
-    "wb_merge_topk_dev": (C.c_int, [C.c_int, C.c_int64, C.c_int64, C.c_int64, _vp, _vp, _vp, _vp, _vp]),
+    "wb_filter_create_ids": (C.c_int, [_vp, C.c_int64, _vp, C.c_int, C.POINTER(_vp)]),
+    "wb_filter_create_range": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int, C.POINTER(_vp)]),
+    "wb_filter_count": (C.c_int64, [_vp]),
+    "wb_filter_free": (C.c_int, [_vp]),
+    "wb_search_filtered": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp]),
+    "wb_search_filtered_dev": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp]),
+    "wb_exch_search_filtered": (C.c_int, [_vp, _vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp]),
+    "wb_exch_search_filtered_dev": (C.c_int, [_vp, _vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp]),
+    "wb_merge_topk_dev":(C.c_int, [C.c_int, C.c_int64, C.c_int64, C.c_int64, _vp, _vp, _vp, _vp, _vp]),
     "wb_exch_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int64, C.POINTER(_vp)]),
     "wb_exch_local_handle": (C.c_int, [_vp, _vp]),
     "wb_exch_open_peers": (C.c_int, [_vp, _vp]),

@@ -535,12 +535,19 @@ static void set_tail(ScanParams& p, wb_index* h, const ScanCfg& c, int S_merge, 
     }
 }
 
+// The rows a filtered search may return (dense filter path, DESIGN.md "Filtered search"): bit p of allow[p / 32] is
+// set for a selected insertion position p, and sel[t] counts the selected positions in [0, t * kGemmBM) (host).
+struct RowMask {
+    const uint32_t* allow;
+    const int64_t* sel;
+};
+
 // Exhaustive top-k of `nq` device queries (row stride ld) against `nrows` rows: K1 with the K3 merge (and, when `ex`
 // is given, the multi-GPU exchange) fused into its tail; K1 + K3 as two launches when the tail cannot be fused.
 // *exchanged tells the caller whether (D, I) already hold the GLOBAL result (written to ex->D / ex->I).
 static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const float* q_dev, int64_t nq, int k,
                          const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed,
-                         const ExchParams* ex = nullptr, bool* exchanged = nullptr) {
+                         const ExchParams* ex = nullptr, bool* exchanged = nullptr, const RowMask* mask = nullptr) {
     if (exchanged) *exchanged = false;
     ScanCfg c;
     TRY(plan_scan(h, nq, k, false, 0, &c));
@@ -558,6 +565,7 @@ static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const fl
     p.ld = h->ld;
     p.k = k;
     p.nparts = (int)S;
+    p.allow = mask ? mask->allow : nullptr;
     int S_merge = 0, heads_bytes = 0;
     const bool fuse = tail_fusable(c, k, S, ex ? ex->world : 1, &S_merge, &heads_bytes);
     if (fuse) {
@@ -642,10 +650,12 @@ static bool gemm_eligible(const wb_index* h, int64_t nrows, int64_t nq, int k, i
 
 template <int BN>
 static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const float* q_ld, int64_t nq, int k, int cap,
-                         const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, bool* overflowed) {
-    // Filter-and-refine (main row store only, whose norms are tracked): after the first epoch the GEMM issues only
-    // the hi x hi term and the compaction re-scores the few hundred candidates per query exactly in fp32.
-    const bool filter = rows == h->rows.get() && env_int("WB_GEMM_FILTER", 1) != 0;
+                         const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, bool* overflowed,
+                         const RowMask* mask) {
+    // Filter-and-refine (rows of the store, or the compact copy of a filter's rows: norm2_max bounds both; not the
+    // centroid table): after the first epoch the GEMM issues only the hi x hi term and the compaction re-scores the few
+    // hundred candidates per query exactly in fp32.
+    const bool filter = rows != h->centroids.get() && env_int("WB_GEMM_FILTER", 1) != 0;
     constexpr bool kFold = kGemmFold<BN, false>;
     using Cfg = GemmCfg<BN, kFold>;
     constexpr int kGemmBN = BN;
@@ -755,6 +765,7 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
     g.k = k;
     g.cap = cap;
     g.kstride = kstride;
+    g.allow = mask ? mask->allow : nullptr;
     CompactParams c{};
     c.k = k;
     c.cap = cap;
@@ -777,9 +788,24 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
     TRY(timing_begin(h, timed && h->timing, st));
     int64_t r0 = 0;
     while (r0 < nrows) {
-        int64_t len = r0 == 0 ? cap : (int64_t)((double)r0 * growth);
-        len = std::max<int64_t>(kGemmBM, (len + kGemmBM - 1) / kGemmBM * kGemmBM);
-        const int64_t r1 = std::min(nrows, r0 + len);
+        int64_t r1;
+        if (mask) {
+            // the same schedule in SELECTED rows: epoch 0 ends before its selected rows (every one of them a candidate)
+            // exceed `cap`, later epochs take growth x the selected rows seen so far.  Counting all rows instead, a
+            // filter that keeps 13 % of the rows leaves fewer than k = 1000 of them in a 4096-row epoch 0, the
+            // threshold stays -inf and the next epoch's candidates overflow `cap`.  (A filter that keeps every row
+            // gets exactly the unfiltered epochs.)
+            const int64_t t0 = r0 / kGemmBM, nt = (nrows + kGemmBM - 1) / kGemmBM;
+            const int64_t seen = mask->sel[t0];
+            const int64_t grow = (int64_t)((double)seen * growth);
+            const int64_t want = seen + (r0 == 0 ? cap : (grow + kGemmBM - 1) / kGemmBM * kGemmBM);
+            const int64_t t1 = std::upper_bound(mask->sel + t0 + 1, mask->sel + nt + 1, want) - mask->sel - 1;
+            r1 = std::min(nrows, std::max(t1, t0 + 1) * kGemmBM);
+        } else {
+            int64_t len = r0 == 0 ? cap : (int64_t)((double)r0 * growth);
+            len = std::max<int64_t>(kGemmBM, (len + kGemmBM - 1) / kGemmBM * kGemmBM);
+            r1 = std::min(nrows, r0 + len);
+        }
         g.row_begin = r0;
         g.row_end = r1;
         const int64_t nwork = ((r1 - r0 + kGemmBM - 1) / kGemmBM) * nqb;
@@ -843,13 +869,14 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
 }
 
 static int run_flat_gemm(wb_index* h, const float* rows, int64_t nrows, const float* q_ld, int64_t nq, int k, int cap,
-                         const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, bool* overflowed) {
+                         const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, bool* overflowed,
+                         const RowMask* mask) {
     // 16-query blocks halve the image traffic and the MMA work of a half-empty 32-query block (K2 is power-capped at
     // small batches: 992 W and 1.37 GHz at batch 16)
-    if (nq <= 16) return run_flat_gemm_t<16>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
-    if (nq <= 32) return run_flat_gemm_t<32>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
-    if (nq <= 64) return run_flat_gemm_t<64>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
-    return run_flat_gemm_t<128>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed);
+    if (nq <= 16) return run_flat_gemm_t<16>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask);
+    if (nq <= 32) return run_flat_gemm_t<32>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask);
+    if (nq <= 64) return run_flat_gemm_t<64>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask);
+    return run_flat_gemm_t<128>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask);
 }
 
 // K4/K6 on the tensor cores: argmax over the centroid table for n device-resident points (row stride ld).
@@ -936,7 +963,7 @@ static int run_assign_gemm(wb_index* h, const float* x_ld, int64_t n, int32_t* a
 // is repaired by re-running the batch through K1.
 static int run_flat_any(wb_index* h, const float* rows, int64_t nrows, const float* q_dev, int64_t nq, int k,
                         const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed,
-                        const ExchParams* ex = nullptr, bool* exchanged = nullptr) {
+                        const ExchParams* ex = nullptr, bool* exchanged = nullptr, const RowMask* mask = nullptr) {
     if (exchanged) *exchanged = false;
     int cap = 0;
     if (gemm_eligible(h, nrows, nq, k, &cap)) {
@@ -946,14 +973,14 @@ static int run_flat_any(wb_index* h, const float* rows, int64_t nrows, const flo
             const int64_t nqc = std::min(max_q, nq - q0);
             bool ovf = false;
             TRY(run_flat_gemm(h, rows, nrows, q_dev + (size_t)q0 * h->ld, nqc, k, cap, ids, D + (size_t)q0 * k,
-                              I + (size_t)q0 * k, st, timed, &ovf));
+                              I + (size_t)q0 * k, st, timed, &ovf, mask));
             any_overflow |= ovf;
         }
         if (!any_overflow) return 0;
         h->gemm_fallbacks++;
     }
     return run_flat_scan(h, rows, nrows, q_dev, nq, k, ids, D, I, st, timed,
-                         ex && nq <= kMaxGridY ? ex : nullptr, exchanged);
+                         ex && nq <= kMaxGridY ? ex : nullptr, exchanged, mask);
 }
 
 // ---- K8: CSR inverted lists, built on the device (csr.cuh) -------------------------------------------------------
@@ -1207,7 +1234,7 @@ static int launch_lm_t(const LmParams& p, int grid, size_t smem, cudaStream_t st
 // Taken when the probes of the batch overlap enough for shared reads to pay (on average every list is probed at
 // least once) and the rows are physically grouped by list.  WB_IVF_LISTMAJOR=0 / 1 forces it off / on.
 static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, int np, float* D, int64_t* I,
-                             cudaStream_t st, bool* done) {
+                             cudaStream_t st, const uint32_t* allow, bool* done) {
     *done = false;
     const int mode = env_int("WB_IVF_LISTMAJOR", -1);
     if (mode == 0 || h->slot_row != nullptr || h->n == 0) return 0;
@@ -1249,6 +1276,7 @@ static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, 
     p.nlist = nlist;
     p.list_off = h->list_off.get();
     p.row_pos = h->row_pos.get();
+    p.allow = allow;
     p.pl_off = h->lmC.as<int64_t>();
     p.pair_src = h->lmB.as<uint32_t>();
     p.item_off = h->lmE.as<int64_t>();
@@ -1295,14 +1323,143 @@ static int run_gather_scan(wb_index* h, const ScanCfg& c, ScanParams& p, int64_t
     return launch_merge_keys(h, nq, (int)k, S, h->parts.as<uint64_t>(), h->ids.get(), D, I, st);
 }
 
+// ---- filters (faiss SearchParameters.sel): a bitmap over insertion positions, DESIGN.md "Filtered search" ---------
+struct wb_filter {
+    wb_index* h = nullptr;          // the index whose rows the filter selects
+    DevPtr<int64_t> set;            // the sorted, unique ids of an id set; null: the range [imin, imax)
+    int64_t nset = 0, imin = 0, imax = 0;
+    bool invert = false;            // IDSelectorNot
+    DevPtr<uint32_t> bits;          // one bit per insertion position
+    DevPtr<uint32_t> tile_cnt;      // selected positions per kFilterTile positions (evaluation output)
+    int64_t words_cap = 0;          // capacity of `bits`, in 32-bit words (tile_cnt holds words_cap / 4)
+    std::vector<int64_t> sel;       // [tiles + 1] selected positions before each tile (host)
+    int64_t count = 0;              // selected rows
+    int64_t built_n = -1;           // ntotal the bitmap describes; a search after an add re-evaluates it
+    DevPtr<float> crows;            // flat sparse path: the selected rows [count, ld] in insertion order ...
+    DevPtr<int64_t> cids;           // ... and their ids
+    int64_t compact_n = -1;         // built_n the compact copy was made at (-1: none)
+};
+static_assert(kFilterTile == kGemmBM, "the K2 epoch schedule reads the per-tile counts of the filter evaluation");
+
+// Below this selected fraction a flat search scans a compact copy of the selected rows instead of masking the full
+// store.  Measured on a B200 (1000 W, 1965 MHz max SM clock; profiles/filtered/bench_filtered.jsonl, 10M x 768, k 100):
+// the mask path costs the unfiltered time (batch 1: 4.05 ms at 1, 1/2 and 1/8 selected vs 4.05 unfiltered); the
+// compact path costs about the selected fraction of it (1/64: 0.087 ms at batch 1, 0.40 ms at 16, 2.2 ms at 1024 vs
+// 4.05 / 4.34 / 24.6 ms) plus a one-time gather (2.3-2.5 ms at batch 1 for 1/64).  Per search the copy wins at every
+// measured fraction; the cutoff bounds the extra memory the copy takes to 1/8 of the store.
+constexpr int64_t kSparseCutoffDen = 8;
+
+// Evaluate the selector over the index's current rows (on the handle's stream, one synchronisation to read the
+// per-tile counts the host needs for dispatch).
+static int filter_eval(wb_filter* f) {
+    wb_index* h = f->h;
+    cudaStream_t st = h->stream;
+    const int64_t n = h->n, ntiles = (n + kFilterTile - 1) / kFilterTile;
+    const int64_t words = ntiles * (kFilterTile / 32);
+    if (words > f->words_cap) {
+        const int64_t cap = std::max<int64_t>(words, (std::max<int64_t>(h->cap, n) + kFilterTile - 1) / kFilterTile *
+                                                         (kFilterTile / 32));
+        DevPtr<uint32_t> bits, cnt;
+        CK(dev_alloc(&bits, (size_t)cap * 4));
+        CK(dev_alloc(&cnt, (size_t)cap / (kFilterTile / 32) * 4));
+        f->bits = std::move(bits);
+        f->tile_cnt = std::move(cnt);
+        f->words_cap = cap;
+    }
+    std::vector<uint32_t> cnt((size_t)ntiles);
+    if (n > 0) {
+        filter_eval_kernel<<<(unsigned)ntiles, kFilterTile, 0, st>>>(h->ids.get(), n, f->set.get(), f->nset, f->imin,
+                                                                    f->imax, f->invert, f->bits.get(), f->tile_cnt.get());
+        CK(cudaGetLastError());
+        h->launches++;
+        CK(cudaMemcpyAsync(cnt.data(), f->tile_cnt.get(), (size_t)ntiles * 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+    }
+    f->sel.assign((size_t)ntiles + 1, 0);
+    for (int64_t t = 0; t < ntiles; ++t) f->sel[t + 1] = f->sel[t] + cnt[t];
+    f->count = f->sel[ntiles];
+    f->built_n = n;
+    f->crows.reset();
+    f->cids.reset();
+    f->compact_n = -1;
+    return 0;
+}
+
+// Bring the bitmap up to date with rows added since it was evaluated.  An add on `st` may still be writing the ids:
+// `st` is synchronised first (this is the one synchronisation a _dev search with a stale filter makes).
+static int filter_current(wb_filter* f, cudaStream_t st) {
+    if (f->built_n == f->h->n) return 0;
+    if (st != f->h->stream) CK(cudaStreamSynchronize(st));
+    return filter_eval(f);
+}
+
+// Flat sparse path: the selected rows gathered, in insertion order, into [count, ld] with their ids, so that index
+// order in the copy is insertion order and ties resolve as in the full store.  Built once per evaluation (repeated
+// searches with one filter pay for it once).  *ok = false when it does not fit in memory: the caller masks instead.
+static int filter_compact(wb_filter* f, bool* ok) {
+    *ok = true;
+    if (f->compact_n == f->built_n) return 0;
+    wb_index* h = f->h;
+    cudaStream_t st = h->stream;
+    const int64_t m = f->count, ntiles = (int64_t)f->sel.size() - 1;
+    DevPtr<float> rows;
+    DevPtr<int64_t> ids, pos, off;
+    if (dev_alloc(&rows, (size_t)m * h->ld * 4) != cudaSuccess || dev_alloc(&ids, (size_t)m * 8) != cudaSuccess ||
+        dev_alloc(&pos, (size_t)m * 8) != cudaSuccess || dev_alloc(&off, (size_t)(ntiles + 1) * 8) != cudaSuccess) {
+        cudaGetLastError();  // (clear the allocation error: the next launch check would report it)
+        *ok = false;
+        return 0;
+    }
+    CK(cudaMemcpyAsync(off.get(), f->sel.data(), (size_t)(ntiles + 1) * 8, cudaMemcpyHostToDevice, st));
+    filter_positions_kernel<<<(unsigned)ntiles, kFilterTile, 0, st>>>(f->bits.get(), h->n, off.get(), h->ids.get(),
+                                                                     pos.get(), ids.get());
+    CK(cudaGetLastError());
+    const int64_t tot = m * h->ld;  // whole rows, padding columns included: the copy has the store's stride
+    gather_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(h->rows.get(), h->ld, h->ld, pos.get(), m, rows.get());
+    CK(cudaGetLastError());
+    h->launches += 2;
+    CK(cudaStreamSynchronize(st));  // a search on another stream reads the copy next; `off` and `pos` are freed on return
+    f->crows = std::move(rows);
+    f->cids = std::move(ids);
+    f->compact_n = f->built_n;
+    return 0;
+}
+
+static int check_filter(const wb_index* h, const wb_filter* f) {
+    if (f && f->h != h) return fail("the filter was created for another index");
+    return 0;
+}
+
 // ---- search --------------------------------------------------------------------------------
 constexpr int64_t kIvfFuseCoarseMaxQ = 4;  // largest IVF batch that runs the coarse quantizer inside the list-scan launch
 
-static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld] */, int64_t k, int64_t nprobe, float* D,
-                           int64_t* I, cudaStream_t st, const ExchParams* ex = nullptr, bool* exchanged = nullptr) {
+// Every search entry point ends here.  `f` (may be null) restricts the result to the rows it selects.
+static int search_dev_impl(wb_index* h, wb_filter* f, int64_t nq, const float* q_ld /* [nq, ld] */, int64_t k,
+                           int64_t nprobe, float* D, int64_t* I, cudaStream_t st, const ExchParams* ex = nullptr,
+                           bool* exchanged = nullptr) {
     if (exchanged) *exchanged = false;
-    if (!h->ivf) return run_flat_any(h, h->rows.get(), h->n, q_ld, nq, (int)k, h->ids.get(), D, I, st, true, ex, exchanged);
-    if (!h->trained) return fail("IndexIVFFlat is not trained");
+    if (h->ivf && !h->trained) return fail("IndexIVFFlat is not trained");
+    RowMask mask{};
+    if (f) {
+        TRY(filter_current(f, st));
+        if (f->count == 0) {  // all padding; a sharded search still takes part in the exchange (*exchanged stays false)
+            const int64_t tot = nq * k;
+            pad_results_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(D, I, tot);
+            CK(cudaGetLastError());
+            h->launches++;
+            return 0;
+        }
+        if (!h->ivf && f->count * kSparseCutoffDen < h->n) {
+            bool ok = false;
+            TRY(filter_compact(f, &ok));
+            if (ok)
+                return run_flat_any(h, f->crows.get(), f->count, q_ld, nq, (int)k, f->cids.get(), D, I, st, true, ex,
+                                    exchanged);
+        }
+        mask = RowMask{f->bits.get(), f->sel.data()};
+    }
+    const RowMask* m = f ? &mask : nullptr;
+    if (!h->ivf) return run_flat_any(h, h->rows.get(), h->n, q_ld, nq, (int)k, h->ids.get(), D, I, st, true, ex, exchanged, m);
     int np = (int)std::min<int64_t>(std::max<int64_t>(nprobe, 1), std::min<int64_t>(h->nlist, WB_MAX_K));
     if (h->csr_dirty) {
         if (st != h->stream) CK(cudaStreamSynchronize(st));
@@ -1329,7 +1486,7 @@ static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld
             // K5, batches: list-major - the probe table is inverted on the device and every probed list is streamed once
             // per group of 8 of the queries that probe it (ivf_lm.cuh)
             bool done = false;
-            TRY(run_ivf_listmajor(h, nq, q_ld, (int)k, np, D, I, st, &done));
+            TRY(run_ivf_listmajor(h, nq, q_ld, (int)k, np, D, I, st, mask.allow, &done));
             if (done) return 0;
         }
         TRY(h->parts.ensure((size_t)nq * S * k * sizeof(uint64_t)));
@@ -1343,6 +1500,7 @@ static int search_dev_impl(wb_index* h, int64_t nq, const float* q_ld /* [nq, ld
         p.row_pos = h->row_pos.get();
         p.list_off = h->list_off.get();
         p.nprobe = np;
+        p.allow = mask.allow;
         if (fuse) {
             TRY(ensure_tail_counters(h, st));
             set_tail(p, h, c, S_merge, heads_bytes, h->ids.get(), ex ? ex->D : D, ex ? ex->I : I, (int)k, ex);
@@ -1467,28 +1625,96 @@ static int search_to_host(wb_index* h, int64_t nq, int64_t k, DevBuf& D_dev, Dev
     return fetch_results(h, nq, k, D_dev.as<float>(), I_dev.as<int64_t>(), D_host, I_host, st);
 }
 
-extern "C" int wb_search_dev(wb_index* h, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe, float* D_dev,
-                             int64_t* I_dev, void* stream) {
+static int search_dev_entry(wb_index* h, wb_filter* f, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
+                            float* D_dev, int64_t* I_dev, void* stream) {
     TRY(check_search_args(h, nq, q_dev, k, D_dev, I_dev));
+    TRY(check_filter(h, f));
     if (nq == 0) return 0;
     TRY(set_dev(h));
     cudaStream_t st = (cudaStream_t)stream;
     const float* q = nullptr;
     TRY(stage_queries(h, nq, q_dev, false, st, &q));
-    return search_dev_impl(h, nq, q, k, nprobe, D_dev, I_dev, st);
+    return search_dev_impl(h, f, nq, q, k, nprobe, D_dev, I_dev, st);
 }
 
-extern "C" int wb_search(wb_index* h, int64_t nq, const float* q_host, int64_t k, int64_t nprobe, float* D_host,
-                         int64_t* I_host) {
+static int search_host_entry(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
+                             float* D_host, int64_t* I_host) {
     TRY(check_search_args(h, nq, q_host, k, D_host, I_host));
+    TRY(check_filter(h, f));
     if (nq == 0) return 0;
     TRY(set_dev(h));
     cudaStream_t st = h->stream;
     const float* q = nullptr;
     TRY(stage_queries(h, nq, q_host, true, st, &q));
     return search_to_host(h, nq, k, h->dbuf, h->ibuf, D_host, I_host, st, [&](float* D, int64_t* I) {
-        return search_dev_impl(h, nq, q, k, nprobe, D, I, st);
+        return search_dev_impl(h, f, nq, q, k, nprobe, D, I, st);
     });
+}
+
+extern "C" int wb_search_dev(wb_index* h, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe, float* D_dev,
+                             int64_t* I_dev, void* stream) {
+    return search_dev_entry(h, nullptr, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
+}
+extern "C" int wb_search(wb_index* h, int64_t nq, const float* q_host, int64_t k, int64_t nprobe, float* D_host,
+                         int64_t* I_host) {
+    return search_host_entry(h, nullptr, nq, q_host, k, nprobe, D_host, I_host);
+}
+extern "C" int wb_search_filtered_dev(wb_index* h, wb_filter* f, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
+                                      float* D_dev, int64_t* I_dev, void* stream) {
+    return search_dev_entry(h, f, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
+}
+extern "C" int wb_search_filtered(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
+                                  float* D_host, int64_t* I_host) {
+    return search_host_entry(h, f, nq, q_host, k, nprobe, D_host, I_host);
+}
+
+// ---- filter objects --------------------------------------------------------------------------
+static int filter_create(wb_index* h, std::unique_ptr<wb_filter> f, wb_filter** out) {
+    TRY(set_dev(h));
+    f->h = h;
+    TRY(filter_eval(f.get()));
+    *out = f.release();
+    return 0;
+}
+
+extern "C" int wb_filter_create_ids(wb_index* h, int64_t n, const int64_t* ids_host, int invert, wb_filter** out) {
+    if (!out) return fail("out is NULL");
+    *out = nullptr;
+    if (!h) return fail("NULL index");
+    if (n < 0 || (n > 0 && !ids_host)) return fail("bad id set");
+    std::vector<int64_t> s(ids_host, ids_host + n);
+    if (!std::is_sorted(s.begin(), s.end())) std::sort(s.begin(), s.end());
+    s.erase(std::unique(s.begin(), s.end()), s.end());
+    TRY(set_dev(h));
+    std::unique_ptr<wb_filter> f(new wb_filter());
+    f->nset = (int64_t)s.size();
+    f->invert = invert != 0;
+    CK(dev_alloc(&f->set, std::max<size_t>(s.size(), 1) * 8));  // (an empty set still has a pointer: it is a set)
+    if (!s.empty()) {
+        CK(cudaMemcpyAsync(f->set.get(), s.data(), s.size() * 8, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaStreamSynchronize(h->stream));  // `s` is freed on return
+    }
+    return filter_create(h, std::move(f), out);
+}
+
+extern "C" int wb_filter_create_range(wb_index* h, int64_t imin, int64_t imax, int invert, wb_filter** out) {
+    if (!out) return fail("out is NULL");
+    *out = nullptr;
+    if (!h) return fail("NULL index");
+    std::unique_ptr<wb_filter> f(new wb_filter());
+    f->imin = imin;
+    f->imax = imax;  // imin >= imax: the empty set
+    f->invert = invert != 0;
+    return filter_create(h, std::move(f), out);
+}
+
+extern "C" int64_t wb_filter_count(const wb_filter* f) { return f ? f->count : -1; }
+
+extern "C" int wb_filter_free(wb_filter* f) {
+    if (!f) return 0;
+    cudaSetDevice(f->h->device);
+    delete f;
+    return 0;
 }
 
 extern "C" int wb_merge_topk_dev(int device, int64_t nq, int64_t k, int64_t nparts, const float* D_parts_dev,
@@ -2129,15 +2355,15 @@ extern "C" int wb_tar_read(const char* path, int64_t d, int64_t cap, int64_t* id
 // Search over a row-sharded index, device buffers: local search + NVLink exchange + merge.  Batches that run the
 // scan kernel (flat batch <= 4, every IVF list scan) do all of it in ONE launch (scan.cuh, fused tail); the others
 // run the local search and then exchange_merge_kernel.  Every rank calls it with the same queries.
-static int exch_search_dev_impl(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_ld, int64_t k, int64_t nprobe,
-                                float* D_dev, int64_t* I_dev, cudaStream_t st) {
+static int exch_search_dev_impl(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_ld, int64_t k,
+                                int64_t nprobe, float* D_dev, int64_t* I_dev, cudaStream_t st) {
     if (ex->device != h->device) return fail("index and exchange live on different devices");
     ExchParams p;
     TRY(exch_prepare(ex, nq, k, D_dev, I_dev, &p));
     TRY(h->dbuf.ensure((size_t)nq * k * sizeof(float)));
     TRY(h->ibuf.ensure((size_t)nq * k * sizeof(int64_t)));
     bool exchanged = false;
-    TRY(search_dev_impl(h, nq, q_ld, k, nprobe, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st, &p, &exchanged));
+    TRY(search_dev_impl(h, f, nq, q_ld, k, nprobe, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st, &p, &exchanged));
     if (exchanged) {
         exch_commit(ex, p);
         return 0;
@@ -2145,23 +2371,33 @@ static int exch_search_dev_impl(wb_index* h, wb_exchange* ex, int64_t nq, const 
     return launch_exchange_kernel(ex, p, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st);
 }
 
-extern "C" int wb_exch_search_dev(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
-                                  float* D_dev, int64_t* I_dev, void* stream) {
+static int exch_search_dev_entry(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_dev, int64_t k,
+                                 int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream) {
     TRY(check_search_args(h, nq, q_dev, k, D_dev, I_dev));
+    TRY(check_filter(h, f));
     if (!ex) return fail("NULL exchange");
     if (nq == 0) return 0;
     TRY(set_dev(h));
     cudaStream_t st = (cudaStream_t)stream;
     const float* q = nullptr;
     TRY(stage_queries(h, nq, q_dev, false, st, &q));
-    return exch_search_dev_impl(h, ex, nq, q, k, nprobe, D_dev, I_dev, st);
+    return exch_search_dev_impl(h, ex, f, nq, q, k, nprobe, D_dev, I_dev, st);
+}
+extern "C" int wb_exch_search_dev(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
+                                  float* D_dev, int64_t* I_dev, void* stream) {
+    return exch_search_dev_entry(h, ex, nullptr, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
+}
+extern "C" int wb_exch_search_filtered_dev(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_dev,
+                                           int64_t k, int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream) {
+    return exch_search_dev_entry(h, ex, f, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
 }
 
 // Host-buffer search over a sharded index: H2D of the queries, local search, NVLink exchange + merge, D2H of the
 // global (D, I) - one call, one stream, one synchronisation.  Every rank calls it with the same queries.
-extern "C" int wb_exch_search(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
-                              float* D_host, int64_t* I_host) {
+static int exch_search_host_entry(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_host, int64_t k,
+                                  int64_t nprobe, float* D_host, int64_t* I_host) {
     TRY(check_search_args(h, nq, q_host, k, D_host, I_host));
+    TRY(check_filter(h, f));
     if (!ex) return fail("NULL exchange");
     if (nq == 0) return 0;
     TRY(set_dev(h));
@@ -2170,8 +2406,16 @@ extern "C" int wb_exch_search(wb_index* h, wb_exchange* ex, int64_t nq, const fl
     TRY(stage_queries(h, nq, q_host, true, st, &q));
     // (eD, eI): exch_search_dev_impl keeps this rank's local results in (dbuf, ibuf)
     TRY(search_to_host(h, nq, k, h->eD, h->eI, D_host, I_host, st, [&](float* D, int64_t* I) {
-        return exch_search_dev_impl(h, ex, nq, q, k, nprobe, D, I, st);
+        return exch_search_dev_impl(h, ex, f, nq, q, k, nprobe, D, I, st);
     }));
     if (*reinterpret_cast<volatile int*>(ex->status.get())) return fail("sharded search: a peer GPU did not join the exchange within 20 s (results invalid)");
     return 0;
+}
+extern "C" int wb_exch_search(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
+                              float* D_host, int64_t* I_host) {
+    return exch_search_host_entry(h, ex, nullptr, nq, q_host, k, nprobe, D_host, I_host);
+}
+extern "C" int wb_exch_search_filtered(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_host,
+                                       int64_t k, int64_t nprobe, float* D_host, int64_t* I_host) {
+    return exch_search_host_entry(h, ex, f, nq, q_host, k, nprobe, D_host, I_host);
 }

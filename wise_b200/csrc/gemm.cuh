@@ -35,6 +35,7 @@
 #include <cuda.h>  // CUtensorMap (types only; the encoder is fetched with cudaGetDriverEntryPoint)
 
 #include "common.cuh"
+#include "filter.cuh"
 
 namespace wb {
 
@@ -107,6 +108,7 @@ struct GemmParams {
     int* overflow;                // set when a candidate list ran out of room
     int k, cap, kstride;
     unsigned int* work_counter;   // dynamic work dispenser of this launch (zero at launch); null: static interleave
+    const uint32_t* allow;        // filtered search: bitmap over rows (= insertion positions); null: every row
 };
 
 // ---- tcgen05 / TMA PTX -----------------------------------------------------------------------
@@ -528,7 +530,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tmap, const GemmParams p) {
         int qb;
         while (next_item(wc, tile, qb)) {
             const int64_t row = p.row_begin + tile * kGemmBM + quarter * 32 + lane;
-            const bool row_ok = row < p.row_end;
+            const bool row_ok = row < p.row_end && row_allowed(p.allow, (uint32_t)row);
             if constexpr (!ARGMAX) {
                 if (etid < BN) {
                     float t = p.thr[qb * BN + etid];
@@ -907,7 +909,7 @@ gemm2_topk_kernel(const __grid_constant__ CUtensorMap tmap, const GemmParams p) 
             int qb;
             work_at(it, tile, qb);
             const int64_t row = p.row_begin + tile * kGemmBM + quarter * 32 + lane;
-            const bool row_ok = row < p.row_end;
+            const bool row_ok = row < p.row_end && row_allowed(p.allow, (uint32_t)row);
             if constexpr (!ARGMAX) {
                 if (etid < BN) thr_s[buf * BN + etid] = p.thr[qb * BN + etid];
                 named_bar_sync(kBarEpilogue, 128);

@@ -247,7 +247,7 @@ filter2_topk_kernel(const __grid_constant__ CUtensorMap tmap, const GemmParams p
             int qb;
             work_at(it, tile, qb);
             const int64_t row = p.row_begin + tile * kGemmBM + quarter * 32 + lane;
-            const bool row_ok = row < p.row_end;
+            const bool row_ok = row < p.row_end && row_allowed(p.allow, (uint32_t)row);
             if constexpr (!ARGMAX) {
                 if (etid < kBN) thr_s[buf * kBN + etid] = p.thr[qb * kBN + etid] - p.margin[qb * kBN + etid];  // +inf for padding
                 named_bar_sync(kBarEpilogue, kF2EpiThreads);

@@ -28,6 +28,7 @@ struct LmParams {
     int64_t nlist;
     const int64_t* list_off;  // [nlist + 1] rows of each list
     const uint32_t* row_pos;  // storage row -> insertion position (null: identity)
+    const uint32_t* allow;    // filtered search: bitmap over insertion positions (filter.cuh); null: every row
     const int64_t* pl_off;    // [nlist + 1] (query, probe) pairs of each list
     const uint32_t* pair_src; // [npairs] pair = query * nprobe + probe slot, grouped by list (queries ascending)
     const int64_t* item_off;  // [nlist + 1] first work item of each list; item_off[nlist] = number of items
@@ -174,7 +175,7 @@ __global__ void __launch_bounds__(kScanThreads, 1) ivf_listmajor_kernel(const Lm
                         uint32_t pos = (uint32_t)(row0 + cpos);
                         if (p.row_pos) pos = p.row_pos[pos];  // ties go by INSERTION position
                         const uint64_t key = make_key(score, pos);
-                        if (key > lists[(size_t)b * P + k - 1]) {
+                        if (key > lists[(size_t)b * P + k - 1] && row_allowed(p.allow, pos)) {
                             const int slot = atomicAdd(&qcnt[b], 1);
                             lists[(size_t)b * P + k + slot] = key;
                             hw = slot + 1 > hw_mark;

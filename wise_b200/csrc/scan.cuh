@@ -22,6 +22,7 @@
 #pragma once
 #include "coarse.cuh"
 #include "exchange.cuh"
+#include "filter.cuh"
 
 namespace wb {
 
@@ -74,6 +75,7 @@ struct ScanParams {
     // works until the rows run out.  The result does not depend on who scans what: keys carry positions.
     unsigned int* group_count; // [gridDim.y], zero between launches (reset with tail_count); null: static partition
     const int64_t* ids;       // position -> external id (null: id = position)
+    const uint32_t* allow;    // filtered search: bitmap over insertion positions (filter.cuh); null: every row
     float* D;                 // [nq][k]
     int64_t* I;
     int exchange;             // 0: emit local results; 1: exch holds the peer mailboxes
@@ -419,7 +421,7 @@ __global__ void __launch_bounds__(kScanThreads, 1) scan_topk_kernel(const ScanPa
                     uint32_t pos = GATHER ? gather_row(G, (uint32_t)cpos) : (uint32_t)cpos;
                     if (GATHER && p.row_pos) pos = p.row_pos[pos];  // grouped store: ties go by INSERTION position
                     const uint64_t key = make_key(score, pos);
-                    if (key > lists[(size_t)b * P + k - 1]) {
+                    if (key > lists[(size_t)b * P + k - 1] && row_allowed(p.allow, pos)) {
                         const int slot = atomicAdd(&qcnt[b], 1);
                         lists[(size_t)b * P + k + slot] = key;
                         hw = slot + 1 > hw_mark;

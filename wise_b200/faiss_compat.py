@@ -5,7 +5,9 @@ INTEGRATION.md).  Mirrored surface (SURVEY.md section 8b):
 
   module : IndexFlatIP(d) | IndexIDMap(index) | IndexIVFFlat(quantizer, d, nlist, metric)
            METRIC_INNER_PRODUCT | IO_FLAG_READ_ONLY | write_index | read_index
-  index  : .d .ntotal .is_trained .train .add .add_with_ids .search
+  index  : .d .ntotal .is_trained .train .add .add_with_ids .search(x, k, params=None)
+  search : SearchParameters(sel) | SearchParametersIVF(sel, nprobe)
+           IDSelectorBatch | IDSelectorRange | IDSelectorNot (filtered search, faiss >= 1.7.3)
            IVF only: .nprobe .parallel_mode .make_direct_map .direct_map .reconstruct_batch
            (Flat/IDMap deliberately have no `nprobe`/`direct_map`: /root/reference/api/routes.py:899
             and :1317 branch on hasattr())
@@ -124,18 +126,33 @@ class Index:
     def _nprobe(self) -> int:
         return 1
 
-    def search(self, x, k: int):
+    def _search_params(self, params):
+        """(nprobe, wb_filter* or None) of a search with faiss SearchParameters `params` (None: the index's own)."""
+        if params is None:
+            return self._nprobe(), None
+        if not isinstance(params, SearchParameters):
+            raise TypeError("params must be a SearchParameters")
+        return self._nprobe(), (params.sel._filter(self._hd) if params.sel is not None else None)
+
+    def search(self, x, k: int, *, params=None):
         """D, I = index.search(x, k)  (/root/reference/src/index/feature_search_index.py:113,
-        /root/reference/api/routes.py:1407): D float32 (n,k) descending, I int64 (n,k), -1 padded."""
+        /root/reference/api/routes.py:1407): D float32 (n,k) descending, I int64 (n,k), -1 padded.
+        params=SearchParameters(sel=...) restricts the result to the rows whose id the selector keeps (exact top-k
+        of those rows; IVF takes SearchParametersIVF, whose nprobe replaces index.nprobe for this call)."""
         x = _as_f32_matrix(x, self.d, "x")
         k = int(k)
         if k <= 0:
             raise AssertionError("k must be positive")  # faiss: assert k > 0
+        nprobe, flt = self._search_params(params)
         n = x.shape[0]
         D = np.empty((n, k), np.float32)
         I = np.empty((n, k), np.int64)
         if n:
-            _capi.check(_capi.lib().wb_search(self._h, n, _capi.ptr(x), k, self._nprobe(), _capi.ptr(D), _capi.ptr(I)))
+            L = _capi.lib()
+            if flt is None:
+                _capi.check(L.wb_search(self._h, n, _capi.ptr(x), k, nprobe, _capi.ptr(D), _capi.ptr(I)))
+            else:
+                _capi.check(L.wb_search_filtered(self._h, flt, n, _capi.ptr(x), k, nprobe, _capi.ptr(D), _capi.ptr(I)))
         return D, I
 
     # -- bulk access used by write_index --------------------------------------------------------
@@ -233,6 +250,14 @@ class IndexIVFFlat(Index):
     def _nprobe(self) -> int:
         return max(1, int(self.nprobe))
 
+    def _search_params(self, params):
+        if params is None:
+            return self._nprobe(), None
+        if not isinstance(params, SearchParametersIVF):
+            raise RuntimeError("IndexIVF params have incorrect type")  # faiss IndexIVF::search
+        _, flt = super()._search_params(params)
+        return max(1, int(params.nprobe)), flt
+
     def train(self, x) -> None:
         """index.train(train_features) (/root/reference/src/index/feature_search_index.py:75): k-means with
         max-inner-product assignment, faiss Clustering defaults in self.cp (niter=10, seed=1234, spherical=False,
@@ -297,6 +322,117 @@ class IndexIVFFlat(Index):
         if self.direct_map.type == DirectMap.NoMap:
             raise RuntimeError("direct map not initialized")
         return _reconstruct(self, keys)
+
+
+class _Filter:
+    """Owns one wb_filter*.  Holds the _Handle of its index, so the filter is freed before the index is."""
+
+    def __init__(self, hd: _Handle, f):
+        self.hd = hd
+        self.f = f
+
+    def __del__(self):
+        f, self.f = getattr(self, "f", None), None
+        if f:
+            try:
+                _capi.lib().wb_filter_free(f)
+            except Exception:  # interpreter shutdown
+                pass
+
+    @property
+    def count(self) -> int:
+        """Rows selected when the filter was last evaluated."""
+        return int(_capi.lib().wb_filter_count(self.f))
+
+
+class IDSelector:
+    """faiss.IDSelector: decides per external id whether a row takes part in a search.  The selectors here are
+    evaluated on the GPU into one bitmap per index (kept while the selector lives, re-evaluated after adds)."""
+
+    _invert = False
+
+    def __init__(self):
+        self._filters: dict[int, _Filter] = {}
+
+    def _create(self, h, invert: bool, out) -> int:
+        raise NotImplementedError
+
+    def _filter(self, hd: _Handle):
+        """This selector's wb_filter* for the index owning `hd`, created on first use."""
+        f = self._filters.get(id(hd))
+        if f is None:
+            p = C.c_void_p()
+            _capi.check(self._create(hd.h, self._invert, C.byref(p)))
+            f = self._filters[id(hd)] = _Filter(hd, p)
+        return f.f
+
+
+class IDSelectorBatch(IDSelector):
+    """faiss.IDSelectorBatch(ids) or (n, ids): the ids in a set (any order, duplicates allowed)."""
+
+    def __init__(self, *args):
+        super().__init__()
+        if len(args) == 2:
+            n, ids = int(args[0]), args[1]
+            ids = np.asarray(ids).reshape(-1)[:n]
+        elif len(args) == 1:
+            ids = np.asarray(args[0]).reshape(-1)
+        else:
+            raise TypeError("IDSelectorBatch(ids) or IDSelectorBatch(n, ids)")
+        if ids.size and ids.dtype.kind not in "iu":
+            raise TypeError(f"ids must be integers (got {ids.dtype})")
+        self.ids = np.unique(ids.astype(np.int64))  # sorted and unique: the device set is searched by bisection
+
+    def _create(self, h, invert, out):
+        return _capi.lib().wb_filter_create_ids(h, self.ids.size, _capi.ptr(self.ids), int(invert), out)
+
+
+class IDSelectorRange(IDSelector):
+    """faiss.IDSelectorRange(imin, imax): imin <= id < imax (empty when imin >= imax)."""
+
+    def __init__(self, imin: int, imax: int):
+        super().__init__()
+        for v in (imin, imax):
+            if not isinstance(v, (int, np.integer)) or isinstance(v, bool):
+                raise TypeError(f"IDSelectorRange bounds must be integers (got {type(v).__name__})")
+        self.imin, self.imax = int(imin), int(imax)
+
+    def _create(self, h, invert, out):
+        return _capi.lib().wb_filter_create_range(h, self.imin, self.imax, int(invert), out)
+
+
+class IDSelectorNot(IDSelector):
+    """faiss.IDSelectorNot(sel): the ids `sel` rejects.  `sel` is an IDSelectorBatch, IDSelectorRange or another
+    IDSelectorNot (Not of Not keeps what the inner selector keeps)."""
+
+    def __init__(self, sel: IDSelector):
+        super().__init__()
+        if not isinstance(sel, (IDSelectorBatch, IDSelectorRange, IDSelectorNot)):
+            raise TypeError("IDSelectorNot takes an IDSelectorBatch, IDSelectorRange or IDSelectorNot")
+        self.sel = sel
+        self._base = sel._base if isinstance(sel, IDSelectorNot) else sel
+        self._invert = not sel._invert
+
+    def _create(self, h, invert, out):
+        return self._base._create(h, invert, out)
+
+
+class SearchParameters:
+    """faiss.SearchParameters(sel=...): per-call search options of a flat index."""
+
+    def __init__(self, sel: IDSelector | None = None):
+        if sel is not None and not isinstance(sel, IDSelector):
+            raise TypeError("sel must be an IDSelector")
+        self.sel = sel
+
+
+class SearchParametersIVF(SearchParameters):
+    """faiss.SearchParametersIVF(sel=..., nprobe=...): an IVF index's per-call options; nprobe (default 1, as in
+    faiss) replaces index.nprobe for the call."""
+
+    def __init__(self, sel: IDSelector | None = None, nprobe: int = 1):
+        super().__init__(sel)
+        self.nprobe = int(nprobe)
 
 
 def _reconstruct(index: Index, keys) -> np.ndarray:

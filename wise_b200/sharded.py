@@ -14,6 +14,10 @@ tests/test_sharded_cpu.py).
 
 IVF: centroids are replicated, each rank keeps its slice of every inverted list; the candidate
 set of a query is the union over ranks, so the same merge applies.
+
+Filtered search (params=SearchParameters(sel=...)): every rank applies the same selector to its own rows, so the
+candidate set is again the union over ranks and the exchange is unchanged.  A rank whose rows the selector rejects
+entirely contributes padding and still takes part in the exchange.
 """
 from __future__ import annotations
 
@@ -30,13 +34,15 @@ def shard_range(n_total: int, rank: int, world: int) -> tuple[int, int]:
     return n_total * rank // world, n_total * (rank + 1) // world
 
 
-def _cuda_local_search(index, q: torch.Tensor, k: int, nprobe: int):
+def _cuda_local_search(index, q: torch.Tensor, k: int, nprobe: int, flt=None):
+    """Local top-k on this rank's GPU; `flt` (a wb_filter* of `index`, or None) restricts the rows."""
     from . import _capi
     nq = q.shape[0]
     D = torch.empty((nq, k), dtype=torch.float32, device=q.device)
     I = torch.empty((nq, k), dtype=torch.int64, device=q.device)
     st = torch.cuda.current_stream(q.device).cuda_stream
-    _capi.check(_capi.lib().wb_search_dev(index._h, nq, q.data_ptr(), k, nprobe, D.data_ptr(), I.data_ptr(), st))
+    _capi.check(_capi.lib().wb_search_filtered_dev(index._h, flt, nq, q.data_ptr(), k, nprobe, D.data_ptr(),
+                                                   I.data_ptr(), st))
     return D, I
 
 
@@ -86,14 +92,15 @@ class PeerExchange:
                                                             Io.data_ptr(), st))
         return Do, Io
 
-    def search_dev(self, index, q: torch.Tensor, k: int, nprobe: int):
-        """Local search + exchange + merge in one C call (one kernel launch for scan-served searches)."""
+    def search_dev(self, index, q: torch.Tensor, k: int, nprobe: int, flt=None):
+        """Local search + exchange + merge in one C call (one kernel launch for scan-served searches); `flt` is an
+        optional wb_filter* of `index`."""
         nq = q.shape[0]
         D = torch.empty((nq, k), dtype=torch.float32, device=q.device)
         I = torch.empty((nq, k), dtype=torch.int64, device=q.device)
         st = torch.cuda.current_stream(q.device).cuda_stream
-        self._capi.check(self._capi.lib().wb_exch_search_dev(index._h, self.h, nq, q.data_ptr(), k, nprobe, D.data_ptr(),
-                                                             I.data_ptr(), st))
+        self._capi.check(self._capi.lib().wb_exch_search_filtered_dev(index._h, self.h, flt, nq, q.data_ptr(), k, nprobe,
+                                                                      D.data_ptr(), I.data_ptr(), st))
         return D, I
 
     def timed_out(self) -> bool:
@@ -151,11 +158,23 @@ class ShardedIndex:
         """Each rank adds ITS OWN rows (the caller partitions the store with shard_range)."""
         self.local.add_with_ids(x, ids)
 
-    def search_dev(self, q: torch.Tensor, k: int, nprobe: int = 1):
-        """q: [nq, d] float32 tensor, replicated on every rank. Returns merged (D, I) tensors on every rank."""
+    def _params(self, nprobe: int, params):
+        """(nprobe, wb_filter* or None): faiss SearchParameters resolved against this rank's index."""
+        if params is None:
+            return nprobe, None
+        return self.local._search_params(params)
+
+    def search_dev(self, q: torch.Tensor, k: int, nprobe: int = 1, params=None):
+        """q: [nq, d] float32 tensor, replicated on every rank. Returns merged (D, I) tensors on every rank.
+        params: faiss SearchParameters / SearchParametersIVF (the same selector on every rank; its nprobe replaces
+        `nprobe`)."""
+        nprobe, flt = self._params(nprobe, params)
         if self.exchange is not None and self.exchange.fits(q.shape[0], k):
-            return self.exchange.search_dev(self.local, q.contiguous(), k, nprobe)
-        D, I = self._local_search(self.local, q, k, nprobe)
+            return self.exchange.search_dev(self.local, q.contiguous(), k, nprobe, flt)
+        if flt is None:
+            D, I = self._local_search(self.local, q, k, nprobe)
+        else:
+            D, I = self._local_search(self.local, q, k, nprobe, flt)
         if self.world == 1:
             return D, I
         nq, kk = D.shape
@@ -165,22 +184,23 @@ class ShardedIndex:
         dist.all_gather_into_tensor(Ip, I.contiguous(), group=self.group)
         return self._merge(Dp.view(self.world, nq, kk), Ip.view(self.world, nq, kk))
 
-    def search(self, x: np.ndarray, k: int):
-        """faiss-style host API: numpy in, numpy out (same on every rank)."""
+    def search(self, x: np.ndarray, k: int, params=None):
+        """faiss-style host API: numpy in, numpy out (same on every rank).  params as in search_dev."""
         x = np.ascontiguousarray(x, np.float32)
         if self.exchange is not None and self.exchange.fits(x.shape[0], int(k)):
             # one C call: H2D, local search, NVLink exchange + merge, D2H (no torch ops on the path)
             from . import _capi
+            nprobe, flt = self._params(int(getattr(self.local, "nprobe", 1)), params)
             nq = x.shape[0]
             D = np.empty((nq, int(k)), np.float32)
             I = np.empty((nq, int(k)), np.int64)
-            _capi.check(_capi.lib().wb_exch_search(self.local._h, self.exchange.h, nq, _capi.ptr(x), int(k),
-                                                  int(getattr(self.local, "nprobe", 1)), _capi.ptr(D), _capi.ptr(I)))
+            _capi.check(_capi.lib().wb_exch_search_filtered(self.local._h, self.exchange.h, flt, nq, _capi.ptr(x), int(k),
+                                                           nprobe, _capi.ptr(D), _capi.ptr(I)))
             return D, I
         dev = self._comm_device()
         q = torch.from_numpy(np.ascontiguousarray(x, np.float32)).to(dev)
         nprobe = getattr(self.local, "nprobe", 1)
-        D, I = self.search_dev(q, int(k), int(nprobe))
+        D, I = self.search_dev(q, int(k), int(nprobe), params)
         return D.cpu().numpy(), I.cpu().numpy()
 
 
