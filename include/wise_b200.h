@@ -141,6 +141,23 @@ int wb_search_filtered(wb_index* h, wb_filter* f, int64_t nq, const float* q_hos
 int wb_search_filtered_dev(wb_index* h, wb_filter* f, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
                            float* D_dev, int64_t* I_dev, void* stream);
 
+/* ---- range search (DESIGN.md "Range search") ----------------------------------------------------
+ * Every row whose fp32 inner product with the query is strictly greater than `thresh` (the score returned in D is the
+ * one compared), per query in score-descending order, equal scores by insertion position.  Flat: every row is a
+ * candidate; IVF: the rows of the nprobe lists the coarse quantizer of wb_search picks; with a filter, only the rows it
+ * selects.  There is no cap on the result size (WB_MAX_K does not apply): query i's results are entries
+ * [lims[i], lims[i+1]) of D and I.  A query whose hits alone exceed the device budget of one call (2^28 hits) is an
+ * error; the index stays usable.
+ * Results come back in a wb_range_result that owns host memory: it does not depend on the index's scratch or lifetime,
+ * so a later search cannot clobber it, and it may outlive the index. */
+typedef struct wb_range_result wb_range_result;
+/* index.range_search(x, thresh, params=...) [faiss-upstream].  f may be NULL (unfiltered); nprobe is ignored by flat
+ * indices.  Synchronises once the hit counts are known; fills lims_host[0..nq] before returning. */
+int wb_range_search(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, float thresh, int64_t nprobe,
+                    int64_t* lims_host, wb_range_result** out);
+int wb_range_result_copy(const wb_range_result* r, float* D_host, int64_t* I_host); /* lims_host[nq] entries each */
+int wb_range_result_free(wb_range_result* r);
+
 /* Merge `nparts` sorted partial results (layout [part][nq][k], e.g. the all-gathered per-GPU
  * top-k) into the global top-k.  Order: score desc, then part asc, then rank-in-part asc - with
  * contiguous row sharding that is exactly "lowest insertion position". */

@@ -23,6 +23,7 @@
 #include "ivf_lm.cuh"
 #include "kmeans.cuh"
 #include "merge.cuh"
+#include "range.cuh"
 #include "scan.cuh"
 #include "tarstore.h"
 
@@ -154,6 +155,7 @@ struct wb_index {
     cudaEvent_t add_ev[kAddSlots] = {};
     bool add_pending[kAddSlots] = {};
     int64_t gemm_launches = 0, gemm_fallbacks = 0;
+    DevBuf rpool, rqid, rgrp, rstate, roff, rrun;  // range search: hit pool, query tags, sort buffer, counters, lims, runs
     DevBuf phase;               // WB_PHASE_TS=1: per-CTA phase stamps of the last fused-tail scan launch (diagnostics)
     DevBuf ckeys;               // fused coarse quantizer: ordered centroid scores of the queries of one launch
     bool coop_ok = false;       // the device takes cooperative launches (fused coarse quantizer, coarse.cuh)
@@ -630,6 +632,11 @@ constexpr double kK2StreamBytesPerS = 6.0e12;
 constexpr double kK2FixedSeconds = 0.3e-3;
 constexpr int64_t kK2MinBatch = 5;  // measured: K2 5.8 ms vs K1 8.1 ms at 5..8 queries (10M x 768)
 
+// Range search (DESIGN.md "Range search"): the hits of one chunk of queries are held on the device at 20 bytes each
+// (pool key + query tag, one sort buffer); a chunk holds at most this many, and so does an enlarged K2 candidate list.
+constexpr int64_t kRangeBudgetHits = (int64_t)1 << 28;
+constexpr int kRangeEpochs = 64;  // K2 range epochs of one batch, re-runs included (12x growth: ~6 + ~6 re-runs)
+
 // Can the tensor-core path take this problem?  (candidate capacity `cap` rows form epoch 0)
 static bool gemm_eligible(const wb_index* h, int64_t nrows, int64_t nq, int k, int* cap_out) {
     if (nq < kK2MinBatch) return false;
@@ -651,11 +658,13 @@ static bool gemm_eligible(const wb_index* h, int64_t nrows, int64_t nq, int k, i
 template <int BN>
 static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const float* q_ld, int64_t nq, int k, int cap,
                          const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, bool* overflowed,
-                         const RowMask* mask) {
+                         const RowMask* mask, const RangeOut* range) {
     // Filter-and-refine (rows of the store, or the compact copy of a filter's rows: norm2_max bounds both; not the
     // centroid table): after the first epoch the GEMM issues only the hi x hi term and the compaction re-scores the few
     // hundred candidates per query exactly in fp32.
-    const bool filter = rows != h->centroids.get() && env_int("WB_GEMM_FILTER", 1) != 0;
+    // A range search (`range`, k = 0) runs every epoch one-term: a 3xTF32 score is not the exact fp32 score, so it must
+    // not decide membership.
+    const bool filter = rows != h->centroids.get() && (range || env_int("WB_GEMM_FILTER", 1) != 0);
     constexpr bool kFold = kGemmFold<BN, false>;
     using Cfg = GemmCfg<BN, kFold>;
     constexpr int kGemmBN = BN;
@@ -676,7 +685,8 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
     const int nq_pad = use_f2 ? nqb2 * kF2BN : nqb * kGemmBN;  // thresholds / margins of padding queries: +inf / 0
     TRY(h->gimg.ensure((size_t)nqb * nchunks * kGemmBBytes));
     TRY(h->gkeys.ensure((size_t)nq * kstride * sizeof(uint64_t)));
-    TRY(h->gstate.ensure((size_t)nq_pad * 4 + (size_t)nq * 4 + 64 + 64 * 4));  // thr | cnt | overflow | one work dispenser per epoch
+    // thr | cnt | overflow | one work dispenser per epoch | range: overflow flag and candidate count of each epoch
+    TRY(h->gstate.ensure((size_t)nq_pad * 4 + (size_t)nq * 4 + 64 + 64 * 4 + (range ? 2 * kRangeEpochs * 4 : 0)));
     float* thr = h->gstate.as<float>();
     float* margin = nullptr;
     if (filter) {
@@ -708,13 +718,17 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
     int* cnt = reinterpret_cast<int*>(thr + (size_t)nq_pad);
     int* overflow = cnt + nq;
     unsigned int* dispensers = reinterpret_cast<unsigned int*>(overflow + 16);  // [64], zeroed once per search
-    CK(cudaMemsetAsync(dispensers, 0, 64 * sizeof(unsigned int), st));
+    int* rflags = range ? reinterpret_cast<int*>(dispensers + 64) : nullptr;  // [kRangeEpochs] flags, then counts
+    CK(cudaMemsetAsync(dispensers, 0, 64 * sizeof(unsigned int) + (range ? 2 * kRangeEpochs * 4 : 0), st));
     int epoch_no = 0;
     uint64_t* keys = h->gkeys.as<uint64_t>();
     {
         const int64_t n1 = std::max<int64_t>((int64_t)nq_pad, nq * (int64_t)k);
-        init_gemm_state_kernel<<<(unsigned)((n1 + 255) / 256), 256, 0, st>>>(thr, (int)nq, nq_pad, cnt, keys, k,
-                                                                            kstride, overflow);
+        if (range)
+            range_gemm_init_kernel<<<(unsigned)((nq_pad + 255) / 256), 256, 0, st>>>(thr, (int)nq, nq_pad, range->thresh, cnt);
+        else
+            init_gemm_state_kernel<<<(unsigned)((n1 + 255) / 256), 256, 0, st>>>(thr, (int)nq, nq_pad, cnt, keys, k,
+                                                                                kstride, overflow);
         CK(cudaGetLastError());
         const int64_t n2 = (int64_t)nqb * nchunks * 8 * kGemmBN;
         if constexpr (BN >= 128) {
@@ -785,34 +799,16 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
     // next epoch = growth x (rows seen so far): a query then collects ~k*ln(1+growth) survivors per epoch, far
     // below `cap`; fewer, larger epochs mean fewer launch gaps and compactions (each costs ~50 us)
     const double growth = std::min(12.0, std::max(0.25, (double)cap / (4.0 * k)));
-    TRY(timing_begin(h, timed && h->timing, st));
-    int64_t r0 = 0;
-    while (r0 < nrows) {
-        int64_t r1;
-        if (mask) {
-            // the same schedule in SELECTED rows: epoch 0 ends before its selected rows (every one of them a candidate)
-            // exceed `cap`, later epochs take growth x the selected rows seen so far.  Counting all rows instead, a
-            // filter that keeps 13 % of the rows leaves fewer than k = 1000 of them in a 4096-row epoch 0, the
-            // threshold stays -inf and the next epoch's candidates overflow `cap`.  (A filter that keeps every row
-            // gets exactly the unfiltered epochs.)
-            const int64_t t0 = r0 / kGemmBM, nt = (nrows + kGemmBM - 1) / kGemmBM;
-            const int64_t seen = mask->sel[t0];
-            const int64_t grow = (int64_t)((double)seen * growth);
-            const int64_t want = seen + (r0 == 0 ? cap : (grow + kGemmBM - 1) / kGemmBM * kGemmBM);
-            const int64_t t1 = std::upper_bound(mask->sel + t0 + 1, mask->sel + nt + 1, want) - mask->sel - 1;
-            r1 = std::min(nrows, std::max(t1, t0 + 1) * kGemmBM);
-        } else {
-            int64_t len = r0 == 0 ? cap : (int64_t)((double)r0 * growth);
-            len = std::max<int64_t>(kGemmBM, (len + kGemmBM - 1) / kGemmBM * kGemmBM);
-            r1 = std::min(nrows, r0 + len);
-        }
+    // one epoch over rows [r0, r1): the K2 launch, the exact re-scoring of its candidates and their compaction
+    auto run_epoch = [&](int64_t r0, int64_t r1) -> int {
         g.row_begin = r0;
         g.row_end = r1;
         const int64_t nwork = ((r1 - r0 + kGemmBM - 1) / kGemmBM) * nqb;
         const unsigned grid = (unsigned)std::min<int64_t>(nwork, h->sm_count);
         // first epoch: 3xTF32 scores select, the winners are re-scored; later epochs: one-term filter, candidates re-scored
-        const bool one_term = filter && r0 > 0;
-        c.rescore = filter ? (r0 == 0 ? 2 : 1) : 0;
+        const bool one_term = filter && (r0 > 0 || range);
+        c.rescore = filter ? (r0 == 0 && !range ? 2 : 1) : 0;
+        if (range) g.overflow = rflags + epoch_no;
         if constexpr (BN >= 128) {
             // with the pair, every filter epoch (one_term) goes to the SS kernel: use_f2 or use_f2h is set
             const int64_t ntp = ((r1 - r0 + kGemmBM - 1) / kGemmBM + 1) / 2;
@@ -853,14 +849,78 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
             CK(cudaGetLastError());
             h->launches++;
         }
-        compact_topk_kernel<<<(unsigned)nq, kMergeThreads, (size_t)c.S * 8, st>>>(c);
+        if (range) {
+            const RangeCollect rc{keys, cnt, g.cap, g.kstride, rflags + epoch_no, rflags + kRangeEpochs + epoch_no, *range};
+            range_collect_kernel<<<(unsigned)nq, kRangeThreads, 0, st>>>(rc);
+        } else {
+            compact_topk_kernel<<<(unsigned)nq, kMergeThreads, (size_t)c.S * 8, st>>>(c);
+        }
         CK(cudaGetLastError());
         h->launches += 2;
         h->gemm_launches++;
         epoch_no++;
+        return 0;
+    };
+    TRY(timing_begin(h, timed && h->timing, st));
+    std::vector<std::pair<int64_t, int64_t>> spans;  // range: the row span of every epoch (overflow repair)
+    int64_t r0 = 0;
+    while (r0 < nrows) {
+        if (range && epoch_no >= kRangeEpochs / 2) {  // (not reached: 12x growth; K1 takes the batch)
+            *overflowed = true;
+            return 0;
+        }
+        int64_t r1;
+        if (mask) {
+            // the same schedule in SELECTED rows: epoch 0 ends before its selected rows (every one of them a candidate)
+            // exceed `cap`, later epochs take growth x the selected rows seen so far.  Counting all rows instead, a
+            // filter that keeps 13 % of the rows leaves fewer than k = 1000 of them in a 4096-row epoch 0, the
+            // threshold stays -inf and the next epoch's candidates overflow `cap`.  (A filter that keeps every row
+            // gets exactly the unfiltered epochs.)
+            const int64_t t0 = r0 / kGemmBM, nt = (nrows + kGemmBM - 1) / kGemmBM;
+            const int64_t seen = mask->sel[t0];
+            const int64_t grow = (int64_t)((double)seen * growth);
+            const int64_t want = seen + (r0 == 0 ? cap : (grow + kGemmBM - 1) / kGemmBM * kGemmBM);
+            const int64_t t1 = std::upper_bound(mask->sel + t0 + 1, mask->sel + nt + 1, want) - mask->sel - 1;
+            r1 = std::min(nrows, std::max(t1, t0 + 1) * kGemmBM);
+        } else {
+            int64_t len = r0 == 0 ? cap : (int64_t)((double)r0 * growth);
+            len = std::max<int64_t>(kGemmBM, (len + kGemmBM - 1) / kGemmBM * kGemmBM);
+            r1 = std::min(nrows, r0 + len);
+        }
+        TRY(run_epoch(r0, r1));
+        if (range) spans.emplace_back(r0, r1);
         r0 = r1;
     }
     TRY(timing_end(h, timed && h->timing, st));
+    if (range) {
+        // An epoch whose candidate list overflowed contributed nothing; its exact candidate count is known, so it is
+        // re-run once with a list that holds them all.  *overflowed: the enlarged lists would exceed the budget (the
+        // caller runs the batch on K1 instead).
+        *overflowed = false;
+        std::vector<int> fl(2 * kRangeEpochs);
+        CK(cudaMemcpyAsync(fl.data(), rflags, fl.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        const int first = epoch_no;
+        for (size_t e = 0; e < spans.size(); ++e) {
+            if (!fl[e]) continue;
+            const int64_t want = ((int64_t)fl[kRangeEpochs + e] + 127) / 128 * 128;
+            if (nq * want > kRangeBudgetHits || epoch_no >= kRangeEpochs) {
+                *overflowed = true;
+                return 0;
+            }
+            TRY(h->gkeys.ensure((size_t)nq * want * sizeof(uint64_t)));
+            keys = h->gkeys.as<uint64_t>();
+            g.keys = c.keys = keys;
+            g.cap = g.kstride = c.cap = c.kstride = (int)want;
+            TRY(run_epoch(spans[e].first, spans[e].second));
+        }
+        if (epoch_no > first) {
+            CK(cudaMemcpyAsync(fl.data(), rflags, kRangeEpochs * sizeof(int), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            for (int e = first; e < epoch_no; ++e) *overflowed |= fl[e] != 0;
+        }
+        return 0;
+    }
     int ovf = 0;
     CK(cudaMemcpyAsync(&ovf, overflow, sizeof(int), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
@@ -870,13 +930,13 @@ static int run_flat_gemm_t(wb_index* h, const float* rows, int64_t nrows, const 
 
 static int run_flat_gemm(wb_index* h, const float* rows, int64_t nrows, const float* q_ld, int64_t nq, int k, int cap,
                          const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, bool* overflowed,
-                         const RowMask* mask) {
+                         const RowMask* mask, const RangeOut* range = nullptr) {
     // 16-query blocks halve the image traffic and the MMA work of a half-empty 32-query block (K2 is power-capped at
     // small batches: 992 W and 1.37 GHz at batch 16)
-    if (nq <= 16) return run_flat_gemm_t<16>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask);
-    if (nq <= 32) return run_flat_gemm_t<32>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask);
-    if (nq <= 64) return run_flat_gemm_t<64>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask);
-    return run_flat_gemm_t<128>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask);
+    if (nq <= 16) return run_flat_gemm_t<16>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask, range);
+    if (nq <= 32) return run_flat_gemm_t<32>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask, range);
+    if (nq <= 64) return run_flat_gemm_t<64>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask, range);
+    return run_flat_gemm_t<128>(h, rows, nrows, q_ld, nq, k, cap, ids, D, I, st, timed, overflowed, mask, range);
 }
 
 // K4/K6 on the tensor cores: argmax over the centroid table for n device-resident points (row stride ld).
@@ -1666,6 +1726,276 @@ extern "C" int wb_search_filtered_dev(wb_index* h, wb_filter* f, int64_t nq, con
 extern "C" int wb_search_filtered(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
                                   float* D_host, int64_t* I_host) {
     return search_host_entry(h, f, nq, q_host, k, nprobe, D_host, I_host);
+}
+
+// ---- range search (DESIGN.md "Range search") --------------------------------------------------------------------
+struct wb_range_result {  // host memory only: independent of the index, its scratch and its lifetime
+    std::vector<float> D;
+    std::vector<int64_t> I;
+};
+
+constexpr int64_t kRangeMaxQ = 32768;  // queries per chunk: one launch (grid.y) per scan
+constexpr int kRangeStage = 256;       // staged hits per query and CTA in the range scan (P of its shared lists)
+
+template <int NQ, int RW, bool GATHER>
+static int launch_range_t(const ScanParams& p, const RangeOut& ro, dim3 grid, size_t smem, cudaStream_t st) {
+    CK(smem_optin<scan_range_kernel<NQ, RW, GATHER>>(232448));
+    scan_range_kernel<NQ, RW, GATHER><<<grid, kScanThreads, smem, st>>>(p, ro);
+    CK(cudaGetLastError());
+    return 0;
+}
+
+template <int NQ, bool GATHER>
+static int launch_range_rw(int RW, const ScanParams& p, const RangeOut& ro, dim3 grid, size_t smem, cudaStream_t st) {
+    switch (RW) {
+        case 4: return launch_range_t<NQ, 4, GATHER>(p, ro, grid, smem, st);
+        case 2: return launch_range_t<NQ, 2, GATHER>(p, ro, grid, smem, st);
+        case 1: return launch_range_t<NQ, 1, GATHER>(p, ro, grid, smem, st);
+    }
+    return fail("bad RW %d", RW);
+}
+
+// K1 / K5 in range mode: `S` CTAs per query group, one launch per <= kMaxGridY groups.  Whole-row stages draw their
+// row groups from the shared dispensers, which every launch leaves at zero as the fused tails do.
+static int run_range_scan(wb_index* h, const ScanCfg& c, bool gather, ScanParams& p, int64_t S, int64_t nq,
+                          const float* q_ld, int np, const RangeOut& ro0, cudaStream_t st) {
+    apply_scan_cfg(c, p);
+    p.k = 0;
+    p.nparts = (int)S;
+    TRY(ensure_tail_counters(h, st));
+    p.group_count = c.nchunks == 1 ? h->tailcnt.as<unsigned int>() + kMaxGridY : nullptr;
+    const int64_t qgroups = (nq + c.NQ - 1) / c.NQ;
+    TRY(timing_begin(h, h->timing, st));
+    for (int64_t g0 = 0; g0 < qgroups; g0 += kMaxGridY) {
+        const int64_t gy = std::min(kMaxGridY, qgroups - g0), qoff = g0 * c.NQ;
+        p.queries = q_ld + (size_t)qoff * h->ld;
+        p.nq = (int)std::min<int64_t>(nq - qoff, gy * c.NQ);
+        if (gather) p.probes = h->pI.as<int64_t>() + (size_t)qoff * np;
+        RangeOut ro = ro0;
+        ro.count += qoff;
+        ro.qbase = (int)qoff;
+        const dim3 grid((unsigned)S, (unsigned)gy);
+        const int rc = gather      ? launch_range_rw<1, true>(c.RW, p, ro, grid, c.smem, st)
+                       : c.NQ == 1 ? launch_range_rw<1, false>(c.RW, p, ro, grid, c.smem, st)
+                       : c.NQ == 2 ? launch_range_rw<2, false>(c.RW, p, ro, grid, c.smem, st)
+                       : c.NQ == 4 ? launch_range_rw<4, false>(c.RW, p, ro, grid, c.smem, st)
+                                   : launch_range_rw<8, false>(c.RW, p, ro, grid, c.smem, st);
+        TRY(rc);
+        h->launches++;
+        if (p.group_count) CK(cudaMemsetAsync(p.group_count, 0, (size_t)gy * sizeof(unsigned int), st));
+    }
+    return timing_end(h, h->timing, st);
+}
+
+// Flat range hits of `nq` queries against `nrows` rows: K2 epochs when search would take K2 for this batch (the same
+// cost model without its k terms), else K1.  A K2 batch whose candidate lists cannot be repaired goes to K1.
+static int range_flat(wb_index* h, const float* rows, int64_t nrows, const float* q_ld, int64_t nq, const RowMask* mask,
+                      const RangeOut& ro, cudaStream_t st) {
+    int cap = 0;
+    if (gemm_eligible(h, nrows, nq, 0, &cap)) {
+        bool ovf = false;
+        TRY(run_flat_gemm(h, rows, nrows, q_ld, nq, 0, cap, nullptr, nullptr, nullptr, st, true, &ovf, mask, &ro));
+        if (!ovf) return 0;
+        h->gemm_fallbacks++;
+        CK(cudaMemsetAsync(ro.cursor, 0, (size_t)(1 + nq) * sizeof(unsigned long long), st));
+    }
+    ScanCfg c;
+    TRY(plan_scan(h, nq, kRangeStage - kMinQueue, false, 0, &c));
+    const int64_t ngroups = (nrows + kConsumerWarps * c.RW - 1) / (kConsumerWarps * c.RW);
+    const int64_t qgroups = (nq + c.NQ - 1) / c.NQ;
+    int64_t S = std::min<int64_t>(std::max<int64_t>(ngroups, 1),
+                                  std::max<int64_t>(1, ((int64_t)h->sm_count * (qgroups > 1 ? 2 : 1) + qgroups - 1) / qgroups));
+    S = std::min<int64_t>(S, (int64_t)h->sm_count);
+    ScanParams p{};
+    p.rows = rows;
+    p.nrows = nrows;
+    p.ld = h->ld;
+    p.allow = mask ? mask->allow : nullptr;
+    return run_range_scan(h, c, false, p, S, nq, q_ld, 0, ro, st);
+}
+
+// IVF range hits: K4 picks the probes exactly as search does, then K5 scans them query-major in range mode.
+static int range_ivf(wb_index* h, int64_t nq, const float* q_ld, int np, const uint32_t* allow, const RangeOut& ro,
+                     cudaStream_t st) {
+    TRY(h->pD.ensure((size_t)nq * np * sizeof(float)));
+    TRY(h->pI.ensure((size_t)nq * np * sizeof(int64_t)));
+    TRY(run_flat_any(h, h->centroids.get(), h->nlist, q_ld, nq, np, nullptr, h->pD.as<float>(), h->pI.as<int64_t>(), st, false));
+    ScanCfg c;
+    TRY(plan_scan(h, 1, kRangeStage - kMinQueue, true, np, &c));
+    const int64_t S = nq >= h->sm_count ? 1 : std::max<int64_t>(1, (int64_t)h->sm_count / nq);
+    ScanParams p{};
+    p.rows = h->rows.get();
+    p.ld = h->ld;
+    p.perm = h->slot_row.get();
+    p.row_pos = h->row_pos.get();
+    p.list_off = h->list_off.get();
+    p.nprobe = np;
+    p.allow = allow;
+    return run_range_scan(h, c, true, p, S, nq, q_ld, np, ro, st);
+}
+
+// Sort the `total` pooled hits of a chunk by query and key, emit them as (D, I) and append them to `res`.
+// off[nq + 1]: exclusive prefix of the per-query counts.
+static int range_assemble(wb_index* h, int64_t nq, const std::vector<int64_t>& off, const int64_t* ids,
+                          wb_range_result* res, cudaStream_t st) {
+    const int64_t total = off[nq];
+    if (total == 0) return 0;
+    uint64_t* pool = h->rpool.as<uint64_t>();
+    TRY(h->rgrp.ensure((size_t)total * sizeof(uint64_t)));
+    TRY(h->roff.ensure((size_t)(nq + 1) * sizeof(int64_t) + (size_t)nq * sizeof(unsigned int)));
+    int64_t* off_dev = h->roff.as<int64_t>();
+    unsigned int* fill = reinterpret_cast<unsigned int*>(off_dev + nq + 1);
+    CK(cudaMemcpyAsync(off_dev, off.data(), (size_t)(nq + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(fill, 0, (size_t)nq * sizeof(unsigned int), st));
+    const unsigned blocks = (unsigned)((total + 255) / 256);
+    uint64_t* cur = h->rgrp.as<uint64_t>();
+    uint64_t* other = pool;
+    range_scatter_kernel<<<blocks, 256, 0, st>>>(pool, h->rqid.as<uint32_t>(), total, off_dev, fill, cur);
+    CK(cudaGetLastError());
+    // runs of <= kRangeRun keys of one query, sorted in shared memory
+    std::vector<int64_t> run_start;
+    std::vector<int> run_len;
+    int64_t longest = 0;
+    for (int64_t q = 0; q < nq; ++q) {
+        const int64_t n = off[q + 1] - off[q];
+        longest = std::max(longest, n);
+        for (int64_t s = 0; s < n; s += kRangeRun) {
+            run_start.push_back(off[q] + s);
+            run_len.push_back((int)std::min<int64_t>(kRangeRun, n - s));
+        }
+    }
+    const size_t nruns = run_start.size();
+    TRY(h->rrun.ensure(nruns * (sizeof(int64_t) + sizeof(int))));
+    int64_t* rs_dev = h->rrun.as<int64_t>();
+    int* rl_dev = reinterpret_cast<int*>(rs_dev + nruns);
+    CK(cudaMemcpyAsync(rs_dev, run_start.data(), nruns * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(rl_dev, run_len.data(), nruns * sizeof(int), cudaMemcpyHostToDevice, st));
+    CK(smem_optin<range_block_sort_kernel>(kRangeRun * 8));
+    for (size_t r0 = 0; r0 < nruns; r0 += (size_t)1 << 30) {
+        const size_t nr = std::min(nruns - r0, (size_t)1 << 30);
+        range_block_sort_kernel<<<(unsigned)nr, kRangeThreads, (size_t)kRangeRun * 8, st>>>(cur, rs_dev + r0, rl_dev + r0);
+        CK(cudaGetLastError());
+    }
+    h->launches += 2;
+    for (int64_t w = kRangeRun; w < longest; w *= 2) {
+        range_merge_kernel<<<blocks, 256, 0, st>>>(cur, other, off_dev, (int)nq, total, w);
+        CK(cudaGetLastError());
+        std::swap(cur, other);
+        h->launches++;
+    }
+    // (D, I) go to the two buffers the sorted keys no longer need: the query tags and the other key buffer
+    float* D_dev = reinterpret_cast<float*>(h->rqid.get());
+    int64_t* I_dev = reinterpret_cast<int64_t*>(other);
+    range_emit_kernel<<<blocks, 256, 0, st>>>(cur, total, ids, D_dev, I_dev);
+    CK(cudaGetLastError());
+    h->launches++;
+    const size_t at = res->D.size();
+    res->D.resize(at + (size_t)total);
+    res->I.resize(at + (size_t)total);
+    CK(cudaMemcpyAsync(res->D.data() + at, D_dev, (size_t)total * sizeof(float), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(res->I.data() + at, I_dev, (size_t)total * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+static int range_search_impl(wb_index* h, wb_filter* f, int64_t nq, const float* q, float thresh, int64_t nprobe,
+                             int64_t* lims, wb_range_result* res, cudaStream_t st) {
+    if (h->ivf && !h->trained) return fail("IndexIVFFlat is not trained");
+    for (int64_t i = 0; i <= nq; ++i) lims[i] = 0;
+    if (nq == 0 || h->n == 0) return 0;
+    // the rows to search, as search_dev_impl picks them
+    const float* rows = h->rows.get();
+    int64_t nrows = h->n;
+    const int64_t* ids = h->ids.get();
+    RowMask mask{};
+    const RowMask* m = nullptr;
+    if (f) {
+        TRY(filter_current(f, st));
+        if (f->count == 0) return 0;
+        bool compact = false;
+        if (!h->ivf && f->count * kSparseCutoffDen < h->n) TRY(filter_compact(f, &compact));
+        if (compact) {
+            rows = f->crows.get();
+            nrows = f->count;
+            ids = f->cids.get();
+        } else {
+            mask = RowMask{f->bits.get(), f->sel.data()};
+            m = &mask;
+        }
+    }
+    const int np = (int)std::min<int64_t>(std::max<int64_t>(nprobe, 1), std::min<int64_t>(h->nlist, WB_MAX_K));
+    if (h->ivf && h->csr_dirty) TRY(ensure_csr(h));
+    TRY(h->rstate.ensure((size_t)(1 + kRangeMaxQ) * sizeof(unsigned long long)));
+    unsigned long long* cursor = h->rstate.as<unsigned long long>();
+    std::vector<unsigned long long> cnt((size_t)(1 + kRangeMaxQ));
+    for (int64_t q0 = 0; q0 < nq;) {
+        int64_t nqc = std::min(kRangeMaxQ, nq - q0);
+        const float* qc = q + (size_t)q0 * h->ld;
+        // run the scan; if the hits exceed the pool, grow it to the exact count and run again
+        for (int attempt = 0;; ++attempt) {
+            TRY(h->rpool.ensure((size_t)std::min<int64_t>(kRangeBudgetHits, nqc * 64) * sizeof(uint64_t)));
+            TRY(h->rqid.ensure(h->rpool.cap / 2));
+            const RangeOut ro{thresh, cursor, cursor + 1, h->rpool.as<uint64_t>(), h->rqid.as<uint32_t>(),
+                              (int64_t)(h->rpool.cap / sizeof(uint64_t)), 0};
+            CK(cudaMemsetAsync(cursor, 0, (size_t)(1 + nqc) * sizeof(unsigned long long), st));
+            if (h->ivf) TRY(range_ivf(h, nqc, qc, np, m ? m->allow : nullptr, ro, st));
+            else TRY(range_flat(h, rows, nrows, qc, nqc, m, ro, st));
+            CK(cudaMemcpyAsync(cnt.data(), cursor, (size_t)(1 + nqc) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            int64_t total = (int64_t)cnt[0];
+            if (total <= ro.cap) break;
+            if (attempt >= 3) return fail("range_search: the hit count of a chunk did not settle");
+            if (total > kRangeBudgetHits) {  // fewer queries: the longest prefix whose hits fit the budget
+                int64_t keep = 0, sum = 0;
+                while (keep < nqc && sum + (int64_t)cnt[1 + keep] <= kRangeBudgetHits) sum += (int64_t)cnt[1 + keep++];
+                if (keep == 0)
+                    return fail("range_search: query %lld has %llu results, more than the %lld one call can hold",
+                                (long long)q0, cnt[1], (long long)kRangeBudgetHits);
+                nqc = keep;
+                total = sum;
+            }
+            TRY(h->rpool.ensure((size_t)total * sizeof(uint64_t)));
+            TRY(h->rqid.ensure((size_t)total * sizeof(uint32_t)));
+        }
+        std::vector<int64_t> off((size_t)nqc + 1, 0);
+        for (int64_t i = 0; i < nqc; ++i) off[i + 1] = off[i] + (int64_t)cnt[1 + i];
+        for (int64_t i = 1; i <= nqc; ++i) lims[q0 + i] = lims[q0] + off[i];
+        TRY(range_assemble(h, nqc, off, ids, res, st));
+        q0 += nqc;
+    }
+    return 0;
+}
+
+extern "C" int wb_range_search(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, float thresh, int64_t nprobe,
+                               int64_t* lims_host, wb_range_result** out) {
+    if (!out) return fail("out is NULL");
+    *out = nullptr;
+    if (!h) return fail("NULL index");
+    if (nq < 0) return fail("negative nq");
+    if (!lims_host || (nq > 0 && !q_host)) return fail("NULL buffer");
+    TRY(check_filter(h, f));
+    TRY(set_dev(h));
+    std::unique_ptr<wb_range_result> res(new wb_range_result());
+    cudaStream_t st = h->stream;
+    const float* q = nullptr;
+    if (nq > 0) TRY(stage_queries(h, nq, q_host, true, st, &q));
+    TRY(range_search_impl(h, f, nq, q, thresh, nprobe, lims_host, res.get(), st));
+    *out = res.release();
+    return 0;
+}
+
+extern "C" int wb_range_result_copy(const wb_range_result* r, float* D_host, int64_t* I_host) {
+    if (!r) return fail("NULL range result");
+    if (r->D.empty()) return 0;
+    if (!D_host || !I_host) return fail("NULL buffer");
+    memcpy(D_host, r->D.data(), r->D.size() * sizeof(float));
+    memcpy(I_host, r->I.data(), r->I.size() * sizeof(int64_t));
+    return 0;
+}
+
+extern "C" int wb_range_result_free(wb_range_result* r) {
+    delete r;
+    return 0;
 }
 
 // ---- filter objects --------------------------------------------------------------------------

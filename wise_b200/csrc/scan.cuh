@@ -18,6 +18,8 @@
 //     queue; when a queue fills, the consumers bitonic-sort [top-k list | queue] in shared
 //     memory and tighten the threshold.  Scores never go to HBM; each CTA writes k keys per
 //     query at the end, merged by merge_topk_kernel (merge.cuh).
+//   * range mode (scan_range_kernel, range search): the same scan with a fixed threshold; every hit is staged in the
+//     shared lists and flushed to a global pool (RangeOut) instead of the fused top-k (DESIGN.md "Range search").
 // Algorithmic bytes per launch: nrows * ld * 4 (the row store is read exactly once per pass).
 #pragma once
 #include "coarse.cuh"
@@ -152,8 +154,53 @@ __device__ __forceinline__ uint32_t gather_row(const GatherCtx& G, uint32_t cpos
     return G.perm ? G.perm[slot] : (uint32_t)slot;  // perm == null: rows are physically grouped by list
 }
 
-template <int NQ, int RW, bool GATHER>
-__global__ void __launch_bounds__(kScanThreads, 1) scan_topk_kernel(const ScanParams p) {
+// Range search (DESIGN.md "Range search"): where the result goes.  Every row with score > thresh (and allowed by the
+// filter) is appended to `keys` / `qid` at a slot drawn from `cursor`; `count[q]` counts the hits of query q.  Both
+// counters keep counting once `cap` slots are used, so the host learns the exact sizes from one read.
+struct RangeOut {
+    float thresh;
+    unsigned long long* cursor;  // pool slots drawn so far
+    unsigned long long* count;   // [nq of this launch] hits per query
+    uint64_t* keys;              // [cap] pool: make_key(score, insertion position)
+    uint32_t* qid;               // [cap] query of each pool entry (chunk-relative)
+    int64_t cap;
+    int qbase;                   // chunk-relative index of this launch's first query
+};
+
+// The scan (K1 flat, K5 gather) with its result stage as a compile-time mode: RANGE = false keeps the fused top-k,
+// RANGE = true stages every hit in the per-query shared lists and flushes them to the range pool (RangeOut).
+// Range mode: move the staged hits of every query of this CTA to the pool - one slot reservation and one count per
+// query and flush - and empty the stages.  Called by all consumer threads at a consumer barrier.  The pool slot bases
+// live in the misc region behind qcnt[] (the range kernel has no thresholds there): round8(4 NQ) + 8 NQ <= 12 NQ + 16.
+template <int NQ>
+__device__ __forceinline__ void range_flush(const ScanSmem& L, unsigned char* smem, const uint64_t* lists, int* qcnt,
+                                            int P, int q0, int nqv, int ctid, const RangeOut& ro) {
+    unsigned long long* base = reinterpret_cast<unsigned long long*>(smem + L.misc + ((NQ * 4 + 7) & ~7));
+    if (ctid < nqv) {
+        const int c = qcnt[ctid];
+        if (c) {
+            base[ctid] = atomicAdd(ro.cursor, (unsigned long long)c);
+            atomicAdd(&ro.count[q0 + ctid], (unsigned long long)c);
+        }
+    }
+    named_bar_sync(kBarConsumers, kConsumerThreads);
+    for (int i = ctid; i < nqv * P; i += kConsumerThreads) {
+        const int l = i / P, j = i - l * P;
+        if (j < qcnt[l]) {
+            const unsigned long long slot = base[l] + (unsigned long long)j;
+            if (slot < (unsigned long long)ro.cap) {
+                ro.keys[slot] = lists[i];
+                ro.qid[slot] = (uint32_t)(ro.qbase + q0 + l);
+            }
+        }
+    }
+    named_bar_sync(kBarConsumers, kConsumerThreads);
+    if (ctid < nqv) qcnt[ctid] = 0;
+    named_bar_sync(kBarConsumers, kConsumerThreads);
+}
+
+template <int NQ, int RW, bool GATHER, bool RANGE>
+__device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& ro) {
     constexpr int kRowsPerWarp = RW;
     constexpr int kGroupRows = kConsumerWarps * RW;
     extern __shared__ __align__(128) unsigned char smem_scan[];
@@ -415,6 +462,22 @@ __global__ void __launch_bounds__(kScanThreads, 1) scan_topk_kernel(const ScanPa
             const bool owner = (lane & ((32 >> LV) - 1)) == 0;
             const int r = vi / NQ, b = vi % NQ;
             bool hw = false;
+            if constexpr (RANGE) {
+                if (owner && b < nqv) {
+                    const int64_t cpos = g * kGroupRows + cw * kRowsPerWarp + r;
+                    if (cpos < total && score > ro.thresh) {
+                        uint32_t pos = GATHER ? gather_row(G, (uint32_t)cpos) : (uint32_t)cpos;
+                        if (GATHER && p.row_pos) pos = p.row_pos[pos];
+                        if (row_allowed(p.allow, pos)) {
+                            const int slot = atomicAdd(&qcnt[b], 1);
+                            lists[(size_t)b * P + slot] = make_key(score, pos);
+                            hw = slot + 1 > hw_mark;
+                        }
+                    }
+                }
+                if (named_bar_or(kBarConsumers, kConsumerThreads, hw)) range_flush<NQ>(L, smem, lists, qcnt, P, q0, nqv, ctid, ro);
+                continue;
+            }
             if (owner) {
                 const int64_t cpos = g * kGroupRows + cw * kRowsPerWarp + r;
                 if (cpos < total && score >= thr_s[b]) {
@@ -446,6 +509,10 @@ __global__ void __launch_bounds__(kScanThreads, 1) scan_topk_kernel(const ScanPa
         // ---- epilogue: final sort, k best keys of this CTA for each query -------------------
         named_bar_sync(kBarConsumers, kConsumerThreads);
         stamp(5);
+        if constexpr (RANGE) {
+            range_flush<NQ>(L, smem, lists, qcnt, P, q0, nqv, ctid, ro);
+            return;
+        }
         if (NQ == 1 && p.rank_sort) rank_sort_desc<kConsumerThreads>(lists, P, ctid, kBarConsumers);
         else bitonic_sort_desc<kConsumerThreads>(lists, P, nqv, ctid, kBarConsumers);
         stamp(6);
@@ -529,6 +596,17 @@ __global__ void __launch_bounds__(kScanThreads, 1) scan_topk_kernel(const ScanPa
         }
         stamp(9);
     }
+}
+
+template <int NQ, int RW, bool GATHER>
+__global__ void __launch_bounds__(kScanThreads, 1) scan_topk_kernel(const ScanParams p) {
+    scan_impl<NQ, RW, GATHER, false>(p, RangeOut{});
+}
+
+// Range mode: P = the staging capacity per query, p.k = 0; no parts, no fused tail.
+template <int NQ, int RW, bool GATHER>
+__global__ void __launch_bounds__(kScanThreads, 1) scan_range_kernel(const ScanParams p, const RangeOut ro) {
+    scan_impl<NQ, RW, GATHER, true>(p, ro);
 }
 
 }  // namespace wb

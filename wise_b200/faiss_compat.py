@@ -6,6 +6,7 @@ INTEGRATION.md).  Mirrored surface (SURVEY.md section 8b):
   module : IndexFlatIP(d) | IndexIDMap(index) | IndexIVFFlat(quantizer, d, nlist, metric)
            METRIC_INNER_PRODUCT | IO_FLAG_READ_ONLY | write_index | read_index
   index  : .d .ntotal .is_trained .train .add .add_with_ids .search(x, k, params=None)
+           .range_search(x, thresh, params=None) -> lims (uint64, n+1), D, I
   search : SearchParameters(sel) | SearchParametersIVF(sel, nprobe)
            IDSelectorBatch | IDSelectorRange | IDSelectorNot (filtered search, faiss >= 1.7.3)
            IVF only: .nprobe .parallel_mode .make_direct_map .direct_map .reconstruct_batch
@@ -154,6 +155,29 @@ class Index:
             else:
                 _capi.check(L.wb_search_filtered(self._h, flt, n, _capi.ptr(x), k, nprobe, _capi.ptr(D), _capi.ptr(I)))
         return D, I
+
+    def range_search(self, x, thresh, *, params=None):
+        """lims, D, I = index.range_search(x, thresh): every row whose inner product with a query is strictly greater
+        than `thresh` (used as float32).  Query i's results are D[lims[i]:lims[i+1]] (float32, descending; equal scores
+        by insertion order) and I[...] (int64).  lims is uint64 of length n+1, as faiss returns it; there is no cap on
+        the number of results.  params as in search (IVF: the rows of the probed lists are the candidates)."""
+        x = _as_f32_matrix(x, self.d, "x")
+        thresh = np.float32(thresh)
+        nprobe, flt = self._search_params(params)
+        n = x.shape[0]
+        lims = np.zeros((n + 1,), np.int64)
+        L = _capi.lib()
+        res = C.c_void_p()
+        _capi.check(L.wb_range_search(self._h, flt, n, _capi.ptr(x) if n else None, float(thresh), nprobe,
+                                      _capi.ptr(lims), C.byref(res)))
+        try:
+            total = int(lims[-1])
+            D = np.empty((total,), np.float32)
+            I = np.empty((total,), np.int64)
+            _capi.check(L.wb_range_result_copy(res, _capi.ptr(D), _capi.ptr(I)))
+        finally:
+            L.wb_range_result_free(res)
+        return lims.astype(np.uint64), D, I
 
     # -- bulk access used by write_index --------------------------------------------------------
     def _export(self, start: int, n: int, want_assign: bool = False, want_ids: bool = True, want_x: bool = True):
