@@ -148,15 +148,34 @@ int wb_search_filtered_dev(wb_index* h, wb_filter* f, int64_t nq, const float* q
  * selects.  There is no cap on the result size (WB_MAX_K does not apply): query i's results are entries
  * [lims[i], lims[i+1]) of D and I.  A query whose hits alone exceed the device budget of one call (2^28 hits) is an
  * error; the index stays usable.
- * Results come back in a wb_range_result that owns host memory: it does not depend on the index's scratch or lifetime,
- * so a later search cannot clobber it, and it may outlive the index. */
+ * Results come back in a wb_range_result that owns its memory (host memory, or device memory for wb_range_search_dev):
+ * it does not depend on the index's scratch or lifetime, so a later search cannot clobber it, and it may outlive the
+ * index. */
 typedef struct wb_range_result wb_range_result;
 /* index.range_search(x, thresh, params=...) [faiss-upstream].  f may be NULL (unfiltered); nprobe is ignored by flat
  * indices.  Synchronises once the hit counts are known; fills lims_host[0..nq] before returning. */
 int wb_range_search(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, float thresh, int64_t nprobe,
                     int64_t* lims_host, wb_range_result** out);
-int wb_range_result_copy(const wb_range_result* r, float* D_host, int64_t* I_host); /* lims_host[nq] entries each */
-int wb_range_result_free(wb_range_result* r);
+/* The same search with queries [nq, d] on the index's GPU, run on `stream`, which is synchronised once per query chunk
+ * to read the hit counts; lims_host is filled before returning.  The result holds D and I in device memory of the
+ * index's GPU, written on `stream`: no host copy is made. */
+int wb_range_search_dev(wb_index* h, wb_filter* f, int64_t nq, const float* q_dev, float thresh, int64_t nprobe,
+                        int64_t* lims_host, wb_range_result** out, void* stream);
+/* Copy a result (host or device) out, lims_host[nq] entries each.  wb_range_result_copy synchronises the device of a
+ * device result first; wb_range_result_copy_dev enqueues the copies on `stream` (for a device result: the stream it
+ * was written on, or one ordered after it). */
+int wb_range_result_copy(const wb_range_result* r, float* D_host, int64_t* I_host);
+int wb_range_result_copy_dev(const wb_range_result* r, float* D_dev, int64_t* I_dev, void* stream);
+int wb_range_result_free(wb_range_result* r); /* a device result's memory is freed on its GPU */
+
+/* Sharded range search: merge the range results of the same nq queries from `nparts` parts (one per rank, rank p
+ * holding the p-th contiguous slice of the rows).  Part p's hits for query q are entries
+ * p * part_stride + [lims_p[q], lims_p[q+1]) of D_parts / I_parts (the padded all-gather layout), lims_p =
+ * lims_parts_dev + p * (nq + 1).  lims_dev[nq + 1] is the sum of the parts' lims.  The result is the single-index
+ * order: score descending, equal scores by part, then by order inside the part.  No synchronisation, no allocation. */
+int wb_range_merge_dev(int device, int64_t nq, int64_t nparts, const int64_t* lims_parts_dev, int64_t part_stride,
+                       const float* D_parts_dev, const int64_t* I_parts_dev, const int64_t* lims_dev, float* D_dev,
+                       int64_t* I_dev, void* stream);
 
 /* Merge `nparts` sorted partial results (layout [part][nq][k], e.g. the all-gathered per-GPU
  * top-k) into the global top-k.  Order: score desc, then part asc, then rank-in-part asc - with

@@ -58,8 +58,11 @@ SIGNATURES = {
     "wb_search_filtered": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp]),
     "wb_search_filtered_dev": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp]),
     "wb_range_search": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_float, C.c_int64, _vp, C.POINTER(_vp)]),
+    "wb_range_search_dev": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_float, C.c_int64, _vp, C.POINTER(_vp), _vp]),
     "wb_range_result_copy": (C.c_int, [_vp, _vp, _vp]),
+    "wb_range_result_copy_dev": (C.c_int, [_vp, _vp, _vp, _vp]),
     "wb_range_result_free": (C.c_int, [_vp]),
+    "wb_range_merge_dev": (C.c_int, [C.c_int, C.c_int64, C.c_int64, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "wb_exch_search_filtered": (C.c_int, [_vp, _vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp]),
     "wb_exch_search_filtered_dev": (C.c_int, [_vp, _vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp]),
     "wb_merge_topk_dev":(C.c_int, [C.c_int, C.c_int64, C.c_int64, C.c_int64, _vp, _vp, _vp, _vp, _vp]),

@@ -1729,9 +1729,18 @@ extern "C" int wb_search_filtered(wb_index* h, wb_filter* f, int64_t nq, const f
 }
 
 // ---- range search (DESIGN.md "Range search") --------------------------------------------------------------------
-struct wb_range_result {  // host memory only: independent of the index, its scratch and its lifetime
+// A result owns its (D, I): in host memory (wb_range_search) or, one part per query chunk with hits, in device memory of
+// the index's GPU (wb_range_search_dev).  Either way it is independent of the index, its scratch and its lifetime.
+struct wb_range_result {
     std::vector<float> D;
     std::vector<int64_t> I;
+    int device = -1;  // >= 0: a device result on this GPU
+    struct Part {
+        DevPtr<float> D;
+        DevPtr<int64_t> I;
+        int64_t n = 0;
+    };
+    std::vector<Part> parts;
 };
 
 constexpr int64_t kRangeMaxQ = 32768;  // queries per chunk: one launch (grid.y) per scan
@@ -1834,7 +1843,8 @@ static int range_ivf(wb_index* h, int64_t nq, const float* q_ld, int np, const u
     return run_range_scan(h, c, true, p, S, nq, q_ld, np, ro, st);
 }
 
-// Sort the `total` pooled hits of a chunk by query and key, emit them as (D, I) and append them to `res`.
+// Sort the `total` pooled hits of a chunk by query and key, emit them as (D, I) and append them to `res`: a host result
+// gets them with one synchronisation, a device result gets a new part that the emit kernel writes on `st`.
 // off[nq + 1]: exclusive prefix of the per-query counts.
 static int range_assemble(wb_index* h, int64_t nq, const std::vector<int64_t>& off, const int64_t* ids,
                           wb_range_result* res, cudaStream_t st) {
@@ -1883,12 +1893,22 @@ static int range_assemble(wb_index* h, int64_t nq, const std::vector<int64_t>& o
         std::swap(cur, other);
         h->launches++;
     }
-    // (D, I) go to the two buffers the sorted keys no longer need: the query tags and the other key buffer
+    // host result: (D, I) go to the two buffers the sorted keys no longer need, the query tags and the other key buffer
     float* D_dev = reinterpret_cast<float*>(h->rqid.get());
     int64_t* I_dev = reinterpret_cast<int64_t*>(other);
+    if (res->device >= 0) {
+        wb_range_result::Part part;
+        CK(dev_alloc(&part.D, (size_t)total * sizeof(float)));
+        CK(dev_alloc(&part.I, (size_t)total * sizeof(int64_t)));
+        part.n = total;
+        D_dev = part.D.get();
+        I_dev = part.I.get();
+        res->parts.push_back(std::move(part));
+    }
     range_emit_kernel<<<blocks, 256, 0, st>>>(cur, total, ids, D_dev, I_dev);
     CK(cudaGetLastError());
     h->launches++;
+    if (res->device >= 0) return 0;
     const size_t at = res->D.size();
     res->D.resize(at + (size_t)total);
     res->I.resize(at + (size_t)total);
@@ -1924,7 +1944,10 @@ static int range_search_impl(wb_index* h, wb_filter* f, int64_t nq, const float*
         }
     }
     const int np = (int)std::min<int64_t>(std::max<int64_t>(nprobe, 1), std::min<int64_t>(h->nlist, WB_MAX_K));
-    if (h->ivf && h->csr_dirty) TRY(ensure_csr(h));
+    if (h->ivf && h->csr_dirty) {
+        if (st != h->stream) CK(cudaStreamSynchronize(st));  // ensure_csr runs on h->stream: rows added on `st` first
+        TRY(ensure_csr(h));
+    }
     TRY(h->rstate.ensure((size_t)(1 + kRangeMaxQ) * sizeof(unsigned long long)));
     unsigned long long* cursor = h->rstate.as<unsigned long long>();
     std::vector<unsigned long long> cnt((size_t)(1 + kRangeMaxQ));
@@ -1966,34 +1989,83 @@ static int range_search_impl(wb_index* h, wb_filter* f, int64_t nq, const float*
     return 0;
 }
 
-extern "C" int wb_range_search(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, float thresh, int64_t nprobe,
-                               int64_t* lims_host, wb_range_result** out) {
+// `host`: q is host memory and the result a host result; else q is on the index's GPU and the result a device result.
+static int range_search_entry(wb_index* h, wb_filter* f, int64_t nq, const float* q_in, bool host, float thresh,
+                              int64_t nprobe, int64_t* lims_host, wb_range_result** out, cudaStream_t st) {
     if (!out) return fail("out is NULL");
     *out = nullptr;
     if (!h) return fail("NULL index");
     if (nq < 0) return fail("negative nq");
-    if (!lims_host || (nq > 0 && !q_host)) return fail("NULL buffer");
+    if (!lims_host || (nq > 0 && !q_in)) return fail("NULL buffer");
     TRY(check_filter(h, f));
     TRY(set_dev(h));
     std::unique_ptr<wb_range_result> res(new wb_range_result());
-    cudaStream_t st = h->stream;
+    if (!host) res->device = h->device;
     const float* q = nullptr;
-    if (nq > 0) TRY(stage_queries(h, nq, q_host, true, st, &q));
+    if (nq > 0) TRY(stage_queries(h, nq, q_in, host, st, &q));
     TRY(range_search_impl(h, f, nq, q, thresh, nprobe, lims_host, res.get(), st));
     *out = res.release();
     return 0;
 }
 
+extern "C" int wb_range_search(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, float thresh, int64_t nprobe,
+                               int64_t* lims_host, wb_range_result** out) {
+    return range_search_entry(h, f, nq, q_host, true, thresh, nprobe, lims_host, out, h ? h->stream : nullptr);
+}
+
+extern "C" int wb_range_search_dev(wb_index* h, wb_filter* f, int64_t nq, const float* q_dev, float thresh,
+                                   int64_t nprobe, int64_t* lims_host, wb_range_result** out, void* stream) {
+    return range_search_entry(h, f, nq, q_dev, false, thresh, nprobe, lims_host, out, (cudaStream_t)stream);
+}
+
+static int64_t range_result_size(const wb_range_result* r) {
+    int64_t n = (int64_t)r->D.size();
+    for (const auto& p : r->parts) n += p.n;
+    return n;
+}
+
 extern "C" int wb_range_result_copy(const wb_range_result* r, float* D_host, int64_t* I_host) {
     if (!r) return fail("NULL range result");
-    if (r->D.empty()) return 0;
+    if (range_result_size(r) == 0) return 0;
     if (!D_host || !I_host) return fail("NULL buffer");
-    memcpy(D_host, r->D.data(), r->D.size() * sizeof(float));
-    memcpy(I_host, r->I.data(), r->I.size() * sizeof(int64_t));
+    if (r->device < 0) {
+        memcpy(D_host, r->D.data(), r->D.size() * sizeof(float));
+        memcpy(I_host, r->I.data(), r->I.size() * sizeof(int64_t));
+        return 0;
+    }
+    CK(cudaSetDevice(r->device));
+    CK(cudaDeviceSynchronize());  // the result was written on the caller's stream, which this call does not know
+    for (const auto& p : r->parts) {
+        CK(cudaMemcpy(D_host, p.D.get(), (size_t)p.n * sizeof(float), cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(I_host, p.I.get(), (size_t)p.n * sizeof(int64_t), cudaMemcpyDeviceToHost));
+        D_host += p.n;
+        I_host += p.n;
+    }
+    return 0;
+}
+
+extern "C" int wb_range_result_copy_dev(const wb_range_result* r, float* D_dev, int64_t* I_dev, void* stream) {
+    if (!r) return fail("NULL range result");
+    if (range_result_size(r) == 0) return 0;
+    if (!D_dev || !I_dev) return fail("NULL buffer");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (r->device < 0) {  // (pageable source: the call returns once the driver has staged it)
+        CK(cudaMemcpyAsync(D_dev, r->D.data(), r->D.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(I_dev, r->I.data(), r->I.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+        return 0;
+    }
+    CK(cudaSetDevice(r->device));
+    for (const auto& p : r->parts) {
+        CK(cudaMemcpyAsync(D_dev, p.D.get(), (size_t)p.n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(I_dev, p.I.get(), (size_t)p.n * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+        D_dev += p.n;
+        I_dev += p.n;
+    }
     return 0;
 }
 
 extern "C" int wb_range_result_free(wb_range_result* r) {
+    if (r && r->device >= 0) cudaSetDevice(r->device);  // the device memory is freed on its own GPU
     delete r;
     return 0;
 }
@@ -2064,6 +2136,24 @@ extern "C" int wb_merge_topk_dev(int device, int64_t nq, int64_t k, int64_t npar
     m.I = I_dev;
     CK(smem_optin<merge_topk_kernel<false>>(8192 * 8));
     merge_topk_kernel<false><<<(unsigned)nq, kMergeThreads, (size_t)m.S * 8, (cudaStream_t)stream>>>(m);
+    CK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int wb_range_merge_dev(int device, int64_t nq, int64_t nparts, const int64_t* lims_parts_dev,
+                                  int64_t part_stride, const float* D_parts_dev, const int64_t* I_parts_dev,
+                                  const int64_t* lims_dev, float* D_dev, int64_t* I_dev, void* stream) {
+    if (nq < 0) return fail("negative nq");
+    if (nparts < 1 || nparts > kMaxGridY) return fail("nparts=%lld out of range [1, %lld]", (long long)nparts,
+                                                      (long long)kMaxGridY);
+    if (part_stride < 0) return fail("negative part stride");
+    if (nq == 0 || part_stride == 0) return 0;  // nothing to merge
+    if (!lims_parts_dev || !D_parts_dev || !I_parts_dev || !lims_dev || !D_dev || !I_dev) return fail("NULL buffer");
+    const int64_t bx = (part_stride + 255) / 256;
+    if (bx > INT32_MAX) return fail("part stride %lld too large", (long long)part_stride);
+    CK(cudaSetDevice(device));
+    range_merge_parts_kernel<<<dim3((unsigned)bx, (unsigned)nparts), 256, 0, (cudaStream_t)stream>>>(
+        lims_parts_dev, nq, part_stride, D_parts_dev, I_parts_dev, lims_dev, D_dev, I_dev);
     CK(cudaGetLastError());
     return 0;
 }

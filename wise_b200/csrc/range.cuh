@@ -9,6 +9,7 @@
 //                             longest query is one run (each key finds its rank in the other run by bisection:
 //                             keys of one query are distinct, so ranks are unique and the result is deterministic);
 //   range_emit_kernel         turns keys into (D, I).
+// A sharded range search merges the per-rank (D, I) with range_merge_parts_kernel.
 #pragma once
 #include "merge.cuh"
 #include "scan.cuh"
@@ -141,6 +142,47 @@ __global__ void range_emit_kernel(const uint64_t* keys, int64_t total, const int
     const uint32_t pos = key_pos(key);
     D[i] = key_score(key);
     I[i] = ids ? ids[pos] : (int64_t)pos;
+}
+
+// Sharded range search: merge the range results of the same nq queries from gridDim.y parts (ranks).  Part p's hits
+// for query q are entries p * stride + [lp[q], lp[q + 1]) of Dp / Ip, lp = lims_parts + p * (nq + 1), in the order
+// range_emit_kernel writes them.  Entry i of part p goes to lims[q] + (i - lp[q]) plus, for every other part, the
+// number of its entries of query q that come first: a larger score (parts after p) or a larger or equal score (parts
+// before p).  Scores compare as order_f32 bits, the map make_key uses, so equal scores tie by part, then by position
+// inside the part: the single-index order when part p holds the p-th contiguous slice of the rows.  The output is a
+// permutation of the input, found by bisection alone.
+__global__ void range_merge_parts_kernel(const int64_t* lims_parts, int64_t nq, int64_t stride, const float* Dp,
+                                         const int64_t* Ip, const int64_t* lims, float* D, int64_t* I) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    const int p = blockIdx.y;
+    const int64_t* lp = lims_parts + (size_t)p * (nq + 1);
+    if (i >= stride || i >= lp[nq]) return;
+    int64_t lo = 0, hi = nq - 1;  // the query of entry i: the largest q with lp[q] <= i
+    while (lo < hi) {
+        const int64_t mid = (lo + hi + 1) >> 1;
+        if (lp[mid] <= i) lo = mid;
+        else hi = mid - 1;
+    }
+    const int64_t q = lo;
+    const float d = Dp[(size_t)p * stride + i];
+    const uint32_t key = order_f32(d);
+    int64_t out = lims[q] + (i - lp[q]);
+    for (int o = 0; o < (int)gridDim.y; ++o) {
+        if (o == p) continue;
+        const int64_t* lo_lims = lims_parts + (size_t)o * (nq + 1);
+        const float* Do = Dp + (size_t)o * stride;
+        const int64_t b = lo_lims[q];
+        int64_t a = b, e = lo_lims[q + 1];  // the run of part o is sorted: the entries before this one are a prefix
+        while (a < e) {
+            const int64_t mid = (a + e) >> 1;
+            const uint32_t km = order_f32(Do[mid]);
+            if (o < p ? km >= key : km > key) a = mid + 1;
+            else e = mid;
+        }
+        out += a - b;
+    }
+    D[out] = d;
+    I[out] = Ip[(size_t)p * stride + i];
 }
 
 }  // namespace wb

@@ -221,6 +221,7 @@ class IndexIDMap(Index):
         self.index = index
         self.d = index.d
         self._hd = index._hd
+        self._device = index._device
 
     def add(self, x) -> None:
         raise RuntimeError("add does not make sense with IndexIDMap, use add_with_ids")

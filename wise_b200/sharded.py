@@ -18,6 +18,14 @@ set of a query is the union over ranks, so the same merge applies.
 Filtered search (params=SearchParameters(sel=...)): every rank applies the same selector to its own rows, so the
 candidate set is again the union over ranks and the exchange is unchanged.  A rank whose rows the selector rejects
 entirely contributes padding and still takes part in the exchange.
+
+Range search (range_search / range_search_dev): every rank runs wb_range_search_dev on its rows, leaving its hits on
+its GPU.  One all-gather of [status, count per query] tells every rank every rank's lims; a non-zero status (the local
+call failed) makes every rank raise.  Two all-gathers then move D and I, each padded to the largest rank total (skipped
+when no rank has a hit), and wb_range_merge_dev places every hit at its rank in the merged result: score descending,
+equal scores by (rank, local order) == global insertion position, as on one index.  The payload varies per call from
+nothing to gigabytes, so it goes through torch.distributed, not through the fixed-size peer mailbox, whose sequence
+range search leaves untouched.
 """
 from __future__ import annotations
 
@@ -55,6 +63,50 @@ def _cuda_merge(Dp: torch.Tensor, Ip: torch.Tensor):
     st = torch.cuda.current_stream(Dp.device).cuda_stream
     _capi.check(_capi.lib().wb_merge_topk_dev(Dp.device.index or 0, nq, k, parts, Dp.data_ptr(), Ip.data_ptr(),
                                               D.data_ptr(), I.data_ptr(), st))
+    return D, I
+
+
+def _cuda_local_range_search(index, q: torch.Tensor, thresh: float, nprobe: int, flt=None):
+    """Local range search on the index's GPU (wb_range_search_dev): lims [nq + 1] int64 CPU tensor, D / I on that GPU.
+    Queries elsewhere (host queries of a single process without an NCCL group) are moved there first."""
+    import ctypes as C
+    from . import _capi
+    L = _capi.lib()
+    dev = torch.device("cuda", index._device)
+    q = q.to(dev).contiguous()
+    nq = q.shape[0]
+    lims = torch.zeros(nq + 1, dtype=torch.int64)
+    st = torch.cuda.current_stream(dev).cuda_stream
+    res = C.c_void_p()
+    _capi.check(L.wb_range_search_dev(index._h, flt, nq, q.data_ptr() if nq else None, float(thresh), nprobe,
+                                      lims.data_ptr(), C.byref(res), st))
+    try:
+        total = int(lims[-1])
+        D = torch.empty(total, dtype=torch.float32, device=q.device)
+        I = torch.empty(total, dtype=torch.int64, device=q.device)
+        _capi.check(L.wb_range_result_copy_dev(res, D.data_ptr(), I.data_ptr(), st))
+    finally:
+        # cudaFree waits for the device, so the copies just enqueued on `st` finish before the result's memory goes;
+        # an asynchronous free would need an explicit synchronisation of `st` here
+        L.wb_range_result_free(res)
+    return lims, D, I
+
+
+def _cuda_range_merge(lims_parts: torch.Tensor, Dp: torch.Tensor, Ip: torch.Tensor, lims: torch.Tensor):
+    """lims_parts [parts, nq + 1] and lims [nq + 1] (int64, CPU); Dp, Ip [parts, stride] on the GPU, part p's hits of
+    query q at [lims_parts[p, q], lims_parts[p, q + 1]) of row p -> merged (D, I) (wb_range_merge_dev)."""
+    from . import _capi
+    parts, stride = Dp.shape
+    nq = lims.shape[0] - 1
+    dev = Dp.device
+    lp = lims_parts.to(dev)
+    ld = lims.to(dev)
+    total = int(lims[-1])
+    D = torch.empty(total, dtype=torch.float32, device=dev)
+    I = torch.empty(total, dtype=torch.int64, device=dev)
+    st = torch.cuda.current_stream(dev).cuda_stream
+    _capi.check(_capi.lib().wb_range_merge_dev(dev.index or 0, nq, parts, lp.data_ptr(), stride, Dp.data_ptr(),
+                                               Ip.data_ptr(), ld.data_ptr(), D.data_ptr(), I.data_ptr(), st))
     return D, I
 
 
@@ -121,18 +173,21 @@ class PeerExchange:
 class ShardedIndex:
     """A faiss-like index whose rows live on `world_size` GPUs (this process owns one shard).
 
-    local_search / merge are injectable so the rank arithmetic and the exchange step can be tested
-    on CPU with the gloo backend; the defaults are the CUDA kernels and nothing else.
+    local_search / merge and local_range_search / range_merge are injectable so the rank arithmetic and the exchange
+    steps can be tested on CPU with the gloo backend; the defaults are the CUDA kernels and nothing else.
     """
 
     def __init__(self, local_index, group=None,
-                 local_search: Callable | None = None, merge: Callable | None = None):
+                 local_search: Callable | None = None, merge: Callable | None = None,
+                 local_range_search: Callable | None = None, range_merge: Callable | None = None):
         self.local = local_index
         self.group = group
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self._local_search = local_search or _cuda_local_search
         self._merge = merge or _cuda_merge
+        self._local_range_search = local_range_search or _cuda_local_range_search
+        self._range_merge = range_merge or _cuda_range_merge
         self.d = local_index.d
         # exchange step: "peer" = one fused kernel over NVLink peer memory (default on GPUs),
         # "nccl" = all-gather + merge kernel.  CPU/gloo tests always take the all-gather path.
@@ -202,6 +257,77 @@ class ShardedIndex:
         nprobe = getattr(self.local, "nprobe", 1)
         D, I = self.search_dev(q, int(k), int(nprobe), params)
         return D.cpu().numpy(), I.cpu().numpy()
+
+    def range_search_dev(self, q: torch.Tensor, thresh, nprobe: int = 1, params=None):
+        """q: [nq, d] float32 tensor, replicated on every rank, with the same thresh on every rank.  Returns, on every
+        rank, (lims [nq + 1] int64 CPU tensor, D, I on q's device): exactly the range search of one index holding all
+        rows (score descending, equal scores by global insertion position).  params as in search_dev.  A failure on
+        any rank raises RuntimeError on every rank; no rank is left waiting in a collective."""
+        thresh = float(np.float32(thresh))
+        try:
+            nprobe, flt = self._params(nprobe, params)
+            if flt is None:
+                lims, D, I = self._local_range_search(self.local, q, thresh, nprobe)
+            else:
+                lims, D, I = self._local_range_search(self.local, q, thresh, nprobe, flt)
+            err = None
+        except Exception as e:  # reported through the counts exchange, so that every rank raises
+            if self.world == 1:
+                raise
+            nq = q.shape[0]
+            lims, D, I, err = torch.zeros(nq + 1, dtype=torch.int64), None, None, e
+        if self.world == 1:
+            return lims, D, I
+        nq = lims.shape[0] - 1
+        dev = self._comm_device()
+        # counts: [status, count_0 .. count_{nq-1}] of every rank
+        mine = torch.empty(nq + 1, dtype=torch.int64)
+        mine[0] = 0 if err is None else 1
+        mine[1:] = lims[1:] - lims[:-1]
+        counts = torch.empty(self.world * (nq + 1), dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(counts, mine.to(dev), group=self.group)
+        counts = counts.cpu().view(self.world, nq + 1)
+        failed = torch.nonzero(counts[:, 0]).flatten().tolist()
+        if failed:
+            msg = f"range_search failed on rank(s) {failed}"
+            raise RuntimeError(msg if err is None else f"{msg}: {err}") from err
+        lims_parts = torch.zeros((self.world, nq + 1), dtype=torch.int64)
+        lims_parts[:, 1:] = torch.cumsum(counts[:, 1:], dim=1)
+        merged = lims_parts.sum(dim=0)
+        stride = int(lims_parts[:, -1].max())
+        if stride == 0:
+            return merged, D, I
+        # payload: D and I of every rank, padded to the largest rank total; every rank learns whether all could
+        # allocate the buffers before any of them enters the gathers
+        try:
+            Ds = torch.empty(stride, dtype=D.dtype, device=D.device)
+            Is = torch.empty(stride, dtype=I.dtype, device=I.device)
+            Ds[:D.shape[0]] = D
+            Is[:I.shape[0]] = I
+            Dp = torch.empty(self.world * stride, dtype=D.dtype, device=D.device)
+            Ip = torch.empty(self.world * stride, dtype=I.dtype, device=I.device)
+            ok = 1
+        except RuntimeError:  # torch.OutOfMemoryError
+            Ds = Is = Dp = Ip = None
+            ok = 0
+        flag = torch.tensor([ok], dtype=torch.int64, device=dev)
+        dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
+        if not int(flag.item()):
+            raise RuntimeError(f"range_search: a rank could not allocate the {stride} x {self.world} result exchange")
+        dist.all_gather_into_tensor(Dp, Ds, group=self.group)
+        dist.all_gather_into_tensor(Ip, Is, group=self.group)
+        del Ds, Is
+        D, I = self._range_merge(lims_parts, Dp.view(self.world, stride), Ip.view(self.world, stride), merged)
+        return merged, D, I
+
+    def range_search(self, x: np.ndarray, thresh, params=None):
+        """faiss-style host API: lims (uint64, nq + 1), D, I = sh.range_search(x, thresh), numpy in and out, the same on
+        every rank (see range_search_dev)."""
+        x = np.ascontiguousarray(x, np.float32)
+        q = torch.from_numpy(x).to(self._comm_device())
+        nprobe = int(getattr(self.local, "nprobe", 1))
+        lims, D, I = self.range_search_dev(q, thresh, nprobe, params)
+        return lims.numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
 
 
 def train_ivf_sharded(index, x_local: torch.Tensor, niter: int = 10, seed: int = 1234, group=None, verbose: bool = False):
