@@ -401,33 +401,46 @@ static int plan_scan(const wb_index* h, int64_t nq, int k, bool gather, int npro
     return fail("scan does not fit shared memory (d=%d, k=%d)", h->d, k);
 }
 
-template <int NQ, int RW, bool GATHER>
-static int launch_scan_t(const ScanParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-    CK(smem_optin<scan_topk_kernel<NQ, RW, GATHER>>(232448));
-    scan_topk_kernel<NQ, RW, GATHER><<<grid, kScanThreads, smem, st>>>(p);
+constexpr int kScanSmemOptin = 232448;  // the scan kernels opt in to the most a block may have (227 KB)
+
+// Opt `Kernel` in to the scans' shared memory, launch it on `st` and check the launch.
+template <auto Kernel, class... Args>
+static int launch(dim3 grid, int block, size_t smem, cudaStream_t st, const Args&... args) {
+    CK(smem_optin<Kernel>(kScanSmemOptin));
+    Kernel<<<grid, block, smem, st>>>(args...);
     CK(cudaGetLastError());
     return 0;
 }
 
-template <int NQ, bool GATHER>
-static int launch_scan_rw(int RW, const ScanParams& p, dim3 grid, size_t smem, cudaStream_t st) {
+template <int V>
+using Int = std::integral_constant<int, V>;
+
+// fn(Int<RW>) for the rows per warp of a scan plan: plan_scan picks 4, 2 or 1; anything else runs as 1.
+template <class Fn>
+static auto with_rw(int RW, Fn&& fn) {
     switch (RW) {
-        case 4: return launch_scan_t<NQ, 4, GATHER>(p, grid, smem, st);
-        case 2: return launch_scan_t<NQ, 2, GATHER>(p, grid, smem, st);
-        case 1: return launch_scan_t<NQ, 1, GATHER>(p, grid, smem, st);
+        case 4: return fn(Int<4>{});
+        case 2: return fn(Int<2>{});
+        default: return fn(Int<1>{});
     }
-    return fail("bad RW %d", RW);
 }
 
-// Cooperative launch of the gather kernel (fused coarse quantizer: the CTAs of a query group meet at a barrier, so all
-// of them must be resident - the cooperative launch guarantees it or fails).
-template <int RW>
-static cudaError_t launch_scan_coop_t(const ScanParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-    const cudaError_t e = smem_optin<scan_topk_kernel<1, RW, true>>(232448);
-    if (e != cudaSuccess) return e;
-    void* args[] = {const_cast<ScanParams*>(&p)};
-    return cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(scan_topk_kernel<1, RW, true>), grid,
-                                       dim3(kScanThreads), args, smem, st);
+// fn(Int<NQ>, Int<RW>, std::bool_constant<GATHER>) for the scan kernel instance of a plan: NQ = 1, 2, 4 or 8 queries per
+// CTA over contiguous rows, or one query per CTA over the rows of its probed lists (GATHER).
+template <class Fn>
+static int with_scan_instance(int NQ, int RW, bool gather, Fn&& fn) {
+    auto rw = [&](auto nq, auto g) -> int {
+        if (RW != 4 && RW != 2 && RW != 1) return fail("bad RW %d", RW);
+        return with_rw(RW, [&](auto rw) { return fn(nq, rw, g); });
+    };
+    if (gather) return rw(Int<1>{}, std::true_type{});
+    switch (NQ) {
+        case 1: return rw(Int<1>{}, std::false_type{});
+        case 2: return rw(Int<2>{}, std::false_type{});
+        case 4: return rw(Int<4>{}, std::false_type{});
+        case 8: return rw(Int<8>{}, std::false_type{});
+    }
+    return fail("bad NQ %d", NQ);
 }
 
 static void apply_scan_cfg(const ScanCfg& c, ScanParams& p) {
@@ -440,25 +453,24 @@ static void apply_scan_cfg(const ScanCfg& c, ScanParams& p) {
     p.rank_sort = c.P <= kConsumerThreads;  // measured: slower than bitonic at P = 512
 }
 
+// Cooperative launch of the gather kernel (fused coarse quantizer: the CTAs of a query group meet at a barrier, so all
+// of them must be resident - the cooperative launch guarantees it or fails).
 static cudaError_t launch_scan_coop(const ScanCfg& c, ScanParams& p, dim3 grid, cudaStream_t st) {
     apply_scan_cfg(c, p);
-    switch (c.RW) {
-        case 4: return launch_scan_coop_t<4>(p, grid, c.smem, st);
-        case 2: return launch_scan_coop_t<2>(p, grid, c.smem, st);
-        default: return launch_scan_coop_t<1>(p, grid, c.smem, st);
-    }
+    return with_rw(c.RW, [&](auto RW) {
+        const cudaError_t e = smem_optin<scan_topk_kernel<1, RW, true>>(kScanSmemOptin);
+        if (e != cudaSuccess) return e;
+        void* args[] = {&p};
+        return cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(scan_topk_kernel<1, RW, true>), grid,
+                                           dim3(kScanThreads), args, c.smem, st);
+    });
 }
 
 static int launch_scan(const ScanCfg& c, bool gather, ScanParams& p, dim3 grid, cudaStream_t st) {
     apply_scan_cfg(c, p);
-    if (gather) return launch_scan_rw<1, true>(c.RW, p, grid, c.smem, st);
-    switch (c.NQ) {
-        case 1: return launch_scan_rw<1, false>(c.RW, p, grid, c.smem, st);
-        case 2: return launch_scan_rw<2, false>(c.RW, p, grid, c.smem, st);
-        case 4: return launch_scan_rw<4, false>(c.RW, p, grid, c.smem, st);
-        case 8: return launch_scan_rw<8, false>(c.RW, p, grid, c.smem, st);
-    }
-    return fail("bad NQ %d", c.NQ);
+    return with_scan_instance(c.NQ, c.RW, gather, [&](auto NQ, auto RW, auto G) {
+        return launch<scan_topk_kernel<NQ, RW, G>>(grid, kScanThreads, c.smem, st, p);
+    });
 }
 
 // Sort-buffer size of the merge: everything at once when it is small, else k + a 2048-entry queue.
@@ -544,22 +556,63 @@ struct RowMask {
     const int64_t* sel;
 };
 
+// CTAs per query group of a scan over `nrows` contiguous rows: enough to fill the SMs (twice over when there are
+// several query groups), at most one per row group.
+static int64_t flat_ctas(const wb_index* h, const ScanCfg& c, int64_t nrows, int64_t nq) {
+    const int gr = kConsumerWarps * c.RW;
+    const int64_t ngroups = (nrows + gr - 1) / gr;
+    const int64_t qgroups = (nq + c.NQ - 1) / c.NQ;
+    const int64_t S = std::min<int64_t>(std::max<int64_t>(ngroups, 1),
+                                        std::max<int64_t>(1, ((int64_t)h->sm_count * (qgroups > 1 ? 2 : 1) + qgroups - 1) / qgroups));
+    return std::min<int64_t>(S, (int64_t)h->sm_count);
+}
+
+// CTAs per query of a list scan: the SMs shared out among the queries.
+static int64_t ivf_ctas(const wb_index* h, int64_t nq) {
+    return nq >= h->sm_count ? 1 : std::max<int64_t>(1, (int64_t)h->sm_count / nq);
+}
+
+// The top-k scan launches of `nq` queries (K1, or K5 when `gather`: the probe table is in h->pI), one per <= kMaxGridY
+// query groups of c.NQ, with p.nparts CTAs per group; then the K3 merge of the per-CTA lists unless p.fuse_tail has
+// the kernel's last CTA merge them.  *exchanged tells the caller whether (D, I) already hold the GLOBAL result
+// (written to ex->D / ex->I).
+static int run_scan_groups(wb_index* h, const ScanCfg& c, bool gather, ScanParams& p, int64_t nq, const float* q_ld,
+                           const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed, const ExchParams* ex,
+                           bool* exchanged) {
+    const int64_t qgroups = (nq + c.NQ - 1) / c.NQ;
+    TRY(timing_begin(h, timed && h->timing, st));
+    for (int64_t g0 = 0; g0 < qgroups; g0 += kMaxGridY) {
+        const int64_t gy = std::min(kMaxGridY, qgroups - g0);
+        const int64_t qoff = g0 * c.NQ;
+        p.queries = q_ld + (size_t)qoff * h->ld;
+        p.nq = (int)std::min<int64_t>(nq - qoff, gy * c.NQ);
+        if (gather) p.probes = h->pI.as<int64_t>() + (size_t)qoff * p.nprobe;
+        p.parts = h->parts.as<uint64_t>() + (size_t)qoff * p.nparts * p.k;
+        if (p.fuse_tail) {  // the tail indexes (D, I) and the mailboxes by the query number inside this launch
+            p.D = (ex ? ex->D : D) + (size_t)qoff * p.k;
+            p.I = (ex ? ex->I : I) + (size_t)qoff * p.k;
+            if (ex && qoff != 0) return fail("exchange-fused scans take at most %lld query groups", (long long)kMaxGridY);
+        }
+        TRY(launch_scan(c, gather, p, dim3((unsigned)p.nparts, (unsigned)gy), st));
+        h->launches++;
+    }
+    TRY(timing_end(h, timed && h->timing, st));
+    if (p.fuse_tail) {
+        if (ex && exchanged) *exchanged = true;
+        return 0;
+    }
+    return launch_merge_keys(h, nq, p.k, p.nparts, h->parts.as<uint64_t>(), ids, D, I, st);
+}
+
 // Exhaustive top-k of `nq` device queries (row stride ld) against `nrows` rows: K1 with the K3 merge (and, when `ex`
 // is given, the multi-GPU exchange) fused into its tail; K1 + K3 as two launches when the tail cannot be fused.
-// *exchanged tells the caller whether (D, I) already hold the GLOBAL result (written to ex->D / ex->I).
 static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const float* q_dev, int64_t nq, int k,
                          const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed,
                          const ExchParams* ex = nullptr, bool* exchanged = nullptr, const RowMask* mask = nullptr) {
     if (exchanged) *exchanged = false;
     ScanCfg c;
     TRY(plan_scan(h, nq, k, false, 0, &c));
-    const int gr = kConsumerWarps * c.RW;
-    const int64_t ngroups = (nrows + gr - 1) / gr;
-    const int64_t qgroups_total = (nq + c.NQ - 1) / c.NQ;
-    int64_t S = std::min<int64_t>(std::max<int64_t>(ngroups, 1),
-                                  std::max<int64_t>(1, ((int64_t)h->sm_count * (qgroups_total > 1 ? 2 : 1) +
-                                                        qgroups_total - 1) / qgroups_total));
-    S = std::min<int64_t>(S, (int64_t)h->sm_count);
+    const int64_t S = flat_ctas(h, c, nrows, nq);
     TRY(h->parts.ensure((size_t)nq * S * k * sizeof(uint64_t)));
     ScanParams p{};
     p.rows = rows;
@@ -569,32 +622,11 @@ static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const fl
     p.nparts = (int)S;
     p.allow = mask ? mask->allow : nullptr;
     int S_merge = 0, heads_bytes = 0;
-    const bool fuse = tail_fusable(c, k, S, ex ? ex->world : 1, &S_merge, &heads_bytes);
-    if (fuse) {
+    if (tail_fusable(c, k, S, ex ? ex->world : 1, &S_merge, &heads_bytes)) {
         TRY(ensure_tail_counters(h, st));
         set_tail(p, h, c, S_merge, heads_bytes, ids, ex ? ex->D : D, ex ? ex->I : I, k, ex);
     }
-    TRY(timing_begin(h, timed && h->timing, st));
-    for (int64_t g0 = 0; g0 < qgroups_total; g0 += kMaxGridY) {
-        const int64_t gy = std::min(kMaxGridY, qgroups_total - g0);
-        const int64_t qoff = g0 * c.NQ;
-        p.queries = q_dev + (size_t)qoff * h->ld;
-        p.nq = (int)std::min<int64_t>(nq - qoff, gy * c.NQ);
-        p.parts = h->parts.as<uint64_t>() + (size_t)qoff * S * k;
-        if (fuse) {  // the tail indexes (D, I) and the mailboxes by the query number inside this launch
-            p.D = (ex ? ex->D : D) + (size_t)qoff * k;
-            p.I = (ex ? ex->I : I) + (size_t)qoff * k;
-            if (ex && qoff != 0) return fail("exchange-fused scans take at most %lld query groups", (long long)kMaxGridY);
-        }
-        TRY(launch_scan(c, false, p, dim3((unsigned)S, (unsigned)gy), st));
-        h->launches++;
-    }
-    TRY(timing_end(h, timed && h->timing, st));
-    if (fuse) {
-        if (ex && exchanged) *exchanged = true;
-        return 0;
-    }
-    return launch_merge_keys(h, nq, k, S, h->parts.as<uint64_t>(), ids, D, I, st);
+    return run_scan_groups(h, c, false, p, nq, q_dev, ids, D, I, st, timed, ex, exchanged);
 }
 
 // ---- K2: tensor-core batched scan ---------------------------------------------------------------
@@ -1283,14 +1315,6 @@ extern "C" int wb_ivf_add_preassigned(wb_index* h, int64_t n, const float* x_hos
 }
 
 // ---- K5 for batches: list-major scan (ivf_lm.cuh) ------------------------------------------------------------------
-template <int RW>
-static int launch_lm_t(const LmParams& p, int grid, size_t smem, cudaStream_t st) {
-    CK(smem_optin<ivf_listmajor_kernel<8, RW>>(232448));
-    ivf_listmajor_kernel<8, RW><<<grid, kScanThreads, smem, st>>>(p);
-    CK(cudaGetLastError());
-    return 0;
-}
-
 // Taken when the probes of the batch overlap enough for shared reads to pay (on average every list is probed at
 // least once) and the rows are physically grouped by list.  WB_IVF_LISTMAJOR=0 / 1 forces it off / on.
 static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, int np, float* D, int64_t* I,
@@ -1346,11 +1370,7 @@ static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, 
     p.parts = h->parts.as<uint64_t>();
     TRY(timing_begin(h, h->timing, st));
     const int grid = (int)std::min<int64_t>(h->sm_count, max_items);
-    switch (c.RW) {
-        case 4: TRY(launch_lm_t<4>(p, grid, c.smem, st)); break;
-        case 2: TRY(launch_lm_t<2>(p, grid, c.smem, st)); break;
-        default: TRY(launch_lm_t<1>(p, grid, c.smem, st)); break;
-    }
+    TRY(with_rw(c.RW, [&](auto RW) { return launch<ivf_listmajor_kernel<8, RW>>(grid, kScanThreads, c.smem, st, p); }));
     TRY(timing_end(h, h->timing, st));
     h->launches += 4;
     TRY(launch_merge_keys(h, nq, k, np, h->parts.as<uint64_t>(), h->ids.get(), D, I, st));
@@ -1358,29 +1378,36 @@ static int run_ivf_listmajor(wb_index* h, int64_t nq, const float* q_ld, int k, 
     return 0;
 }
 
-// The query-major list scan: one launch per <= 32768 queries (the probe table is in h->pI), tail merge fused or not.
-static int run_gather_scan(wb_index* h, const ScanCfg& c, ScanParams& p, int64_t S, bool fuse, int64_t nq, const float* q_ld,
-                           int k, int np, float* D, int64_t* I, cudaStream_t st, const ExchParams* ex, bool* exchanged) {
-    TRY(timing_begin(h, h->timing, st));
-    for (int64_t q0 = 0; q0 < nq; q0 += kMaxGridY) {
-        const int64_t gy = std::min(kMaxGridY, nq - q0);
-        p.queries = q_ld + (size_t)q0 * h->ld;
-        p.nq = (int)gy;
-        p.probes = h->pI.as<int64_t>() + (size_t)q0 * np;
-        p.parts = h->parts.as<uint64_t>() + (size_t)q0 * S * k;
-        if (fuse) {
-            p.D = (ex ? ex->D : D) + (size_t)q0 * k;
-            p.I = (ex ? ex->I : I) + (size_t)q0 * k;
-        }
-        TRY(launch_scan(c, true, p, dim3((unsigned)S, (unsigned)gy), st));
-        h->launches++;
+// ---- IVF set-up shared by search and range search ------------------------------------------------------------------
+// The lists to probe per query, nprobe clamped to [1, min(nlist, WB_MAX_K)], and the inverted lists made current.
+// ensure_csr works on the handle's stream, so rows added on `st` are waited for first.
+static int ivf_prepare(wb_index* h, int64_t nprobe, cudaStream_t st, int* np) {
+    *np = (int)std::min<int64_t>(std::max<int64_t>(nprobe, 1), std::min<int64_t>(h->nlist, WB_MAX_K));
+    if (h->csr_dirty) {
+        if (st != h->stream) CK(cudaStreamSynchronize(st));
+        TRY(ensure_csr(h));
     }
-    TRY(timing_end(h, h->timing, st));
-    if (fuse) {
-        if (ex && exchanged) *exchanged = true;
-        return 0;
-    }
-    return launch_merge_keys(h, nq, (int)k, S, h->parts.as<uint64_t>(), h->ids.get(), D, I, st);
+    return 0;
+}
+
+// K4: the coarse quantizer, an exhaustive top-`np` scan of the centroids, into the probe table (h->pD, h->pI).
+static int ivf_probes(wb_index* h, int64_t nq, const float* q_ld, int np, cudaStream_t st) {
+    TRY(h->pD.ensure((size_t)nq * np * sizeof(float)));
+    TRY(h->pI.ensure((size_t)nq * np * sizeof(int64_t)));
+    return run_flat_any(h, h->centroids.get(), h->nlist, q_ld, nq, np, nullptr, h->pD.as<float>(), h->pI.as<int64_t>(), st, false);
+}
+
+// The fields of a K5 list scan that describe the inverted lists; `allow` as in RowMask.
+static ScanParams ivf_scan_params(const wb_index* h, int np, const uint32_t* allow) {
+    ScanParams p{};
+    p.rows = h->rows.get();
+    p.ld = h->ld;
+    p.perm = h->slot_row.get();
+    p.row_pos = h->row_pos.get();
+    p.list_off = h->list_off.get();
+    p.nprobe = np;
+    p.allow = allow;
+    return p;
 }
 
 // ---- filters (faiss SearchParameters.sel): a bitmap over insertion positions, DESIGN.md "Filtered search" ---------
@@ -1490,6 +1517,40 @@ static int check_filter(const wb_index* h, const wb_filter* f) {
     return 0;
 }
 
+// The rows a search scans: without a filter the whole store.  With filter `f`, once it is current: nothing (`none`),
+// the compact copy of its rows (a flat store of which fewer than 1/kSparseCutoffDen are selected, when the copy fits in
+// memory) or the store under its bitmap (`mask`).
+struct RowSel {
+    bool none;
+    const float* rows;
+    int64_t nrows;
+    const int64_t* ids;
+    RowMask mask;  // mask.allow null: every row of `rows`
+    const RowMask* masked() const { return mask.allow ? &mask : nullptr; }
+};
+
+static int select_rows(wb_index* h, wb_filter* f, cudaStream_t st, RowSel* s) {
+    *s = RowSel{false, h->rows.get(), h->n, h->ids.get(), RowMask{}};
+    if (!f) return 0;
+    TRY(filter_current(f, st));
+    if (f->count == 0) {
+        s->none = true;
+        return 0;
+    }
+    if (!h->ivf && f->count * kSparseCutoffDen < h->n) {
+        bool ok = false;
+        TRY(filter_compact(f, &ok));
+        if (ok) {
+            s->rows = f->crows.get();
+            s->nrows = f->count;
+            s->ids = f->cids.get();
+            return 0;
+        }
+    }
+    s->mask = RowMask{f->bits.get(), f->sel.data()};
+    return 0;
+}
+
 // ---- search --------------------------------------------------------------------------------
 constexpr int64_t kIvfFuseCoarseMaxQ = 4;  // largest IVF batch that runs the coarse quantizer inside the list-scan launch
 
@@ -1499,36 +1560,22 @@ static int search_dev_impl(wb_index* h, wb_filter* f, int64_t nq, const float* q
                            bool* exchanged = nullptr) {
     if (exchanged) *exchanged = false;
     if (h->ivf && !h->trained) return fail("IndexIVFFlat is not trained");
-    RowMask mask{};
-    if (f) {
-        TRY(filter_current(f, st));
-        if (f->count == 0) {  // all padding; a sharded search still takes part in the exchange (*exchanged stays false)
-            const int64_t tot = nq * k;
-            pad_results_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(D, I, tot);
-            CK(cudaGetLastError());
-            h->launches++;
-            return 0;
-        }
-        if (!h->ivf && f->count * kSparseCutoffDen < h->n) {
-            bool ok = false;
-            TRY(filter_compact(f, &ok));
-            if (ok)
-                return run_flat_any(h, f->crows.get(), f->count, q_ld, nq, (int)k, f->cids.get(), D, I, st, true, ex,
-                                    exchanged);
-        }
-        mask = RowMask{f->bits.get(), f->sel.data()};
+    RowSel s;
+    TRY(select_rows(h, f, st, &s));
+    if (s.none) {  // all padding; a sharded search still takes part in the exchange (*exchanged stays false)
+        const int64_t tot = nq * k;
+        pad_results_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(D, I, tot);
+        CK(cudaGetLastError());
+        h->launches++;
+        return 0;
     }
-    const RowMask* m = f ? &mask : nullptr;
-    if (!h->ivf) return run_flat_any(h, h->rows.get(), h->n, q_ld, nq, (int)k, h->ids.get(), D, I, st, true, ex, exchanged, m);
-    int np = (int)std::min<int64_t>(std::max<int64_t>(nprobe, 1), std::min<int64_t>(h->nlist, WB_MAX_K));
-    if (h->csr_dirty) {
-        if (st != h->stream) CK(cudaStreamSynchronize(st));
-        TRY(ensure_csr(h));
-    }
+    if (!h->ivf) return run_flat_any(h, s.rows, s.nrows, q_ld, nq, (int)k, s.ids, D, I, st, true, ex, exchanged, s.masked());
+    int np = 0;
+    TRY(ivf_prepare(h, nprobe, st, &np));
     // K5 plan: gather-scan of the probed lists, S CTAs per query
     ScanCfg c;
     TRY(plan_scan(h, 1, (int)k, true, np, &c));
-    int64_t S = nq >= h->sm_count ? 1 : std::max<int64_t>(1, (int64_t)h->sm_count / nq);
+    const int64_t S = ivf_ctas(h, nq);
     if (ex && nq > kMaxGridY) ex = nullptr;
     int S_merge = 0, heads_bytes = 0;
     const bool fuse = tail_fusable(c, (int)k, S, ex ? ex->world : 1, &S_merge, &heads_bytes);
@@ -1539,28 +1586,17 @@ static int search_dev_impl(wb_index* h, wb_filter* f, int64_t nq, const float* q
                        env_int("WB_IVF_FUSE_COARSE", 1) && env_int("WB_IVF_LISTMAJOR", -1) != 1;
     for (int attempt = 0; attempt < 2; ++attempt) {
         if (!fuse_coarse) {
-            // K4: coarse quantizer = exhaustive scan of the centroids, top-nprobe
-            TRY(h->pD.ensure((size_t)nq * np * sizeof(float)));
-            TRY(h->pI.ensure((size_t)nq * np * sizeof(int64_t)));
-            TRY(run_flat_any(h, h->centroids.get(), h->nlist, q_ld, nq, np, nullptr, h->pD.as<float>(), h->pI.as<int64_t>(), st, false));
+            TRY(ivf_probes(h, nq, q_ld, np, st));
             // K5, batches: list-major - the probe table is inverted on the device and every probed list is streamed once
             // per group of 8 of the queries that probe it (ivf_lm.cuh)
             bool done = false;
-            TRY(run_ivf_listmajor(h, nq, q_ld, (int)k, np, D, I, st, mask.allow, &done));
+            TRY(run_ivf_listmajor(h, nq, q_ld, (int)k, np, D, I, st, s.mask.allow, &done));
             if (done) return 0;
         }
         TRY(h->parts.ensure((size_t)nq * S * k * sizeof(uint64_t)));
-        ScanParams p{};
-        p.rows = h->rows.get();
-        p.nrows = 0;
-        p.ld = h->ld;
+        ScanParams p = ivf_scan_params(h, np, s.mask.allow);
         p.k = (int)k;
         p.nparts = (int)S;
-        p.perm = h->slot_row.get();
-        p.row_pos = h->row_pos.get();
-        p.list_off = h->list_off.get();
-        p.nprobe = np;
-        p.allow = mask.allow;
         if (fuse) {
             TRY(ensure_tail_counters(h, st));
             set_tail(p, h, c, S_merge, heads_bytes, h->ids.get(), ex ? ex->D : D, ex ? ex->I : I, (int)k, ex);
@@ -1589,11 +1625,173 @@ static int search_dev_impl(wb_index* h, wb_filter* f, int64_t nq, const float* q
             if (ex && exchanged) *exchanged = true;
             return 0;
         }
-        return run_gather_scan(h, c, p, S, fuse, nq, q_ld, (int)k, np, D, I, st, ex, exchanged);
+        return run_scan_groups(h, c, true, p, nq, q_ld, h->ids.get(), D, I, st, true, ex, exchanged);
     }
     return fail("unreachable");
 }
 
+// ---- multi-GPU exchange over peer memory ----------------------------------------------------------
+struct wb_exchange {
+    int device = 0, rank = 0, world = 1;
+    size_t region_bytes = 0, flags_bytes = 0, cap_entries = 0, nq_cap = 0, total_bytes = 0;
+    DevPtr<unsigned char> local;
+    unsigned char* peers[kExchMaxWorld] = {};
+    bool opened[kExchMaxWorld] = {};
+    uint32_t seq = 0;       // sequence number of the last exchange that was LAUNCHED (all ranks advance in lockstep)
+    PinPtr<int> status;     // pinned (device-visible) host word raised by a kernel whose wait for the peers timed out
+    int64_t launches = 0;   // exchange_merge_kernel launches (the fused path needs none)
+};
+
+extern "C" int wb_exch_create(int device, int rank, int world, int64_t max_queries, int64_t max_entries,
+                              wb_exchange** out) {
+    if (!out) return fail("out is NULL");
+    *out = nullptr;
+    if (world < 1 || world > kExchMaxWorld || rank < 0 || rank >= world) return fail("bad rank/world %d/%d", rank, world);
+    if (max_queries < 1 || max_entries < max_queries) return fail("bad exchange capacity");
+    CK(cudaSetDevice(device));
+    std::unique_ptr<wb_exchange> ex(new wb_exchange());
+    ex->device = device;
+    ex->rank = rank;
+    ex->world = world;
+    ex->nq_cap = (size_t)max_queries;
+    ex->cap_entries = ((size_t)max_entries + 3) & ~(size_t)3;
+    ex->flags_bytes = ((size_t)max_queries * 4 + 255) & ~(size_t)255;
+    ex->region_bytes = (ex->flags_bytes + ex->cap_entries * 12 + 255) & ~(size_t)255;
+    ex->total_bytes = ex->region_bytes * 2 * world;
+    CK(dev_alloc(&ex->local, ex->total_bytes));
+    CK(cudaMemset(ex->local.get(), 0, ex->total_bytes));
+    int* status = nullptr;
+    CK(cudaHostAlloc(&status, sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
+    ex->status.reset(status);
+    *status = 0;
+    CK(cudaDeviceSynchronize());
+    ex->peers[rank] = ex->local.get();
+    *out = ex.release();
+    return 0;
+}
+
+extern "C" int wb_exch_local_handle(wb_exchange* ex, void* handle64) {
+    if (!ex || !handle64) return fail("NULL argument");
+    CK(cudaSetDevice(ex->device));
+    static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
+    cudaIpcMemHandle_t hnd;
+    CK(cudaIpcGetMemHandle(&hnd, ex->local.get()));
+    memcpy(handle64, &hnd, 64);
+    return 0;
+}
+
+extern "C" int wb_exch_open_peers(wb_exchange* ex, const void* handles /* [world][64] */) {
+    if (!ex || !handles) return fail("NULL argument");
+    CK(cudaSetDevice(ex->device));
+    for (int r = 0; r < ex->world; ++r) {
+        if (r == ex->rank) continue;
+        cudaIpcMemHandle_t hnd;
+        memcpy(&hnd, (const char*)handles + (size_t)r * 64, 64);
+        void* ptr = nullptr;
+        CK(cudaIpcOpenMemHandle(&ptr, hnd, cudaIpcMemLazyEnablePeerAccess));
+        ex->peers[r] = (unsigned char*)ptr;
+        ex->opened[r] = true;
+    }
+    return 0;
+}
+
+extern "C" int wb_exch_free(wb_exchange* ex) {
+    if (!ex) return 0;
+    cudaSetDevice(ex->device);
+    cudaDeviceSynchronize();
+    for (int r = 0; r < ex->world; ++r)
+        if (ex->opened[r]) cudaIpcCloseMemHandle(ex->peers[r]);
+    delete ex;
+    return 0;
+}
+
+// Parameters of the NEXT exchange (sequence number ex->seq + 1).  The caller commits the sequence number with
+// exch_commit() only after the kernel that carries these parameters has been launched successfully: a rank whose
+// launch failed must not drift out of lockstep with its peers.
+static int exch_prepare(wb_exchange* ex, int64_t nq, int64_t k, float* D_dev, int64_t* I_dev, ExchParams* out) {
+    if (!ex) return fail("NULL exchange");
+    if (k < 1 || k > WB_MAX_K) return fail("k=%lld out of range [1, %d]", (long long)k, WB_MAX_K);
+    if (nq < 1 || (size_t)nq > ex->nq_cap || (size_t)(nq * k) > ex->cap_entries)
+        return fail("exchange capacity exceeded (nq=%lld, k=%lld)", (long long)nq, (long long)k);
+    for (int r = 0; r < ex->world; ++r)
+        if (!ex->peers[r]) return fail("peer %d is not mapped: call wb_exch_open_peers first", r);
+    ExchParams p{};
+    p.rank = ex->rank;
+    p.world = ex->world;
+    p.nq = nq;
+    p.k = (int)k;
+    p.S = merge_buffer_entries((int)k, ex->world);
+    p.seq = ex->seq + 1;
+    if (p.seq == 0) p.seq = 1;
+    for (int r = 0; r < ex->world; ++r) p.mailbox[r] = ex->peers[r];
+    p.region_bytes = ex->region_bytes;
+    p.flags_bytes = ex->flags_bytes;
+    p.cap_entries = ex->cap_entries;
+    p.D = D_dev;
+    p.I = I_dev;
+    p.status = ex->status.get();
+    *out = p;
+    return 0;
+}
+static void exch_commit(wb_exchange* ex, const ExchParams& p) { ex->seq = p.seq; }
+
+static int launch_exchange_kernel(wb_exchange* ex, ExchParams& p, const float* D_local, const int64_t* I_local,
+                                  cudaStream_t st) {
+    p.D_local = D_local;
+    p.I_local = I_local;
+    p.S = merge_buffer_entries(p.k, p.world);
+    CK(smem_optin<exchange_merge_kernel>(8192 * 8));
+    int sms = 148;
+    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ex->device));
+    const unsigned grid = (unsigned)std::min<int64_t>(p.nq, sms);  // one resident CTA per SM at most (1024 threads)
+    exchange_merge_kernel<<<grid, kMergeThreads, (size_t)p.S * 8, st>>>(p);
+    CK(cudaGetLastError());
+    exch_commit(ex, p);
+    ex->launches++;
+    return 0;
+}
+
+// Global top-k from this rank's local (D, I): one kernel does the NVLink exchange and the merge.
+// Every rank must call this the same number of times with the same nq and k.
+extern "C" int wb_exch_merge_dev(wb_exchange* ex, int64_t nq, int64_t k, const float* D_local_dev,
+                                 const int64_t* I_local_dev, float* D_dev, int64_t* I_dev, void* stream) {
+    ExchParams p;
+    TRY(exch_prepare(ex, nq, k, D_dev, I_dev, &p));
+    CK(cudaSetDevice(ex->device));
+    return launch_exchange_kernel(ex, p, D_local_dev, I_local_dev, (cudaStream_t)stream);
+}
+
+// 1 when a kernel of this exchange gave up waiting for a peer (a rank that never launched): the results of that
+// search are invalid.  The word lives in pinned host memory that the kernels write through; it is current for every
+// kernel the caller has synchronised with.
+extern "C" int64_t wb_exch_launch_count(const wb_exchange* ex) { return ex ? ex->launches : -1; }
+
+extern "C" int wb_exch_status(wb_exchange* ex, int* timed_out) {
+    if (!ex || !timed_out) return fail("NULL argument");
+    *timed_out = *reinterpret_cast<volatile int*>(ex->status.get());
+    return 0;
+}
+
+// Search over a row-sharded index, device buffers: local search + NVLink exchange + merge.  Batches that run the
+// scan kernel (flat batch <= 4, every IVF list scan) do all of it in ONE launch (scan.cuh, fused tail); the others
+// run the local search and then exchange_merge_kernel.  Every rank calls it with the same queries.
+static int exch_search_dev_impl(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_ld, int64_t k,
+                                int64_t nprobe, float* D_dev, int64_t* I_dev, cudaStream_t st) {
+    if (ex->device != h->device) return fail("index and exchange live on different devices");
+    ExchParams p;
+    TRY(exch_prepare(ex, nq, k, D_dev, I_dev, &p));
+    TRY(h->dbuf.ensure((size_t)nq * k * sizeof(float)));
+    TRY(h->ibuf.ensure((size_t)nq * k * sizeof(int64_t)));
+    bool exchanged = false;
+    TRY(search_dev_impl(h, f, nq, q_ld, k, nprobe, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st, &p, &exchanged));
+    if (exchanged) {
+        exch_commit(ex, p);
+        return 0;
+    }
+    return launch_exchange_kernel(ex, p, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st);
+}
+
+// ---- search entry points -------------------------------------------------------------------
 static int check_search_args(const wb_index* h, int64_t nq, const void* q, int64_t k, const void* D, const void* I) {
     if (!h) return fail("NULL index");
     if (nq < 0) return fail("negative nq");
@@ -1685,8 +1883,10 @@ static int search_to_host(wb_index* h, int64_t nq, int64_t k, DevBuf& D_dev, Dev
     return fetch_results(h, nq, k, D_dev.as<float>(), I_dev.as<int64_t>(), D_host, I_host, st);
 }
 
-static int search_dev_entry(wb_index* h, wb_filter* f, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
-                            float* D_dev, int64_t* I_dev, void* stream) {
+// With an exchange `ex` (may be null) the search runs over a row-sharded index: every rank calls it with the same
+// queries, and (D, I) receive the global result.
+static int search_dev_entry(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_dev, int64_t k,
+                            int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream) {
     TRY(check_search_args(h, nq, q_dev, k, D_dev, I_dev));
     TRY(check_filter(h, f));
     if (nq == 0) return 0;
@@ -1694,11 +1894,14 @@ static int search_dev_entry(wb_index* h, wb_filter* f, int64_t nq, const float* 
     cudaStream_t st = (cudaStream_t)stream;
     const float* q = nullptr;
     TRY(stage_queries(h, nq, q_dev, false, st, &q));
+    if (ex) return exch_search_dev_impl(h, ex, f, nq, q, k, nprobe, D_dev, I_dev, st);
     return search_dev_impl(h, f, nq, q, k, nprobe, D_dev, I_dev, st);
 }
 
-static int search_host_entry(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
-                             float* D_host, int64_t* I_host) {
+// Host buffers: H2D of the queries, the search (with `ex`: local search, NVLink exchange + merge), D2H of (D, I) - one
+// call, one stream, one synchronisation.
+static int search_host_entry(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_host, int64_t k,
+                             int64_t nprobe, float* D_host, int64_t* I_host) {
     TRY(check_search_args(h, nq, q_host, k, D_host, I_host));
     TRY(check_filter(h, f));
     if (nq == 0) return 0;
@@ -1706,26 +1909,51 @@ static int search_host_entry(wb_index* h, wb_filter* f, int64_t nq, const float*
     cudaStream_t st = h->stream;
     const float* q = nullptr;
     TRY(stage_queries(h, nq, q_host, true, st, &q));
-    return search_to_host(h, nq, k, h->dbuf, h->ibuf, D_host, I_host, st, [&](float* D, int64_t* I) {
-        return search_dev_impl(h, f, nq, q, k, nprobe, D, I, st);
-    });
+    if (!ex)
+        return search_to_host(h, nq, k, h->dbuf, h->ibuf, D_host, I_host, st, [&](float* D, int64_t* I) {
+            return search_dev_impl(h, f, nq, q, k, nprobe, D, I, st);
+        });
+    // (eD, eI): exch_search_dev_impl keeps this rank's local results in (dbuf, ibuf)
+    TRY(search_to_host(h, nq, k, h->eD, h->eI, D_host, I_host, st, [&](float* D, int64_t* I) {
+        return exch_search_dev_impl(h, ex, f, nq, q, k, nprobe, D, I, st);
+    }));
+    if (*reinterpret_cast<volatile int*>(ex->status.get())) return fail("sharded search: a peer GPU did not join the exchange within 20 s (results invalid)");
+    return 0;
 }
 
 extern "C" int wb_search_dev(wb_index* h, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe, float* D_dev,
                              int64_t* I_dev, void* stream) {
-    return search_dev_entry(h, nullptr, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
+    return wb_search_filtered_dev(h, nullptr, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
 }
 extern "C" int wb_search(wb_index* h, int64_t nq, const float* q_host, int64_t k, int64_t nprobe, float* D_host,
                          int64_t* I_host) {
-    return search_host_entry(h, nullptr, nq, q_host, k, nprobe, D_host, I_host);
+    return wb_search_filtered(h, nullptr, nq, q_host, k, nprobe, D_host, I_host);
 }
 extern "C" int wb_search_filtered_dev(wb_index* h, wb_filter* f, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
                                       float* D_dev, int64_t* I_dev, void* stream) {
-    return search_dev_entry(h, f, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
+    return search_dev_entry(h, nullptr, f, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
 }
 extern "C" int wb_search_filtered(wb_index* h, wb_filter* f, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
                                   float* D_host, int64_t* I_host) {
-    return search_host_entry(h, f, nq, q_host, k, nprobe, D_host, I_host);
+    return search_host_entry(h, nullptr, f, nq, q_host, k, nprobe, D_host, I_host);
+}
+extern "C" int wb_exch_search_dev(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
+                                  float* D_dev, int64_t* I_dev, void* stream) {
+    return wb_exch_search_filtered_dev(h, ex, nullptr, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
+}
+extern "C" int wb_exch_search(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
+                              float* D_host, int64_t* I_host) {
+    return wb_exch_search_filtered(h, ex, nullptr, nq, q_host, k, nprobe, D_host, I_host);
+}
+extern "C" int wb_exch_search_filtered_dev(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_dev,
+                                           int64_t k, int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream) {
+    if (!ex) return fail("NULL exchange");
+    return search_dev_entry(h, ex, f, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
+}
+extern "C" int wb_exch_search_filtered(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_host,
+                                       int64_t k, int64_t nprobe, float* D_host, int64_t* I_host) {
+    if (!ex) return fail("NULL exchange");
+    return search_host_entry(h, ex, f, nq, q_host, k, nprobe, D_host, I_host);
 }
 
 // ---- range search (DESIGN.md "Range search") --------------------------------------------------------------------
@@ -1746,28 +1974,10 @@ struct wb_range_result {
 constexpr int64_t kRangeMaxQ = 32768;  // queries per chunk: one launch (grid.y) per scan
 constexpr int kRangeStage = 256;       // staged hits per query and CTA in the range scan (P of its shared lists)
 
-template <int NQ, int RW, bool GATHER>
-static int launch_range_t(const ScanParams& p, const RangeOut& ro, dim3 grid, size_t smem, cudaStream_t st) {
-    CK(smem_optin<scan_range_kernel<NQ, RW, GATHER>>(232448));
-    scan_range_kernel<NQ, RW, GATHER><<<grid, kScanThreads, smem, st>>>(p, ro);
-    CK(cudaGetLastError());
-    return 0;
-}
-
-template <int NQ, bool GATHER>
-static int launch_range_rw(int RW, const ScanParams& p, const RangeOut& ro, dim3 grid, size_t smem, cudaStream_t st) {
-    switch (RW) {
-        case 4: return launch_range_t<NQ, 4, GATHER>(p, ro, grid, smem, st);
-        case 2: return launch_range_t<NQ, 2, GATHER>(p, ro, grid, smem, st);
-        case 1: return launch_range_t<NQ, 1, GATHER>(p, ro, grid, smem, st);
-    }
-    return fail("bad RW %d", RW);
-}
-
 // K1 / K5 in range mode: `S` CTAs per query group, one launch per <= kMaxGridY groups.  Whole-row stages draw their
 // row groups from the shared dispensers, which every launch leaves at zero as the fused tails do.
 static int run_range_scan(wb_index* h, const ScanCfg& c, bool gather, ScanParams& p, int64_t S, int64_t nq,
-                          const float* q_ld, int np, const RangeOut& ro0, cudaStream_t st) {
+                          const float* q_ld, const RangeOut& ro0, cudaStream_t st) {
     apply_scan_cfg(c, p);
     p.k = 0;
     p.nparts = (int)S;
@@ -1779,17 +1989,14 @@ static int run_range_scan(wb_index* h, const ScanCfg& c, bool gather, ScanParams
         const int64_t gy = std::min(kMaxGridY, qgroups - g0), qoff = g0 * c.NQ;
         p.queries = q_ld + (size_t)qoff * h->ld;
         p.nq = (int)std::min<int64_t>(nq - qoff, gy * c.NQ);
-        if (gather) p.probes = h->pI.as<int64_t>() + (size_t)qoff * np;
+        if (gather) p.probes = h->pI.as<int64_t>() + (size_t)qoff * p.nprobe;
         RangeOut ro = ro0;
         ro.count += qoff;
         ro.qbase = (int)qoff;
         const dim3 grid((unsigned)S, (unsigned)gy);
-        const int rc = gather      ? launch_range_rw<1, true>(c.RW, p, ro, grid, c.smem, st)
-                       : c.NQ == 1 ? launch_range_rw<1, false>(c.RW, p, ro, grid, c.smem, st)
-                       : c.NQ == 2 ? launch_range_rw<2, false>(c.RW, p, ro, grid, c.smem, st)
-                       : c.NQ == 4 ? launch_range_rw<4, false>(c.RW, p, ro, grid, c.smem, st)
-                                   : launch_range_rw<8, false>(c.RW, p, ro, grid, c.smem, st);
-        TRY(rc);
+        TRY(with_scan_instance(c.NQ, c.RW, gather, [&](auto NQ, auto RW, auto G) {
+            return launch<scan_range_kernel<NQ, RW, G>>(grid, kScanThreads, c.smem, st, p, ro);
+        }));
         h->launches++;
         if (p.group_count) CK(cudaMemsetAsync(p.group_count, 0, (size_t)gy * sizeof(unsigned int), st));
     }
@@ -1810,37 +2017,22 @@ static int range_flat(wb_index* h, const float* rows, int64_t nrows, const float
     }
     ScanCfg c;
     TRY(plan_scan(h, nq, kRangeStage - kMinQueue, false, 0, &c));
-    const int64_t ngroups = (nrows + kConsumerWarps * c.RW - 1) / (kConsumerWarps * c.RW);
-    const int64_t qgroups = (nq + c.NQ - 1) / c.NQ;
-    int64_t S = std::min<int64_t>(std::max<int64_t>(ngroups, 1),
-                                  std::max<int64_t>(1, ((int64_t)h->sm_count * (qgroups > 1 ? 2 : 1) + qgroups - 1) / qgroups));
-    S = std::min<int64_t>(S, (int64_t)h->sm_count);
     ScanParams p{};
     p.rows = rows;
     p.nrows = nrows;
     p.ld = h->ld;
     p.allow = mask ? mask->allow : nullptr;
-    return run_range_scan(h, c, false, p, S, nq, q_ld, 0, ro, st);
+    return run_range_scan(h, c, false, p, flat_ctas(h, c, nrows, nq), nq, q_ld, ro, st);
 }
 
 // IVF range hits: K4 picks the probes exactly as search does, then K5 scans them query-major in range mode.
 static int range_ivf(wb_index* h, int64_t nq, const float* q_ld, int np, const uint32_t* allow, const RangeOut& ro,
                      cudaStream_t st) {
-    TRY(h->pD.ensure((size_t)nq * np * sizeof(float)));
-    TRY(h->pI.ensure((size_t)nq * np * sizeof(int64_t)));
-    TRY(run_flat_any(h, h->centroids.get(), h->nlist, q_ld, nq, np, nullptr, h->pD.as<float>(), h->pI.as<int64_t>(), st, false));
+    TRY(ivf_probes(h, nq, q_ld, np, st));
     ScanCfg c;
     TRY(plan_scan(h, 1, kRangeStage - kMinQueue, true, np, &c));
-    const int64_t S = nq >= h->sm_count ? 1 : std::max<int64_t>(1, (int64_t)h->sm_count / nq);
-    ScanParams p{};
-    p.rows = h->rows.get();
-    p.ld = h->ld;
-    p.perm = h->slot_row.get();
-    p.row_pos = h->row_pos.get();
-    p.list_off = h->list_off.get();
-    p.nprobe = np;
-    p.allow = allow;
-    return run_range_scan(h, c, true, p, S, nq, q_ld, np, ro, st);
+    ScanParams p = ivf_scan_params(h, np, allow);
+    return run_range_scan(h, c, true, p, ivf_ctas(h, nq), nq, q_ld, ro, st);
 }
 
 // Sort the `total` pooled hits of a chunk by query and key, emit them as (D, I) and append them to `res`: a host result
@@ -1923,31 +2115,11 @@ static int range_search_impl(wb_index* h, wb_filter* f, int64_t nq, const float*
     if (h->ivf && !h->trained) return fail("IndexIVFFlat is not trained");
     for (int64_t i = 0; i <= nq; ++i) lims[i] = 0;
     if (nq == 0 || h->n == 0) return 0;
-    // the rows to search, as search_dev_impl picks them
-    const float* rows = h->rows.get();
-    int64_t nrows = h->n;
-    const int64_t* ids = h->ids.get();
-    RowMask mask{};
-    const RowMask* m = nullptr;
-    if (f) {
-        TRY(filter_current(f, st));
-        if (f->count == 0) return 0;
-        bool compact = false;
-        if (!h->ivf && f->count * kSparseCutoffDen < h->n) TRY(filter_compact(f, &compact));
-        if (compact) {
-            rows = f->crows.get();
-            nrows = f->count;
-            ids = f->cids.get();
-        } else {
-            mask = RowMask{f->bits.get(), f->sel.data()};
-            m = &mask;
-        }
-    }
-    const int np = (int)std::min<int64_t>(std::max<int64_t>(nprobe, 1), std::min<int64_t>(h->nlist, WB_MAX_K));
-    if (h->ivf && h->csr_dirty) {
-        if (st != h->stream) CK(cudaStreamSynchronize(st));  // ensure_csr runs on h->stream: rows added on `st` first
-        TRY(ensure_csr(h));
-    }
+    RowSel s;
+    TRY(select_rows(h, f, st, &s));
+    if (s.none) return 0;
+    int np = 0;
+    if (h->ivf) TRY(ivf_prepare(h, nprobe, st, &np));
     TRY(h->rstate.ensure((size_t)(1 + kRangeMaxQ) * sizeof(unsigned long long)));
     unsigned long long* cursor = h->rstate.as<unsigned long long>();
     std::vector<unsigned long long> cnt((size_t)(1 + kRangeMaxQ));
@@ -1961,8 +2133,8 @@ static int range_search_impl(wb_index* h, wb_filter* f, int64_t nq, const float*
             const RangeOut ro{thresh, cursor, cursor + 1, h->rpool.as<uint64_t>(), h->rqid.as<uint32_t>(),
                               (int64_t)(h->rpool.cap / sizeof(uint64_t)), 0};
             CK(cudaMemsetAsync(cursor, 0, (size_t)(1 + nqc) * sizeof(unsigned long long), st));
-            if (h->ivf) TRY(range_ivf(h, nqc, qc, np, m ? m->allow : nullptr, ro, st));
-            else TRY(range_flat(h, rows, nrows, qc, nqc, m, ro, st));
+            if (h->ivf) TRY(range_ivf(h, nqc, qc, np, s.mask.allow, ro, st));
+            else TRY(range_flat(h, s.rows, s.nrows, qc, nqc, s.masked(), ro, st));
             CK(cudaMemcpyAsync(cnt.data(), cursor, (size_t)(1 + nqc) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
             int64_t total = (int64_t)cnt[0];
@@ -1983,7 +2155,7 @@ static int range_search_impl(wb_index* h, wb_filter* f, int64_t nq, const float*
         std::vector<int64_t> off((size_t)nqc + 1, 0);
         for (int64_t i = 0; i < nqc; ++i) off[i + 1] = off[i] + (int64_t)cnt[1 + i];
         for (int64_t i = 1; i <= nqc; ++i) lims[q0 + i] = lims[q0] + off[i];
-        TRY(range_assemble(h, nqc, off, ids, res, st));
+        TRY(range_assemble(h, nqc, off, s.ids, res, st));
         q0 += nqc;
     }
     return 0;
@@ -2554,148 +2726,6 @@ extern "C" int wb_tf32_peak(int device, int iters, int reps, double* tflops_burs
     return 0;
 }
 
-// ---- multi-GPU exchange over peer memory ----------------------------------------------------------
-struct wb_exchange {
-    int device = 0, rank = 0, world = 1;
-    size_t region_bytes = 0, flags_bytes = 0, cap_entries = 0, nq_cap = 0, total_bytes = 0;
-    DevPtr<unsigned char> local;
-    unsigned char* peers[kExchMaxWorld] = {};
-    bool opened[kExchMaxWorld] = {};
-    uint32_t seq = 0;       // sequence number of the last exchange that was LAUNCHED (all ranks advance in lockstep)
-    PinPtr<int> status;     // pinned (device-visible) host word raised by a kernel whose wait for the peers timed out
-    int64_t launches = 0;   // exchange_merge_kernel launches (the fused path needs none)
-};
-
-extern "C" int wb_exch_create(int device, int rank, int world, int64_t max_queries, int64_t max_entries,
-                              wb_exchange** out) {
-    if (!out) return fail("out is NULL");
-    *out = nullptr;
-    if (world < 1 || world > kExchMaxWorld || rank < 0 || rank >= world) return fail("bad rank/world %d/%d", rank, world);
-    if (max_queries < 1 || max_entries < max_queries) return fail("bad exchange capacity");
-    CK(cudaSetDevice(device));
-    std::unique_ptr<wb_exchange> ex(new wb_exchange());
-    ex->device = device;
-    ex->rank = rank;
-    ex->world = world;
-    ex->nq_cap = (size_t)max_queries;
-    ex->cap_entries = ((size_t)max_entries + 3) & ~(size_t)3;
-    ex->flags_bytes = ((size_t)max_queries * 4 + 255) & ~(size_t)255;
-    ex->region_bytes = (ex->flags_bytes + ex->cap_entries * 12 + 255) & ~(size_t)255;
-    ex->total_bytes = ex->region_bytes * 2 * world;
-    CK(dev_alloc(&ex->local, ex->total_bytes));
-    CK(cudaMemset(ex->local.get(), 0, ex->total_bytes));
-    int* status = nullptr;
-    CK(cudaHostAlloc(&status, sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
-    ex->status.reset(status);
-    *status = 0;
-    CK(cudaDeviceSynchronize());
-    ex->peers[rank] = ex->local.get();
-    *out = ex.release();
-    return 0;
-}
-
-extern "C" int wb_exch_local_handle(wb_exchange* ex, void* handle64) {
-    if (!ex || !handle64) return fail("NULL argument");
-    CK(cudaSetDevice(ex->device));
-    static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
-    cudaIpcMemHandle_t hnd;
-    CK(cudaIpcGetMemHandle(&hnd, ex->local.get()));
-    memcpy(handle64, &hnd, 64);
-    return 0;
-}
-
-extern "C" int wb_exch_open_peers(wb_exchange* ex, const void* handles /* [world][64] */) {
-    if (!ex || !handles) return fail("NULL argument");
-    CK(cudaSetDevice(ex->device));
-    for (int r = 0; r < ex->world; ++r) {
-        if (r == ex->rank) continue;
-        cudaIpcMemHandle_t hnd;
-        memcpy(&hnd, (const char*)handles + (size_t)r * 64, 64);
-        void* ptr = nullptr;
-        CK(cudaIpcOpenMemHandle(&ptr, hnd, cudaIpcMemLazyEnablePeerAccess));
-        ex->peers[r] = (unsigned char*)ptr;
-        ex->opened[r] = true;
-    }
-    return 0;
-}
-
-extern "C" int wb_exch_free(wb_exchange* ex) {
-    if (!ex) return 0;
-    cudaSetDevice(ex->device);
-    cudaDeviceSynchronize();
-    for (int r = 0; r < ex->world; ++r)
-        if (ex->opened[r]) cudaIpcCloseMemHandle(ex->peers[r]);
-    delete ex;
-    return 0;
-}
-
-// Parameters of the NEXT exchange (sequence number ex->seq + 1).  The caller commits the sequence number with
-// exch_commit() only after the kernel that carries these parameters has been launched successfully: a rank whose
-// launch failed must not drift out of lockstep with its peers.
-static int exch_prepare(wb_exchange* ex, int64_t nq, int64_t k, float* D_dev, int64_t* I_dev, ExchParams* out) {
-    if (!ex) return fail("NULL exchange");
-    if (k < 1 || k > WB_MAX_K) return fail("k=%lld out of range [1, %d]", (long long)k, WB_MAX_K);
-    if (nq < 1 || (size_t)nq > ex->nq_cap || (size_t)(nq * k) > ex->cap_entries)
-        return fail("exchange capacity exceeded (nq=%lld, k=%lld)", (long long)nq, (long long)k);
-    for (int r = 0; r < ex->world; ++r)
-        if (!ex->peers[r]) return fail("peer %d is not mapped: call wb_exch_open_peers first", r);
-    ExchParams p{};
-    p.rank = ex->rank;
-    p.world = ex->world;
-    p.nq = nq;
-    p.k = (int)k;
-    p.S = merge_buffer_entries((int)k, ex->world);
-    p.seq = ex->seq + 1;
-    if (p.seq == 0) p.seq = 1;
-    for (int r = 0; r < ex->world; ++r) p.mailbox[r] = ex->peers[r];
-    p.region_bytes = ex->region_bytes;
-    p.flags_bytes = ex->flags_bytes;
-    p.cap_entries = ex->cap_entries;
-    p.D = D_dev;
-    p.I = I_dev;
-    p.status = ex->status.get();
-    *out = p;
-    return 0;
-}
-static void exch_commit(wb_exchange* ex, const ExchParams& p) { ex->seq = p.seq; }
-
-static int launch_exchange_kernel(wb_exchange* ex, ExchParams& p, const float* D_local, const int64_t* I_local,
-                                  cudaStream_t st) {
-    p.D_local = D_local;
-    p.I_local = I_local;
-    p.S = merge_buffer_entries(p.k, p.world);
-    CK(smem_optin<exchange_merge_kernel>(8192 * 8));
-    int sms = 148;
-    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ex->device));
-    const unsigned grid = (unsigned)std::min<int64_t>(p.nq, sms);  // one resident CTA per SM at most (1024 threads)
-    exchange_merge_kernel<<<grid, kMergeThreads, (size_t)p.S * 8, st>>>(p);
-    CK(cudaGetLastError());
-    exch_commit(ex, p);
-    ex->launches++;
-    return 0;
-}
-
-// Global top-k from this rank's local (D, I): one kernel does the NVLink exchange and the merge.
-// Every rank must call this the same number of times with the same nq and k.
-extern "C" int wb_exch_merge_dev(wb_exchange* ex, int64_t nq, int64_t k, const float* D_local_dev,
-                                 const int64_t* I_local_dev, float* D_dev, int64_t* I_dev, void* stream) {
-    ExchParams p;
-    TRY(exch_prepare(ex, nq, k, D_dev, I_dev, &p));
-    CK(cudaSetDevice(ex->device));
-    return launch_exchange_kernel(ex, p, D_local_dev, I_local_dev, (cudaStream_t)stream);
-}
-
-// 1 when a kernel of this exchange gave up waiting for a peer (a rank that never launched): the results of that
-// search are invalid.  The word lives in pinned host memory that the kernels write through; it is current for every
-// kernel the caller has synchronised with.
-extern "C" int64_t wb_exch_launch_count(const wb_exchange* ex) { return ex ? ex->launches : -1; }
-
-extern "C" int wb_exch_status(wb_exchange* ex, int* timed_out) {
-    if (!ex || !timed_out) return fail("NULL argument");
-    *timed_out = *reinterpret_cast<volatile int*>(ex->status.get());
-    return 0;
-}
-
 // ---- FeatureStore fast ingest (host only) ------------------------------------------------------------
 // Count the feature rows of one WebdatasetStore shard and report their dimension.
 extern "C" int wb_tar_scan(const char* path, int64_t* rows_out, int64_t* members_out, int64_t* d_out) {
@@ -2770,72 +2800,4 @@ extern "C" int wb_tar_read(const char* path, int64_t d, int64_t cap, int64_t* id
     if (rc) return fail("wb_tar_read(%s): %s (code %d)", path, why.c_str(), rc), rc + 1;
     *rows_out = n;
     return 0;
-}
-
-// Search over a row-sharded index, device buffers: local search + NVLink exchange + merge.  Batches that run the
-// scan kernel (flat batch <= 4, every IVF list scan) do all of it in ONE launch (scan.cuh, fused tail); the others
-// run the local search and then exchange_merge_kernel.  Every rank calls it with the same queries.
-static int exch_search_dev_impl(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_ld, int64_t k,
-                                int64_t nprobe, float* D_dev, int64_t* I_dev, cudaStream_t st) {
-    if (ex->device != h->device) return fail("index and exchange live on different devices");
-    ExchParams p;
-    TRY(exch_prepare(ex, nq, k, D_dev, I_dev, &p));
-    TRY(h->dbuf.ensure((size_t)nq * k * sizeof(float)));
-    TRY(h->ibuf.ensure((size_t)nq * k * sizeof(int64_t)));
-    bool exchanged = false;
-    TRY(search_dev_impl(h, f, nq, q_ld, k, nprobe, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st, &p, &exchanged));
-    if (exchanged) {
-        exch_commit(ex, p);
-        return 0;
-    }
-    return launch_exchange_kernel(ex, p, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st);
-}
-
-static int exch_search_dev_entry(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_dev, int64_t k,
-                                 int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream) {
-    TRY(check_search_args(h, nq, q_dev, k, D_dev, I_dev));
-    TRY(check_filter(h, f));
-    if (!ex) return fail("NULL exchange");
-    if (nq == 0) return 0;
-    TRY(set_dev(h));
-    cudaStream_t st = (cudaStream_t)stream;
-    const float* q = nullptr;
-    TRY(stage_queries(h, nq, q_dev, false, st, &q));
-    return exch_search_dev_impl(h, ex, f, nq, q, k, nprobe, D_dev, I_dev, st);
-}
-extern "C" int wb_exch_search_dev(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_dev, int64_t k, int64_t nprobe,
-                                  float* D_dev, int64_t* I_dev, void* stream) {
-    return exch_search_dev_entry(h, ex, nullptr, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
-}
-extern "C" int wb_exch_search_filtered_dev(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_dev,
-                                           int64_t k, int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream) {
-    return exch_search_dev_entry(h, ex, f, nq, q_dev, k, nprobe, D_dev, I_dev, stream);
-}
-
-// Host-buffer search over a sharded index: H2D of the queries, local search, NVLink exchange + merge, D2H of the
-// global (D, I) - one call, one stream, one synchronisation.  Every rank calls it with the same queries.
-static int exch_search_host_entry(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_host, int64_t k,
-                                  int64_t nprobe, float* D_host, int64_t* I_host) {
-    TRY(check_search_args(h, nq, q_host, k, D_host, I_host));
-    TRY(check_filter(h, f));
-    if (!ex) return fail("NULL exchange");
-    if (nq == 0) return 0;
-    TRY(set_dev(h));
-    cudaStream_t st = h->stream;
-    const float* q = nullptr;
-    TRY(stage_queries(h, nq, q_host, true, st, &q));
-    // (eD, eI): exch_search_dev_impl keeps this rank's local results in (dbuf, ibuf)
-    TRY(search_to_host(h, nq, k, h->eD, h->eI, D_host, I_host, st, [&](float* D, int64_t* I) {
-        return exch_search_dev_impl(h, ex, f, nq, q, k, nprobe, D, I, st);
-    }));
-    if (*reinterpret_cast<volatile int*>(ex->status.get())) return fail("sharded search: a peer GPU did not join the exchange within 20 s (results invalid)");
-    return 0;
-}
-extern "C" int wb_exch_search(wb_index* h, wb_exchange* ex, int64_t nq, const float* q_host, int64_t k, int64_t nprobe,
-                              float* D_host, int64_t* I_host) {
-    return exch_search_host_entry(h, ex, nullptr, nq, q_host, k, nprobe, D_host, I_host);
-}
-extern "C" int wb_exch_search_filtered(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q_host,
-                                       int64_t k, int64_t nprobe, float* D_host, int64_t* I_host) {
-    return exch_search_host_entry(h, ex, f, nq, q_host, k, nprobe, D_host, I_host);
 }

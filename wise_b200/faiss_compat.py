@@ -150,10 +150,7 @@ class Index:
         I = np.empty((n, k), np.int64)
         if n:
             L = _capi.lib()
-            if flt is None:
-                _capi.check(L.wb_search(self._h, n, _capi.ptr(x), k, nprobe, _capi.ptr(D), _capi.ptr(I)))
-            else:
-                _capi.check(L.wb_search_filtered(self._h, flt, n, _capi.ptr(x), k, nprobe, _capi.ptr(D), _capi.ptr(I)))
+            _capi.check(L.wb_search_filtered(self._h, flt, n, _capi.ptr(x), k, nprobe, _capi.ptr(D), _capi.ptr(I)))
         return D, I
 
     def range_search(self, x, thresh, *, params=None):
