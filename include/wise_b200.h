@@ -261,6 +261,11 @@ int wb_gemm_stats(const wb_index* h, int64_t* epochs, int64_t* fallbacks);
  * of IndexIVF::search, reached from /root/reference/src/index/feature_search_index.py:113) is the prologue of the list
  * scan.  Number of searches served that way so far (the others took the coarse scan + list scan launches). */
 int64_t wb_ivf_fused_searches(const wb_index* h);
+/* The CUDA-core scan plan of a search of nq queries with k results (k = 0: a range search) over the whole store
+ * (gather = 0) or over nprobe probed lists (gather = 1): out = {queries per CTA, rows per warp, floats per staged row
+ * chunk, chunks per row, ring stages}.  Chunks per row > 1 is the fallback for rows too wide for two whole-row stages.
+ * Fails with the planner's message when no plan fits shared memory.  Read-only. */
+int wb_scan_plan(wb_index* h, int64_t nq, int64_t k, int gather, int64_t nprobe, int out[5]);
 /* Diagnostics (replaces nothing in the reference): with WB_PHASE_TS=1 in the environment the scan kernel's CTAs stamp
  * %globaltimer at their phase boundaries (scan.cuh ScanParams::phase_ts lists the 10 phases); this copies the stamps of
  * the first `ctas` CTAs of the last scan-served search, 16 uint64 per CTA (scripts/phase_times.py prints them). */

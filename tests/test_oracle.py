@@ -154,3 +154,31 @@ def test_one_term_tf32_filter_margin_bound():
         assert np.all(one_term[:500, :2] <= exact[:500, :2])  # all-positive operands: truncation only shrinks the sum
         worst = max(worst, float((np.abs(exact - one_term) / bound).max()))
     assert 0.05 < worst <= 1.0  # the bound is within ~20x of what same-sign vectors actually reach: not vacuous
+
+
+def test_chunked_fp64_references_match_the_oracle():
+    """The torch fp64 references of tests/test_limits_gpu.py (run here on the CPU) agree exactly with O.flat_search /
+    O.ivf_search, ties by insertion position included, across several query chunks and with k > ntotal."""
+    from test_limits_gpu import coarse_fp64, ivf_topk_fp64, topk_fp64
+    xb = O.unit_gaussian(700, 24, 1)
+    xb[[10, 300, 650]] = xb[5]  # exact ties, decided by position
+    xq = np.concatenate([O.unit_gaussian(40, 24, 2), xb[5:6]])
+    ids = np.arange(700, dtype=np.int64) * 3 + 1
+    for k in (1, 10, 64):
+        D, I = topk_fp64(xb, xq, k, ids, device="cpu")
+        Dr, Ir = O.flat_search(xb, xq, k, ids)
+        assert np.array_equal(D, Dr) and np.array_equal(I, Ir), k
+    assert I[-1, :4].tolist() == [ids[5], ids[10], ids[300], ids[650]]
+    D, I = topk_fp64(xb[:30], xq, 64, device="cpu")
+    Dr, Ir = O.flat_search(xb[:30], xq, 64)
+    assert np.array_equal(D, Dr) and np.array_equal(I, Ir) and np.all(I[:, 30:] == -1)
+    cent = O.unit_gaussian(16, 24, 3)
+    assign = O.ivf_assign(xb, cent)
+    for nprobe in (1, 3, 16):
+        probes, gaps = coarse_fp64(cent, xq, nprobe, device="cpu")
+        _, Pr = O.ivf_coarse(xq, cent, nprobe)
+        assert np.array_equal(probes, Pr) and np.all(gaps >= 0)
+        for k in (5, 200):
+            D, I = ivf_topk_fp64(xb, ids, assign, probes, xq, k, device="cpu")
+            Dr, Ir = O.ivf_search(xb, ids, assign, cent, xq, k, nprobe)
+            assert np.array_equal(D, Dr) and np.array_equal(I, Ir), (nprobe, k)

@@ -67,3 +67,31 @@ def test_ivf_reference_with_every_list_is_flat():
 def test_range_search_is_declared():
     for name in ("wb_range_search", "wb_range_result_copy", "wb_range_result_free"):
         assert name in _capi.SIGNATURES
+
+
+def test_check_accepts_the_reference_and_rejects_errors():
+    """range_oracle.check, the rule every GPU range test applies: it accepts the fp64 reference's own output and
+    rejects a missing row, a row of another query, a wrong score and a broken tie order."""
+    from range_oracle import check
+    xb = O.unit_gaussian(3000, 16, 1)
+    xb[2500] = xb[7]
+    xq = np.concatenate([O.unit_gaussian(5, 16, 2), xb[7:8]])
+    ids = np.arange(3000, dtype=np.int64) * 2 + 1
+    t = np.float32(0.3)
+    lims, D, I = range_search(xb, xq, t, ids)
+    assert lims[-1] > 50
+    check(lims, D, I, xb, xq, t, ids)
+    check(lims, D, I, xb, xq, t, ids, cand=[np.arange(3000)] * len(xq))
+    a = int(lims[-2])  # the query equal to row 7: rows 7 and 2500 lead, tied
+    assert I[a] == ids[7] and I[a + 1] == ids[2500]
+    bad = [(lims, D, np.roll(I, 1)), (lims, D + np.float32(1e-3) * (np.arange(D.size) == 3), I)]
+    I2 = I.copy()
+    I2[a], I2[a + 1] = I[a + 1], I[a]
+    bad.append((lims, D, I2))
+    l3 = lims.copy()
+    l3[1:] -= 1
+    l3[0] = 0
+    bad.append((l3, D[1:], I[1:]))  # query 0 loses its best row
+    for lb, Db, Ib in bad:
+        with pytest.raises(AssertionError):
+            check(lb, Db, Ib, xb, xq, t, ids)

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from range_oracle import ivf_range_search, range_search
+from range_oracle import check as _check, ivf_range_search, range_search
 from wise_b200 import _capi
 from wise_b200 import faiss_compat as faiss
 
@@ -15,32 +15,6 @@ pytestmark = pytest.mark.gpu
 
 N, D = 200_000, 126
 BAND = {False: 2e-6, True: 4e-6}  # scan path, tensor-core path
-
-
-def _check(lims, Dg, Ig, xb, xq, thresh, ids, cand=None, band=4e-6):
-    """Every query's results against fp64 over its candidate rows (cand[i]: row indices; None: all rows)."""
-    n = len(xq)
-    assert lims.dtype == np.uint64 and lims.shape == (n + 1,) and lims[0] == 0
-    assert Dg.dtype == np.float32 and Ig.dtype == np.int64 and Dg.size == Ig.size == int(lims[-1])
-    assert np.all(np.diff(lims.astype(np.int64)) >= 0)
-    pos_of = np.empty(int(ids.max()) + 1, np.int64)
-    pos_of[ids] = np.arange(ids.size)
-    xb64 = xb.astype(np.float64)
-    for i in range(n):
-        a, b = int(lims[i]), int(lims[i + 1])
-        d, p = Dg[a:b], pos_of[Ig[a:b]]
-        assert np.all(d > np.float32(thresh))
-        rows = np.arange(xb.shape[0]) if cand is None else cand[i]
-        s = xb64[rows] @ xq[i].astype(np.float64)
-        assert np.all(np.isin(p, rows)) and np.unique(p).size == p.size
-        s_ret = xb64[p] @ xq[i].astype(np.float64)
-        assert np.all(np.abs(d - s_ret) <= 1e-5)
-        must = rows[s > thresh + band]
-        assert np.all(np.isin(must, p)), f"query {i}: {np.setdiff1d(must, p).size} rows missing"
-        assert np.all(s_ret > thresh - band)
-        assert np.all(np.diff(d.astype(np.float64)) <= 0)
-        tie = np.diff(d) == 0
-        assert np.all(np.diff(p)[tie] > 0), "equal scores must come in insertion order"
 
 
 @pytest.fixture(scope="module")

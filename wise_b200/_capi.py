@@ -86,6 +86,7 @@ SIGNATURES = {
     "wb_storage": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(C.c_int64)]),
     "wb_launch_count": (C.c_int64, [_vp]),
     "wb_ivf_fused_searches": (C.c_int64, [_vp]),
+    "wb_scan_plan": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int, C.c_int64, _i32p]),
     "wb_phase_stamps": (C.c_int, [_vp, _vp, C.c_int]),
     "wb_gemm_stats": (C.c_int, [_vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "wb_set_timing": (C.c_int, [_vp, C.c_int]),

@@ -401,6 +401,20 @@ static int plan_scan(const wb_index* h, int64_t nq, int k, bool gather, int npro
     return fail("scan does not fit shared memory (d=%d, k=%d)", h->d, k);
 }
 
+constexpr int kRangeStage = 256;  // staged hits per query and CTA in the range scan (P of its shared lists)
+
+// The plan plan_scan makes for a search of `nq` queries (k = 0: a range search), so that tests can choose shapes by the
+// path they take: out = {NQ, RW, ck, nchunks, stages}.
+extern "C" int wb_scan_plan(wb_index* h, int64_t nq, int64_t k, int gather, int64_t nprobe, int out[5]) {
+    if (!h || !out) return fail("NULL argument");
+    if (nq < 1 || k < 0 || k > WB_MAX_K || nprobe < 0 || nprobe > WB_MAX_K) return fail("bad scan plan arguments");
+    ScanCfg c;
+    TRY(plan_scan(h, nq, k == 0 ? kRangeStage - kMinQueue : (int)k, gather != 0, (int)nprobe, &c));
+    const int v[5] = {c.NQ, c.RW, c.ck, c.nchunks, c.stages};
+    for (int i = 0; i < 5; ++i) out[i] = v[i];
+    return 0;
+}
+
 constexpr int kScanSmemOptin = 232448;  // the scan kernels opt in to the most a block may have (227 KB)
 
 // Opt `Kernel` in to the scans' shared memory, launch it on `st` and check the launch.
@@ -1972,7 +1986,6 @@ struct wb_range_result {
 };
 
 constexpr int64_t kRangeMaxQ = 32768;  // queries per chunk: one launch (grid.y) per scan
-constexpr int kRangeStage = 256;       // staged hits per query and CTA in the range scan (P of its shared lists)
 
 // K1 / K5 in range mode: `S` CTAs per query group, one launch per <= kMaxGridY groups.  Whole-row stages draw their
 // row groups from the shared dispensers, which every launch leaves at zero as the fused tails do.
