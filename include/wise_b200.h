@@ -11,6 +11,9 @@
  *   - the caller owns every buffer; "host" pointers are ordinary (pageable or pinned) host
  *     memory, "_dev" variants take device pointers on the index's GPU and a cudaStream_t
  *     (passed as void*) and do not synchronise.
+ *   - a buffer (host or device) needs only the natural alignment of its element type: 4 bytes for float and int32,
+ *     8 bytes for int64.  Any view into a larger allocation at such an offset is a valid argument.
+ *   - one handle must not be used from two threads at the same time; different handles (also of one GPU) may be.
  *   - one index lives on one GPU (one process per GPU; rows are sharded across processes by
  *     the host layer, wise_b200/sharded.py; the per-GPU top-k lists are exchanged and merged through
  *     NVLink peer memory by wb_exch_search*, below - NCCL is not on the search path).

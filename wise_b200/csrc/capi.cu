@@ -1816,9 +1816,14 @@ static int check_search_args(const wb_index* h, int64_t nq, const void* q, int64
 
 constexpr size_t kPinStageMax = (size_t)4 << 20;  // larger transfers are bandwidth-bound anyway: copy them directly
 
+// The scan, list-major, SS-image and re-scoring kernels load query rows 16 bytes at a time, and the assignment GEMM
+// maps the points with TMA (16-byte base): a caller's device buffer goes to them as is only when it is 16-byte
+// aligned.  The C API asks for no more than the alignment of a float, so other buffers are staged like padded ones.
+static bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
+
 // queries arrive with row stride d; the kernels want stride ld
 static int stage_queries(wb_index* h, int64_t nq, const float* q, bool host, cudaStream_t st, const float** out) {
-    if (!host && h->ld == h->d) {
+    if (!host && h->ld == h->d && aligned16(q)) {
         *out = q;
         return 0;
     }
@@ -1830,8 +1835,8 @@ static int stage_queries(wb_index* h, int64_t nq, const float* q, bool host, cud
         q = reinterpret_cast<const float*>(pb.get());
     }
     TRY(h->qbuf.ensure((size_t)nq * h->ld * sizeof(float)));
-    if (h->ld == h->d) {
-        CK(cudaMemcpyAsync(h->qbuf.get(), q, qbytes, cudaMemcpyHostToDevice, st));
+    if (h->ld == h->d) {  // (device queries get here only when unaligned: a copy takes any alignment)
+        CK(cudaMemcpyAsync(h->qbuf.get(), q, qbytes, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st));
     } else {
         const float* src = q;
         if (host) {
@@ -2481,17 +2486,21 @@ extern "C" int wb_ivf_get_centroids(const wb_index* h, float* c) {
     return 0;
 }
 
-// x_dev has row stride d; kernels need stride ld
+// x_dev has row stride d; kernels need stride ld and a 16-byte aligned base (see stage_queries)
 static int stage_points(wb_index* h, int64_t n, const float* x_dev, cudaStream_t st, const float** out) {
-    if (h->ld == h->d) {
+    if (h->ld == h->d && aligned16(x_dev)) {
         *out = x_dev;
         return 0;
     }
     TRY(h->xbuf.ensure((size_t)n * h->ld * sizeof(float)));
-    const int64_t tot = n * h->ld;
-    pad_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(x_dev, h->xbuf.as<float>(), n, h->d, h->ld);
-    CK(cudaGetLastError());
-    h->launches++;
+    if (h->ld == h->d) {
+        CK(cudaMemcpyAsync(h->xbuf.get(), x_dev, (size_t)n * h->d * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    } else {
+        const int64_t tot = n * h->ld;
+        pad_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(x_dev, h->xbuf.as<float>(), n, h->d, h->ld);
+        CK(cudaGetLastError());
+        h->launches++;
+    }
     *out = h->xbuf.as<float>();
     return 0;
 }

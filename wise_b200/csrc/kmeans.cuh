@@ -11,15 +11,16 @@
 namespace wb {
 
 // sums[c, 0:d] = sum over slots of list c of x[perm[slot], 0:d]; counts[c] = list size.
-// One CTA per list; a thread owns 4 adjacent columns (one 128-bit load per row) when d and ldx allow it, rows are
-// taken four at a time into four accumulators per column that are combined as (a0 + a1) + (a2 + a3): the order is
-// static, so the sums do not depend on the schedule.
+// One CTA per list; a thread owns 4 adjacent columns (one 128-bit load per row) when d, ldx and the alignment of x and
+// sums allow it, rows are taken four at a time into four accumulators per column that are combined as
+// (a0 + a1) + (a2 + a3): the order is static, so the sums do not depend on the schedule (and the scalar branch, which
+// uses the same order, gives the same bits).
 __global__ void __launch_bounds__(256) segment_sum_kernel(const float* x, int ldx, int d, const uint32_t* perm,
                                                           const int64_t* off, float* sums, int64_t* counts) {
     const int64_t c = blockIdx.x;
     const int64_t b = off[c], e = off[c + 1];
     if (threadIdx.x == 0) counts[c] = e - b;
-    if (((d | ldx) & 3) == 0) {
+    if ((((d | ldx) & 3) | (((uintptr_t)x | (uintptr_t)sums) & 15)) == 0) {
         const int d4 = d >> 2, ld4 = ldx >> 2;
         const float4* x4 = reinterpret_cast<const float4*>(x);
         for (int col = threadIdx.x; col < d4; col += blockDim.x) {
