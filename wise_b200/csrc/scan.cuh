@@ -20,7 +20,12 @@
 //     query at the end, merged by merge_topk_kernel (merge.cuh).
 //   * range mode (scan_range_kernel, range search): the same scan with a fixed threshold; every hit is staged in the
 //     shared lists and flushed to a global pool (RangeOut) instead of the fused top-k (DESIGN.md "Range search").
-// Algorithmic bytes per launch: nrows * ld * 4 (the row store is read exactly once per pass).
+//   * bf16 filter (flat top-k of 1-2 queries, DESIGN.md "K1"): the ring streams the bf16 image of the rows instead, the
+//     consumers score it approximately, and only the (row, query) pairs whose approximation can reach the threshold
+//     are queued and re-scored from the fp32 rows with the arithmetic of the fp32 scan; every CTA's list is therefore
+//     the top-k of the exact keys of its rows, as without the filter.
+// Algorithmic bytes per launch: nrows * ld * 4 (the row store is read exactly once per pass); with the bf16 filter
+// nrows * ld * 2 plus the re-scored rows.
 #pragma once
 #include "coarse.cuh"
 #include "exchange.cuh"
@@ -87,14 +92,23 @@ struct ScanParams {
     // 10-13 inside block_merge_heads: staged, T0 found, candidates compacted, ranked
     unsigned long long* phase_ts;
     ExchParams exch;
+    // bf16 filter (scan_topk_kernel<..., IMG = true>): `img` is the bf16 image of `rows`, row stride 2 * ck bf16 (a
+    // multiple of 8, zero padded); `rows` is read only to re-score the queued candidates
+    const uint16_t* img;
+    const float* norm2_max;          // device scalar: max |row|^2 over the store (the filter's error bound)
+    unsigned long long* rescored;    // += (row, query) pairs re-scored by this launch
 };
+
+constexpr int kRescoreCap = 256;    // queued (row, query) pairs of the bf16 filter per CTA
+constexpr int kRescoreChunk = 32;   // pairs re-scored per insertion round: 4 rows in flight per consumer warp
 
 struct ScanSmem {
-    size_t ring, queries, lists, bars, misc, prefix, total;
+    size_t ring, queries, lists, bars, misc, prefix, rescore, total;
 };
 
+// `ld`: stride of the queries in shared memory (floats).  `rescore`: the bf16 filter's queue and margins.
 __host__ __device__ inline ScanSmem scan_smem_layout(int NQ, int ld, int P, int ck, int stages, int nprobe,
-                                                     int group_rows) {
+                                                     int group_rows, bool rescore = false) {
     ScanSmem L;
     size_t o = 0;
     L.ring = o;    o += (size_t)stages * group_rows * ck * 4;
@@ -105,6 +119,8 @@ __host__ __device__ inline ScanSmem scan_smem_layout(int NQ, int ld, int P, int 
     L.misc = o;    o += (size_t)NQ * 12 + 16;  // qcnt[NQ] (int) + thr_s[NQ] (float) + 4 ints (fused tail / work item) + pair[NQ] (list-major)
     o = (o + 7) & ~(size_t)7;
     L.prefix = o;  o += nprobe > 0 ? (size_t)nprobe * 8 + (size_t)(nprobe + 1) * 4 : 0;  // pbase[np] i64 + prefix[np+1] u32
+    o = (o + 15) & ~(size_t)15;
+    L.rescore = o; o += rescore ? (size_t)kRescoreCap * 8 + (size_t)NQ * 4 + 16 : 0;  // queue [cap] u64 + margin[NQ] + count
     L.total = (o + 15) & ~(size_t)15;
     return L;
 }
@@ -199,13 +215,56 @@ __device__ __forceinline__ void range_flush(const ScanSmem& L, unsigned char* sm
     named_bar_sync(kBarConsumers, kConsumerThreads);
 }
 
-template <int NQ, int RW, bool GATHER, bool RANGE>
+// The exact fp32 score of J rows, each against its own query (queries in shared memory, stride dq4 float4), with the
+// arithmetic of the fp32 scan's whole-row stages: lane l accumulates float4 l, l + 32, ... in order with fmaf in x, y,
+// z, w order, then the xor butterfly 16, 8, 4, 2, 1 (the sums multi_reduce_step forms, so the same bits).  Every lane
+// gets every score.  The loads of all J rows are in flight together.
+template <int J>
+__device__ __forceinline__ void exact_scores(const float* rows, int ld, const float4* q4, int dq4, const uint64_t* ent,
+                                             const bool* valid, int lane, float* a) {
+    const float4* xr[J];
+    const float4* qr[J];
+#pragma unroll
+    for (int j = 0; j < J; ++j) {
+        xr[j] = reinterpret_cast<const float4*>(rows + (size_t)(ent[j] >> 8) * ld);
+        qr[j] = q4 + (size_t)(ent[j] & 0xff) * dq4;
+        a[j] = 0.f;
+    }
+    const int d4 = ld >> 2;
+#pragma unroll 2
+    for (int i = lane; i < d4; i += 32) {
+        float4 x[J];
+#pragma unroll
+        for (int j = 0; j < J; ++j) x[j] = valid[j] ? __ldg(xr[j] + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+        for (int j = 0; j < J; ++j) {
+            const float4 q = qr[j][i];
+            a[j] = fmaf(x[j].x, q.x, a[j]);
+            a[j] = fmaf(x[j].y, q.y, a[j]);
+            a[j] = fmaf(x[j].z, q.z, a[j]);
+            a[j] = fmaf(x[j].w, q.w, a[j]);
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+        for (int j = 0; j < J; ++j) a[j] += __shfl_xor_sync(0xffffffffu, a[j], o);
+}
+
+// bf16 -> fp32 of the low / high half of a word of two packed bf16 values (element 2i is the low half)
+__device__ __forceinline__ float bf16_lo(uint32_t w) { return __uint_as_float(w << 16); }
+__device__ __forceinline__ float bf16_hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }
+
+template <int NQ, int RW, bool GATHER, bool RANGE, bool IMG = false>
 __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& ro) {
+    static_assert(!(IMG && (GATHER || RANGE)), "the bf16 filter serves flat top-k scans only");
     constexpr int kRowsPerWarp = RW;
     constexpr int kGroupRows = kConsumerWarps * RW;
     extern __shared__ __align__(128) unsigned char smem_scan[];
     unsigned char* smem = smem_scan;
-    const ScanSmem L = scan_smem_layout(NQ, p.ld, p.P, p.ck, p.stages, GATHER ? p.nprobe : 0, kGroupRows);
+    // queries in shared memory: stride ld, or with the bf16 filter the image's row length 2 * ck (zero padded)
+    const int ldq = IMG ? 2 * p.ck : p.ld, dq4 = ldq >> 2;
+    const ScanSmem L = scan_smem_layout(NQ, ldq, p.P, p.ck, p.stages, GATHER ? p.nprobe : 0, kGroupRows, IMG);
     float* ring = reinterpret_cast<float*>(smem + L.ring);
     float* qs = reinterpret_cast<float*>(smem + L.queries);
     uint64_t* lists = reinterpret_cast<uint64_t*>(smem + L.lists);
@@ -216,6 +275,9 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
     float* thr_s = reinterpret_cast<float*>(smem + L.misc) + NQ;
     int64_t* pbase = reinterpret_cast<int64_t*>(smem + L.prefix);
     uint32_t* prefix = reinterpret_cast<uint32_t*>(pbase + (GATHER ? p.nprobe : 0));
+    uint64_t* rq = reinterpret_cast<uint64_t*>(smem + L.rescore);  // bf16 filter: queued (row << 8 | query) pairs
+    float* margin_s = reinterpret_cast<float*>(rq + kRescoreCap);   // [NQ]
+    int* rq_cnt = reinterpret_cast<int*>(margin_s + NQ);
 
     const int tid = threadIdx.x;
     const int warp = tid >> 5, lane = tid & 31;
@@ -228,7 +290,8 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
     const int ld = p.ld, d4 = ld >> 2, ck = p.ck, ck4 = ck >> 2;
     const int k = p.k, P = p.P;
     const int qcap = P - k;
-    const int hw_mark = qcap - kGroupRows;
+    // insertions into a queue between two checks: one per row of a group, or one per pair of a re-scoring round
+    const int hw_mark = qcap - (IMG ? kRescoreChunk : kGroupRows);
 
     // ---- prologue: barriers, queries, empty lists ------------------------------------------
     if (tid == 0) {
@@ -238,10 +301,10 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
         }
         fence_mbar_init();
     }
-    for (int i = tid; i < NQ * d4; i += kScanThreads) {
-        const int b = i / d4, c = i - b * d4;
+    for (int i = tid; i < NQ * dq4; i += kScanThreads) {
+        const int b = i / dq4, c = i - b * dq4;
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (b < nqv) v = reinterpret_cast<const float4*>(p.queries + (size_t)(q0 + b) * ld)[c];
+        if (b < nqv && c < d4) v = reinterpret_cast<const float4*>(p.queries + (size_t)(q0 + b) * ld)[c];
         reinterpret_cast<float4*>(qs)[i] = v;
     }
     for (int i = tid; i < NQ * P; i += kScanThreads) lists[i] = 0ull;
@@ -249,6 +312,7 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
         qcnt[tid] = 0;
         thr_s[tid] = tid < nqv ? -INFINITY : INFINITY;
     }
+    if (IMG && tid == 0) *rq_cnt = 0;
     int64_t total = p.nrows;
     GatherCtx G{prefix, pbase, p.perm, p.nprobe};
     if constexpr (GATHER && NQ == 1) {
@@ -371,7 +435,7 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
             // CSR loads are in flight while this group's copies are issued
             const int64_t g_next = draw(g);
             if (g_next < ngroups) row_next = lookup(g_next);
-            const float* src = p.rows + (size_t)row * ld;
+            const float* src = IMG ? reinterpret_cast<const float*>(p.img) + (size_t)row * ck : p.rows + (size_t)row * ld;
             for (int ch = 0; ch < p.nchunks; ++ch) {
                 if (lane == 0) {
                     mbar_wait(&empty[s], ph ^ 1u);
@@ -418,6 +482,88 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
         int s = 0;
         uint32_t ph = 0;
         const bool dyn = p.group_count != nullptr;
+        // [list | queue] of every query sorted, queues emptied, thresholds tightened (all consumers, at a barrier)
+        auto tighten = [&]() {
+            if (NQ == 1 && p.rank_sort) rank_sort_desc<kConsumerThreads>(lists, P, ctid, kBarConsumers);
+            else bitonic_sort_desc<kConsumerThreads>(lists, P, nqv, ctid, kBarConsumers);
+            for (int i = ctid; i < nqv * qcap; i += kConsumerThreads) {
+                const int l = i / qcap, j = i - l * qcap;
+                lists[(size_t)l * P + k + j] = 0ull;
+            }
+            if (ctid < nqv) {
+                qcnt[ctid] = 0;
+                const uint64_t t = lists[(size_t)ctid * P + k - 1];
+                thr_s[ctid] = t ? key_score(t) : -INFINITY;
+            }
+            named_bar_sync(kBarConsumers, kConsumerThreads);
+        };
+        // bf16 filter.  Error bound of an approximate score (the image and the query in fp32, DESIGN.md "K1"):
+        //   |exact - approx| <= (2^-8 + ld 2^-23 1.1 + 1e-5) |q| sqrt(norm2_max)   one bf16 rounding of every element,
+        //                                                                          both fp32 sums, their comparison
+        //                       + 2^-134 (sqrt(ld) |q| + ld)                       rows with fp32-subnormal elements
+        // times 1.001 for the rounding of |q| and of the margin itself.  |q|^2 and norm2_max are fp32 sums of squares
+        // that may underflow (elements below ~1e-19): ld 2^-149 added to each bounds what the underflow lost, so a store
+        // of tiny rows keeps a margin of their true size.  A NaN row does not enter norm2_max (its
+        // approximation is NaN and is re-scored); norm2_max = +Inf (a |row|^2 overflowed) or a NaN query makes the margin
+        // Inf or NaN and every row is re-scored.  One warp per query, before the first group.
+        unsigned long long nrescored = 0;
+        if constexpr (IMG) {
+            if (cw < NQ) {
+                float s2 = 0.f;
+                for (int t = lane; t < dq4; t += 32) {
+                    const float4 v = q4[cw * dq4 + t];
+                    s2 += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
+                }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+                if (lane == 0) {
+                    const float c = 3.90625e-3f + (float)ld * 1.1920929e-7f * 1.1f + 1e-5f;
+                    const float lost = (float)ld * 0x1p-149f;
+                    const float qn = sqrtf(s2 + lost);
+                    margin_s[cw] = 1.001f * (c * qn * sqrtf(*p.norm2_max + lost) + 0x1p-134f * (sqrtf((float)ld) * qn + (float)ld));
+                }
+            }
+            named_bar_sync(kBarConsumers, kConsumerThreads);
+        }
+        // Re-score the queued pairs exactly, kRescoreChunk at a time (insertion as in the fp32 scan), and empty the
+        // queue.  All consumers, at a barrier.
+        auto rescore_queue = [&]() {
+            const int n = *rq_cnt;
+            nrescored += (unsigned long long)n;
+            for (int c0 = 0; c0 < n; c0 += kRescoreChunk) {
+                constexpr int J = kRescoreChunk / kConsumerWarps;
+                uint64_t ent[J];
+                bool valid[J];
+#pragma unroll
+                for (int j = 0; j < J; ++j) {
+                    const int e = c0 + cw + kConsumerWarps * j;
+                    valid[j] = e < n;
+                    ent[j] = valid[j] ? rq[e] : 0ull;
+                }
+                float a[J];
+                exact_scores<J>(p.rows, ld, q4, dq4, ent, valid, lane, a);
+                bool hw = false;
+#pragma unroll
+                for (int j = 0; j < J; ++j) {
+                    if (lane == j && valid[j]) {
+                        const float score = a[j];
+                        const int b = (int)(ent[j] & 0xff);
+                        const uint32_t pos = (uint32_t)(ent[j] >> 8);
+                        if (score >= thr_s[b]) {
+                            const uint64_t key = make_key(score, pos);
+                            if (key > lists[(size_t)b * P + k - 1] && row_allowed(p.allow, pos)) {
+                                const int slot = atomicAdd(&qcnt[b], 1);
+                                lists[(size_t)b * P + k + slot] = key;
+                                hw = slot + 1 > hw_mark;
+                            }
+                        }
+                    }
+                }
+                if (named_bar_or(kBarConsumers, kConsumerThreads, hw)) tighten();
+            }
+            if (ctid == 0 && n) *rq_cnt = 0;
+            named_bar_sync(kBarConsumers, kConsumerThreads);
+        };
         for (int64_t g = blockIdx.x; dyn || g < ngroups; g += gridDim.x) {
             float acc[V];
 #pragma unroll
@@ -429,10 +575,41 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
             }
             for (int ch = 0; ch < p.nchunks; ++ch) {
                 if (!dyn) mbar_wait(&full[s], ph);
+                if constexpr (IMG) {  // whole rows of bf16: 8 elements per 16-byte load, unpacked by a shift or a mask
+                    const uint4* tile = reinterpret_cast<const uint4*>(ring + (size_t)s * stage_floats) +
+                                        (size_t)(cw * kRowsPerWarp) * ck4;
+#pragma unroll 2
+                    for (int i = lane; i < ck4; i += 32) {
+                        uint4 x[kRowsPerWarp];
+#pragma unroll
+                        for (int r = 0; r < kRowsPerWarp; ++r) x[r] = tile[r * ck4 + i];
+#pragma unroll
+                        for (int b = 0; b < NQ; ++b) {
+                            const float4 qa = q4[b * dq4 + 2 * i], qb = q4[b * dq4 + 2 * i + 1];
+#pragma unroll
+                            for (int r = 0; r < kRowsPerWarp; ++r) {
+                                float a = acc[r * NQ + b];
+                                a = fmaf(bf16_lo(x[r].x), qa.x, a);
+                                a = fmaf(bf16_hi(x[r].x), qa.y, a);
+                                a = fmaf(bf16_lo(x[r].y), qa.z, a);
+                                a = fmaf(bf16_hi(x[r].y), qa.w, a);
+                                a = fmaf(bf16_lo(x[r].z), qb.x, a);
+                                a = fmaf(bf16_hi(x[r].z), qb.y, a);
+                                a = fmaf(bf16_lo(x[r].w), qb.z, a);
+                                a = fmaf(bf16_hi(x[r].w), qb.w, a);
+                                acc[r * NQ + b] = a;
+                            }
+                        }
+                    }
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(&empty[s]);
+                    if (++s == p.stages) { s = 0; ph ^= 1u; }
+                    continue;
+                }
                 const float4* tile =
                     reinterpret_cast<const float4*>(ring + (size_t)s * stage_floats) + (size_t)(cw * kRowsPerWarp) * ck4;
                 const int c4n = min(ck4, d4 - ch * ck4);
-                const float4* qb = q4 + ch * ck4;
+                const float4* qb = q4 + ch * ck4;  // (stride dq4 == d4 without the bf16 filter)
 #pragma unroll 2
                 for (int i = lane; i < c4n; i += 32) {
                     float4 x[kRowsPerWarp];
@@ -478,6 +655,22 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
                 if (named_bar_or(kBarConsumers, kConsumerThreads, hw)) range_flush<NQ>(L, smem, lists, qcnt, P, q0, nqv, ctid, ro);
                 continue;
             }
+            if constexpr (IMG) {
+                // queue the pair unless the bound shows that its exact score is below the threshold (a NaN or Inf
+                // approximation, a non-finite margin and a threshold of -inf all queue it)
+                bool full_q = false;
+                if (owner && b < nqv) {
+                    const int64_t cpos = g * kGroupRows + cw * kRowsPerWarp + r;
+                    if (cpos < total && row_allowed(p.allow, (uint32_t)cpos) &&
+                        !(fabsf(score) <= FLT_MAX && score + margin_s[b] < thr_s[b])) {
+                        const int slot = atomicAdd(rq_cnt, 1);
+                        rq[slot] = (uint64_t)cpos << 8 | (uint64_t)b;
+                        full_q = slot + 1 > kRescoreCap - kGroupRows * NQ;
+                    }
+                }
+                if (named_bar_or(kBarConsumers, kConsumerThreads, full_q)) rescore_queue();
+                continue;
+            }
             if (owner) {
                 const int64_t cpos = g * kGroupRows + cw * kRowsPerWarp + r;
                 if (cpos < total && score >= thr_s[b]) {
@@ -491,20 +684,7 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
                     }
                 }
             }
-            if (named_bar_or(kBarConsumers, kConsumerThreads, hw)) {
-                if (NQ == 1 && p.rank_sort) rank_sort_desc<kConsumerThreads>(lists, P, ctid, kBarConsumers);
-                else bitonic_sort_desc<kConsumerThreads>(lists, P, nqv, ctid, kBarConsumers);
-                for (int i = ctid; i < nqv * qcap; i += kConsumerThreads) {
-                    const int l = i / qcap, j = i - l * qcap;
-                    lists[(size_t)l * P + k + j] = 0ull;
-                }
-                if (ctid < nqv) {
-                    qcnt[ctid] = 0;
-                    const uint64_t t = lists[(size_t)ctid * P + k - 1];
-                    thr_s[ctid] = t ? key_score(t) : -INFINITY;
-                }
-                named_bar_sync(kBarConsumers, kConsumerThreads);
-            }
+            if (named_bar_or(kBarConsumers, kConsumerThreads, hw)) tighten();
         }
         // ---- epilogue: final sort, k best keys of this CTA for each query -------------------
         named_bar_sync(kBarConsumers, kConsumerThreads);
@@ -512,6 +692,10 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
         if constexpr (RANGE) {
             range_flush<NQ>(L, smem, lists, qcnt, P, q0, nqv, ctid, ro);
             return;
+        }
+        if constexpr (IMG) {
+            rescore_queue();
+            if (ctid == 0 && nrescored) atomicAdd(p.rescored, nrescored);
         }
         if (NQ == 1 && p.rank_sort) rank_sort_desc<kConsumerThreads>(lists, P, ctid, kBarConsumers);
         else bitonic_sort_desc<kConsumerThreads>(lists, P, nqv, ctid, kBarConsumers);
@@ -598,9 +782,35 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
     }
 }
 
-template <int NQ, int RW, bool GATHER>
+// The bf16 image of n rows: out[r][c] = bf16(rows[r][c]) rounded to nearest even (NaN stays NaN, a value within half a
+// bf16 ulp of FLT_MAX rounds to Inf), columns [ld, ldh) zero.  One thread per 8 elements.
+__global__ void bf16_image_kernel(const float* rows, int ld, int ldh, int64_t n, uint16_t* out) {
+    const int c8n = ldh >> 3;
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n * c8n) return;
+    const int64_t r = i / c8n;
+    const int c = (int)(i - r * c8n) * 8;
+    uint32_t w[4];
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (c + 4 * h < ld) v = *reinterpret_cast<const float4*>(rows + (size_t)r * ld + c + 4 * h);
+        const float f[4] = {v.x, v.y, v.z, v.w};
+        uint32_t b[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const uint32_t u = __float_as_uint(f[e]);
+            b[e] = (f[e] != f[e]) ? 0x7fc0u : (u + 0x7fffu + ((u >> 16) & 1u)) >> 16;
+        }
+        w[2 * h] = b[0] | b[1] << 16;
+        w[2 * h + 1] = b[2] | b[3] << 16;
+    }
+    *reinterpret_cast<uint4*>(out + (size_t)r * ldh + c) = make_uint4(w[0], w[1], w[2], w[3]);
+}
+
+template <int NQ, int RW, bool GATHER, bool IMG = false>
 __global__ void __launch_bounds__(kScanThreads, 1) scan_topk_kernel(const ScanParams p) {
-    scan_impl<NQ, RW, GATHER, false>(p, RangeOut{});
+    scan_impl<NQ, RW, GATHER, false, IMG>(p, RangeOut{});
 }
 
 // Range mode: P = the staging capacity per query, p.k = 0; no parts, no fused tail.
