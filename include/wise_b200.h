@@ -14,9 +14,10 @@
  *   - a buffer (host or device) needs only the natural alignment of its element type: 4 bytes for float and int32,
  *     8 bytes for int64.  Any view into a larger allocation at such an offset is a valid argument.
  *   - one handle must not be used from two threads at the same time; different handles (also of one GPU) may be.
- *   - one index lives on one GPU (one process per GPU; rows are sharded across processes by
- *     the host layer, wise_b200/sharded.py; the per-GPU top-k lists are exchanged and merged through
- *     NVLink peer memory by wb_exch_search*, below - NCCL is not on the search path).
+ *   - one index lives on one GPU.  Several GPUs serve one set of rows either from one process per GPU (rows are
+ *     sharded across processes by the host layer, wise_b200/sharded.py; the per-GPU top-k lists are exchanged and
+ *     merged through NVLink peer memory by wb_exch_search*, below - NCCL is not on the search path) or from one
+ *     process through a shard group (wb_group_*, below).
  *   - results: D float32[nq*k] sorted by score descending, ties broken by lowest insertion
  *     position; I int64[nq*k]; unfilled slots are (-FLT_MAX, -1) exactly like faiss.
  *   - there is no CPU fallback: without a CUDA device every compute call fails.
@@ -62,6 +63,9 @@ int wb_is_ivf(const wb_index* h);
 /* Pre-size HBM for n rows (FeatureStore.feature_count is known before the add loop,
  * feature_search_index.py:44) so adds never re-allocate. Optional. */
 int wb_reserve(wb_index* h, int64_t n);
+/* Rows the store holds without growing, and the free memory of the index's GPU (a growth allocates the new store,
+ * at least 1.5x the old, before it frees the old one): lets a multi-GPU index decide when a shard is full. */
+int wb_capacity(wb_index* h, int64_t* cap_rows, int64_t* free_bytes);
 /* index.add_with_ids(X, ids)   feature_search_index.py:81.  ids may be NULL (index.add).
  * IVF: also assigns each row to its max-inner-product centroid (ties -> lowest list). */
 int wb_add_with_ids(wb_index* h, int64_t n, const float* x_host, const int64_t* ids_host);
@@ -218,10 +222,44 @@ int wb_exch_status(wb_exchange* ex, int* timed_out);
 int64_t wb_exch_launch_count(const wb_exchange* ex);
 int wb_exch_free(wb_exchange* ex);
 
+/* ---- in-process shard group: one index over several GPUs of one process (DESIGN.md "Shard group") -----------------
+ * faiss index_cpu_to_all_gpus(index, co) with co.shard = True.  shards[0..n) are indices of the same kind (flat / IVF),
+ * the same d (and nlist) and, for IVF, bit-identical centroids, each on its own GPU; shard s holds the s-th contiguous
+ * slice of insertion order.  A search of the group returns exactly what one index holding all the rows in that order
+ * returns (equal scores by shard, then by local order == global insertion position).
+ *   - shards[0]'s GPU is the root: the _dev queries, the results and the caller's stream live there.
+ *   - creation enables peer access between every ordered pair of the GPUs and builds one exchange (rank s of n) whose
+ *     mailboxes are the other shards' device memory.  Searches of at most max_queries queries and max_entries = nq * k
+ *     results run the exchange in the search kernels' tail; larger ones, and every search of a group with a pair of
+ *     GPUs without peer access, search each shard locally, copy the results to the root (cudaMemcpyPeerAsync) and
+ *     merge them there (wb_merge_topk_dev).  With n = 1 every call is the plain single-index call.
+ *   - filters: NULL (unfiltered) or filters[s] = a wb_filter of shards[s] (NULL entries allowed), each built from the
+ *     same selector over its shard's rows.
+ *   - threads: searches of 1-4 queries (flat or IVF) are enqueued on every GPU from the calling thread.  Larger
+ *     batches may take the tensor-core path (the flat scan, or the coarse step of IVF), which synchronises once: the
+ *     group keeps one host thread per non-root shard (created here, joined by wb_group_free) that runs those shards'
+ *     searches.  One group must not be
+ *     used from two threads at the same time, and its shards must not be used elsewhere during a group call.
+ *   - streams: wb_group_search runs on the shards' own streams and returns synchronised on every GPU; a time-out of
+ *     the exchange (wb_exch_status) is its error.  wb_group_search_dev does not synchronise for searches of 1-4 queries:
+ *     the non-root shards' streams wait for `stream`, copy q_dev to their GPUs, and `stream` waits for those copies,
+ *     so the caller may overwrite q_dev with later work on `stream`; D_dev / I_dev are complete when `stream` is.
+ *   - wb_group_free comes before the free of its shards; shards grow (add) only between group calls. */
+typedef struct wb_group wb_group;
+int wb_group_create(int n, wb_index* const* shards, int64_t max_queries, int64_t max_entries, wb_group** out);
+int wb_group_search(wb_group* g, wb_filter* const* filters /* [n] or NULL */, int64_t nq, const float* q_host,
+                    int64_t k, int64_t nprobe, float* D_host, int64_t* I_host);
+int wb_group_search_dev(wb_group* g, wb_filter* const* filters, int64_t nq, const float* q_dev, int64_t k,
+                        int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream);
+int wb_group_free(wb_group* g);
+
 /* ---- row access ------------------------------------------------------------------------- */
 /* index.reconstruct_batch(ids)   api/routes.py:1078 (after index.make_direct_map, :907).
  * Looks rows up by external id; an unknown id is an error (faiss raises). */
 int wb_reconstruct_batch(wb_index* h, int64_t m, const int64_t* ids_host, float* out_host /* [m*d] */);
+/* The insertion position of each id, -1 for an id the index does not hold (the shard lookup of a group's
+ * reconstruct_batch: an unknown id is not an error here). */
+int wb_lookup_ids(wb_index* h, int64_t m, const int64_t* ids_host, int64_t* pos_host /* [m] */);
 /* Bulk export for faiss.write_index (feature_search_index.py:84): storage rows [start,start+n), their ids, and (IVF)
  * their list assignment.  Storage order is insertion order for flat indices and for IVF indices that have not been
  * searched / finalized yet; afterwards it is list by list.  Any output may be NULL. */

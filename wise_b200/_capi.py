@@ -32,6 +32,7 @@ SIGNATURES = {
     "wb_nlist": (C.c_int64, [_vp]),
     "wb_is_ivf": (C.c_int, [_vp]),
     "wb_reserve": (C.c_int, [_vp, C.c_int64]),
+    "wb_capacity": (C.c_int, [_vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "wb_add_with_ids": (C.c_int, [_vp, C.c_int64, _vp, _vp]),
     "wb_add_with_ids_dev": (C.c_int, [_vp, C.c_int64, _vp, _vp, _vp]),
     "wb_pinned_alloc": (C.c_int, [C.c_int64, C.POINTER(_vp)]),
@@ -75,7 +76,12 @@ SIGNATURES = {
     "wb_exch_launch_count": (C.c_int64, [_vp]),
     "wb_exch_status": (C.c_int, [_vp, C.POINTER(C.c_int)]),
     "wb_exch_free": (C.c_int, [_vp]),
+    "wb_group_create": (C.c_int, [C.c_int, _vp, C.c_int64, C.c_int64, C.POINTER(_vp)]),
+    "wb_group_search": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp]),
+    "wb_group_search_dev": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp]),
+    "wb_group_free": (C.c_int, [_vp]),
     "wb_reconstruct_batch": (C.c_int, [_vp, C.c_int64, _vp, _vp]),
+    "wb_lookup_ids": (C.c_int, [_vp, C.c_int64, _vp, _vp]),
     "wb_export_rows": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp, _vp, _vp]),
     "wb_ivf_add_preassigned": (C.c_int, [_vp, C.c_int64, _vp, _vp, _vp]),
     "wb_ivf_finalize": (C.c_int, [_vp]),

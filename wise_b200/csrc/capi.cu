@@ -9,9 +9,13 @@
 #include <string.h>
 
 #include <algorithm>
+#include <condition_variable>
+#include <functional>
 #include <memory>
+#include <mutex>
 #include <random>
 #include <string>
+#include <thread>
 #include <type_traits>
 #include <vector>
 
@@ -372,6 +376,16 @@ extern "C" int wb_reserve(wb_index* h, int64_t n) {
     if (!h) return fail("NULL index");
     TRY(set_dev(h));
     return ensure_capacity(h, n);
+}
+
+extern "C" int wb_capacity(wb_index* h, int64_t* cap_rows, int64_t* free_bytes) {
+    if (!h || !cap_rows || !free_bytes) return fail("NULL argument");
+    TRY(set_dev(h));
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    *cap_rows = h->cap;
+    *free_bytes = (int64_t)free_b;
+    return 0;
 }
 
 // ---- scan launch ---------------------------------------------------------------------------
@@ -2076,6 +2090,315 @@ extern "C" int wb_exch_search_filtered(wb_index* h, wb_exchange* ex, wb_filter* 
     return search_host_entry(h, ex, f, nq, q_host, k, nprobe, D_host, I_host);
 }
 
+// ---- in-process shard group (DESIGN.md "Shard group") ------------------------------------------------------------
+// A host thread of a group: runs a non-root shard's search when that search synchronises its stream (K2 reads its
+// overflow flag), so that the shards' searches overlap instead of running one GPU at a time.
+struct GroupWorker {
+    std::mutex mu;
+    std::condition_variable cv;
+    std::function<int()> job;
+    bool busy = false, quit = false;
+    int rc = 0;
+    std::string err;
+    std::thread th;  // declared last: the thread starts once the members above exist
+
+    GroupWorker() : th([this] { loop(); }) {}
+    ~GroupWorker() {
+        {
+            std::lock_guard<std::mutex> lk(mu);
+            quit = true;
+        }
+        cv.notify_all();
+        th.join();
+    }
+    void loop() {
+        std::unique_lock<std::mutex> lk(mu);
+        for (;;) {
+            cv.wait(lk, [&] { return quit || (bool)job; });
+            if (quit) return;
+            std::function<int()> j = std::move(job);
+            job = nullptr;
+            lk.unlock();
+            const int r = j();
+            lk.lock();
+            rc = r;
+            err = r ? g_err : std::string();  // g_err is per thread: hand the message to the caller
+            busy = false;
+            cv.notify_all();
+        }
+    }
+    void post(std::function<int()> j) {
+        std::lock_guard<std::mutex> lk(mu);
+        job = std::move(j);
+        busy = true;
+        cv.notify_all();
+    }
+    int wait() {
+        std::unique_lock<std::mutex> lk(mu);
+        cv.wait(lk, [&] { return !busy; });
+        if (rc) g_err = err;
+        return rc;
+    }
+};
+
+struct wb_group {
+    std::vector<wb_index*> shards;                      // [s] on its own GPU; [0] is the root
+    bool p2p = true;                                    // every ordered pair of the GPUs has peer access
+    std::vector<wb_exchange*> ex;                       // [s]: rank s of the group's exchange (p2p only)
+    std::vector<std::unique_ptr<GroupWorker>> workers;  // [s >= 1]
+    std::vector<DevBuf> qpeer;                          // [s >= 1]: the _dev queries, copied from the root
+    std::vector<EventPtr> ev;                           // [0]: the caller's stream reached the call; [s]: shard s's copies
+    DevBuf pD, pI;                                      // fallback merge: the shards' local results on the root, [n][nq][k]
+
+    ~wb_group() {
+        workers.clear();
+        for (size_t s = 0; s < shards.size(); ++s) {
+            cudaSetDevice(shards[s]->device);
+            if (s < ex.size()) wb_exch_free(ex[s]);  // waits for the device
+            if (s < qpeer.size()) qpeer[s].mem.reset();
+            if (s < ev.size()) ev[s].reset();
+        }
+        if (!shards.empty()) cudaSetDevice(shards[0]->device);
+    }
+};
+
+extern "C" int wb_group_create(int n, wb_index* const* shards, int64_t max_queries, int64_t max_entries, wb_group** out) {
+    if (!out) return fail("out is NULL");
+    *out = nullptr;
+    if (n < 1 || n > kExchMaxWorld) return fail("a group holds 1 to %d shards (got %d)", kExchMaxWorld, n);
+    if (!shards) return fail("NULL shards");
+    for (int s = 0; s < n; ++s) {
+        const wb_index* h = shards[s];
+        if (!h) return fail("shard %d is NULL", s);
+        if (h->ivf != shards[0]->ivf || h->d != shards[0]->d || h->nlist != shards[0]->nlist)
+            return fail("shard %d differs from shard 0 in kind, d or nlist", s);
+        for (int r = 0; r < s; ++r)
+            if (shards[r]->device == h->device) return fail("shards %d and %d are both on GPU %d", r, s, h->device);
+    }
+    if (shards[0]->ivf) {  // every shard must probe the same lists: identical centroids, bit for bit
+        const size_t row = (size_t)shards[0]->d * sizeof(float), bytes = (size_t)shards[0]->nlist * row;
+        std::vector<unsigned char> c0(bytes), cs(bytes);
+        for (int s = 0; s < n; ++s) {
+            TRY(set_dev(shards[s]));
+            CK(cudaStreamSynchronize(shards[s]->stream));
+            CK(cudaMemcpy2D(s ? cs.data() : c0.data(), row, shards[s]->centroids.get(), (size_t)shards[s]->ld * sizeof(float),
+                            row, (size_t)shards[0]->nlist, cudaMemcpyDeviceToHost));
+            if (s && memcmp(c0.data(), cs.data(), bytes) != 0) return fail("shard %d has other centroids than shard 0", s);
+        }
+    }
+    std::unique_ptr<wb_group> g(new wb_group());
+    g->shards.assign(shards, shards + n);
+    for (int s = 0; s < n; ++s)
+        for (int r = 0; r < n; ++r) {
+            if (r == s) continue;
+            int can = 0;
+            CK(cudaDeviceCanAccessPeer(&can, shards[s]->device, shards[r]->device));
+            if (!can) {
+                g->p2p = false;
+                continue;
+            }
+            TRY(set_dev(shards[s]));
+            const cudaError_t e = cudaDeviceEnablePeerAccess(shards[r]->device, 0);
+            if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+            else CK(e);
+        }
+    g->qpeer.resize(n);
+    g->ev.resize(n);
+    g->workers.resize(n);
+    for (int s = 0; s < n; ++s) {
+        TRY(set_dev(shards[s]));
+        cudaEvent_t e = nullptr;
+        CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        g->ev[s].reset(e);
+        if (s) {
+            try {
+                g->workers[s].reset(new GroupWorker());
+            } catch (const std::exception& ex) {  // std::system_error when no thread can be started
+                return fail("group: could not start a host thread for shard %d: %s", s, ex.what());
+            }
+        }
+    }
+    if (g->p2p && n > 1) {  // the mailboxes of the exchange are plain device pointers of the peers
+        for (int s = 0; s < n; ++s) {
+            wb_exchange* ex = nullptr;
+            TRY(wb_exch_create(shards[s]->device, s, n, max_queries, max_entries, &ex));
+            g->ex.push_back(ex);
+        }
+        for (int s = 0; s < n; ++s)
+            for (int r = 0; r < n; ++r) g->ex[s]->peers[r] = g->ex[r]->local.get();
+    }
+    TRY(set_dev(shards[0]));
+    *out = g.release();
+    return 0;
+}
+
+extern "C" int wb_group_free(wb_group* g) {
+    delete g;
+    return 0;
+}
+
+// Shard s's part of an exchange.  A shard whose search fails before it has launched its part joins the exchange with
+// padding, so that the shards already launched are not left waiting and every rank keeps its place in the sequence.
+static int group_exch_part(wb_index* h, wb_exchange* ex, wb_filter* f, int64_t nq, const float* q, int64_t k,
+                           int64_t nprobe, float* D, int64_t* I, cudaStream_t st) {
+    const uint32_t seq0 = ex->seq;
+    int rc = set_dev(h);
+    if (rc == 0) rc = exch_search_dev_impl(h, ex, f, nq, q, k, nprobe, D, I, st);
+    if (rc != 0 && ex->seq == seq0) {
+        const std::string err = g_err;
+        ExchParams p;
+        if (cudaSetDevice(h->device) == cudaSuccess && exch_prepare(ex, nq, k, D, I, &p) == 0) {
+            pad_results_kernel<<<(unsigned)((nq * k + 255) / 256), 256, 0, st>>>(h->dbuf.as<float>(), h->ibuf.as<int64_t>(),
+                                                                              nq * k);
+            launch_exchange_kernel(ex, p, h->dbuf.as<float>(), h->ibuf.as<int64_t>(), st);
+        }
+        g_err = err;
+    }
+    return rc;
+}
+
+// Batches above this may run K2 (flat search, or the coarse step of IVF), which synchronises its stream: they run each
+// non-root shard on a host thread.  Smaller ones never synchronise and are enqueued from the calling thread.
+constexpr int64_t kGroupInlineMaxQ = 4;
+
+// Search of a group: `host` says whether q / D / I are host buffers (else device buffers of the root, ordered on
+// `caller`).  Every shard gets the queries on its own stream (the root: `caller`, or its own for host buffers), then
+// either every shard searches with the exchange in its tail (root: into D / I) or, when the mailbox is too small or a
+// pair of GPUs has no peer access, every shard searches locally, copies its result to the root and the root merges.
+static int group_search(wb_group* g, wb_filter* const* filters, int64_t nq, const float* q, bool host, int64_t k,
+                        int64_t nprobe, float* D, int64_t* I, cudaStream_t caller) {
+    if (!g) return fail("NULL group");
+    const int n = (int)g->shards.size();
+    wb_index* h0 = g->shards[0];
+    auto filt = [&](int s) { return filters ? filters[s] : nullptr; };
+    if (n == 1)
+        return host ? search_host_entry(h0, nullptr, filt(0), nq, q, k, nprobe, D, I)
+                    : search_dev_entry(h0, nullptr, filt(0), nq, q, k, nprobe, D, I, caller);
+    // every check and allocation comes before the first launch: an argument error leaves no shard waiting
+    for (int s = 0; s < n; ++s) {
+        TRY(check_search_args(g->shards[s], nq, q, k, D, I));
+        TRY(check_filter(g->shards[s], filt(s)));
+        if (g->shards[s]->ivf && !g->shards[s]->trained) return fail("IndexIVFFlat is not trained");
+    }
+    if (nq == 0) return 0;
+    const bool exch = g->p2p && (size_t)nq <= g->ex[0]->nq_cap && (size_t)(nq * k) <= g->ex[0]->cap_entries;
+    const bool threaded = nq > kGroupInlineMaxQ;
+    const size_t dbytes = (size_t)nq * k * sizeof(float), ibytes = (size_t)nq * k * sizeof(int64_t);
+    cudaStream_t st[kExchMaxWorld];
+    const float* qs[kExchMaxWorld];
+    for (int s = 0; s < n; ++s) {
+        wb_index* h = g->shards[s];
+        st[s] = s ? h->stream : host ? h->stream : caller;
+        TRY(set_dev(h));
+        TRY(h->dbuf.ensure(dbytes));
+        TRY(h->ibuf.ensure(ibytes));
+        TRY(h->eD.ensure(dbytes));
+        TRY(h->eI.ensure(ibytes));
+    }
+    TRY(set_dev(h0));
+    if (!exch) {
+        TRY(g->pD.ensure(n * dbytes));
+        TRY(g->pI.ensure(n * ibytes));
+    }
+    if (!host) CK(cudaEventRecord(g->ev[0].get(), caller));
+    for (int s = 0; s < n; ++s) {
+        wb_index* h = g->shards[s];
+        TRY(set_dev(h));
+        if (host || s == 0) {
+            TRY(stage_queries(h, nq, q, host, st[s], &qs[s]));
+            continue;
+        }
+        // _dev: the copy waits for the caller's stream, and the caller's stream waits for the copy (so that a later
+        // write of q_dev cannot race it)
+        const size_t qbytes = (size_t)nq * h->d * sizeof(float);
+        TRY(g->qpeer[s].ensure(qbytes));
+        CK(cudaStreamWaitEvent(st[s], g->ev[0].get(), 0));
+        CK(cudaMemcpyPeerAsync(g->qpeer[s].get(), h->device, q, h0->device, qbytes, st[s]));
+        TRY(stage_queries(h, nq, g->qpeer[s].as<float>(), false, st[s], &qs[s]));
+        CK(cudaEventRecord(g->ev[s].get(), st[s]));
+    }
+    if (!host) {
+        TRY(set_dev(h0));
+        for (int s = 1; s < n; ++s) CK(cudaStreamWaitEvent(caller, g->ev[s].get(), 0));
+    }
+
+    // Shard s's search.  Exchange: the global top-k lands in (D0, I0) on the root and in eD / eI elsewhere.  Fallback:
+    // the local top-k lands in part s of (pD, pI) on the root.
+    auto part = [&](int s, float* D0, int64_t* I0) -> int {
+        wb_index* h = g->shards[s];
+        if (exch)
+            return group_exch_part(h, g->ex[s], filt(s), nq, qs[s], k, nprobe, s ? h->eD.as<float>() : D0,
+                                   s ? h->eI.as<int64_t>() : I0, st[s]);
+        TRY(set_dev(h));
+        float* Dl = s ? h->eD.as<float>() : g->pD.as<float>();
+        int64_t* Il = s ? h->eI.as<int64_t>() : g->pI.as<int64_t>();
+        TRY(search_dev_impl(h, filt(s), nq, qs[s], k, nprobe, Dl, Il, st[s]));
+        if (s == 0) return 0;
+        CK(cudaMemcpyPeerAsync(g->pD.as<unsigned char>() + s * dbytes, h0->device, Dl, h->device, dbytes, st[s]));
+        CK(cudaMemcpyPeerAsync(g->pI.as<unsigned char>() + s * ibytes, h0->device, Il, h->device, ibytes, st[s]));
+        CK(cudaEventRecord(g->ev[s].get(), st[s]));
+        return 0;
+    };
+    // Searches of 1-4 queries are enqueued on every GPU from this thread, root last (no thread hand-off on the latency
+    // path); larger batches run each non-root shard on its own thread.  Every shard runs even when another one failed.
+    auto run = [&](float* D0, int64_t* I0) -> int {
+        int rc = 0;
+        std::string err;
+        auto keep = [&](int r) {
+            if (r && !rc) {
+                rc = r;
+                err = g_err;
+            }
+        };
+        if (threaded) {
+            for (int s = 1; s < n; ++s) g->workers[s]->post([&part, s, D0, I0] { return part(s, D0, I0); });
+            keep(part(0, D0, I0));
+            for (int s = 1; s < n; ++s) keep(g->workers[s]->wait());
+        } else {
+            for (int s = n - 1; s >= 0; --s) keep(part(s, D0, I0));
+        }
+        if (rc) {
+            g_err = err;
+            return rc;
+        }
+        if (exch) return 0;
+        TRY(set_dev(h0));
+        for (int s = 1; s < n; ++s) CK(cudaStreamWaitEvent(st[0], g->ev[s].get(), 0));
+        return wb_merge_topk_dev(h0->device, nq, k, n, g->pD.as<float>(), g->pI.as<int64_t>(), D0, I0, st[0]);
+    };
+    if (!host) {
+        const int rc = run(D, I);
+        if (set_dev(h0) != 0) return 1;
+        return rc;
+    }
+    int rc = search_to_host(h0, nq, k, h0->eD, h0->eI, D, I, st[0], run);
+    std::string err = g_err;
+    for (int s = 1; s < n; ++s) {  // host calls return synchronised on every GPU
+        const cudaError_t e = cudaStreamSynchronize(st[s]);
+        if (e != cudaSuccess && !rc) {
+            rc = fail("group search: shard %d: %s", s, cudaGetErrorString(e));
+            err = g_err;
+        }
+    }
+    if (!rc && exch)
+        for (int s = 0; s < n; ++s)
+            if (*reinterpret_cast<volatile int*>(g->ex[s]->status.get()))
+                return fail("group search: GPU %d did not join the exchange within 20 s (results invalid)",
+                            g->shards[s]->device);
+    g_err = err;
+    if (set_dev(h0) != 0) return 1;
+    return rc;
+}
+
+extern "C" int wb_group_search(wb_group* g, wb_filter* const* filters, int64_t nq, const float* q_host, int64_t k,
+                               int64_t nprobe, float* D_host, int64_t* I_host) {
+    return group_search(g, filters, nq, q_host, true, k, nprobe, D_host, I_host, nullptr);
+}
+extern "C" int wb_group_search_dev(wb_group* g, wb_filter* const* filters, int64_t nq, const float* q_dev, int64_t k,
+                                   int64_t nprobe, float* D_dev, int64_t* I_dev, void* stream) {
+    return group_search(g, filters, nq, q_dev, false, k, nprobe, D_dev, I_dev, (cudaStream_t)stream);
+}
+
 // ---- range search (DESIGN.md "Range search") --------------------------------------------------------------------
 // A result owns its (D, I): in host memory (wb_range_search) or, one part per query chunk with hits, in device memory of
 // the index's GPU (wb_range_search_dev).  Either way it is independent of the index, its scratch and its lifetime.
@@ -2486,22 +2809,39 @@ static int find_positions(wb_index* h, void (*kernel)(const T*, int64_t, const i
     }
     return 0;
 }
+// Insertion positions of ids_host[0, m) into hpos (-1: absent), and on the device into h->idbuf[m, 2m).
+static int lookup_ids(wb_index* h, int64_t m, const int64_t* ids_host, int64_t* hpos) {
+    TRY(set_dev(h));
+    cudaStream_t st = h->stream;
+    TRY(h->idbuf.ensure((size_t)m * 2 * sizeof(int64_t)));
+    int64_t* tgt = h->idbuf.as<int64_t>();
+    unsigned long long* pos = reinterpret_cast<unsigned long long*>(tgt + m);
+    CK(cudaMemcpyAsync(tgt, ids_host, (size_t)m * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    TRY(find_positions(h, find_ids_kernel<int64_t>, h->ids.get(), tgt, m, pos, st));
+    CK(cudaMemcpyAsync(hpos, pos, (size_t)m * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int wb_lookup_ids(wb_index* h, int64_t m, const int64_t* ids_host, int64_t* pos_host) {
+    if (!h) return fail("NULL index");
+    if (m < 0) return fail("negative m");
+    if (m == 0) return 0;
+    if (!ids_host || !pos_host) return fail("NULL buffer");
+    return lookup_ids(h, m, ids_host, pos_host);
+}
+
 extern "C" int wb_reconstruct_batch(wb_index* h, int64_t m, const int64_t* ids_host, float* out_host) {
     if (!h) return fail("NULL index");
     if (m < 0) return fail("negative m");
     if (m == 0) return 0;
     if (!ids_host || !out_host) return fail("NULL buffer");
-    TRY(set_dev(h));
+    std::vector<int64_t> hpos((size_t)m);
+    TRY(lookup_ids(h, m, ids_host, hpos.data()));
     cudaStream_t st = h->stream;
-    TRY(h->idbuf.ensure((size_t)m * 2 * sizeof(int64_t)));
     TRY(h->xbuf.ensure((size_t)m * h->d * sizeof(float)));
     int64_t* tgt = h->idbuf.as<int64_t>();
     unsigned long long* pos = reinterpret_cast<unsigned long long*>(tgt + m);
-    CK(cudaMemcpyAsync(tgt, ids_host, (size_t)m * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    TRY(find_positions(h, find_ids_kernel<int64_t>, h->ids.get(), tgt, m, pos, st));
-    std::vector<int64_t> hpos((size_t)m);
-    CK(cudaMemcpyAsync(hpos.data(), pos, (size_t)m * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
     for (int64_t j = 0; j < m; ++j)
         if (hpos[j] < 0) return fail("reconstruct: id %lld not found in the index", (long long)ids_host[j]);
     if (h->row_pos) {  // grouped IVF store: insertion position -> storage row

@@ -76,7 +76,13 @@ def _write_flat(f, index, centroids: np.ndarray | None = None) -> None:
     n, d = index.ntotal, index.d
     _hdr(f, d, n, True, fc.METRIC_INNER_PRODUCT)
     f.write(struct.pack("<Q", n * d))
-    _stream_rows_out(f, index, 0, n)
+    for sh in _parts(index):  # a multi-GPU index: the shards in order are the rows in insertion order
+        _stream_rows_out(f, sh, 0, sh.ntotal)
+
+
+def _parts(index) -> list:
+    """The single-GPU indices that hold `index`'s rows, in insertion order."""
+    return index._shards if index._shards is not None else [index]
 
 
 def _stream_rows_out(f, index, start: int, n: int) -> None:
@@ -116,9 +122,11 @@ def write_index(index, fname: str) -> None:
             _hdr(f, index.d, n, True, fc.METRIC_INNER_PRODUCT)
             _write_flat(f, index)
             f.write(struct.pack("<Q", n))
-            for s in range(0, n, _CHUNK_ROWS):
-                _, ids, _ = index._export(s, min(_CHUNK_ROWS, n - s), want_x=False)
-                _write_array(f, ids)
+            for sh in _parts(index):
+                m = sh.ntotal
+                for s in range(0, m, _CHUNK_ROWS):
+                    _, ids, _ = sh._export(s, min(_CHUNK_ROWS, m - s), want_x=False)
+                    _write_array(f, ids)
         elif isinstance(index, fc.IndexFlatIP):
             _write_flat(f, index)
         elif isinstance(index, fc.IndexIVFFlat):
@@ -130,12 +138,14 @@ def write_index(index, fname: str) -> None:
 
 def _write_ivf(f, index) -> None:
     n, d, nlist = index.ntotal, index.d, index.nlist
+    parts = [sh for sh in _parts(index) if sh.ntotal]
     if n and index.is_trained:
         # group the row store list by list first (K8 on the device): every inverted list is then ONE contiguous run of
         # storage rows and is exported with one copy per chunk.  Without it (train, add, write - no search in between,
         # which is exactly /root/reference/src/index/feature_search_index.py:75-84) the rows are still in insertion order
         # and a list would be gathered row by row.
-        _capi.check(_capi.lib().wb_ivf_finalize(index._h))
+        for sh in parts:
+            _capi.check(_capi.lib().wb_ivf_finalize(sh._hd.h))
     f.write(b"IwFl")
     _hdr(f, d, n, index.is_trained, fc.METRIC_INNER_PRODUCT)
     f.write(struct.pack("<QQ", nlist, int(index.nprobe)))
@@ -143,21 +153,33 @@ def _write_ivf(f, index) -> None:
     # direct map: only the type byte and an (empty or sequential) array
     dm_type = index.direct_map.type
     f.write(struct.pack("<B", dm_type))
-    # list membership
-    assign = np.empty((n,), np.int32)
-    ids = np.empty((n,), np.int64)
-    for s in range(0, n, 1 << 20):
-        m = min(1 << 20, n - s)
-        _capi.check(_capi.lib().wb_export_rows(index._h, s, m, None, _capi.ptr(ids[s:s + m]), _capi.ptr(assign[s:s + m])))
-    order = np.argsort(assign, kind="stable")  # CSR: rows of each list in insertion order
-    sizes = np.bincount(assign, minlength=nlist).astype(np.uint64)
+    # list membership, per part: a list of a multi-GPU index is its rows of every shard in shard order, which is its
+    # rows in insertion order
+    members = []  # (part, ids, assign, order, sizes)
+    for sh in parts:
+        m_all = sh.ntotal
+        assign = np.empty((m_all,), np.int32)
+        ids = np.empty((m_all,), np.int64)
+        for s in range(0, m_all, 1 << 20):
+            m = min(1 << 20, m_all - s)
+            _capi.check(_capi.lib().wb_export_rows(sh._hd.h, s, m, None, _capi.ptr(ids[s:s + m]),
+                                                   _capi.ptr(assign[s:s + m])))
+        order = np.argsort(assign, kind="stable")  # CSR: rows of each list in insertion order
+        members.append((sh, ids, assign, order, np.bincount(assign, minlength=nlist).astype(np.uint64)))
+    sizes = np.zeros(nlist, np.uint64)
+    for *_, sz in members:
+        sizes += sz
     if dm_type == fc.DirectMap.Array:
         # lo_build(list, offset) = list << 32 | offset, indexed by id (ids are 0..n-1 here)
-        off_in_list = np.empty(n, np.int64)
-        starts = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
-        off_in_list[order] = np.arange(n, dtype=np.int64) - starts[assign[order]]
         arr = np.full(n, -1, np.int64)
-        arr[ids] = (assign.astype(np.int64) << 32) | off_in_list
+        before = np.zeros(nlist, np.int64)  # rows of each list in the earlier parts
+        for _, ids, assign, order, sz in members:
+            m_all = ids.shape[0]
+            off_in_list = np.empty(m_all, np.int64)
+            starts = np.concatenate([[0], np.cumsum(sz)[:-1]]).astype(np.int64)
+            off_in_list[order] = np.arange(m_all, dtype=np.int64) - starts[assign[order]]
+            arr[ids] = (assign.astype(np.int64) << 32) | (off_in_list + before[assign])
+            before += sz.astype(np.int64)
         f.write(struct.pack("<Q", n))
         f.write(arr.tobytes())
     else:
@@ -175,19 +197,24 @@ def _write_ivf(f, index) -> None:
         pairs = np.stack([nz, sizes[nz]], axis=1).reshape(-1)
         f.write(struct.pack("<Q", pairs.size))
         f.write(pairs.tobytes())
-    pos = 0
+    pos = [0] * len(members)
     for l in range(nlist):
-        m = int(sizes[l])
-        if m == 0:
+        if int(sizes[l]) == 0:
             continue
-        rows = order[pos:pos + m]
-        pos += m
-        if m > 4096 and rows[-1] - rows[0] == m - 1:  # one long contiguous run (a finalized store): pinned streaming
-            _stream_rows_out(f, index, int(rows[0]), m)
-        else:
-            for s in range(0, m, _CHUNK_ROWS):
-                _write_array(f, _gather_rows(index, rows[s:s + _CHUNK_ROWS]))
-        _write_array(f, ids[rows])
+        runs = []
+        for j, (sh, ids, _, order, sz) in enumerate(members):
+            m = int(sz[l])
+            runs.append((sh, ids, order[pos[j]:pos[j] + m]))
+            pos[j] += m
+        for sh, _, rows in runs:
+            m = rows.shape[0]
+            if m > 4096 and rows[-1] - rows[0] == m - 1:  # one long contiguous run (a finalized store): pinned streaming
+                _stream_rows_out(f, sh, int(rows[0]), m)
+            else:
+                for s in range(0, m, _CHUNK_ROWS):
+                    _write_array(f, _gather_rows(sh, rows[s:s + _CHUNK_ROWS]))
+        for _, ids, rows in runs:
+            _write_array(f, ids[rows])
 
 
 def _gather_rows(index, rows: np.ndarray) -> np.ndarray:
@@ -245,17 +272,17 @@ def _stream_rows_in(f, index, d: int, n: int, rows_at: int, ids_at: int | None) 
         for i, s0 in enumerate(range(0, n, chunk)):
             m = min(chunk, n - s0)
             slot = i % RING
-            _capi.check(L.wb_add_slot_wait(index._h, slot))
+            index._slot_wait(slot)
             f.seek(rows_at + s0 * d * 4)
             _readinto(f, ring.x[slot][:m])
             if ids_at is not None:
                 f.seek(ids_at + s0 * 8)
                 _readinto(f, ring.ids[slot][:m])
-            _capi.check(L.wb_add_with_ids_pinned(index._h, m, _capi.ptr(ring.x[slot]),
-                                                 _capi.ptr(ring.ids[slot]) if ids_at is not None else None, slot))
-        _capi.check(L.wb_sync(index._h))
+            index._add_pinned(m, ring.x[slot], ring.ids[slot] if ids_at is not None else None, slot,
+                              pos_buf=ring.ids[slot])
+        index._sync()
     finally:
-        L.wb_sync(index._h)
+        index._sync(check=False)
         ring.close()
 
 
@@ -306,7 +333,6 @@ def _read_ivf_lists(f, index, d: int, sizes: np.ndarray) -> None:
     into one pinned buffer together with their list number and handed to wb_ivf_add_preassigned_pinned, which only
     enqueues - a build with tens of thousands of short lists no longer pays one synchronous call per list."""
     from .ingest import PinnedRing, RING
-    L = _capi.lib()
     total = int(sizes.sum())
     if total == 0:
         return
@@ -317,11 +343,10 @@ def _read_ivf_lists(f, index, d: int, sizes: np.ndarray) -> None:
     def flush():
         slot = state["i"] % RING
         if state["fill"]:
-            _capi.check(L.wb_ivf_add_preassigned_pinned(index._h, state["fill"], _capi.ptr(ring.x[slot]),
-                                                        _capi.ptr(ring.ids[slot]), _capi.ptr(ring.assign[slot]), slot))
+            index._add_pinned(state["fill"], ring.x[slot], ring.ids[slot], slot, assign=ring.assign[slot])
         state["i"] += 1
         state["fill"] = 0
-        _capi.check(L.wb_add_slot_wait(index._h, state["i"] % RING))
+        index._slot_wait(state["i"] % RING)
 
     try:
         for l in range(sizes.shape[0]):
@@ -336,9 +361,9 @@ def _read_ivf_lists(f, index, d: int, sizes: np.ndarray) -> None:
             ring.assign[slot][o:o + m] = l
             state["fill"] = o + m
         flush()
-        _capi.check(L.wb_sync(index._h))
+        index._sync()
     finally:
-        L.wb_sync(index._h)
+        index._sync(check=False)
         ring.close()
 
 

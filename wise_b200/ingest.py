@@ -64,7 +64,6 @@ def add_store_pipelined(index, store) -> int:
     Threads: the helper thread only decodes and calls wb_add_slot_wait (an event wait on a slot the main thread is not
     using); every call that changes the index (wb_add_with_ids_pinned, add_with_ids) is made by the calling thread, in
     shard order, and the future hand-off orders the two."""
-    L = _capi.lib()
     files = list(store.shard_files())
     rows_by = getattr(store, "_shard_rows", {})
     if not files:
@@ -72,12 +71,11 @@ def add_store_pipelined(index, store) -> int:
     cap = max([rows_by.get(fn, 0) for fn in files] + [1])
     d = store.feature_dim
     ring = PinnedRing(cap, d)
-    h = index._h
     added = 0
 
     def decode(i):
         slot = i % RING
-        _capi.check(L.wb_add_slot_wait(h, slot))  # the GPU has finished reading this buffer (two shards ago)
+        index._slot_wait(slot)  # the GPU has finished reading this buffer (two shards ago)
         return store.decode_shard_into(files[i], ring.ids[slot], ring.x[slot])
 
     try:
@@ -94,11 +92,11 @@ def add_store_pipelined(index, store) -> int:
                         index.add_with_ids(np.ascontiguousarray(x, np.float32), np.ascontiguousarray(ids, np.int64))
                     added += len(ids)
                     continue
-                if n:
-                    _capi.check(L.wb_add_with_ids_pinned(h, n, _capi.ptr(ring.x[slot]), _capi.ptr(ring.ids[slot]), slot))
+                if n:  # (a multi-GPU index splits the shard at its shard boundaries)
+                    index._add_pinned(n, ring.x[slot], ring.ids[slot], slot)
                 added += n
-        _capi.check(L.wb_sync(h))
+        index._sync()
     finally:
-        L.wb_sync(h)
+        index._sync(check=False)
         ring.close()
     return added

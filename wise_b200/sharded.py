@@ -36,10 +36,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-
-def shard_range(n_total: int, rank: int, world: int) -> tuple[int, int]:
-    """Contiguous row range [lo, hi) of `rank` (balanced to within one row)."""
-    return n_total * rank // world, n_total * (rank + 1) // world
+from .routing import shard_range  # noqa: F401  (part of this module's interface)
 
 
 def _cuda_local_search(index, q: torch.Tensor, k: int, nprobe: int, flt=None):
