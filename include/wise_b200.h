@@ -292,7 +292,7 @@ int wb_tar_read(const char* path, int64_t d, int64_t cap, int64_t* ids_host, flo
  * pair; sustained (optional) = the second half of `reps` back-to-back launches, i.e. under the settled power cap. */
 int wb_tf32_peak(int device, int iters, int reps, double* tflops_burst_out, double* tflops_sustained_out);
 /* Device pointer and row stride (floats) of the resident row store, for reading.  Writing rows through it is not
- * supported: the bf16 image that 1-2 query flat searches stream would no longer match the rows. */
+ * supported: the int8 image that 1-2 query flat searches stream would no longer match the rows. */
 int wb_storage(wb_index* h, void** rows_dev, int64_t* ld);
 /* Number of this library's kernels launched on behalf of `h` since creation. */
 int64_t wb_launch_count(const wb_index* h);
@@ -303,10 +303,12 @@ int wb_gemm_stats(const wb_index* h, int64_t* epochs, int64_t* fallbacks);
  * of IndexIVF::search, reached from /root/reference/src/index/feature_search_index.py:113) is the prologue of the list
  * scan.  Number of searches served that way so far (the others took the coarse scan + list scan launches). */
 int64_t wb_ivf_fused_searches(const wb_index* h);
-/* Flat searches of 1-2 queries over a large store stream a bf16 image of it and re-score the candidates exactly in
+/* Flat searches of 1-2 queries over a large store stream an int8 image of it and re-score the candidates exactly in
  * fp32: the number of searches served by the image so far, and the (row, query) pairs they re-scored.  Waits for the
- * device. */
+ * device.  (The name predates the int8 image, which replaced a bf16 one.) */
 int wb_flat_bf16_stats(wb_index* h, int64_t* searches, int64_t* rescored);
+/* Device bytes held by that image: 0 until a search builds it, then capacity x (16 + d rounded up to 16). */
+int64_t wb_flat_image_bytes(const wb_index* h);
 /* The CUDA-core scan plan of a search of nq queries with k results (k = 0: a range search) over the whole store
  * (gather = 0) or over nprobe probed lists (gather = 1): out = {queries per CTA, rows per warp, floats per staged row
  * chunk, chunks per row, ring stages}.  Chunks per row > 1 is the fallback for rows too wide for two whole-row stages.

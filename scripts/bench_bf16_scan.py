@@ -1,4 +1,4 @@
-"""The bf16 filter of K1 on bench.py's flagship store (10M x 768 clustered rows, top-100): per search of 1 and 2
+"""The int8 filter of K1 on bench.py's flagship store (10M x 768 clustered rows, top-100): per search of 1 and 2
 queries, the image bytes streamed, the (row, query) pairs re-scored in fp32 (wb_flat_bf16_stats), the bytes actually
 read (image + re-scored rows) over the scan kernel's time, and the image's memory.  One JSON line per batch size.
 
@@ -51,7 +51,7 @@ def main():
     L.wb_set_timing(index._h, 1)
     search = ShardedIndex(index).search_dev  # device queries in, device (D, I) out: the path bench.py times
     ld = (a.dim + 3) & ~3
-    ldh = (ld + 7) & ~7
+    row_bytes = 16 + ((ld + 15) & ~15)  # img_row_bytes (scan.cuh): a 16-byte header and the codes
 
     def stats():
         s, r = C.c_int64(0), C.c_int64(0)
@@ -72,7 +72,7 @@ def main():
         buf = (C.c_float * 128)()
         n = L.wb_scan_ms_history(index._h, buf, min(a.searches, 128))
         scan_ms = float(np.mean([buf[i] for i in range(n)]))
-        img_bytes = a.rows * ldh * 2
+        img_bytes = a.rows * row_bytes
         pairs = (r1 - r0) / max(1, s1 - s0)
         read = img_bytes + pairs * ld * 4  # a pair re-scored reads its fp32 row (from L2 when queries share it)
         line = {"batch": nq, "searches_on_image": s1 - s0, "searches": a.searches, "scan_ms": scan_ms,

@@ -96,6 +96,7 @@ SIGNATURES = {
     "wb_phase_stamps": (C.c_int, [_vp, _vp, C.c_int]),
     "wb_gemm_stats": (C.c_int, [_vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "wb_flat_bf16_stats": (C.c_int, [_vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "wb_flat_image_bytes": (C.c_int64, [_vp]),
     "wb_set_timing": (C.c_int, [_vp, C.c_int]),
     "wb_last_scan_ms": (C.c_float, [_vp]),
     "wb_scan_ms_history": (C.c_int, [_vp, _f32p, C.c_int]),

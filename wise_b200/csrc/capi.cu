@@ -141,16 +141,17 @@ struct wb_index {
     DevPtr<int64_t> ids;
     DevPtr<int32_t> assign;  // IVF: list of each row
     int64_t n = 0, cap = 0;
-    DevPtr<float> norm2_max;  // device scalar: max |row|^2 over everything ever added (K2 and bf16 filter margins)
-    // bf16 image of a flat store (the filter rows of 1-2 query scans, DESIGN.md "K1"): row r is rows[r] rounded to bf16,
-    // stride ld rounded up to 8, padding zero; img_cap rows allocated.  Built lazily by the first search that uses it:
+    DevPtr<float> norm2_max;  // device scalar: max |row|^2 over everything ever added (K2 filter margin)
+    // int8 image of a flat store (the filter rows of 1-2 query scans, DESIGN.md "K1"): row r is the header and int8 codes
+    // of rows[r] (int8_image_kernel), stride img_row_bytes(ld); img_cap rows allocated.  Built lazily by the first search
+    // that uses it:
     // rows [img_n, n) are converted before such a search.  Rows reach the store only through add_common (appended at
     // n), which keeps img_n <= n right; anything that rewrites or removes stored rows must reset img_n to 0.
-    DevPtr<uint16_t> img;
+    DevPtr<uint8_t> img;
     int64_t img_n = 0, img_cap = 0;
     cudaEvent_t img_ev = nullptr;    // recorded after the last conversion, on img_st: searches on other streams wait
     cudaStream_t img_st = nullptr;
-    DevPtr<unsigned long long> img_rescored;  // device counter: (row, query) pairs the bf16 filter re-scored
+    DevPtr<unsigned long long> img_rescored;  // device counter: (row, query) pairs the int8 filter re-scored
     int64_t img_searches = 0;                 // searches served by the image
     // IVF quantizer + inverted lists.  `ids` always stay in INSERTION order.  After a (re)grouping the rows are
     // stored list by list (insertion order kept inside a list): row_pos[row] is then the insertion position of a
@@ -294,6 +295,9 @@ extern "C" int wb_flat_bf16_stats(wb_index* h, int64_t* searches, int64_t* resco
     if (rescored) *rescored = (int64_t)r;
     return 0;
 }
+extern "C" int64_t wb_flat_image_bytes(const wb_index* h) {
+    return h ? h->img_cap * img_row_bytes(h->ld) : 0;
+}
 extern "C" int wb_set_timing(wb_index* h, int on) {
     if (!h) return fail("NULL index");
     h->timing = on != 0;
@@ -400,8 +404,8 @@ static int env_int(const char* name, int dflt) {
 }
 
 // Pick queries-per-CTA, rows-per-warp and ring depth so that everything fits the 227 KB of
-// shared memory: [ring | queries | top-k lists + queues | barriers].  `img`: the ring holds rows of the bf16 image
-// (ck = half the image's row length, in floats); whole-row stages only.
+// shared memory: [ring | queries | top-k lists + queues | barriers].  `img`: the ring holds rows of the int8 image
+// (ck = the image's row length img_row_bytes(ld), in floats); whole-row stages only.
 // Measured on B200 (profiles/r01_scan_sweep.md): one bulk copy engine request costs the producer
 // ~27 cycles, so stages hold WHOLE rows - a flat row group is then one contiguous copy (7.2 TB/s);
 // chunked stages (one 1 KB copy per row and chunk) top out at 4.0 TB/s and are only the fallback
@@ -412,18 +416,17 @@ static int plan_scan(const wb_index* h, int64_t nq, int k, bool gather, int npro
     int NQ = gather ? 1 : (nq >= 8 ? 8 : nq > 2 ? 4 : nq > 1 ? 2 : 1);
     const int P = pow2_ceil(k + kMinQueue);
     const int np = gather ? nprobe : 0;
-    const int ldq = img ? (ld + 7) & ~7 : ld;  // query stride in shared memory
-    const int rowf = img ? ldq / 2 : ld;       // ring floats per row
+    const int rowf = img ? img_row_bytes(ld) / 4 : ld;  // ring floats per row
     for (; NQ >= 1; NQ >>= 1) {
         for (int RW = kMaxRowsPerWarp; RW >= 1; RW >>= 1) {  // whole-row stages
             const int gr = kConsumerWarps * RW;
-            const size_t fixed = scan_smem_layout(NQ, ldq, P, rowf, 0, np, gr, img).total;
+            const size_t fixed = scan_smem_layout(NQ, ld, P, rowf, 0, np, gr, img).total;
             const size_t stage_bytes = (size_t)gr * rowf * 4;
             if (fixed + 2 * stage_bytes + 64 > (size_t)h->smem_max) continue;
             if (stage_bytes >= (1u << 20)) continue;  // mbarrier tx-count limit
             const int stages = (int)std::min<size_t>(kMaxStages, ((size_t)h->smem_max - fixed - 64) / (stage_bytes + 24));
             *c = ScanCfg{NQ, RW, P, rowf, 1, stages, gather ? 0 : 1, 0};
-            c->smem = scan_smem_layout(NQ, ldq, P, rowf, stages, np, gr, img).total;
+            c->smem = scan_smem_layout(NQ, ld, P, rowf, stages, np, gr, img).total;
             return 0;
         }
         if (img) continue;
@@ -521,14 +524,14 @@ static cudaError_t launch_scan_coop(const ScanCfg& c, ScanParams& p, dim3 grid, 
     });
 }
 
-// p.img set: the bf16 filter instance (flat, NQ <= 2)
+// p.img set: the int8 filter instance (flat, NQ <= 2)
 static int launch_scan(const ScanCfg& c, bool gather, ScanParams& p, dim3 grid, cudaStream_t st) {
     apply_scan_cfg(c, p);
     return with_scan_instance(c.NQ, c.RW, gather, [&](auto NQ, auto RW, auto G) {
         if constexpr (!G && NQ <= 2) {
             if (p.img) return launch<scan_topk_kernel<NQ, RW, false, true>>(grid, kScanThreads, c.smem, st, p);
         }
-        if (p.img) return fail("no bf16 filter scan for NQ %d", (int)NQ);
+        if (p.img) return fail("no int8 filter scan for NQ %d", (int)NQ);
         return launch<scan_topk_kernel<NQ, RW, G>>(grid, kScanThreads, c.smem, st, p);
     });
 }
@@ -666,23 +669,24 @@ static int run_scan_groups(wb_index* h, const ScanCfg& c, bool gather, ScanParam
 
 constexpr size_t kMemReserve = (size_t)1 << 30;  // free device memory an optional copy of the rows must leave
 
-// The bf16 filter pays a fixed cost per CTA - its first few hundred rows are re-scored while the threshold is still
-// loose, 32 latency-bound rows at a time - and saves half the bytes of every row.  Measured on a B200 (1000 W, 1965 MHz
-// max SM clock; profiles/r03): one query over 100k x 512 took 110 us on the image against 59 us in fp32, 1M x 768 was
-// even (0.44 ms), 2.5M x 768 0.82 against 1.06 ms, 10M x 768 2.60-2.72 against 4.11 ms.  Batches of 3-4 queries were slower on the image (4.35-4.50 ms against ~4.1 at
-// 10M x 768: four queries double the shared-memory reads per byte), so the image serves 1-2 queries.
-constexpr int64_t kImageMinRowsPerSm = 16384;
+// The int8 filter pays a fixed cost per CTA - its first few hundred rows are re-scored while the threshold is still
+// loose, 32 latency-bound rows at a time - and saves three quarters of the bytes of every row.  Measured on a B200
+// (1000 W, 1965 MHz max SM clock; profiles/r05), one query over N x 768, image against the fp32 scan: 0.5M rows (3378
+// per SM) 0.285 against 0.242 ms, 1M (6757 per SM) 0.418 against 0.449 ms, 1.5M 0.538 against 0.653 ms.  The cutoff
+// sits just below the smallest store measured to gain.  Batches of 3-4 queries were slower on the bf16 image that
+// preceded this one (four queries double the shared-memory reads per byte), so the image serves 1-2 queries.
+constexpr int64_t kImageMinRowsPerSm = 6144;
 constexpr int64_t kImageMaxQueries = 2;
 
-// Bring the bf16 image of a flat store up to date for a search on `st` (rows [img_n, n) converted on `st`).  *ok =
+// Bring the int8 image of a flat store up to date for a search on `st` (rows [img_n, n) converted on `st`).  *ok =
 // false when the image does not fit: it is allocated at the store's capacity only if that leaves kMemReserve free
 // (else the index keeps no image); a failed allocation leaves the handle as it was.
 static int ensure_image(wb_index* h, cudaStream_t st, bool* ok) {
     *ok = false;
     if (h->n == 0) return 0;
-    const int ldh = (h->ld + 7) & ~7;
+    const int rb = img_row_bytes(h->ld);
     if (h->n > h->img_cap) {
-        const size_t bytes = (size_t)h->cap * ldh * 2;
+        const size_t bytes = (size_t)h->cap * rb;
         size_t free_b = 0, total_b = 0;
         CK(cudaMemGetInfo(&free_b, &total_b));
         if (free_b < bytes + kMemReserve) {
@@ -690,7 +694,7 @@ static int ensure_image(wb_index* h, cudaStream_t st, bool* ok) {
             h->img_cap = h->img_n = 0;
             return 0;
         }
-        DevPtr<uint16_t> img;
+        DevPtr<uint8_t> img;
         if (dev_alloc(&img, bytes) != cudaSuccess) {
             cudaGetLastError();  // (clear the allocation error: the next launch check would report it)
             return 0;
@@ -707,9 +711,9 @@ static int ensure_image(wb_index* h, cudaStream_t st, bool* ok) {
     }
     if (!h->img_ev) CK(cudaEventCreateWithFlags(&h->img_ev, cudaEventDisableTiming));
     if (h->img_n < h->n) {
-        const int64_t m = h->n - h->img_n, tot = m * (ldh / 8);
-        bf16_image_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(h->rows.get() + (size_t)h->img_n * h->ld, h->ld,
-                                                                        ldh, m, h->img.get() + (size_t)h->img_n * ldh);
+        const int64_t m = h->n - h->img_n;  // one warp per row
+        int8_image_kernel<<<(unsigned)((m + 7) / 8), 256, 0, st>>>(h->rows.get() + (size_t)h->img_n * h->ld, h->ld, rb, m,
+                                                                  h->img.get() + (size_t)h->img_n * rb);
         CK(cudaGetLastError());
         CK(cudaEventRecord(h->img_ev, st));
         h->launches++;
@@ -724,7 +728,7 @@ static int ensure_image(wb_index* h, cudaStream_t st, bool* ok) {
 
 // Exhaustive top-k of `nq` device queries (row stride ld) against `nrows` rows: K1 with the K3 merge (and, when `ex`
 // is given, the multi-GPU exchange) fused into its tail; K1 + K3 as two launches when the tail cannot be fused.
-// A search of 1-2 queries over a flat store's own rows, when the store is large, streams its bf16 image and re-scores
+// A search of 1-2 queries over a flat store's own rows, when the store is large, streams its int8 image and re-scores
 // the candidates in fp32 (DESIGN.md "K1"); the fp32 scan serves everything else, and searches whose image does not fit.
 static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const float* q_dev, int64_t nq, int k,
                          const int64_t* ids, float* D, int64_t* I, cudaStream_t st, bool timed,
@@ -746,7 +750,6 @@ static int run_flat_scan(wb_index* h, const float* rows, int64_t nrows, const fl
     p.allow = mask ? mask->allow : nullptr;
     if (img) {
         p.img = h->img.get();
-        p.norm2_max = h->norm2_max.get();
         p.rescored = h->img_rescored.get();
         h->img_searches++;
     }

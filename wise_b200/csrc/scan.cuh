@@ -20,13 +20,14 @@
 //     query at the end, merged by merge_topk_kernel (merge.cuh).
 //   * range mode (scan_range_kernel, range search): the same scan with a fixed threshold; every hit is staged in the
 //     shared lists and flushed to a global pool (RangeOut) instead of the fused top-k (DESIGN.md "Range search").
-//   * bf16 filter (flat top-k of 1-2 queries, DESIGN.md "K1"): the ring streams the bf16 image of the rows instead, the
-//     consumers score it approximately, and only the (row, query) pairs whose approximation can reach the threshold
-//     are queued and re-scored from the fp32 rows with the arithmetic of the fp32 scan; every CTA's list is therefore
-//     the top-k of the exact keys of its rows, as without the filter.
-// Algorithmic bytes per launch: nrows * ld * 4 (the row store is read exactly once per pass); with the bf16 filter
-// nrows * ld * 2 plus the re-scored rows.
+//   * int8 filter (flat top-k of 1-2 queries, DESIGN.md "K1"): the ring streams the int8 image of the rows instead,
+//     the consumers score it approximately, and only the (row, query) pairs whose approximation can reach the
+//     threshold are queued and re-scored from the fp32 rows with the arithmetic of the fp32 scan; every CTA's list is
+//     therefore the top-k of the exact keys of its rows, as without the filter.
+// Algorithmic bytes per launch: nrows * ld * 4 (the row store is read exactly once per pass); with the int8 filter
+// nrows * img_row_bytes(ld) plus the re-scored rows.
 #pragma once
+#include <cuda_fp16.h>
 #include "coarse.cuh"
 #include "exchange.cuh"
 #include "filter.cuh"
@@ -92,21 +93,27 @@ struct ScanParams {
     // 10-13 inside block_merge_heads: staged, T0 found, candidates compacted, ranked
     unsigned long long* phase_ts;
     ExchParams exch;
-    // bf16 filter (scan_topk_kernel<..., IMG = true>): `img` is the bf16 image of `rows`, row stride 2 * ck bf16 (a
-    // multiple of 8, zero padded); `rows` is read only to re-score the queued candidates
-    const uint16_t* img;
-    const float* norm2_max;          // device scalar: max |row|^2 over the store (the filter's error bound)
+    // int8 filter (scan_topk_kernel<..., IMG = true>): `img` is the int8 image of `rows` (int8_image_kernel), row
+    // stride img_row_bytes(ld) = 4 * ck; `rows` is read only to re-score the queued candidates
+    const uint8_t* img;
     unsigned long long* rescored;    // += (row, query) pairs re-scored by this launch
 };
 
-constexpr int kRescoreCap = 256;    // queued (row, query) pairs of the bf16 filter per CTA
+constexpr int kRescoreCap = 256;    // queued (row, query) pairs of the int8 filter per CTA
 constexpr int kRescoreChunk = 32;   // pairs re-scored per insertion round: 4 rows in flight per consumer warp
+
+// A row of the int8 image: a 16-byte header {s, resid, xhat, 0} (fp32) and the codes u_i = n_i + 128 (n_i in
+// [-127, 127], offset binary), zero codes (128) up to a multiple of 16 bytes.  The row's approximation is s * n;
+// resid >= |x - s n| and xhat >= |s n| (both rounded up); s is NaN for a row with a NaN or Inf element.
+constexpr int kImgHeader = 16;
+__host__ __device__ inline int img_row_bytes(int ld) { return kImgHeader + ((ld + 15) & ~15); }
 
 struct ScanSmem {
     size_t ring, queries, lists, bars, misc, prefix, rescore, total;
 };
 
-// `ld`: stride of the queries in shared memory (floats).  `rescore`: the bf16 filter's queue and margins.
+// `ld`: stride of the queries in shared memory (floats).  `rescore`: the int8 filter's queue, per-query margin terms
+// (8 floats) and fp16 queries (img_row_bytes(ld) - kImgHeader halves each).
 __host__ __device__ inline ScanSmem scan_smem_layout(int NQ, int ld, int P, int ck, int stages, int nprobe,
                                                      int group_rows, bool rescore = false) {
     ScanSmem L;
@@ -120,7 +127,7 @@ __host__ __device__ inline ScanSmem scan_smem_layout(int NQ, int ld, int P, int 
     o = (o + 7) & ~(size_t)7;
     L.prefix = o;  o += nprobe > 0 ? (size_t)nprobe * 8 + (size_t)(nprobe + 1) * 4 : 0;  // pbase[np] i64 + prefix[np+1] u32
     o = (o + 15) & ~(size_t)15;
-    L.rescore = o; o += rescore ? (size_t)kRescoreCap * 8 + (size_t)NQ * 4 + 16 : 0;  // queue [cap] u64 + margin[NQ] + count
+    L.rescore = o; o += rescore ? (size_t)kRescoreCap * 8 + (size_t)NQ * (32 + 2 * (img_row_bytes(ld) - kImgHeader)) + 16 : 0;
     L.total = (o + 15) & ~(size_t)15;
     return L;
 }
@@ -251,20 +258,41 @@ __device__ __forceinline__ void exact_scores(const float* rows, int ld, const fl
         for (int j = 0; j < J; ++j) a[j] += __shfl_xor_sync(0xffffffffu, a[j], o);
 }
 
-// bf16 -> fp32 of the low / high half of a word of two packed bf16 values (element 2i is the low half)
-__device__ __forceinline__ float bf16_lo(uint32_t w) { return __uint_as_float(w << 16); }
-__device__ __forceinline__ float bf16_hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }
+// a + the dot product of 8 image codes (offset binary, element 8i + j in byte j) with 8 fp16 query elements, in fp32.
+// PRMT puts two codes u under the exponent byte of fp16 1024 (0x64: 1024 + u exactly), HADD2 subtracts 1152 (exact
+// fp16 n = u - 128), and fma.rn.f32.f16 (FHFMA) adds the exact product n q to the fp32 sum with one rounding: 2
+// instructions per element at one query, 3 at two (the unpack is shared).
+__device__ __forceinline__ float fma_f32_f16(uint32_t a, uint32_t b, bool hi, float c) {
+    const uint16_t x = (uint16_t)(hi ? a >> 16 : a), y = (uint16_t)(hi ? b >> 16 : b);
+    float d;
+    asm("fma.rn.f32.f16 %0, %1, %2, %3;" : "=f"(d) : "h"(x), "h"(y), "f"(c));
+    return d;
+}
+__device__ __forceinline__ float dot8_i8_f16(uint2 x, uint4 q, float a) {
+    const uint32_t w[2] = {x.x, x.y}, qw[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+    for (int h = 0; h < 4; ++h) {
+        uint32_t v = __byte_perm(w[h >> 1], 0x64646464u, (h & 1) ? 0x7342 : 0x5140);
+        const __half2 n = __hsub2(*reinterpret_cast<const __half2*>(&v), __half2half2(__ushort_as_half(0x6480)));
+        v = *reinterpret_cast<const uint32_t*>(&n);
+        a = fma_f32_f16(v, qw[h], false, a);
+        a = fma_f32_f16(v, qw[h], true, a);
+    }
+    return a;
+}
+
+// 2^e as an fp32, e in [-126, 127]
+__device__ __forceinline__ float pow2f(int e) { return __uint_as_float((uint32_t)(e + 127) << 23); }
 
 template <int NQ, int RW, bool GATHER, bool RANGE, bool IMG = false>
 __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& ro) {
-    static_assert(!(IMG && (GATHER || RANGE)), "the bf16 filter serves flat top-k scans only");
+    static_assert(!(IMG && (GATHER || RANGE)), "the int8 filter serves flat top-k scans only");
     constexpr int kRowsPerWarp = RW;
     constexpr int kGroupRows = kConsumerWarps * RW;
     extern __shared__ __align__(128) unsigned char smem_scan[];
     unsigned char* smem = smem_scan;
-    // queries in shared memory: stride ld, or with the bf16 filter the image's row length 2 * ck (zero padded)
-    const int ldq = IMG ? 2 * p.ck : p.ld, dq4 = ldq >> 2;
-    const ScanSmem L = scan_smem_layout(NQ, ldq, p.P, p.ck, p.stages, GATHER ? p.nprobe : 0, kGroupRows, IMG);
+    const int dq4 = p.ld >> 2;  // queries in shared memory: stride ld
+    const ScanSmem L = scan_smem_layout(NQ, p.ld, p.P, p.ck, p.stages, GATHER ? p.nprobe : 0, kGroupRows, IMG);
     float* ring = reinterpret_cast<float*>(smem + L.ring);
     float* qs = reinterpret_cast<float*>(smem + L.queries);
     uint64_t* lists = reinterpret_cast<uint64_t*>(smem + L.lists);
@@ -275,9 +303,11 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
     float* thr_s = reinterpret_cast<float*>(smem + L.misc) + NQ;
     int64_t* pbase = reinterpret_cast<int64_t*>(smem + L.prefix);
     uint32_t* prefix = reinterpret_cast<uint32_t*>(pbase + (GATHER ? p.nprobe : 0));
-    uint64_t* rq = reinterpret_cast<uint64_t*>(smem + L.rescore);  // bf16 filter: queued (row << 8 | query) pairs
-    float* margin_s = reinterpret_cast<float*>(rq + kRescoreCap);   // [NQ]
-    int* rq_cnt = reinterpret_cast<int*>(margin_s + NQ);
+    uint64_t* rq = reinterpret_cast<uint64_t*>(smem + L.rescore);  // int8 filter: queued (row << 8 | query) pairs
+    float* qc_s = reinterpret_cast<float*>(rq + kRescoreCap);       // [NQ][8] margin terms and scale of each query
+    const int nc8 = (4 * p.ck - kImgHeader) >> 3;                   // int8 filter: 8-code words per image row
+    uint4* qh_s = reinterpret_cast<uint4*>(qc_s + NQ * 8);          // [NQ][nc8] fp16 queries, 8 per uint4
+    int* rq_cnt = reinterpret_cast<int*>(qh_s + NQ * nc8);
 
     const int tid = threadIdx.x;
     const int warp = tid >> 5, lane = tid & 31;
@@ -442,7 +472,7 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
                     if (dyn) stage_group[s] = g;  // published to the consumers by the arrive below
                 }
                 __syncwarp();
-                const int cfl = min(ck, ld - ch * ck);
+                const int cfl = IMG ? ck : min(ck, ld - ch * ck);
                 const uint32_t cbytes = (uint32_t)cfl * 4u;
                 if (lane == 0) mbar_arrive_expect_tx(&full[s], cbytes * (uint32_t)nvalid);
                 __syncwarp();
@@ -497,30 +527,69 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
             }
             named_bar_sync(kBarConsumers, kConsumerThreads);
         };
-        // bf16 filter.  Error bound of an approximate score (the image and the query in fp32, DESIGN.md "K1"):
-        //   |exact - approx| <= (2^-8 + ld 2^-23 1.1 + 1e-5) |q| sqrt(norm2_max)   one bf16 rounding of every element,
-        //                                                                          both fp32 sums, their comparison
-        //                       + 2^-134 (sqrt(ld) |q| + ld)                       rows with fp32-subnormal elements
-        // times 1.001 for the rounding of |q| and of the margin itself.  |q|^2 and norm2_max are fp32 sums of squares
-        // that may underflow (elements below ~1e-19): ld 2^-149 added to each bounds what the underflow lost, so a store
-        // of tiny rows keeps a margin of their true size.  A NaN row does not enter norm2_max (its
-        // approximation is NaN and is re-scored); norm2_max = +Inf (a |row|^2 overflowed) or a NaN query makes the margin
-        // Inf or NaN and every row is re-scored.  One warp per query, before the first group.
+        // int8 filter.  Row x has the image s n (header: s, resid >= |x - s n|, xhat >= |s n|); query q is scaled by
+        // 2^e (e per query: max |q_i| 2^e in [2^14, 2^15), e <= 126) and rounded to fp16, q^ = fp16(q 2^e), and the
+        // approximation is approx = s 2^-e (q^ . n), the dot product summed in fp32 from exact products (FHFMA).  With
+        // q' = 2^-e q^ and h = ld + 64 (the depth of every summation tree of the fp32 scan and of this sum, butterfly
+        // included), gamma = 1.01 h 2^-24:
+        //   |exact - approx| <= |q| resid                          quantisation residual: q . (x - s n)
+        //                     + |q - q'| xhat                       query rounding: (q - q') . s n
+        //                     + gamma |q| (resid + xhat)            the fp32 scan's sum (|x| <= resid + xhat)
+        //                     + gamma |q'| xhat                     the fp32 sum of q^ . n (scaled by s 2^-e)
+        //                     + 2^-21 |q'| xhat                     the two products forming approx, approx + margin
+        //                     + h 2^-148                            underflow: every rounding above that lands below
+        //                                                           2^-126 errs by at most 2^-150 absolute
+        // With |q'| <= T = |q| + |q - q'| and g = 2 gamma + 2^-21 this is margin = A resid + B xhat + C, A = |q| + g T,
+        // B = |q - q'| + g T, C = h 2^-148, all times 1.001 for the rounding of the norms (fp32 sums of squares, ld
+        // 2^-149 added for the squares that underflowed), of A, B, C and of the margin itself.  The sum q^ . n cannot
+        // underflow (its terms are multiples of 2^-24), and approx multiplies by 2^-e first when 2^-e > 1 (exactly) so
+        // that an underflow of a product is never scaled up.  The bound assumes that no partial sum overflows: a pair
+        // with T (resid + xhat) > 2^126 gets an infinite margin.  A NaN or Inf row (s = NaN) has a NaN approximation
+        // and a NaN or Inf query a NaN or Inf margin: both are always re-scored.  One warp per query, before the first
+        // group; qc_s[b] = {A, B, C, 2^-e, T}.
         unsigned long long nrescored = 0;
         if constexpr (IMG) {
             if (cw < NQ) {
-                float s2 = 0.f;
-                for (int t = lane; t < dq4; t += 32) {
-                    const float4 v = q4[cw * dq4 + t];
-                    s2 += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
+                const float* qf = qs + (size_t)cw * ld;
+                float s2 = 0.f, mx = 0.f;
+                for (int t = lane; t < ld; t += 32) {
+                    s2 = fmaf(qf[t], qf[t], s2);
+                    mx = fmaxf(mx, fabsf(qf[t]));
                 }
 #pragma unroll
-                for (int o = 16; o > 0; o >>= 1) s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+                for (int o = 16; o > 0; o >>= 1) {
+                    s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+                    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+                }
+                const int e = min(141 - (int)((__float_as_uint(mx) >> 23) & 0xffu), 126);
+                float d2 = 0.f;
+                __half* qh = reinterpret_cast<__half*>(qh_s + (size_t)cw * nc8);
+                for (int t = lane; t < 8 * nc8; t += 32) {
+                    const float x = t < ld ? qf[t] : 0.f;
+                    const float v = e > 63 ? x * pow2f(63) * pow2f(e - 63) : x * pow2f(e);  // |v| < 2^15
+                    const __half h = __float2half_rn(v);
+                    qh[t] = h;
+                    const float d = v - __half2float(h);  // exact
+                    d2 = fmaf(d, d, d2);
+                }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) d2 += __shfl_xor_sync(0xffffffffu, d2, o);
                 if (lane == 0) {
-                    const float c = 3.90625e-3f + (float)ld * 1.1920929e-7f * 1.1f + 1e-5f;
-                    const float lost = (float)ld * 0x1p-149f;
+                    const float h = (float)(ld + 64), lost = (float)ld * 0x1p-149f;
+                    const float g = 2.f * 1.01f * h * 0x1p-24f + 0x1p-21f;
+                    const float qs_e = pow2f(-e);
                     const float qn = sqrtf(s2 + lost);
-                    margin_s[cw] = 1.001f * (c * qn * sqrtf(*p.norm2_max + lost) + 0x1p-134f * (sqrtf((float)ld) * qn + (float)ld));
+                    // |q - q'|: the scaled rounding errors (v itself may have underflowed by 2^-150 when e <= 0), scaled
+                    // back by 2^-e (that product may underflow by 2^-150 too).  2^-149 stands for 2^-150: nvcc folds the
+                    // literal 0x1p-150f to +Inf.
+                    const float dqn = (sqrtf(d2 + lost) + sqrtf((float)ld) * 0x1p-149f) * qs_e + 0x1p-149f;
+                    const float T = qn + dqn;
+                    float* c = qc_s + cw * 8;
+                    c[0] = 1.001f * (qn + g * T);
+                    c[1] = 1.001f * (dqn + g * T);
+                    c[2] = 1.001f * h * 0x1p-148f;
+                    c[3] = qs_e;
+                    c[4] = T;
                 }
             }
             named_bar_sync(kBarConsumers, kConsumerThreads);
@@ -566,6 +635,7 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
         };
         for (int64_t g = blockIdx.x; dyn || g < ngroups; g += gridDim.x) {
             float acc[V];
+            float4 hdr;  // int8 filter: header {s, resid, xhat, 0} of this lane's row
 #pragma unroll
             for (int i = 0; i < V; ++i) acc[i] = 0.f;
             if (dyn) {  // (whole-row stages only: one stage per group)
@@ -575,32 +645,23 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
             }
             for (int ch = 0; ch < p.nchunks; ++ch) {
                 if (!dyn) mbar_wait(&full[s], ph);
-                if constexpr (IMG) {  // whole rows of bf16: 8 elements per 16-byte load, unpacked by a shift or a mask
-                    const uint4* tile = reinterpret_cast<const uint4*>(ring + (size_t)s * stage_floats) +
-                                        (size_t)(cw * kRowsPerWarp) * ck4;
+                if constexpr (IMG) {  // whole image rows: 8 codes per 8-byte load, the header of this lane's row
+                    const unsigned char* tile = reinterpret_cast<const unsigned char*>(ring + (size_t)s * stage_floats) +
+                                                (size_t)(cw * kRowsPerWarp) * (4 * ck);
+                    const uint2* codes = reinterpret_cast<const uint2*>(tile + kImgHeader);
 #pragma unroll 2
-                    for (int i = lane; i < ck4; i += 32) {
-                        uint4 x[kRowsPerWarp];
+                    for (int i = lane; i < nc8; i += 32) {
+                        uint2 x[kRowsPerWarp];
 #pragma unroll
-                        for (int r = 0; r < kRowsPerWarp; ++r) x[r] = tile[r * ck4 + i];
+                        for (int r = 0; r < kRowsPerWarp; ++r) x[r] = codes[r * (ck >> 1) + i];
 #pragma unroll
                         for (int b = 0; b < NQ; ++b) {
-                            const float4 qa = q4[b * dq4 + 2 * i], qb = q4[b * dq4 + 2 * i + 1];
+                            const uint4 q = qh_s[b * nc8 + i];
 #pragma unroll
-                            for (int r = 0; r < kRowsPerWarp; ++r) {
-                                float a = acc[r * NQ + b];
-                                a = fmaf(bf16_lo(x[r].x), qa.x, a);
-                                a = fmaf(bf16_hi(x[r].x), qa.y, a);
-                                a = fmaf(bf16_lo(x[r].y), qa.z, a);
-                                a = fmaf(bf16_hi(x[r].y), qa.w, a);
-                                a = fmaf(bf16_lo(x[r].z), qb.x, a);
-                                a = fmaf(bf16_hi(x[r].z), qb.y, a);
-                                a = fmaf(bf16_lo(x[r].w), qb.z, a);
-                                a = fmaf(bf16_hi(x[r].w), qb.w, a);
-                                acc[r * NQ + b] = a;
-                            }
+                            for (int r = 0; r < kRowsPerWarp; ++r) acc[r * NQ + b] = dot8_i8_f16(x[r], q, acc[r * NQ + b]);
                         }
                     }
+                    hdr = *reinterpret_cast<const float4*>(tile + (size_t)(((lane >> (5 - LV)) / NQ) * (4 * ck)));
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&empty[s]);
                     if (++s == p.stages) { s = 0; ph ^= 1u; }
@@ -609,7 +670,7 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
                 const float4* tile =
                     reinterpret_cast<const float4*>(ring + (size_t)s * stage_floats) + (size_t)(cw * kRowsPerWarp) * ck4;
                 const int c4n = min(ck4, d4 - ch * ck4);
-                const float4* qb = q4 + ch * ck4;  // (stride dq4 == d4 without the bf16 filter)
+                const float4* qb = q4 + ch * ck4;
 #pragma unroll 2
                 for (int i = lane; i < c4n; i += 32) {
                     float4 x[kRowsPerWarp];
@@ -661,8 +722,12 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
                 bool full_q = false;
                 if (owner && b < nqv) {
                     const int64_t cpos = g * kGroupRows + cw * kRowsPerWarp + r;
+                    const float* c = qc_s + b * 8;
+                    const float approx = c[3] > 1.f ? score * c[3] * hdr.x : score * hdr.x * c[3];
+                    float margin = fmaf(c[0], hdr.y, fmaf(c[1], hdr.z, c[2]));
+                    if (!(c[4] * (hdr.y + hdr.z) <= 0x1p126f)) margin = INFINITY;
                     if (cpos < total && row_allowed(p.allow, (uint32_t)cpos) &&
-                        !(fabsf(score) <= FLT_MAX && score + margin_s[b] < thr_s[b])) {
+                        !(fabsf(approx) <= FLT_MAX && approx + margin < thr_s[b])) {
                         const int slot = atomicAdd(rq_cnt, 1);
                         rq[slot] = (uint64_t)cpos << 8 | (uint64_t)b;
                         full_q = slot + 1 > kRescoreCap - kGroupRows * NQ;
@@ -782,30 +847,60 @@ __device__ __forceinline__ void scan_impl(const ScanParams& p, const RangeOut& r
     }
 }
 
-// The bf16 image of n rows: out[r][c] = bf16(rows[r][c]) rounded to nearest even (NaN stays NaN, a value within half a
-// bf16 ulp of FLT_MAX rounds to Inf), columns [ld, ldh) zero.  One thread per 8 elements.
-__global__ void bf16_image_kernel(const float* rows, int ld, int ldh, int64_t n, uint16_t* out) {
-    const int c8n = ldh >> 3;
-    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i >= n * c8n) return;
-    const int64_t r = i / c8n;
-    const int c = (int)(i - r * c8n) * 8;
-    uint32_t w[4];
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (c + 4 * h < ld) v = *reinterpret_cast<const float4*>(rows + (size_t)r * ld + c + 4 * h);
-        const float f[4] = {v.x, v.y, v.z, v.w};
-        uint32_t b[4];
+// The int8 image of n rows (row layout at kImgHeader), one warp per row.  s = max |x_i| / 127 (at least the smallest
+// subnormal), n_i = rint(x_i / s) clamped to [-127, 127]; resid = |x - s n| and xhat = s |n| are summed in fp64 (every
+// term exact) and rounded up to fp32, so rounding can only make them larger; an xhat beyond FLT_MAX becomes +Inf.
+// An all-zero row has s = 0, n = 0, resid = xhat = 0; a row with a NaN or Inf element has s = NaN, n = 0 and
+// resid = +Inf.  `rb` = img_row_bytes(ld).
+__global__ void int8_image_kernel(const float* rows, int ld, int rb, int64_t n, uint8_t* out) {
+    const int64_t r = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (r >= n) return;
+    const float4* x4 = reinterpret_cast<const float4*>(rows + (size_t)r * ld);
+    const int d4 = ld >> 2, w4 = (rb - kImgHeader) >> 2;  // float4s of the row, 4-code words of the image row
+    float mx = 0.f;
+    bool bad = false;
+    for (int t = lane; t < d4; t += 32) {
+        const float4 v = x4[t];
+        const float a[4] = {fabsf(v.x), fabsf(v.y), fabsf(v.z), fabsf(v.w)};
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
-            const uint32_t u = __float_as_uint(f[e]);
-            b[e] = (f[e] != f[e]) ? 0x7fc0u : (u + 0x7fffu + ((u >> 16) & 1u)) >> 16;
+            bad |= !(a[e] <= FLT_MAX);
+            mx = fmaxf(mx, a[e]);
         }
-        w[2 * h] = b[0] | b[1] << 16;
-        w[2 * h + 1] = b[2] | b[3] << 16;
     }
-    *reinterpret_cast<uint4*>(out + (size_t)r * ldh + c) = make_uint4(w[0], w[1], w[2], w[3]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    bad = __any_sync(0xffffffffu, bad);
+    const float s = bad ? NAN : mx == 0.f ? 0.f : fmaxf(mx / 127.f, 0x1p-149f);
+    double r2 = 0.0, n2 = 0.0;
+    uint32_t* w = reinterpret_cast<uint32_t*>(out + (size_t)r * rb + kImgHeader);
+    for (int t = lane; t < w4; t += 32) {
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (t < d4) v = x4[t];
+        const float f[4] = {v.x, v.y, v.z, v.w};
+        uint32_t u = 0;
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const float c = s > 0.f ? fminf(fmaxf(rintf(f[e] / s), -127.f), 127.f) : 0.f;  // (s NaN: 0)
+            const double d = (double)f[e] - (double)s * (double)c;
+            r2 = fma(d, d, r2);
+            n2 = fma((double)c, (double)c, n2);
+            u |= (uint32_t)((int)c + 128) << (8 * e);
+        }
+        w[t] = u;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        r2 += __shfl_xor_sync(0xffffffffu, r2, o);
+        n2 += __shfl_xor_sync(0xffffffffu, n2, o);
+    }
+    if (lane == 0) {
+        constexpr double up = 1.0 + 0x1p-30;  // the fp64 sums' and square roots' rounding
+        const float resid = bad ? INFINITY : __double2float_ru(sqrt(r2) * up);
+        const float xhat = bad ? 0.f : __double2float_ru((double)s * sqrt(n2) * up);
+        *reinterpret_cast<float4*>(out + (size_t)r * rb) = make_float4(s, resid, xhat, 0.f);
+    }
 }
 
 template <int NQ, int RW, bool GATHER, bool IMG = false>

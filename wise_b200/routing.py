@@ -7,7 +7,7 @@ no GPU, no torch.
 """
 from __future__ import annotations
 
-_MEM_RESERVE = 1 << 30  # free memory a shard leaves for search scratch (the bf16 image keeps the same margin)
+_MEM_RESERVE = 1 << 30  # free memory a shard leaves for search scratch (the int8 image keeps the same margin)
 
 
 def shard_range(n_total: int, rank: int, world: int) -> tuple[int, int]:
